@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- document graphs/s of the fused CAGGC+MAGGC graph blocks (fwd+bwd) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -33,6 +33,7 @@ cannot travel to the GPU box; oracle/gcgcn_oracle.py issues the same ATen ops, s
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -53,8 +54,12 @@ VARIANTS = {"glove": (2, 8), "bert": (4, 4)}
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps (or calls) of every GPU measurement of the run")
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (y1, y2, a0, a1, dx0, de0, "
+                         "de1 and every parameter gradient) as DIR/<name>.npy in float32: whole when an array has at "
+                         "most 2^20 elements, else a fixed seeded sample of 2^20 of its elements (rank 0's shard)")
     ap.add_argument("--impl", default="gcgcn_b200", choices=["gcgcn_b200", "reference"])
     ap.add_argument("--variant", default="glove", choices=list(VARIANTS))
     ap.add_argument("--dtype", default="fp32", choices=["fp32", "bf16"], help="edge-tensor storage")
@@ -77,7 +82,12 @@ def parse():
     ap.add_argument("--no-aux", action="store_true", help="skip the separate pooling / pair-gather timings")
     ap.add_argument("--no-sweep", action="store_true", help="skip the configs[2] / configs[3] points of the aux section")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
-    return ap.parse_args()
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "gcgcn_b200" or args.train_docs):
+        ap.error("--dump-outputs applies to the graph-block step of the gcgcn_b200 arm")
+    return args
 
 
 def claim_stdout():
@@ -121,7 +131,7 @@ def cpu_oracle_rate(variant: str, seconds: float, max_passes: int = 1000, warmup
                                        f"fwd+bwd, one document at a time, median pass {med * 1e3:.1f} ms"}
 
 
-def cuda_oracle_rate(variant: str, dev, passes: int = 5):
+def cuda_oracle_rate(variant: str, dev, passes: int):
     """SURVEY 8d, config 2: the reference's own PyTorch path on the B200 itself -- the oracle's ATen ops (the same
     calls the reference modules make, pinned bit-exact to them) issued eagerly on `dev`, documents one at a time
     like the reference trainer (C:339), fwd+bwd, inputs resident on the device, CUDA_LAUNCH_BLOCKING unset.
@@ -218,6 +228,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(
                 ["nvidia-smi", "-i", str(index), f"--query-gpu={self.FIELDS}", "--format=csv,noheader,nounits",
                  "-lms", "25"], stdout=self.tmp, stderr=subprocess.DEVNULL)
+            atexit.register(self.proc.kill)     # no sampler outlives a run that fails before stop()
         except OSError:
             self.proc = None
 
@@ -315,7 +326,7 @@ def kernel_roofline(name, launches, ms, flop, bt, H, L, esz, steps, hbm_peak, te
 
 
 # ------------------------------------------------------------------------------- pooling / pair gathers
-def aux_rates(dev, hbm_peak, tensor_peak, tiles=128, iters=10):
+def aux_rates(dev, hbm_peak, tensor_peak, iters, tiles=128):
     """SURVEY 8d: the mention->entity pooling (a1) and the classifier-side pair gathers (a8) are timed apart from
     the graph blocks, each against its own algorithmic bytes.  12-document batch x `tiles`, device-resident,
     CUDA events around `iters` back-to-back calls after 3 warm-up calls (outputs of the gathers are 2.7 GB per
@@ -486,7 +497,7 @@ def aux_rates(dev, hbm_peak, tensor_peak, tiles=128, iters=10):
 
 
 # ------------------------------------------------------------------------------- configs[2] / configs[3] inside the default run
-def graph_block_point(dev, layers, heads, sizes, edge_dtype, hbm_peak, steps=5, warmup=3):
+def graph_block_point(dev, layers, heads, sizes, edge_dtype, hbm_peak, steps, warmup=3):
     """One device-resident measurement of the graph blocks (fwd+bwd, eval mode) on a batch of `sizes` entity counts:
     graphs/s and the whole-path fraction of the HBM roofline (SURVEY 8d algorithmic bytes / step time)."""
     import torch
@@ -531,7 +542,7 @@ def graph_block_point(dev, layers, heads, sizes, edge_dtype, hbm_peak, steps=5, 
     return res
 
 
-def sweep_and_variants(dev, hbm_peak, edge_gb=4.0):
+def sweep_and_variants(dev, hbm_peak, steps, edge_gb=4.0):
     """BASELINE.json configs[3] (entity-count sweep 42/128/256 x 4/8 heads, fully connected, n^2 edge tensors of
     `edge_gb` GB each so that every point streams far more than L2) and configs[2] (the BERT graph head L_s=4, H=4 with
     bf16 edge storage on the DocRED-shaped batch), measured inside the default run so that the driver's record carries
@@ -539,18 +550,18 @@ def sweep_and_variants(dev, hbm_peak, edge_gb=4.0):
     import numpy as np
     import torch
     from gcgcn_b200 import synthetic
-    out = {"sweep": [], "note": "device-resident inputs, CUDA events around 5 steps after 3 warm-up steps; path_frac = "
-                                "SURVEY 8d algorithmic bytes / step time / measured HBM peak"}
+    out = {"sweep": [], "note": f"device-resident inputs, CUDA events around {steps} steps after 3 warm-up steps; "
+                                "path_frac = SURVEY 8d algorithmic bytes / step time / measured HBM peak"}
     for n in (42, 128, 256):
         for h in (4, 8):
             ndoc = max(1, int(edge_gb * 1e9 // (n * n * 512)))
-            r = graph_block_point(dev, 2, h, np.full(ndoc, n, dtype=np.int64), torch.float32, hbm_peak)
+            r = graph_block_point(dev, 2, h, np.full(ndoc, n, dtype=np.int64), torch.float32, hbm_peak, steps)
             r["workload"] = f"configs[3]: {ndoc} fully connected graphs of {n} entities, {h} heads"
             out["sweep"].append(r)
-    r = graph_block_point(dev, 4, 4, synthetic.shard_doc_sizes(12 * 512), torch.bfloat16, hbm_peak)
+    r = graph_block_point(dev, 4, 4, synthetic.shard_doc_sizes(12 * 512), torch.bfloat16, hbm_peak, steps)
     r["workload"] = "configs[2]: GCGCN_Bert graph head (L_s=4, H=4), bf16 edge storage, fp32 accumulate, 6144 documents"
     out["config2_bert_bf16"] = r
-    r = graph_block_point(dev, 4, 4, synthetic.shard_doc_sizes(12 * 512), torch.float32, hbm_peak)
+    r = graph_block_point(dev, 4, 4, synthetic.shard_doc_sizes(12 * 512), torch.float32, hbm_peak, steps)
     r["workload"] = "GCGCN_Bert graph head shapes (L_s=4, H=4), fp32 edge storage, 6144 documents"
     out["bert_head_fp32"] = r
     return out
@@ -656,12 +667,12 @@ def run_e2e(args, dev, gb, bt, gb_params, timed, world, ndocs):
     def e2e_window(count):
         window.update(i=0, count=count)
         copy_stream.synchronize()
-        ms_w, launches, _ = timed(e2e_step, count)
+        ms_w, launches, _, _ = timed(e2e_step, count)
         copy_stream.synchronize()
         return ms_w, launches
 
     e2e_window(3)                                         # warm-up window (pinned pages touched, pools grown)
-    steps = max(20, args.steps)
+    steps = args.steps
     ms_e, launches = e2e_window(steps)
     # the same pipeline with the inputs already resident (no copies): what the copies cost on top of the kernels
     def dev_step():
@@ -678,13 +689,13 @@ def run_e2e(args, dev, gb, bt, gb_params, timed, world, ndocs):
         torch.autograd.backward([y1, y2], [st.dy1, st.dy2])
     for _ in range(3):
         dev_step()
-    ms_d, _, _ = timed(dev_step, max(10, args.steps))
+    ms_d, _, _, _ = timed(dev_step, steps)
     for p in gb_params:
         p.grad = None
     return {"value": world * ndocs * steps / (ms_e * 1e-3), "unit": UNIT, "h2d_bytes_per_step": h2d,
             "d2h_bytes_per_step": d2h, "ms_per_step": ms_e / steps, "steps": steps,
             "h2d_gbs": h2d * steps / (ms_e * 1e-3) / 1e9, "gpu_launches_per_step": launches / steps,
-            "device_resident_ms_per_step": ms_d / max(10, args.steps),
+            "device_resident_ms_per_step": ms_d / steps,
             "active_slots": sets[0].edge.num_slots, "active_tokens": sets[0].edge.num_tokens, "tokens": tok,
             "wire_bytes_per_doc": sum(w.nbytes for w in wires12) / 12.0,
             "note": "inputs from pinned host memory every step: context_output of all documents (fp32), the upstream "
@@ -695,6 +706,26 @@ def run_e2e(args, dev, gb, bt, gb_params, timed, world, ndocs):
                     "device (its consumer, the encoder's backward, lives there).  Double-buffered: the copy of step "
                     "i+1 overlaps the kernels of step i; exactly one full input copy per timed step, none staged "
                     "before the window opens; the window closes after the last device->host read."}
+
+
+# ------------------------------------------------------------------------------- --dump-outputs
+DUMP_ELEMENTS = 1 << 20      # 4 MB of float32 per array: the seven step outputs + the parameter gradients stay < 64 MB
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """Write every tensor as out_dir/<name>.npy in float32 (float64 stays float64): whole when it has at most
+    DUMP_ELEMENTS elements, else its elements at DUMP_ELEMENTS sorted positions drawn by a generator of fixed seed
+    (the same positions in every run with the same arguments), flattened."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_ELEMENTS:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_ELEMENTS, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        t = t.to(torch.float64 if t.dtype == torch.float64 else torch.float32)
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.cpu().numpy())
 
 
 # ------------------------------------------------------------------------------- GPU arm
@@ -779,6 +810,7 @@ def run_gpu_arm(args):
         torch.cuda.synchronize()
 
     def timed(fn, steps, with_kernel_events=False):
+        """(ms, launches, per-kernel table, what the last of the `steps` calls of fn returned)"""
         barrier()
         stream = torch.cuda.current_stream().cuda_stream
         launches0 = _lib.launch_count()
@@ -786,8 +818,9 @@ def run_gpu_arm(args):
         if with_kernel_events:
             _lib.timing_begin(stream)
         ev0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        last = fn()
         ev1.record()
         barrier()
         kern = _lib.timing_end(stream) if with_kernel_events else {}
@@ -796,14 +829,14 @@ def run_gpu_arm(args):
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms, _lib.launch_count() - launches0, kern
+        return ms, _lib.launch_count() - launches0, kern, last
 
     # nvidia-smi needs ~1 s to start: the sampler runs from the warm-up steps to the end of the timed region
     sampler = ClockSampler(local) if rank == 0 else None
     for _ in range(max(args.warmup, 3)):
         step()
     # per-kernel breakdown: an eager pass with the library's per-launch events (not the headline)
-    ms_eager, launches, kern = timed(step, args.steps, with_kernel_events=True)
+    ms_eager, launches, kern, _ = timed(step, args.steps, with_kernel_events=True)
     graphed = None
     if args.graph:
         from gcgcn_b200.graphs import GraphedPass
@@ -833,11 +866,17 @@ def run_gpu_arm(args):
         while sampler.count() < 3 and time.perf_counter() < t_wait:
             step()
         torch.cuda.synchronize()
-    ms, _, _ = timed(step, args.steps)
+    ms, _, _, last = timed(step, args.steps)
     clocks = sampler.stop() if sampler else {}
     if clocks:
         clocks["window"] = "warm-up steps + timed region (same kernels, back to back)"
     value = world * ndocs * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        grads = {"dx0": x0.grad, "de0": e0.grad, "de1": e1.grad}
+        grads.update((f"grad.{n}", p.grad) for n, p in gb.named_parameters() if p.grad is not None)
+        dump_outputs(args.dump_outputs, {"y1": last["y1"], "y2": last["y2"], "a0": last["a0"], "a1": last["a1"],
+                                         **grads})
+    del last
 
     # ---- end to end from pinned host buffers: what the caller of the plugin holds on the host is the encoder output
     # (context_output) and the wire format of the documents; the edge tensors e0/e1 are produced ON the device by the
@@ -908,16 +947,16 @@ def run_gpu_arm(args):
     if not args.no_aux and not args.nodes:
         for t in (x0, e0, e1):
             t.grad = None
-        aux = aux_rates(dev, hbm_peak, tensor_peak)
+        aux = aux_rates(dev, hbm_peak, tensor_peak, args.steps)
         if not args.no_sweep and world == 1:
             del x0, e0, e1, dy1, dy2
             torch.cuda.empty_cache()
-            aux.update(sweep_and_variants(dev, hbm_peak))
+            aux.update(sweep_and_variants(dev, hbm_peak, args.steps))
     cpu = None
     if not args.no_cpu_baseline:
         rate, info = cpu_oracle_rate(args.variant, args.cpu_seconds)
         cpu = {"value": rate, "unit": UNIT, "cores": info["cores"], "kind": "port", "sample": info["sample"],
-               "host_cpus": info["host_cpus"], "reference_eager_cuda": cuda_oracle_rate(args.variant, dev)}
+               "host_cpus": info["host_cpus"], "reference_eager_cuda": cuda_oracle_rate(args.variant, dev, args.steps)}
 
     line = {
         "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps,

@@ -61,6 +61,16 @@ class EdgeTablesC(ctypes.Structure):
     ]
 
 
+class RankResult(ctypes.Structure):
+    """struct gcgcn_rank_result"""
+    _fields_ = [
+        ("count", c_int64), ("total_recall", c_int64), ("best_pos", c_int64), ("w", c_int64),
+        ("auc", ctypes.c_double), ("ign_auc", ctypes.c_double),
+        ("f1", c_float), ("theta", c_float), ("f1_at_w", c_float), ("precision_at_w", c_float),
+        ("recall_at_w", c_float), ("ign_f1", c_float), ("ign_f1_at_w", c_float), ("reserved", c_float),
+    ]
+
+
 def sources():
     return sorted(glob.glob(os.path.join(CSRC, "*.cu")))
 
@@ -177,6 +187,11 @@ SIGNATURES = {
     "gcgcn_doc_bias_bwd": (c_int32, [_BT, _P, c_int32, _P, _P]),
     "gcgcn_pair_bce_fwd": (c_int32, [_BT, _P, _P, c_int32, _P, _P]),
     "gcgcn_pair_bce_bwd": (c_int32, [_BT, _P, _P, c_int32, _P, _P, _P]),
+    "gcgcn_rank_ws_bytes": (c_size_t, [c_int64]),
+    "gcgcn_rank_candidates": (c_int32, [_BT, _P, c_int32, _P, _P, c_int64, _P, _P, _P, _P]),
+    "gcgcn_rank_sort": (c_int32, [_P, _P, c_int64, _P, _P, _P, c_size_t, _P]),
+    "gcgcn_rank_curve": (c_int32, [_P, _P, c_int64, c_int64, c_int32, ctypes.c_double, _P, _P, c_size_t, _P]),
+    "gcgcn_rank_decode": (c_int32, [_P, _P, c_int64, c_int64, _P, _P, c_int32, c_int32, _P, _P, _P, _P, _P, _P]),
     "gcgcn_adam_step": (c_int32, [_P, _P, _P, _P, c_int64] + [c_float] * 6 + [c_int32, _P]),
     "gcgcn_gemm": (c_int32, [c_int32, c_int32, c_int32, c_int32, c_int32, c_float, _P, c_int32, _P,
                              c_int32, c_float, _P, c_int32, _P, _P, c_size_t, _P]),

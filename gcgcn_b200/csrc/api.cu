@@ -120,6 +120,17 @@ int launch_gat_collapse_bwd(const float* Wh, const float* bh, const float* Wt, c
                             const float* br, const float* w, const float* dout, int hid, float* dWh, float* dbh, float* dWt,
                             float* dbt, float* dWr, float* dbr, float* dw, float* db, cudaStream_t st);
 int launch_pack_rows(const float* const* ptrs, int count, int elems, float* out, cudaStream_t st);
+size_t rank_ws_bytes(long long count);
+int launch_rank_candidates(const gcgcn_batch* bt, const float* z, const float* labels, const uint8_t* intrain, int R,
+                           long long base_id, float* score, uint32_t* payload, unsigned long long* counters,
+                           cudaStream_t st);
+int launch_rank_sort(const float* score, const uint32_t* payload, long long count, uint32_t* sorted_key,
+                     uint32_t* sorted_payload, void* ws, size_t ws_bytes, cudaStream_t st);
+int launch_rank_curve(const uint32_t* key, const uint32_t* pay, long long count, long long T, int has_intrain,
+                      double input_theta, gcgcn_rank_result* res, void* ws, size_t ws_bytes, cudaStream_t st);
+int launch_rank_decode(const uint32_t* key, const uint32_t* pay, long long rows, const long long* doc_off,
+                       const int* doc_n, int docs, int R, int* doc, int* row, int* col, int* rel, float* score,
+                       cudaStream_t st);
 
 // ---- error text, launch counter, device cache --------------------------------------------------
 std::atomic<uint64_t> g_launches{0};
@@ -1212,6 +1223,83 @@ int gcgcn_pair_bce_bwd(const gcgcn_batch* bt, const float* logits, const float* 
     GCGCN_TRY(check_device_ptr(dloss, "dloss"));
     GCGCN_TRY(check_device_ptr(dlogits, "dlogits"));
     return launch_pair_bce_bwd(bt, logits, labels, relations, dloss, dlogits, static_cast<cudaStream_t>(stream));
+}
+
+// ---- relation evaluation ---------------------------------------------------------------------
+size_t gcgcn_rank_ws_bytes(int64_t count) { return rank_ws_bytes(count); }
+int gcgcn_rank_candidates(const gcgcn_batch* bt, const float* logits, int32_t relations, const float* labels,
+                          const uint8_t* intrain, int64_t base_id, float* score, uint32_t* payload, int64_t* counters,
+                          void* stream) {
+    GCGCN_API_ENTER(stream);
+    GCGCN_TRY(check_batch(bt));
+    GCGCN_REQUIRE(relations >= 2, "rank_candidates: relations < 2 (relation 0 is not a candidate)");
+    GCGCN_REQUIRE(base_id >= 0, "rank_candidates: negative base_id");
+    const long long count = (bt->total_pairs - bt->total_nodes) * static_cast<long long>(relations - 1);
+    GCGCN_REQUIRE(count >= 0, "rank_candidates: total_pairs < total_nodes");
+    if (base_id + count >= GCGCN_RANK_MAX_CANDIDATES)
+        return fail(GCGCN_ERR_UNSUPPORTED, "rank_candidates: %lld + %lld candidates, one evaluation holds fewer than 2^30",
+                    static_cast<long long>(base_id), count);
+    GCGCN_TRY(check_device_ptr(counters, "counters"));
+    if (count == 0) return GCGCN_OK;
+    GCGCN_TRY(check_device_ptr(logits, "logits"));
+    if (labels != nullptr) GCGCN_TRY(check_device_ptr(labels, "labels"));
+    if (intrain != nullptr) GCGCN_TRY(check_device_ptr(intrain, "intrain"));
+    GCGCN_TRY(check_device_ptr(score, "score"));
+    GCGCN_TRY(check_device_ptr(payload, "payload"));
+    return launch_rank_candidates(bt, logits, labels, intrain, relations, base_id, score, payload,
+                                  reinterpret_cast<unsigned long long*>(counters), static_cast<cudaStream_t>(stream));
+}
+int gcgcn_rank_sort(const float* score, const uint32_t* payload, int64_t count, uint32_t* sorted_key,
+                    uint32_t* sorted_payload, void* ws, size_t ws_bytes, void* stream) {
+    GCGCN_API_ENTER(stream);
+    GCGCN_REQUIRE(count >= 0 && count < GCGCN_RANK_MAX_CANDIDATES, "rank_sort: count %lld outside [0, 2^30)",
+                  static_cast<long long>(count));
+    if (count == 0) return GCGCN_OK;
+    GCGCN_TRY(check_device_ptr(score, "score"));
+    GCGCN_TRY(check_device_ptr(payload, "payload"));
+    GCGCN_TRY(check_device_ptr(sorted_key, "sorted_key"));
+    GCGCN_TRY(check_device_ptr(sorted_payload, "sorted_payload"));
+    GCGCN_TRY(check_device_ptr(ws, "ws"));
+    GCGCN_REQUIRE(ws_bytes >= rank_ws_bytes(count), "rank_sort: ws_bytes %zu < gcgcn_rank_ws_bytes = %zu", ws_bytes,
+                  rank_ws_bytes(count));
+    return launch_rank_sort(score, payload, count, sorted_key, sorted_payload, ws, ws_bytes,
+                            static_cast<cudaStream_t>(stream));
+}
+int gcgcn_rank_curve(const uint32_t* sorted_key, const uint32_t* sorted_payload, int64_t count, int64_t total_recall,
+                     int32_t has_intrain, double input_theta, gcgcn_rank_result* result, void* ws, size_t ws_bytes,
+                     void* stream) {
+    GCGCN_API_ENTER(stream);
+    GCGCN_REQUIRE(count >= 1 && count < GCGCN_RANK_MAX_CANDIDATES, "rank_curve: count %lld outside [1, 2^30)",
+                  static_cast<long long>(count));
+    GCGCN_TRY(check_device_ptr(sorted_key, "sorted_key"));
+    GCGCN_TRY(check_device_ptr(sorted_payload, "sorted_payload"));
+    GCGCN_REQUIRE((reinterpret_cast<uintptr_t>(sorted_payload) & 15) == 0, "rank_curve: sorted_payload not 16-byte aligned");
+    GCGCN_TRY(check_device_ptr(result, "result"));
+    GCGCN_TRY(check_device_ptr(ws, "ws"));
+    GCGCN_REQUIRE(ws_bytes >= rank_ws_bytes(count), "rank_curve: ws_bytes %zu < gcgcn_rank_ws_bytes = %zu", ws_bytes,
+                  rank_ws_bytes(count));
+    return launch_rank_curve(sorted_key, sorted_payload, count, total_recall < 1 ? 1 : total_recall, has_intrain ? 1 : 0,
+                             input_theta, result, ws, ws_bytes, static_cast<cudaStream_t>(stream));
+}
+int gcgcn_rank_decode(const uint32_t* sorted_key, const uint32_t* sorted_payload, int64_t rows, int64_t count,
+                      const int64_t* doc_offsets, const int32_t* doc_n, int32_t num_docs, int32_t relations, int32_t* doc,
+                      int32_t* row, int32_t* col, int32_t* relation, float* score, void* stream) {
+    GCGCN_API_ENTER(stream);
+    GCGCN_REQUIRE(rows >= 0 && num_docs >= 1 && relations >= 2, "rank_decode: bad shape");
+    GCGCN_REQUIRE(rows <= count, "rank_decode: rows %lld > count %lld of the ranking", static_cast<long long>(rows),
+                  static_cast<long long>(count));
+    if (rows == 0) return GCGCN_OK;
+    GCGCN_TRY(check_device_ptr(sorted_key, "sorted_key"));
+    GCGCN_TRY(check_device_ptr(sorted_payload, "sorted_payload"));
+    GCGCN_TRY(check_device_ptr(doc_offsets, "doc_offsets"));
+    GCGCN_TRY(check_device_ptr(doc_n, "doc_n"));
+    GCGCN_TRY(check_device_ptr(doc, "doc"));
+    GCGCN_TRY(check_device_ptr(row, "row"));
+    GCGCN_TRY(check_device_ptr(col, "col"));
+    GCGCN_TRY(check_device_ptr(relation, "relation"));
+    GCGCN_TRY(check_device_ptr(score, "score"));
+    return launch_rank_decode(sorted_key, sorted_payload, rows, reinterpret_cast<const long long*>(doc_offsets), doc_n,
+                              num_docs, relations, doc, row, col, relation, score, static_cast<cudaStream_t>(stream));
 }
 
 // ---- dense projection ------------------------------------------------------------------------

@@ -78,12 +78,12 @@ bilinear_dt_kernel(const float* __restrict__ dout, int ldd, const float* __restr
 // ---- the trainer's loss (C:355-364): per document, mean over the ordered pairs i != j of BCELoss(sigmoid(z), y) ----
 // torch's arithmetic: p = sigmoid(z); bce = (y - 1) max(log1p(-p), -100) - y max(log(p), -100)   (ATen Loss.cpp)
 __device__ __forceinline__ float bce_of(float z, float y) {
-    const float p = 1.0f / (1.0f + expf(-z));
+    const float p = logit_sigmoid(z);
     return (y - 1.f) * fmaxf(log1pf(-p), -100.f) - y * fmaxf(logf(p), -100.f);
 }
 // d bce / d z = (p - y) / max((1 - p) p, 1e-12) * p (1 - p)      (binary_cross_entropy_backward, then sigmoid')
 __device__ __forceinline__ float dbce_of(float z, float y) {
-    const float p = 1.0f / (1.0f + expf(-z));
+    const float p = logit_sigmoid(z);
     const float pq = (1.f - p) * p;
     return (p - y) / fmaxf(pq, 1e-12f) * pq;
 }

@@ -118,6 +118,8 @@ struct Arena {
 static inline int ceil_div(long long a, long long b) { return static_cast<int>((a + b - 1) / b); }
 
 // ---- device helpers ------------------------------------------------------------------------
+// sigmoid of a logit (C:355), within 1 ulp of torch.sigmoid: one definition for the loss kernels and the evaluation
+__device__ __forceinline__ float logit_sigmoid(float z) { return 1.0f / (1.0f + expf(-z)); }
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -1,0 +1,639 @@
+// Relation evaluation of GCGCN (the DocRED baseline evaluation of config/Config.py:432-561 and its Ign variant,
+// config/Config_bert.py:626-650): every (document, i != j, relation r >= 1) candidate is scored with sigmoid, ranked by
+// score (descending, stable: equal scores keep insertion order, as Python's list.sort(reverse=True) does), and the
+// precision/recall curve over that ranking gives the best F1, its threshold, the AUC and the F1 at a given threshold.
+//
+//   candidates  logits/labels/intrain [total_pairs, R] -> score f32 + payload (id << 2 | intrain << 1 | correct)
+//   sort        stable LSD radix sort of (~bits(score), payload): 4 passes of 8-bit digits, reduce-then-scan
+//               (per-tile digit counts -> one digit-major exclusive scan -> stable in-tile ranking and scatter)
+//   curve       per-tile flag counts -> exclusive scan -> x, y, f1 (+ Ign) per position, per-tile first argmax and
+//               float64 AUC partials -> one-block finish (fixed-order reduction, w, result struct)
+//   decode      ranked ids of the first w + 1 candidates -> (doc, row, col, relation, score)
+//
+// Everything is deterministic: integer counts, a stable sort and float64 sums in a fixed order.
+#include "common.cuh"
+
+namespace gcgcn {
+
+constexpr int RK_THREADS = 256;                    // sort and curve tiles: 8 warps x 32 lanes x 16 items
+constexpr int RK_IPT = 16;
+constexpr int RK_TILE = RK_THREADS * RK_IPT;       // = GCGCN_RANK_TILE
+constexpr int RK_WARPS = RK_THREADS / WARP;
+constexpr int RK_RADIX = 256;
+constexpr int SCAN_THREADS = 1024;                 // device-wide exclusive scan: 1024 threads x 16 values per block
+constexpr int SCAN_CHUNK = SCAN_THREADS * 16;
+static_assert(RK_TILE == GCGCN_RANK_TILE, "header and kernels disagree on the tile");
+static_assert(RK_THREADS == RK_RADIX, "the downsweep gives every thread one digit");
+static_assert(RK_IPT == 16, "curve threads own 16 positions (load16)");
+
+__device__ __forceinline__ uint32_t score_key(float s) { return ~__float_as_uint(s); }
+__device__ __forceinline__ float key_score(uint32_t k) { return __uint_as_float(~k); }
+
+// ---- candidates --------------------------------------------------------------------------------------------------
+// One CTA per pair row (document b, row i): its n pairs x R cells are contiguous in logits.  Candidates of document b
+// start at base_id + (pair_ptr[b] - node_ptr[b]) (R - 1) (every earlier document has n(n-1) off-diagonal pairs).
+__global__ void __launch_bounds__(256)
+rank_candidates_kernel(const int* __restrict__ node_ptr, const long long* __restrict__ pair_ptr,
+                       const int* __restrict__ row_doc, const float* __restrict__ z, const float* __restrict__ labels,
+                       const uint8_t* __restrict__ intrain, int R, long long base_id, float* __restrict__ score,
+                       uint32_t* __restrict__ payload, unsigned long long* __restrict__ counters) {
+    __shared__ unsigned int red[2][8];
+    const int row = blockIdx.x;
+    const int b = row_doc[row];
+    const int n = node_ptr[b + 1] - node_ptr[b], i = row - node_ptr[b];
+    const long long cell0 = (pair_ptr[b] + static_cast<long long>(i) * n) * R;
+    const long long doc_base = base_id + (pair_ptr[b] - node_ptr[b]) * (R - 1);
+    const long long row_base = doc_base + static_cast<long long>(i) * (n - 1) * (R - 1);
+    const int cells = n * R;
+    unsigned int pos = 0, nan = 0;
+    for (int c = threadIdx.x; c < cells; c += blockDim.x) {
+        const int j = c / R, r = c - j * R;
+        if (j == i || r == 0) continue;
+        const float s = logit_sigmoid(z[cell0 + c]);
+        const uint32_t corr = (labels != nullptr && labels[cell0 + c] > 0.5f) ? 1u : 0u;
+        const uint32_t intr = (intrain != nullptr && intrain[cell0 + c] != 0) ? 2u : 0u;
+        const long long id = row_base + static_cast<long long>(j - (j > i)) * (R - 1) + (r - 1);
+        score[id - base_id] = s;
+        payload[id - base_id] = (static_cast<uint32_t>(id) << 2) | intr | corr;
+        pos += corr;
+        nan += (s != s) ? 1u : 0u;
+    }
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        pos += __shfl_xor_sync(0xffffffffu, pos, o);
+        nan += __shfl_xor_sync(0xffffffffu, nan, o);
+    }
+    if (lane == 0) { red[0][warp] = pos; red[1][warp] = nan; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        unsigned int p = 0, q = 0;
+        for (int w = 0; w < 8; ++w) { p += red[0][w]; q += red[1][w]; }
+        if (p) atomicAdd(counters, static_cast<unsigned long long>(p));
+        if (q) atomicAdd(counters + 1, static_cast<unsigned long long>(q));
+    }
+}
+
+// ---- block-wide exclusive scan of one value per thread (blockDim.x = NT) -----------------------------------------
+template <typename T, int NT>
+__device__ __forceinline__ T block_excl_scan(T v, T* s_warp, T* total) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    T inc = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const T t = __shfl_up_sync(0xffffffffu, inc, o);
+        if (lane >= o) inc += t;
+    }
+    if (lane == 31) s_warp[warp] = inc;
+    __syncthreads();
+    if (warp == 0) {
+        T w = lane < NT / 32 ? s_warp[lane] : T(0);
+        T wi = w;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const T t = __shfl_up_sync(0xffffffffu, wi, o);
+            if (lane >= o) wi += t;
+        }
+        if (lane < NT / 32) s_warp[lane] = wi - w;
+        if (lane == NT / 32 - 1) s_warp[32] = wi;
+    }
+    __syncthreads();
+    const T out = s_warp[warp] + inc - v;
+    if (total != nullptr) *total = s_warp[32];
+    __syncthreads();
+    return out;
+}
+
+// v[k] = x[base + k] for the 16 values a thread owns (0 past n): 16-byte loads when all 16 exist (base is a multiple of
+// 16 values and x is 256-byte aligned), so a warp's load touches 16-byte pieces instead of one word per lane
+template <typename T>
+__device__ __forceinline__ void load16(const T* __restrict__ x, long long base, long long n, T (&v)[16]) {
+    if (base + 16 <= n) {
+        const uint4* x4 = reinterpret_cast<const uint4*>(x + base);
+#pragma unroll
+        for (int q = 0; q < 16 * static_cast<int>(sizeof(T)) / 16; ++q) reinterpret_cast<uint4*>(v)[q] = x4[q];
+    } else {
+#pragma unroll
+        for (int k = 0; k < 16; ++k) v[k] = base + k < n ? x[base + k] : T(0);
+    }
+}
+
+// ---- device-wide exclusive scan in place (the sort's digit-major tile counts, the curve's packed flag counts) ------
+template <typename T>
+__global__ void __launch_bounds__(SCAN_THREADS)
+scan_reduce_kernel(const T* __restrict__ x, long long n, T* __restrict__ block_sums) {
+    __shared__ T s_warp[33];
+    const long long base = static_cast<long long>(blockIdx.x) * SCAN_CHUNK + threadIdx.x * 16LL;
+    T v[16];
+    load16(x, base, n, v);
+    T acc = 0;
+#pragma unroll
+    for (int k = 0; k < 16; ++k) acc += v[k];
+    T total;
+    block_excl_scan<T, SCAN_THREADS>(acc, s_warp, &total);
+    if (threadIdx.x == 0) block_sums[blockIdx.x] = total;
+}
+
+template <typename T>
+__global__ void __launch_bounds__(SCAN_THREADS)
+scan_top_kernel(T* __restrict__ sums, int n) {
+    __shared__ T s_warp[33];
+    T carry = 0;
+    for (int c0 = 0; c0 < n; c0 += SCAN_THREADS) {
+        const int idx = c0 + threadIdx.x;
+        const T v = idx < n ? sums[idx] : T(0);
+        T total;
+        const T ex = block_excl_scan<T, SCAN_THREADS>(v, s_warp, &total);
+        if (idx < n) sums[idx] = carry + ex;
+        carry += total;
+    }
+}
+
+template <typename T>
+__global__ void __launch_bounds__(SCAN_THREADS)
+scan_down_kernel(T* __restrict__ x, long long n, const T* __restrict__ block_sums) {
+    __shared__ T s_warp[33];
+    const long long base = static_cast<long long>(blockIdx.x) * SCAN_CHUNK + threadIdx.x * 16LL;
+    T v[16];
+    load16(x, base, n, v);
+    T acc = 0;
+#pragma unroll
+    for (int k = 0; k < 16; ++k) acc += v[k];
+    T run = block_excl_scan<T, SCAN_THREADS>(acc, s_warp, nullptr) + block_sums[blockIdx.x];
+#pragma unroll
+    for (int k = 0; k < 16; ++k) {
+        if (base + k < n) x[base + k] = run;
+        run += v[k];
+    }
+}
+
+template <typename T>
+static int launch_scan(T* x, long long n, T* block_sums, cudaStream_t st) {
+    const int blocks = ceil_div(n, SCAN_CHUNK);
+    scan_reduce_kernel<T><<<blocks, SCAN_THREADS, 0, st>>>(x, n, block_sums);
+    GCGCN_CHECK_LAUNCH("rank_scan_reduce");
+    scan_top_kernel<T><<<1, SCAN_THREADS, 0, st>>>(block_sums, blocks);
+    GCGCN_CHECK_LAUNCH("rank_scan_top");
+    scan_down_kernel<T><<<blocks, SCAN_THREADS, 0, st>>>(x, n, block_sums);
+    GCGCN_CHECK_LAUNCH("rank_scan_down");
+    return GCGCN_OK;
+}
+
+// ---- radix sort -------------------------------------------------------------------------------------------------
+// Pass 0 reads the float scores and forms the keys ~bits(s) (scores are >= 0, so the bit pattern is monotone and its
+// complement ascends as the score descends); later passes read the keys of the previous pass.
+template <bool FIRST>
+__device__ __forceinline__ uint32_t load_key(const void* in, long long idx) {
+    if (FIRST) return score_key(reinterpret_cast<const float*>(in)[idx]);
+    return reinterpret_cast<const uint32_t*>(in)[idx];
+}
+
+// counts[d * tiles + tile] = number of keys of the tile whose digit at `shift` is d
+template <bool FIRST>
+__global__ void __launch_bounds__(RK_THREADS)
+radix_upsweep_kernel(const void* __restrict__ keys_in, long long count, int shift, int tiles,
+                     uint32_t* __restrict__ counts) {
+    __shared__ uint32_t hist[RK_WARPS][RK_RADIX];
+    const int warp = threadIdx.x >> 5;
+    for (int t = threadIdx.x; t < RK_WARPS * RK_RADIX; t += RK_THREADS) (&hist[0][0])[t] = 0u;
+    __syncthreads();
+    const long long base = static_cast<long long>(blockIdx.x) * RK_TILE;
+#pragma unroll 4
+    for (int k = 0; k < RK_IPT; ++k) {
+        const long long idx = base + k * RK_THREADS + threadIdx.x;
+        if (idx < count) atomicAdd(&hist[warp][(load_key<FIRST>(keys_in, idx) >> shift) & 255u], 1u);
+    }
+    __syncthreads();
+    uint32_t s = 0;
+#pragma unroll
+    for (int w = 0; w < RK_WARPS; ++w) s += hist[w][threadIdx.x];
+    counts[static_cast<long long>(threadIdx.x) * tiles + blockIdx.x] = s;
+}
+
+// Stable scatter of one tile.  Warp w owns the tile's items [512 w, 512 w + 512), visited in 16 rounds of 32 in input
+// order; in each round the lanes holding the same digit find each other with match.any and take consecutive ranks
+// after the warp's running count of that digit.  Tile rank = start of the digit in the tile + the counts of that
+// digit in earlier warps + the warp rank.  The tile is staged in shared memory in digit order, then written out so
+// that each digit's run is contiguous at offsets[d * tiles + tile] (the digit-major exclusive scan of the counts).
+template <bool FIRST>
+__global__ void __launch_bounds__(RK_THREADS)
+radix_downsweep_kernel(const void* __restrict__ keys_in, const uint32_t* __restrict__ vals_in, long long count, int shift,
+                       int tiles, const uint32_t* __restrict__ offsets, uint32_t* __restrict__ keys_out,
+                       uint32_t* __restrict__ vals_out) {
+    __shared__ uint32_t s_keys[RK_TILE];
+    __shared__ uint32_t s_vals[RK_TILE];
+    __shared__ uint32_t s_whist[RK_WARPS][RK_RADIX];
+    __shared__ uint32_t s_start[RK_RADIX];
+    __shared__ uint32_t s_gout[RK_RADIX];
+    __shared__ uint32_t s_warp[33];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const long long base = static_cast<long long>(blockIdx.x) * RK_TILE;
+    const int valid = static_cast<int>(min(static_cast<long long>(RK_TILE), count - base));
+    for (int t = threadIdx.x; t < RK_WARPS * RK_RADIX; t += RK_THREADS) (&s_whist[0][0])[t] = 0u;
+    __syncthreads();
+
+    const uint32_t lt_mask = (1u << lane) - 1u;
+    uint32_t key[RK_IPT], val[RK_IPT];
+    uint32_t rank[RK_IPT];
+#pragma unroll
+    for (int k = 0; k < RK_IPT; ++k) {
+        const int t = warp * (RK_IPT * WARP) + k * WARP + lane;
+        const bool ok = t < valid;
+        key[k] = ok ? load_key<FIRST>(keys_in, base + t) : 0u;
+        val[k] = ok ? vals_in[base + t] : 0u;
+        const uint32_t d = ok ? ((key[k] >> shift) & 255u) : 256u;
+        const uint32_t peers = __match_any_sync(0xffffffffu, d);
+        const uint32_t before = ok ? s_whist[warp][d] : 0u;
+        __syncwarp();
+        if (ok && (peers & lt_mask) == 0u) s_whist[warp][d] = before + __popc(peers);
+        __syncwarp();
+        rank[k] = before + __popc(peers & lt_mask);
+    }
+    __syncthreads();
+    // thread d: counts of digit d in earlier warps, the digit's start in the tile, its global offset
+    {
+        const int d = threadIdx.x;
+        uint32_t run = 0;
+#pragma unroll
+        for (int w = 0; w < RK_WARPS; ++w) {
+            const uint32_t c = s_whist[w][d];
+            s_whist[w][d] = run;
+            run += c;
+        }
+        const uint32_t start = block_excl_scan<uint32_t, RK_THREADS>(run, s_warp, nullptr);
+        s_start[d] = start;
+        s_gout[d] = offsets[static_cast<long long>(d) * tiles + blockIdx.x];
+    }
+    __syncthreads();
+#pragma unroll
+    for (int k = 0; k < RK_IPT; ++k) {
+        const int t = warp * (RK_IPT * WARP) + k * WARP + lane;
+        if (t < valid) {
+            const uint32_t d = (key[k] >> shift) & 255u;
+            const uint32_t p = s_start[d] + s_whist[warp][d] + rank[k];
+            s_keys[p] = key[k];
+            s_vals[p] = val[k];
+        }
+    }
+    __syncthreads();
+    for (int t = threadIdx.x; t < valid; t += RK_THREADS) {
+        const uint32_t k = s_keys[t];
+        const uint32_t d = (k >> shift) & 255u;
+        const long long o = static_cast<long long>(s_gout[d]) + (t - static_cast<int>(s_start[d]));
+        keys_out[o] = k;
+        vals_out[o] = s_vals[t];
+    }
+}
+
+struct SortWs {
+    uint32_t *keys, *vals, *counts, *sums;
+};
+static int rank_tiles(long long count) { return ceil_div(count, RK_TILE); }
+
+static bool sort_ws_take(Arena& a, long long count, SortWs* w) {
+    const long long tiles = rank_tiles(count);
+    const long long counts = tiles * RK_RADIX;
+    w->keys = a.take<uint32_t>(count);
+    w->vals = a.take<uint32_t>(count);
+    w->counts = a.take<uint32_t>(counts);
+    w->sums = a.take<uint32_t>(ceil_div(counts, SCAN_CHUNK));
+    return w->keys && w->vals && w->counts && w->sums;
+}
+
+// curve workspace: per tile the packed flag count (correct | (correct & intrain) << 32) and its scan, the tile's
+// first argmax of f1 (value, position), the max of the Ign f1 and the two float64 AUC partials
+struct CurveWs {
+    unsigned long long *flags, *sums;
+    float *best_f1, *best_ign;
+    long long* best_pos;
+    double *auc, *ign_auc;
+};
+static bool curve_ws_take(Arena& a, long long count, CurveWs* w) {
+    const long long tiles = rank_tiles(count);
+    w->flags = a.take<unsigned long long>(tiles);
+    w->sums = a.take<unsigned long long>(ceil_div(tiles, SCAN_CHUNK));
+    w->best_f1 = a.take<float>(tiles);
+    w->best_ign = a.take<float>(tiles);
+    w->best_pos = a.take<long long>(tiles);
+    w->auc = a.take<double>(tiles);
+    w->ign_auc = a.take<double>(tiles);
+    return w->flags && w->sums && w->best_f1 && w->best_ign && w->best_pos && w->auc && w->ign_auc;
+}
+
+// The scans and the curve read their workspace arrays with 16-byte loads: the arena starts at the first 256-byte
+// boundary of the caller's workspace, whatever its alignment (rank_ws_bytes includes the slack).
+static Arena rank_arena(void* ws, size_t ws_bytes) {
+    const uintptr_t p = reinterpret_cast<uintptr_t>(ws);
+    const size_t skip = ((p + 255) & ~uintptr_t(255)) - p;
+    if (ws == nullptr || ws_bytes < skip) return Arena(nullptr, 0);
+    return Arena(static_cast<char*>(ws) + skip, ws_bytes - skip);
+}
+
+size_t rank_ws_bytes(long long count) {
+    if (count <= 0) return 512;
+    Arena probe(reinterpret_cast<void*>(256), ~size_t(0) >> 1);
+    SortWs s;
+    sort_ws_take(probe, count, &s);
+    const size_t sort_bytes = probe.off;
+    Arena probe2(reinterpret_cast<void*>(256), ~size_t(0) >> 1);
+    CurveWs c;
+    curve_ws_take(probe2, count, &c);
+    return std::max(sort_bytes, probe2.off) + 256;
+}
+
+int launch_rank_candidates(const gcgcn_batch* bt, const float* z, const float* labels, const uint8_t* intrain, int R,
+                           long long base_id, float* score, uint32_t* payload, unsigned long long* counters,
+                           cudaStream_t st) {
+    if (bt->total_nodes <= 0) return GCGCN_OK;
+    rank_candidates_kernel<<<bt->total_nodes, 256, 0, st>>>(bt->node_ptr, reinterpret_cast<const long long*>(bt->pair_ptr),
+                                                            bt->row_doc, z, labels, intrain, R, base_id, score, payload,
+                                                            counters);
+    GCGCN_CHECK_LAUNCH("rank_candidates");
+    return GCGCN_OK;
+}
+
+int launch_rank_sort(const float* score, const uint32_t* payload, long long count, uint32_t* sorted_key,
+                     uint32_t* sorted_payload, void* ws, size_t ws_bytes, cudaStream_t st) {
+    if (count <= 0) return GCGCN_OK;
+    Arena a = rank_arena(ws, ws_bytes);
+    SortWs w;
+    if (!sort_ws_take(a, count, &w)) return fail(GCGCN_ERR_WORKSPACE, "rank_sort: workspace too small (%zu bytes)", ws_bytes);
+    const int tiles = rank_tiles(count);
+    const long long ncounts = static_cast<long long>(tiles) * RK_RADIX;
+    // passes: scores -> ws -> out -> ws -> out
+    const void* kin = score;
+    const uint32_t* vin = payload;
+    for (int pass = 0; pass < 4; ++pass) {
+        uint32_t* kout = (pass & 1) ? sorted_key : w.keys;
+        uint32_t* vout = (pass & 1) ? sorted_payload : w.vals;
+        const int shift = 8 * pass;
+        if (pass == 0) radix_upsweep_kernel<true><<<tiles, RK_THREADS, 0, st>>>(kin, count, shift, tiles, w.counts);
+        else radix_upsweep_kernel<false><<<tiles, RK_THREADS, 0, st>>>(kin, count, shift, tiles, w.counts);
+        GCGCN_CHECK_LAUNCH("rank_radix_upsweep");
+        GCGCN_TRY(launch_scan<uint32_t>(w.counts, ncounts, w.sums, st));
+        if (pass == 0)
+            radix_downsweep_kernel<true><<<tiles, RK_THREADS, 0, st>>>(kin, vin, count, shift, tiles, w.counts, kout, vout);
+        else
+            radix_downsweep_kernel<false><<<tiles, RK_THREADS, 0, st>>>(kin, vin, count, shift, tiles, w.counts, kout, vout);
+        GCGCN_CHECK_LAUNCH("rank_radix_downsweep");
+        kin = kout;
+        vin = vout;
+    }
+    return GCGCN_OK;
+}
+
+// ---- curve -------------------------------------------------------------------------------------------------------
+// x = f32(c / T), y = f32(c / (k + 1)): one double division, rounded once.  f1 = 2 x y / ((x + y) + 1e-20) in float32,
+// each operation rounded (no contraction): NumPy's  2 * pr_x * pr_y / (pr_x + pr_y + 1e-20)  on float32 arrays.
+__device__ __forceinline__ float curve_ratio(long long a, long long b) {
+    return __double2float_rn(static_cast<double>(a) / static_cast<double>(b));
+}
+__device__ __forceinline__ float curve_f1(float x, float y) {
+    return __fdiv_rn(__fmul_rn(__fmul_rn(2.f, x), y), __fadd_rn(__fadd_rn(x, y), 1e-20f));
+}
+// Ign precision: facts seen in training are left out of the numerator and the denominator
+__device__ __forceinline__ float curve_ign(long long c, long long t, long long k1) {
+    return t == c ? 0.f : curve_ratio(c - t, k1 - t);
+}
+// one np.trapezoid term in float32:  (x1 - x0) * (y1 + y0) / 2
+__device__ __forceinline__ double curve_trap(float x0, float x1, float y0, float y1) {
+    return static_cast<double>(__fdiv_rn(__fmul_rn(__fsub_rn(x1, x0), __fadd_rn(y1, y0)), 2.f));
+}
+
+// per-tile packed flag counts: correct in the low word, correct & intrain in the high word (both < 2^30)
+__global__ void __launch_bounds__(RK_THREADS)
+curve_count_kernel(const uint32_t* __restrict__ pay, long long count, unsigned long long* __restrict__ flags) {
+    __shared__ unsigned long long s_warp[33];
+    const long long base = static_cast<long long>(blockIdx.x) * RK_TILE + threadIdx.x * static_cast<long long>(RK_IPT);
+    uint32_t p[RK_IPT];
+    load16(pay, base, count, p);
+    unsigned long long acc = 0;
+#pragma unroll
+    for (int k = 0; k < RK_IPT; ++k) acc += (p[k] & 1u) + (static_cast<unsigned long long>((p[k] & 3u) == 3u) << 32);
+    unsigned long long total;
+    block_excl_scan<unsigned long long, RK_THREADS>(acc, s_warp, &total);
+    if (threadIdx.x == 0) flags[blockIdx.x] = total;
+}
+
+// Thread t of tile b owns positions [b TILE + 16 t, +16).  prefix = the scanned tile counts + an in-tile scan.
+__global__ void __launch_bounds__(RK_THREADS)
+curve_main_kernel(const uint32_t* __restrict__ pay, long long count, long long T, int has_intrain,
+                  const unsigned long long* __restrict__ tile_prefix, float* __restrict__ best_f1,
+                  long long* __restrict__ best_pos, float* __restrict__ best_ign, double* __restrict__ auc,
+                  double* __restrict__ ign_auc) {
+    __shared__ unsigned long long s_warp[33];
+    __shared__ float s_f1[RK_THREADS], s_ign[RK_THREADS];
+    __shared__ long long s_pos[RK_THREADS];
+    __shared__ double s_auc[RK_THREADS], s_iauc[RK_THREADS];
+    const long long base = static_cast<long long>(blockIdx.x) * RK_TILE + threadIdx.x * static_cast<long long>(RK_IPT);
+    uint32_t p[RK_IPT + 1];
+    load16(pay, base, count, *reinterpret_cast<uint32_t(*)[RK_IPT]>(p));
+    p[RK_IPT] = base + RK_IPT < count ? pay[base + RK_IPT] : 0u;
+    unsigned long long acc = 0;
+#pragma unroll
+    for (int k = 0; k < RK_IPT; ++k) acc += (p[k] & 1u) + (static_cast<unsigned long long>((p[k] & 3u) == 3u) << 32);
+    const unsigned long long pre = block_excl_scan<unsigned long long, RK_THREADS>(acc, s_warp, nullptr) +
+                                   tile_prefix[blockIdx.x];
+    long long c = static_cast<long long>(pre & 0xffffffffull), t = static_cast<long long>(pre >> 32);
+    float f1_best = -1.f, ign_best = -1.f;
+    long long pos_best = -1;
+    double a = 0.0, ai = 0.0;
+    // (x, y, yi) at position k carried to the trapezoid term of (k, k + 1)
+    float xk = 0.f, yk = 0.f, yik = 0.f;
+#pragma unroll
+    for (int k = 0; k <= RK_IPT; ++k) {
+        const long long pos = base + k;
+        if (pos < count) {
+            c += p[k] & 1u;
+            t += (p[k] & 3u) == 3u;
+            const float x = curve_ratio(c, T), y = curve_ratio(c, pos + 1);
+            const float yi = has_intrain ? curve_ign(c, t, pos + 1) : 0.f;
+            if (k > 0) {
+                a += curve_trap(xk, x, yk, y);
+                if (has_intrain) ai += curve_trap(xk, x, yik, yi);
+            }
+            if (k < RK_IPT) {            // k == RK_IPT is the next thread's first position: only the term is ours
+                const float f = curve_f1(x, y);
+                if (f > f1_best) { f1_best = f; pos_best = pos; }
+                if (has_intrain) ign_best = fmaxf(ign_best, curve_f1(x, yi));
+                xk = x; yk = y; yik = yi;
+            }
+        }
+    }
+    s_f1[threadIdx.x] = f1_best;
+    s_pos[threadIdx.x] = pos_best;
+    s_ign[threadIdx.x] = ign_best;
+    s_auc[threadIdx.x] = a;
+    s_iauc[threadIdx.x] = ai;
+    __syncthreads();
+    for (int s = RK_THREADS / 2; s > 0; s >>= 1) {
+        if (threadIdx.x < s) {
+            const int o = threadIdx.x + s;
+            // first argmax: on equal f1 the smaller position wins
+            if (s_f1[o] > s_f1[threadIdx.x] || (s_f1[o] == s_f1[threadIdx.x] && s_pos[o] < s_pos[threadIdx.x])) {
+                s_f1[threadIdx.x] = s_f1[o];
+                s_pos[threadIdx.x] = s_pos[o];
+            }
+            s_ign[threadIdx.x] = fmaxf(s_ign[threadIdx.x], s_ign[o]);
+            s_auc[threadIdx.x] += s_auc[o];
+            s_iauc[threadIdx.x] += s_iauc[o];
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        best_f1[blockIdx.x] = s_f1[0];
+        best_pos[blockIdx.x] = s_pos[0];
+        best_ign[blockIdx.x] = s_ign[0];
+        auc[blockIdx.x] = s_auc[0];
+        ign_auc[blockIdx.x] = s_iauc[0];
+    }
+}
+
+// One block: fixed-order reduction of the tile partials, w, and the curve values at w.
+__global__ void __launch_bounds__(1024)
+curve_finish_kernel(const uint32_t* __restrict__ key, const uint32_t* __restrict__ pay, long long count, long long T,
+                    int has_intrain, double input_theta, int tiles, const unsigned long long* __restrict__ tile_prefix,
+                    const float* __restrict__ best_f1, const long long* __restrict__ best_pos,
+                    const float* __restrict__ best_ign, const double* __restrict__ auc,
+                    const double* __restrict__ ign_auc, gcgcn_rank_result* __restrict__ res) {
+    __shared__ float s_f1[1024], s_ign[1024];
+    __shared__ long long s_pos[1024];
+    __shared__ double s_auc[1024], s_iauc[1024];
+    __shared__ long long s_w;
+    __shared__ unsigned long long s_warp[33];
+    float f = -1.f, g = -1.f;
+    long long bp = -1;
+    double a = 0.0, ai = 0.0;
+    for (int i = threadIdx.x; i < tiles; i += 1024) {       // ascending tiles per thread: strict > keeps the first
+        if (best_f1[i] > f) { f = best_f1[i]; bp = best_pos[i]; }
+        g = fmaxf(g, best_ign[i]);
+        a += auc[i];
+        ai += ign_auc[i];
+    }
+    s_f1[threadIdx.x] = f; s_pos[threadIdx.x] = bp; s_ign[threadIdx.x] = g;
+    s_auc[threadIdx.x] = a; s_iauc[threadIdx.x] = ai;
+    __syncthreads();
+    for (int s = 512; s > 0; s >>= 1) {
+        if (threadIdx.x < s) {
+            const int o = threadIdx.x + s;
+            // equal f1: the smaller position wins (the tree does not keep positions in order)
+            if (s_f1[o] > s_f1[threadIdx.x] || (s_f1[o] == s_f1[threadIdx.x] && s_pos[o] < s_pos[threadIdx.x])) {
+                s_f1[threadIdx.x] = s_f1[o];
+                s_pos[threadIdx.x] = s_pos[o];
+            }
+            s_ign[threadIdx.x] = fmaxf(s_ign[threadIdx.x], s_ign[o]);
+            s_auc[threadIdx.x] += s_auc[o];
+            s_iauc[threadIdx.x] += s_iauc[o];
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        long long w;
+        if (input_theta == -1.0) {
+            w = s_pos[0];
+        } else {
+            // scores descend along the ranking: count the prefix with score > input_theta
+            long long lo = 0, hi = count;
+            while (lo < hi) {
+                const long long mid = (lo + hi) >> 1;
+                if (static_cast<double>(key_score(key[mid])) > input_theta) lo = mid + 1;
+                else hi = mid;
+            }
+            w = lo > 0 ? lo - 1 : 0;
+        }
+        s_w = w;
+    }
+    __syncthreads();
+    // flag counts up to and including w: the scanned tile prefix + this tile's positions <= w
+    const long long w = s_w;
+    const long long t0 = (w / RK_TILE) * RK_TILE;
+    unsigned long long acc = 0;
+    for (long long i = t0 + threadIdx.x; i <= w; i += 1024) {
+        const uint32_t p = pay[i];
+        acc += (p & 1u) + (static_cast<unsigned long long>((p & 3u) == 3u) << 32);
+    }
+    unsigned long long total;
+    block_excl_scan<unsigned long long, 1024>(acc, s_warp, &total);
+    if (threadIdx.x == 0) {
+        const unsigned long long pre = total + tile_prefix[w / RK_TILE];
+        const long long c = static_cast<long long>(pre & 0xffffffffull), t = static_cast<long long>(pre >> 32);
+        const float x = curve_ratio(c, T), y = curve_ratio(c, w + 1);
+        gcgcn_rank_result r;
+        r.count = count;
+        r.total_recall = T;
+        r.best_pos = s_pos[0];
+        r.w = w;
+        r.auc = s_auc[0];
+        r.ign_auc = has_intrain ? s_iauc[0] : 0.0;
+        r.f1 = s_f1[0];
+        r.theta = key_score(key[s_pos[0]]);
+        r.f1_at_w = curve_f1(x, y);
+        r.precision_at_w = y;
+        r.recall_at_w = x;
+        r.ign_f1 = has_intrain ? s_ign[0] : 0.f;
+        r.ign_f1_at_w = has_intrain ? curve_f1(x, curve_ign(c, t, w + 1)) : 0.f;
+        r.reserved = 0;
+        *res = r;
+    }
+}
+
+int launch_rank_curve(const uint32_t* key, const uint32_t* pay, long long count, long long T, int has_intrain,
+                      double input_theta, gcgcn_rank_result* res, void* ws, size_t ws_bytes, cudaStream_t st) {
+    Arena a = rank_arena(ws, ws_bytes);
+    CurveWs w;
+    if (!curve_ws_take(a, count, &w)) return fail(GCGCN_ERR_WORKSPACE, "rank_curve: workspace too small (%zu bytes)", ws_bytes);
+    const int tiles = rank_tiles(count);
+    curve_count_kernel<<<tiles, RK_THREADS, 0, st>>>(pay, count, w.flags);
+    GCGCN_CHECK_LAUNCH("rank_curve_count");
+    GCGCN_TRY(launch_scan<unsigned long long>(w.flags, tiles, w.sums, st));
+    curve_main_kernel<<<tiles, RK_THREADS, 0, st>>>(pay, count, T, has_intrain, w.flags, w.best_f1, w.best_pos,
+                                                    w.best_ign, w.auc, w.ign_auc);
+    GCGCN_CHECK_LAUNCH("rank_curve_main");
+    curve_finish_kernel<<<1, 1024, 0, st>>>(key, pay, count, T, has_intrain, input_theta, tiles, w.flags, w.best_f1,
+                                            w.best_pos, w.best_ign, w.auc, w.ign_auc, res);
+    GCGCN_CHECK_LAUNCH("rank_curve_finish");
+    return GCGCN_OK;
+}
+
+// ---- decode -----------------------------------------------------------------------------------------------------
+// doc_off [docs + 1]: first candidate id of every document (in add() order); the document of an id is the last one
+// whose offset is <= id (documents with n <= 1 own no ids and share their successor's offset).
+__global__ void __launch_bounds__(256)
+rank_decode_kernel(const uint32_t* __restrict__ key, const uint32_t* __restrict__ pay, long long rows,
+                   const long long* __restrict__ doc_off, const int* __restrict__ doc_n, int docs, int R,
+                   int* __restrict__ doc, int* __restrict__ row, int* __restrict__ col, int* __restrict__ rel,
+                   float* __restrict__ score) {
+    const long long k = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (k >= rows) return;
+    const long long id = pay[k] >> 2;
+    int lo = 0, hi = docs;                           // first document whose offset is > id, minus one
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (doc_off[mid] <= id) lo = mid + 1;
+        else hi = mid;
+    }
+    const int b = lo - 1;
+    const int n = doc_n[b];
+    const long long local = id - doc_off[b];
+    const long long per_row = static_cast<long long>(n - 1) * (R - 1);
+    const int i = static_cast<int>(local / per_row);
+    const long long rem = local - i * per_row;
+    const int jj = static_cast<int>(rem / (R - 1));
+    doc[k] = b;
+    row[k] = i;
+    col[k] = jj + (jj >= i);
+    rel[k] = static_cast<int>(rem - static_cast<long long>(jj) * (R - 1)) + 1;
+    score[k] = key_score(key[k]);
+}
+
+int launch_rank_decode(const uint32_t* key, const uint32_t* pay, long long rows, const long long* doc_off,
+                       const int* doc_n, int docs, int R, int* doc, int* row, int* col, int* rel, float* score,
+                       cudaStream_t st) {
+    if (rows <= 0) return GCGCN_OK;
+    rank_decode_kernel<<<ceil_div(rows, 256), 256, 0, st>>>(key, pay, rows, doc_off, doc_n, docs, R, doc, row, col, rel,
+                                                           score);
+    GCGCN_CHECK_LAUNCH("rank_decode");
+    return GCGCN_OK;
+}
+
+}  // namespace gcgcn

@@ -447,6 +447,70 @@ int gcgcn_pair_bce_fwd(const gcgcn_batch* bt, const float* logits, const float* 
 int gcgcn_pair_bce_bwd(const gcgcn_batch* bt, const float* logits, const float* labels, int32_t relations,
                        const float* dloss, float* dlogits, void* stream);
 
+/* ---- relation evaluation (config/Config.py:432-561; Ign F1 of config/Config_bert.py:626-650) ---------------------
+ * The DocRED baseline evaluation on the device.  A candidate is (document, row i, column j, relation r) with i != j and
+ * 1 <= r < R; its id is its position in insertion order (batches in call order, then documents, i, j, r ascending).
+ *   score   = 1 / (1 + exp(-logit))                float32, the loss kernel's sigmoid
+ *   correct = labels[p][r] > 0.5;  intrain = intrain[p][r] != 0 (counts only where correct)
+ * Ranking: score descending, stable (equal scores keep id order).  At ranked position k (0-based), with c_k / t_k the
+ * running counts of correct / correct-and-intrain candidates and T = total_recall:
+ *   x_k = f32(c_k / T), y_k = f32(c_k / (k + 1))   (double division, one rounding)
+ *   f1_k = (2 x_k y_k) / ((x_k + y_k) + 1e-20)       (float32, every operation rounded, no contraction)
+ *   yi_k = 0 if t_k == c_k, else f32((c_k - t_k) / (k + 1 - t_k))   (Ign precision; the x axis stays x_k)
+ *   best_pos = first argmax of f1_k, theta = its score, auc = sum_k f32((x_{k+1} - x_k) (y_{k+1} + y_k) / 2) (terms as
+ *   np.trapezoid forms them in float32, summed in float64 in a fixed order; 0 for one candidate)
+ *   w = best_pos if input_theta == -1, else the last position whose score > input_theta (0 if none).
+ * One evaluator holds fewer than 2^30 candidates (the payload packs id << 2 | intrain << 1 | correct):
+ * GCGCN_ERR_UNSUPPORTED beyond that.  Every result is bit-reproducible.                                             */
+#define GCGCN_RANK_TILE 4096          /* candidates per CTA of the sort and curve kernels */
+#define GCGCN_RANK_MAX_CANDIDATES (1LL << 30)
+
+typedef struct gcgcn_rank_result {    /* 80 bytes, written on the device by gcgcn_rank_curve                */
+    int64_t count;                    /*  0: candidates N                                                 */
+    int64_t total_recall;             /*  8: T actually used (>= 1)                                       */
+    int64_t best_pos;                 /* 16: first argmax of f1_k                                         */
+    int64_t w;                        /* 24: position the *_at_w fields are read at                       */
+    double auc;                       /* 32                                                               */
+    double ign_auc;                   /* 40: 0 without intrain                                            */
+    float f1;                         /* 48: f1_k at best_pos                                             */
+    float theta;                      /* 52: score at best_pos                                            */
+    float f1_at_w;                    /* 56                                                               */
+    float precision_at_w;             /* 60: y_w                                                          */
+    float recall_at_w;                /* 64: x_w                                                          */
+    float ign_f1;                     /* 68: max_k of the Ign f1 (0 without intrain)                      */
+    float ign_f1_at_w;                /* 72: (0 without intrain)                                          */
+    float reserved;                   /* 76                                                               */
+} gcgcn_rank_result;
+
+/* workspace of gcgcn_rank_sort and gcgcn_rank_curve for `count` candidates (about 8 bytes per candidate; any
+ * alignment: the library aligns inside it)                                                                         */
+size_t gcgcn_rank_ws_bytes(int64_t count);
+/* Scores and payloads of every candidate of one batch: logits / labels [total_pairs, relations] float32, intrain
+ * [total_pairs, relations] uint8.  labels NULL: nothing is correct (unlabeled sets); intrain NULL: nothing is.
+ * Candidate ids start at base_id (the count of earlier batches); score / payload receive this batch's
+ * (total_pairs - total_nodes) (relations - 1) candidates at [id - base_id].  counters[0] += correct candidates,
+ * counters[1] += NaN scores (int64, accumulated across batches).                                                    */
+int gcgcn_rank_candidates(const gcgcn_batch* bt, const float* logits, int32_t relations, const float* labels,
+                          const uint8_t* intrain, int64_t base_id, float* score, uint32_t* payload, int64_t* counters,
+                          void* stream);
+/* Stable ranking of `count` candidates: sorted_key[k] = ~bits(score) of the k-th ranked candidate (ascending keys =
+ * descending scores), sorted_payload[k] its payload.  ws >= gcgcn_rank_ws_bytes(count).                           */
+int gcgcn_rank_sort(const float* score, const uint32_t* payload, int64_t count, uint32_t* sorted_key,
+                    uint32_t* sorted_payload, void* ws, size_t ws_bytes, void* stream);
+/* The curve over a ranking from gcgcn_rank_sort; writes *result (device memory) on the stream.  total_recall < 1
+ * means 1.  has_intrain = 0 leaves the Ign fields 0.  The result is meaningless if any score is NaN.
+ * sorted_payload 16-byte aligned.                                                                               */
+int gcgcn_rank_curve(const uint32_t* sorted_key, const uint32_t* sorted_payload, int64_t count, int64_t total_recall,
+                     int32_t has_intrain, double input_theta, gcgcn_rank_result* result, void* ws, size_t ws_bytes,
+                     void* stream);
+/* The first `rows` ranked candidates (rows <= count, the ranking's length) as (doc, row, col, relation, score) int32 /
+ * float32 [rows].  doc_offsets
+ * [num_docs + 1] int64: first candidate id of each document, (n_b^2 - n_b)(relations - 1) apart; doc_n [num_docs]
+ * int32 entity counts.  doc is the document's index in doc_offsets.                                               */
+int gcgcn_rank_decode(const uint32_t* sorted_key, const uint32_t* sorted_payload, int64_t rows, int64_t count,
+                      const int64_t* doc_offsets, const int32_t* doc_n, int32_t num_docs, int32_t relations, int32_t* doc,
+                      int32_t* row, int32_t* col, int32_t* relation, float* score, void* stream);
+
 /* ---- training step of config 5 (new work: the reference has no multi-GPU path, SURVEY.md 8e) ----
  * Fused Adam over ONE flat float32 buffer holding every hot-path parameter, with the semantics of
  * torch.optim.Adam as the reference's trainer constructs it (config/Config.py:300: lr only, betas

@@ -47,7 +47,7 @@ size_t block_frag_floats(int heads, int layers);
 enum { ATT_GRAD_DA = 0, ATT_GRAD_DS = 1, ATT_GRAD_DQ = 2 };   // == BK_OUT_* of gcn_block.cu
 int launch_gemm(int ta, int tb, int M, int N, int K, float alpha, const float* A, int lda, const float* B,
                 int ldb, float beta, float* C, int ldc, const float* bias, void* ws, size_t ws_bytes,
-                cudaStream_t st, void* pre_ws = nullptr, size_t pre_bytes = 0);
+                cudaStream_t st);
 size_t gemm_presplit_bytes(int rows);
 int launch_colsum(const float* X, int M, int N, int ldx, float* out, void* ws, size_t ws_bytes, cudaStream_t st);
 int launch_gemm_batched(int ta, int tb, int M, int N, int K, float alpha, const float* A, int lda, const float* B,
@@ -329,7 +329,6 @@ size_t gcgcn_workspace_bytes(int32_t total_nodes, int64_t total_pairs, int32_t h
     b += GEMM_WS_BYTES + (size_t(8) << 20);                            // split-K and reduction partials
     b += size_t(4) << 20;                                              // fragment-ordered dense-connect weights
     b += size_t(256) << 10;                                            // head-summed output weights
-    b += align256(gemm_presplit_bytes(total_nodes < 0 ? 0 : total_nodes));   // pre-split [rows,128] operand of the weight-gradient GEMMs
     return b;
 }
 
@@ -611,16 +610,13 @@ static int stack_bwd_impl(const gcgcn_batch* bt, int32_t heads, int32_t layers, 
     float* dE = ar.take<float>(static_cast<size_t>(M) * HD);
     float* gws = ar.take<float>(GEMM_WS_BYTES / sizeof(float));
     float* frag = (slab == D && layers > 1 && D % layers == 0) ? ar.take<float>(block_frag_floats(heads, layers)) : nullptr;
-    const size_t pre_bytes = gemm_presplit_bytes(M);         // pre-split copy of a [rows, 128] operand (optional)
-    void* pre = ar.take<uint8_t>(pre_bytes);
     if ((linear && dFbuf == nullptr) || dZ == nullptr || dE == nullptr || gws == nullptr)
         return fail(GCGCN_ERR_WORKSPACE, "stack_bwd: workspace too small");
     const float* dF = dy;
     if (linear) {
         GCGCN_TRY(launch_gemm(0, 0, M, HD, D, 1.f, dy, D, Wout, HD, 0.f, dFbuf, HD, nullptr, gws, GEMM_WS_BYTES, st));
         if (dWout != nullptr)
-            GCGCN_TRY(launch_gemm(1, 0, D, HD, M, 1.f, dy, D, F, HD, 0.f, dWout, HD, nullptr, gws, GEMM_WS_BYTES, st, pre,
-                                  pre == nullptr ? 0 : pre_bytes));
+            GCGCN_TRY(launch_gemm(1, 0, D, HD, M, 1.f, dy, D, F, HD, 0.f, dWout, HD, nullptr, gws, GEMM_WS_BYTES, st));
         if (dbout != nullptr) GCGCN_TRY(launch_colsum(dy, M, D, D, dbout, gws, GEMM_WS_BYTES, st));
         dF = dFbuf;
     }
@@ -644,11 +640,9 @@ static int stack_bwd_impl(const gcgcn_batch* bt, int32_t heads, int32_t layers, 
     GCGCN_TRY(launch_gemm(0, 1, M, in_dim, HD, 1.f, dZ, HD, WnX, HD, beta, dx, in_dim, nullptr, gws, GEMM_WS_BYTES, st));
     GCGCN_TRY(launch_gemm(0, 1, M, D, HD, 1.f, dE, HD, We, HD, 0.f, debar, D, nullptr, gws, GEMM_WS_BYTES, st));
     if (dWnX != nullptr)
-        GCGCN_TRY(launch_gemm(1, 0, in_dim, HD, M, 1.f, x, in_dim, dZ, HD, 0.f, dWnX, HD, nullptr, gws, GEMM_WS_BYTES, st, pre,
-                              pre == nullptr ? 0 : pre_bytes));
+        GCGCN_TRY(launch_gemm(1, 0, in_dim, HD, M, 1.f, x, in_dim, dZ, HD, 0.f, dWnX, HD, nullptr, gws, GEMM_WS_BYTES, st));
     if (dWe != nullptr)
-        GCGCN_TRY(launch_gemm(1, 0, D, HD, M, 1.f, ebar, D, dE, HD, 0.f, dWe, HD, nullptr, gws, GEMM_WS_BYTES, st, pre,
-                              pre == nullptr ? 0 : pre_bytes));
+        GCGCN_TRY(launch_gemm(1, 0, D, HD, M, 1.f, ebar, D, dE, HD, 0.f, dWe, HD, nullptr, gws, GEMM_WS_BYTES, st));
     if (dWinner != nullptr && layers > 1) {
         GCGCN_TRY(cuda_ok(cudaMemsetAsync(dWinner, 0, static_cast<size_t>(heads) * layers * slab * gd * sizeof(float), st),
                           "memset dWinner"));
@@ -1347,12 +1341,11 @@ int gcgcn_gemm(int32_t ta, int32_t tb, int32_t M, int32_t N, int32_t K, float al
         GCGCN_TRY(check_device_ptr(A, "A"));
         GCGCN_TRY(check_device_ptr(B, "B"));
     }
-    // the first GEMM_WS_BYTES of ws hold split-K partials / pre-split weight blobs; anything beyond may hold the
-    // pre-split short operand of a weight-gradient shaped product
+    // only the first GEMM_WS_BYTES of ws are used (split-K partials / pre-split weight blobs).  The split-K count and the
+    // choice of kernel depend on the size passed; the cap keeps them independent of how large a workspace the caller has
     const size_t head = ws_bytes < GEMM_WS_BYTES ? ws_bytes : GEMM_WS_BYTES;
-    void* pre = (ws != nullptr && ws_bytes > head) ? static_cast<char*>(ws) + head : nullptr;
     return launch_gemm(ta, tb, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, bias, ws, head,
-                       static_cast<cudaStream_t>(stream), pre, pre == nullptr ? 0 : ws_bytes - head);
+                       static_cast<cudaStream_t>(stream));
 }
 
 // ---- block-level composites ------------------------------------------------------------------

@@ -106,17 +106,6 @@ static size_t mha_smem(int n, int dh) {
     return (static_cast<size_t>(n) * (dh + 1) + static_cast<size_t>(MHA_WARPS) * n) * sizeof(float);
 }
 
-template <typename K>
-static int set_smem(K kernel, size_t bytes, const char* name) {
-    if (bytes > 227 * 1024)
-        return fail(GCGCN_ERR_UNSUPPORTED, "%s needs %zu bytes of shared memory (> 227 KB): documents "
-                    "this large are not supported", name, bytes);
-    if (bytes > 48 * 1024)
-        return cuda_ok(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                            static_cast<int>(bytes)), name);
-    return GCGCN_OK;
-}
-
 int launch_mha_fwd(const gcgcn_batch* bt, int heads, const float* q, const float* keep, float* P,
                    float* A, cudaStream_t st) {
     if (bt->num_docs == 0) return GCGCN_OK;

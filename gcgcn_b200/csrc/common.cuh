@@ -77,6 +77,27 @@ inline void device_mark_prepared(std::atomic<unsigned long long>& mask) {
     mask.fetch_or(1ULL << dev, std::memory_order_release);
 }
 
+// Dynamic shared memory above the default 48 KB must be enabled per kernel; more than an SM has (227 KB) is refused.
+template <typename K>
+inline int set_smem(K kernel, size_t bytes, const char* name) {
+    if (bytes > 227 * 1024)
+        return fail(GCGCN_ERR_UNSUPPORTED, "%s needs %zu bytes of shared memory (> 227 KB): documents "
+                    "this large are not supported", name, bytes);
+    if (bytes > 48 * 1024)
+        return cuda_ok(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                            static_cast<int>(bytes)), name);
+    return GCGCN_OK;
+}
+// set_smem for a kernel that always launches with the same size, once per device; `mask` is a static of the caller,
+// one per kernel instantiation
+template <typename K>
+inline int set_smem_once(std::atomic<unsigned long long>& mask, K kernel, size_t bytes, const char* name) {
+    if (device_prepared(mask)) return GCGCN_OK;
+    const int rc = set_smem(kernel, bytes, name);
+    if (rc == GCGCN_OK) device_mark_prepared(mask);
+    return rc;
+}
+
 #define GCGCN_API_ENTER(stream)                                                          \
     ::gcgcn::StreamDeviceGuard device_guard__(static_cast<cudaStream_t>(stream));        \
     do {                                                                                 \
@@ -116,6 +137,21 @@ struct Arena {
 };
 
 static inline int ceil_div(long long a, long long b) { return static_cast<int>((a + b - 1) / b); }
+
+// One launch per size class (padded n = 64, 48, 32, 16) when the batch carries the doc_order hint, so that small
+// documents do not reserve the shared memory of the largest one: fn(count, first, nmax, order).
+template <class LaunchFn>
+inline int for_each_size_class(const gcgcn_batch* bt, LaunchFn fn) {
+    if (bt->doc_order == nullptr) return fn(bt->num_docs, 0, bt->max_nodes, static_cast<const int*>(nullptr));
+    static const int cap[4] = {64, 48, 32, 16};
+    int first = 0;
+    for (int c = 0; c < 4; ++c) {
+        const int count = bt->class_end[c] - first;
+        if (count > 0) GCGCN_TRY(fn(count, first, cap[c] < bt->max_nodes ? cap[c] : bt->max_nodes, bt->doc_order));
+        first = bt->class_end[c] > first ? bt->class_end[c] : first;
+    }
+    return GCGCN_OK;
+}
 
 // ---- device helpers ------------------------------------------------------------------------
 // sigmoid of a logit (C:355), within 1 ulp of torch.sigmoid: one definition for the loss kernels and the evaluation

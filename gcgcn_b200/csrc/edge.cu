@@ -360,10 +360,7 @@ static int edge_fwd_t(const gcgcn_batch* bt, const T* e, const float* v, const f
                       cudaStream_t st) {
     size_t smem = (EDGE_WARPS * D + bt->max_nodes) * sizeof(float);
     if (v != nullptr) {
-        if (smem > 48 * 1024)
-            GCGCN_TRY(cuda_ok(cudaFuncSetAttribute(edge_row_fwd_kernel<T, true>,
-                                                   cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                   static_cast<int>(smem)), "edge_fwd smem"));
+        GCGCN_TRY(set_smem(edge_row_fwd_kernel<T, true>, smem, "edge_fwd smem"));
         edge_row_fwd_kernel<T, true><<<bt->total_nodes, EDGE_THREADS, smem, st>>>(
             e, bt->node_ptr, reinterpret_cast<const long long*>(bt->pair_ptr), bt->row_doc, v, ux,
             mask, keep, P, A, ebar);

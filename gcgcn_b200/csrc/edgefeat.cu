@@ -602,20 +602,13 @@ static bool word_pool_doc_path(const gcgcn_edge_tables* t) {
     return t->num_active_docs > 0 && t->max_active_len > 0 && t->max_active_len <= WP_MAX_LEN && t->adoc_tok0 != nullptr &&
            t->adoc_len != nullptr && t->adoc_slot_lo != nullptr && t->adoc_slot_hi != nullptr;
 }
-template <typename K>
-static int word_pool_smem_attr(K kernel, size_t bytes, const char* name) {
-    // (the attribute is per device and the size varies with the batch: set it on every launch that needs it)
-    if (bytes > 48 * 1024)
-        return cuda_ok(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(bytes)), name);
-    return GCGCN_OK;
-}
 
 int launch_word_pool_fwd(const gcgcn_edge_tables* t, const float* T, const float* ctx, float* att, float* cwa,
                          cudaStream_t st) {
     if (t->num_slots <= 0) return GCGCN_OK;
     if (word_pool_doc_path(t)) {
         const size_t smem = static_cast<size_t>(t->max_active_len) * (D + EF_BUCKETS) * sizeof(float);
-        GCGCN_TRY(word_pool_smem_attr(word_pool_fwd_doc_kernel, smem, "word_pool_fwd smem"));
+        GCGCN_TRY(set_smem(word_pool_fwd_doc_kernel, smem, "word_pool_fwd smem"));   // (the size varies with the batch)
         word_pool_fwd_doc_kernel<<<t->num_active_docs, 256, smem, st>>>(make_tabs(t), T, ctx, att, cwa);
         GCGCN_CHECK_LAUNCH("word_pool_fwd<doc>");
         return GCGCN_OK;
@@ -632,7 +625,7 @@ int launch_word_pool_bwd(const gcgcn_edge_tables* t, const float* ctx, const flo
     if (word_pool_doc_path(t)) {
         const size_t L = static_cast<size_t>(t->max_active_len);
         const size_t smem = (L * (D + 32) + WP_ENT * D + 2 * WP_ENT * (L + 1)) * sizeof(float);
-        GCGCN_TRY(word_pool_smem_attr(word_pool_bwd_doc_kernel, smem, "word_pool_bwd smem"));
+        GCGCN_TRY(set_smem(word_pool_bwd_doc_kernel, smem, "word_pool_bwd smem"));
         word_pool_bwd_doc_kernel<<<t->num_active_docs, 256, smem, st>>>(tb, ctx, att, dcwa, dctx, dT);
         GCGCN_CHECK_LAUNCH("word_pool_bwd<doc>");
         return GCGCN_OK;

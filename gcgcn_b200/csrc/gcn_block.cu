@@ -784,12 +784,7 @@ static size_t block_bwd_smem(int np, int layers, int gd) {
 // Block kernels cover: documents of <= 64 nodes, slab 128 cut into 2 x 64 or 4 x 32 sub-layers, and -- when
 // the attention is computed in-kernel -- heads of width 16 or 32.
 bool block_kernels_usable(const gcgcn_batch* bt, int heads, int layers, int slab, bool mha) {
-    static int enabled = -1;
-    if (enabled < 0) {
-        const char* e = getenv("GCGCN_STACK");
-        enabled = (e != nullptr && e[0] != 0 && e[0] != 'b' && e[0] != 'B') ? 0 : 1;   // GCGCN_STACK=mma|simt disables
-    }
-    if (!enabled || slab != D || layers < 1 || slab % layers != 0) return false;
+    if (slab != D || layers < 1 || slab % layers != 0) return false;
     const int gd = slab / layers;
     if (bt->max_nodes > 64 || !(gd == 32 || gd == 64)) return false;
     if (mha) {
@@ -800,33 +795,14 @@ bool block_kernels_usable(const gcgcn_batch* bt, int heads, int layers, int slab
     return true;
 }
 
-template <class LaunchFn>
-static int for_each_size_class(const gcgcn_batch* bt, LaunchFn fn) {
-    if (bt->doc_order == nullptr) return fn(bt->num_docs, 0, bt->max_nodes, static_cast<const int*>(nullptr));
-    static const int cap[4] = {64, 48, 32, 16};
-    int first = 0;
-    for (int c = 0; c < 4; ++c) {
-        const int count = bt->class_end[c] - first;
-        if (count > 0) GCGCN_TRY(fn(count, first, cap[c] < bt->max_nodes ? cap[c] : bt->max_nodes, bt->doc_order));
-        first = bt->class_end[c] > first ? bt->class_end[c] : first;
-    }
-    return GCGCN_OK;
-}
-
-template <typename K>
-static int prepare_kernel(K kernel, size_t max_bytes, const char* name) {
-    return cuda_ok(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                        static_cast<int>(max_bytes)), name);
-}
-
 template <int GD, int DH, int MTC>
 static int launch_fwd_class(const gcgcn_batch* bt, int heads, int count, int first, const int* order, const float* A,
                             const float* q, float* P, float* Z, const float* E, const float* Winner, const float* x,
                             float* G, float* F, float scale, const BlockDrop& drop, cudaStream_t st) {
     constexpr int layers = D / GD;
     const size_t smem = block_fwd_smem(16 * MTC, layers, GD);
-    static std::atomic<unsigned long long> ready{0};        // per device: the attribute is a per-device setting
-    if (!device_prepared(ready)) { GCGCN_TRY(prepare_kernel(block_fwd_kernel<GD, DH, MTC>, smem, "block_fwd")); device_mark_prepared(ready); }
+    static std::atomic<unsigned long long> prepared{0};
+    GCGCN_TRY(set_smem_once(prepared, block_fwd_kernel<GD, DH, MTC>, smem, "block_fwd"));
     block_fwd_kernel<GD, DH, MTC><<<dim3(count, heads), BK_THREADS, smem, st>>>(
         bt->node_ptr, reinterpret_cast<const long long*>(bt->pair_ptr), A, q, P, Z, E, Winner, x, G, F, heads,
         bt->total_pairs, order, first, scale, drop);
@@ -896,8 +872,8 @@ static int launch_bwd_class(const gcgcn_batch* bt, int heads, int count, int fir
                             float* dZ, float* dE, float* dOut, float scale, const BlockDrop& drop, cudaStream_t st) {
     constexpr int layers = D / GD;
     const size_t smem = block_bwd_smem(16 * MTC, layers, GD);
-    static std::atomic<unsigned long long> ready{0};
-    if (!device_prepared(ready)) { GCGCN_TRY(prepare_kernel(block_bwd_kernel<GD, DH, OUT, MTC>, smem, "block_bwd")); device_mark_prepared(ready); }
+    static std::atomic<unsigned long long> prepared{0};
+    GCGCN_TRY(set_smem_once(prepared, block_bwd_kernel<GD, DH, OUT, MTC>, smem, "block_bwd"));
     block_bwd_kernel<GD, DH, OUT, MTC><<<dim3(count, heads), BK_THREADS, smem, st>>>(
         bt->node_ptr, reinterpret_cast<const long long*>(bt->pair_ptr), A, q, Z, G, Winner, dF, dZ, dE, dOut, heads,
         bt->total_pairs, order, first, scale, drop);

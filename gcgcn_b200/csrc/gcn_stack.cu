@@ -403,17 +403,6 @@ static size_t stack_bwd_smem(int n, int layers, int gd) {
     return fl * sizeof(float);
 }
 
-template <typename K>
-static int prep_smem(K kernel, size_t bytes, const char* name) {
-    if (bytes > 227 * 1024)
-        return fail(GCGCN_ERR_UNSUPPORTED,
-                    "%s: a document this large needs %zu bytes of shared memory (> 227 KB)", name, bytes);
-    if (bytes > 48 * 1024)
-        return cuda_ok(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                            static_cast<int>(bytes)), name);
-    return GCGCN_OK;
-}
-
 // tensor-core (mma.sync 3xTF32) versions for n <= 64, gcn_stack_mma.cu
 bool stack_mma_usable(const gcgcn_batch* bt, int layers, int slab);
 int launch_stack_fwd_mma(const gcgcn_batch* bt, int heads, int layers, int slab, int flags, const float* A,
@@ -464,7 +453,7 @@ int launch_stack_fwd(const gcgcn_batch* bt, int heads, int layers, int slab, int
     const long long* pp = reinterpret_cast<const long long*>(bt->pair_ptr);
 #define GCGCN_STACK_FWD(GDV)                                                                        \
     case GDV:                                                                                       \
-        GCGCN_TRY(prep_smem(gcn_stack_fwd_kernel<GDV>, smem, "gcn_stack_fwd"));                     \
+        GCGCN_TRY(set_smem(gcn_stack_fwd_kernel<GDV>, smem, "gcn_stack_fwd"));                      \
         gcn_stack_fwd_kernel<GDV><<<grid, ST_THREADS, smem, st>>>(bt->node_ptr, pp, A, Z, E, Winner, \
                                                                    keep, x, G, F, layers, heads,    \
                                                                    flags, bt->total_pairs);         \
@@ -502,7 +491,7 @@ int launch_stack_bwd(const gcgcn_batch* bt, int heads, int layers, int slab, int
     const long long* pp = reinterpret_cast<const long long*>(bt->pair_ptr);
 #define GCGCN_STACK_BWD(GDV)                                                                        \
     case GDV:                                                                                       \
-        GCGCN_TRY(prep_smem(gcn_stack_bwd_kernel<GDV>, smem, "gcn_stack_bwd"));                     \
+        GCGCN_TRY(set_smem(gcn_stack_bwd_kernel<GDV>, smem, "gcn_stack_bwd"));                      \
         gcn_stack_bwd_kernel<GDV><<<grid, ST_THREADS, smem, st>>>(bt->node_ptr, pp, A, Z, G, Winner, \
                                                                    keep, dF, dZ, dE, dA, layers,    \
                                                                    heads, flags, bt->total_pairs);  \

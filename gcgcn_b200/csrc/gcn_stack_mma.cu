@@ -320,37 +320,9 @@ static size_t bwd_mma_smem(int n, int layers, int gd) {
 }
 
 bool stack_mma_usable(const gcgcn_batch* bt, int layers, int slab) {
-    static int enabled = -1;
-    if (enabled < 0) {
-        const char* e = getenv("GCGCN_STACK");
-        enabled = (e != nullptr && (e[0] == 's' || e[0] == 'S')) ? 0 : 1;    // GCGCN_STACK=simt disables
-    }
-    if (!enabled || layers < 1 || slab % layers != 0) return false;
+    if (layers < 1 || slab % layers != 0) return false;
     const int gd = slab / layers;
     return bt->max_nodes <= 64 && (gd == 32 || gd == 64);
-}
-
-template <typename K>
-static int set_dyn_smem(K kernel, size_t bytes, const char* name) {
-    if (bytes > 48 * 1024)
-        return cuda_ok(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                            static_cast<int>(bytes)), name);
-    return GCGCN_OK;
-}
-
-// One launch per size class (padded n = 64, 48, 32, 16) when the batch carries the doc_order hint, so
-// that small documents do not reserve the shared memory of the largest one.
-template <class LaunchFn>
-static int for_each_class(const gcgcn_batch* bt, LaunchFn fn) {
-    if (bt->doc_order == nullptr) return fn(bt->num_docs, 0, bt->max_nodes, static_cast<const int*>(nullptr));
-    static const int cap[4] = {64, 48, 32, 16};
-    int first = 0;
-    for (int c = 0; c < 4; ++c) {
-        const int count = bt->class_end[c] - first;
-        if (count > 0) GCGCN_TRY(fn(count, first, cap[c] < bt->max_nodes ? cap[c] : bt->max_nodes, bt->doc_order));
-        first = bt->class_end[c] > first ? bt->class_end[c] : first;
-    }
-    return GCGCN_OK;
 }
 
 int launch_stack_fwd_mma(const gcgcn_batch* bt, int heads, int layers, int slab, int flags, const float* A,
@@ -358,9 +330,9 @@ int launch_stack_fwd_mma(const gcgcn_batch* bt, int heads, int layers, int slab,
                          float* G, float* F, cudaStream_t st) {
     const int gd = slab / layers;
     const long long* pp = reinterpret_cast<const long long*>(bt->pair_ptr);
-    GCGCN_TRY(set_dyn_smem(stack_fwd_mma_kernel<64>, fwd_mma_smem(64, layers, 64), "stack_fwd_mma"));
-    GCGCN_TRY(set_dyn_smem(stack_fwd_mma_kernel<32>, fwd_mma_smem(64, layers, 32), "stack_fwd_mma"));
-    return for_each_class(bt, [&](int count, int first, int nmax, const int* order) -> int {
+    GCGCN_TRY(set_smem(stack_fwd_mma_kernel<64>, fwd_mma_smem(64, layers, 64), "stack_fwd_mma"));
+    GCGCN_TRY(set_smem(stack_fwd_mma_kernel<32>, fwd_mma_smem(64, layers, 32), "stack_fwd_mma"));
+    return for_each_size_class(bt, [&](int count, int first, int nmax, const int* order) -> int {
         const size_t smem = fwd_mma_smem(nmax, layers, gd);
         dim3 grid(count, heads);
         if (gd == 64)
@@ -379,9 +351,9 @@ int launch_stack_bwd_mma(const gcgcn_batch* bt, int heads, int layers, int slab,
                          float* dZ, float* dE, float* dA, cudaStream_t st) {
     const int gd = slab / layers;
     const long long* pp = reinterpret_cast<const long long*>(bt->pair_ptr);
-    GCGCN_TRY(set_dyn_smem(stack_bwd_mma_kernel<64>, bwd_mma_smem(64, layers, 64), "stack_bwd_mma"));
-    GCGCN_TRY(set_dyn_smem(stack_bwd_mma_kernel<32>, bwd_mma_smem(64, layers, 32), "stack_bwd_mma"));
-    return for_each_class(bt, [&](int count, int first, int nmax, const int* order) -> int {
+    GCGCN_TRY(set_smem(stack_bwd_mma_kernel<64>, bwd_mma_smem(64, layers, 64), "stack_bwd_mma"));
+    GCGCN_TRY(set_smem(stack_bwd_mma_kernel<32>, bwd_mma_smem(64, layers, 32), "stack_bwd_mma"));
+    return for_each_size_class(bt, [&](int count, int first, int nmax, const int* order) -> int {
         const size_t smem = bwd_mma_smem(nmax, layers, gd);
         dim3 grid(count, heads);
         if (gd == 64)

@@ -497,25 +497,11 @@ static size_t tile_cols_smem(int n, int layers, int gd) {
     return std::max(static_cast<size_t>(k8) * (gd + 8) + static_cast<size_t>(k8) * (TL_ROWS + 8), recycled) * sizeof(float);
 }
 
-// graphs of 65 .. 256 entities with sub-layer width 32 or 64 (GCGCN_STACK=simt keeps gcn_stack.cu)
+// graphs of 65 .. 256 entities with sub-layer width 32 or 64
 bool stack_tiled_usable(const gcgcn_batch* bt, int layers, int slab) {
-    static int enabled = -1;
-    if (enabled < 0) {
-        const char* e = getenv("GCGCN_STACK");
-        enabled = (e != nullptr && (e[0] == 's' || e[0] == 'S')) ? 0 : 1;
-    }
-    if (!enabled || layers < 1 || slab % layers != 0) return false;
+    if (layers < 1 || slab % layers != 0) return false;
     const int gd = slab / layers;
     return bt->max_nodes > 64 && bt->max_nodes <= 256 && bt->num_docs <= 65535 && (gd == 32 || gd == 64);
-}
-
-template <typename K>
-static int tile_smem_attr(K kernel, size_t bytes, const char* name) {
-    if (bytes > 227 * 1024) return fail(GCGCN_ERR_UNSUPPORTED, "%s: %zu bytes of shared memory (> 227 KB)", name, bytes);
-    if (bytes > 48 * 1024)
-        return cuda_ok(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                            static_cast<int>(bytes)), name);
-    return GCGCN_OK;
 }
 
 int launch_stack_fwd_tiled(const gcgcn_batch* bt, int heads, int layers, int slab, int flags, const float* A,
@@ -525,8 +511,8 @@ int launch_stack_fwd_tiled(const gcgcn_batch* bt, int heads, int layers, int sla
     const long long* pp = reinterpret_cast<const long long*>(bt->pair_ptr);
     const dim3 grid(ceil_div(nmax, TL_ROWS), heads, bt->num_docs);
     const size_t smem = tile_fwd_smem(nmax, layers, gd);
-    if (gd == 64) GCGCN_TRY(tile_smem_attr(stack_tile_fwd_kernel<64>, smem, "stack_tile_fwd"));
-    else GCGCN_TRY(tile_smem_attr(stack_tile_fwd_kernel<32>, smem, "stack_tile_fwd"));
+    if (gd == 64) GCGCN_TRY(set_smem(stack_tile_fwd_kernel<64>, smem, "stack_tile_fwd"));
+    else GCGCN_TRY(set_smem(stack_tile_fwd_kernel<32>, smem, "stack_tile_fwd"));
     for (int l = 0; l < layers; ++l) {
         if (gd == 64)
             stack_tile_fwd_kernel<64><<<grid, TL_THREADS, smem, st>>>(bt->node_ptr, pp, A, Z, E, Winner, keep, x, G, F, l,
@@ -548,11 +534,11 @@ int launch_stack_bwd_tiled(const gcgcn_batch* bt, int heads, int layers, int sla
     const dim3 grid_r(ceil_div(nmax, 64), heads, bt->num_docs);
     const size_t smem_r = tile_rows_smem(nmax, gd), smem_c = tile_cols_smem(nmax, layers, gd);
     if (gd == 64) {
-        GCGCN_TRY(tile_smem_attr(stack_tile_bwd_rows_kernel<64>, smem_r, "stack_tile_bwd_rows"));
-        GCGCN_TRY(tile_smem_attr(stack_tile_bwd_cols_kernel<64>, smem_c, "stack_tile_bwd_cols"));
+        GCGCN_TRY(set_smem(stack_tile_bwd_rows_kernel<64>, smem_r, "stack_tile_bwd_rows"));
+        GCGCN_TRY(set_smem(stack_tile_bwd_cols_kernel<64>, smem_c, "stack_tile_bwd_cols"));
     } else {
-        GCGCN_TRY(tile_smem_attr(stack_tile_bwd_rows_kernel<32>, smem_r, "stack_tile_bwd_rows"));
-        GCGCN_TRY(tile_smem_attr(stack_tile_bwd_cols_kernel<32>, smem_c, "stack_tile_bwd_cols"));
+        GCGCN_TRY(set_smem(stack_tile_bwd_rows_kernel<32>, smem_r, "stack_tile_bwd_rows"));
+        GCGCN_TRY(set_smem(stack_tile_bwd_cols_kernel<32>, smem_c, "stack_tile_bwd_cols"));
     }
     for (int l = layers - 1; l >= 0; --l) {
         if (gd == 64)
@@ -650,10 +636,10 @@ int launch_mha_bwd_tiled(const gcgcn_batch* bt, int heads, const float* q, const
     const dim3 grid(ceil_div(nmax, TL_ROWS), heads, bt->num_docs);
     const long long* pp = reinterpret_cast<const long long*>(bt->pair_ptr);
     if (dh == 16) {
-        GCGCN_TRY(tile_smem_attr(mha_bwd_tile_kernel<16>, smem, "mha_bwd_tile"));
+        GCGCN_TRY(set_smem(mha_bwd_tile_kernel<16>, smem, "mha_bwd_tile"));
         mha_bwd_tile_kernel<16><<<grid, TL_THREADS, smem, st>>>(bt->node_ptr, pp, q, dS, dq, bt->total_pairs, scale);
     } else {
-        GCGCN_TRY(tile_smem_attr(mha_bwd_tile_kernel<32>, smem, "mha_bwd_tile"));
+        GCGCN_TRY(set_smem(mha_bwd_tile_kernel<32>, smem, "mha_bwd_tile"));
         mha_bwd_tile_kernel<32><<<grid, TL_THREADS, smem, st>>>(bt->node_ptr, pp, q, dS, dq, bt->total_pairs, scale);
     }
     GCGCN_CHECK_LAUNCH("mha_bwd_tile");

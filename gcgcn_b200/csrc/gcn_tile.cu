@@ -502,14 +502,9 @@ int launch_tile_fwd(const gcgcn_batch* bt, int heads, int layers, const float* q
     uint8_t* blob = static_cast<uint8_t*>(wblob_ws);
     tile_wprep_kernel<<<heads, 256, 0, st>>>(Winner_rowmajor, layers, blob);
     GCGCN_CHECK_LAUNCH("tile_wprep");
-    static std::atomic<unsigned long long> ready{0};
-    if (!device_prepared(ready)) {
-        GCGCN_TRY(cuda_ok(cudaFuncSetAttribute(tile_fwd_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, TL_SMEM_BYTES),
-                          "tile_fwd"));
-        GCGCN_TRY(cuda_ok(cudaFuncSetAttribute(tile_fwd_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, TL_SMEM_BYTES),
-                          "tile_fwd"));
-        device_mark_prepared(ready);
-    }
+    static std::atomic<unsigned long long> prepared16{0}, prepared32{0};
+    GCGCN_TRY(set_smem_once(prepared16, tile_fwd_kernel<16>, TL_SMEM_BYTES, "tile_fwd"));
+    GCGCN_TRY(set_smem_once(prepared32, tile_fwd_kernel<32>, TL_SMEM_BYTES, "tile_fwd"));
     TileFwdArgs a;
     a.tile_doc = bt->tile_doc;
     a.node_ptr = bt->node_ptr;

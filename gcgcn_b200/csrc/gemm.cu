@@ -3,9 +3,9 @@
 // These are the only genuinely dense contractions on the path once the edge einsum is collapsed
 // (SURVEY.md section 8a): node rows of the whole batch x [128 x 128*(1+H)] projection matrices in
 // the forward pass, the transposed products for dX, and the K = (all node rows) reductions for
-// the weight gradients.  This file holds the CUDA-core reference implementation (64x64x16 tiles,
-// 4x4 register blocking, deterministic split-K); gemm_tc.cu routes the large aligned shapes to
-// the tcgen05/TMEM kernel when that path is enabled.
+// the weight gradients.  This file holds the CUDA-core kernel (64x64x16 tiles, 4x4 register
+// blocking, deterministic split-K); gemm_tc.cu runs every product with K >= 1 and M*N*K >= 2e6 on
+// the tcgen05/TMEM kernels, so this one serves the smaller products and K = 0.
 #include "common.cuh"
 
 namespace gcgcn {
@@ -306,12 +306,12 @@ int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float
 
 int launch_gemm(int ta, int tb, int M, int N, int K, float alpha, const float* A, int lda,
                 const float* B, int ldb, float beta, float* C, int ldc, const float* bias, void* ws,
-                size_t ws_bytes, cudaStream_t st, void* pre_ws, size_t pre_bytes) {
+                size_t ws_bytes, cudaStream_t st) {
     if (M <= 0 || N <= 0) return GCGCN_OK;
     if (K < 0) return fail(GCGCN_ERR_INVALID_ARG, "gemm: K < 0");
     int taken = 0;
     GCGCN_TRY(launch_gemm_tc(ta, tb, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, bias, ws, ws_bytes, st, &taken,
-                             1, 0, 0, 0, pre_ws, pre_bytes));
+                             1, 0, 0, 0, nullptr, 0));
     if (taken) return GCGCN_OK;
     const int tiles = ceil_div(M, GM) * ceil_div(N, GN);
     int splits = 1;
@@ -371,7 +371,7 @@ int launch_gemm_batched(int ta, int tb, int M, int N, int K, float alpha, const 
     if (taken) return GCGCN_OK;
     for (int b = 0; b < batch; ++b)
         GCGCN_TRY(launch_gemm(ta, tb, M, N, K, alpha, A + b * sA, lda, B + b * sB, ldb, beta, C + b * sC, ldc, nullptr,
-                              ws, ws_bytes, st, nullptr, 0));
+                              ws, ws_bytes, st));
     return GCGCN_OK;
 }
 

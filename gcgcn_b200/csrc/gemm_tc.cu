@@ -38,8 +38,8 @@ constexpr int TC_EPI_WARP_FLOATS = 32 * 32;
 constexpr int TC_EPI_BYTES = 4 * TC_EPI_WARP_FLOATS * 4;
 // GROUPS producer groups of 4 warps (one K block of global loads in flight each), then 1 MMA warp, then 4
 // epilogue warps (warp index 4*GROUPS+1.. so that warp % 4 covers the TMEM lane quarters 1,2,3,0).
-// Three groups for K-contiguous operands; two when both operands are transposed on the way in (the scalar
-// loads of that path need more registers per thread than a 17-warp CTA leaves).
+// Three groups, except on the presplit-A route: two there, because its producers double-buffer the scalar-loaded
+// generated operand and need more registers per thread (128) than a 17-warp CTA leaves.
 constexpr int tc_threads(int groups) { return (4 * groups + 5) * 32; }
 constexpr int TC_TMEM_COLS = 256;                           // 2 accumulators x 128 fp32 columns
 constexpr size_t TC_SMEM_BYTES = size_t(TC_STAGES) * TC_STAGE_BYTES + TC_EPI_BYTES + 1024 /*align*/ + 256 /*barriers*/;
@@ -318,8 +318,8 @@ __device__ __forceinline__ void tc_epilogue_tile(const TcArgs& args, uint32_t tm
 // producers' work, and the registers it frees double-buffer the A loads (two K blocks in flight per group).
 constexpr uint32_t TC_B_BLOB_BYTES = 2 * TC_PART_BYTES;     // B_hi part, B_lo part
 
-// APRE: the mirror image for the weight-gradient products (K = every node row): the small [rows, 128] operand is
-// pre-split into blobs, the producers keep the wide M/N-contiguous operand (double-buffered), one tile per CTA.
+// APRE: the mirror image for the generated-operand weight gradient of the bilinear form (K = every pair): the small
+// [rows, 128] operand is pre-split into blobs, the producers generate the wide operand (double-buffered).
 // MNMAJ: both operands stored [K][MN] (C = A^T B) and fed to the tensor core MN-major (A_KCONTIG = B_KCONTIG = false).
 template <bool A_KCONTIG, bool B_KCONTIG, int GROUPS, bool BPRE, bool APRE = false, bool MNMAJ = false>
 __global__ void __launch_bounds__(tc_threads(GROUPS), 1) gemm_tc_kernel(const TcArgs args) {
@@ -579,149 +579,15 @@ __global__ void __launch_bounds__(tc_threads(GROUPS), 1) gemm_tc_kernel(const Tc
     if (warp == TC_MMA_WARP) tmem_dealloc(tmem_base, TC_TMEM_COLS);
 }
 
-// ---- K <= 128 projections with a weight operand: resident row operand -------------------------------------
-// x W with W = [128, H*128]: the H column tiles of a 128-row tile share the row operand, so it is split ONCE per
-// row tile into a resident shared-memory copy (up to 4 K blocks x hi/lo) while the weight blobs stream through two
-// stages by bulk copy.  The producers work once per H tiles instead of once per tile; what remains is MMA issue
-// and the 64 KB-per-tile store.  Roles: warps 0-7 producers (two groups, K blocks g and g+2), warp 8 blob loader,
-// warp 9 MMA issuer, warps 10-13 epilogue (TMEM lane quarters 2,3,0,1).
-constexpr int RA_PRODUCER_WARPS = 8, RA_LOADER_WARP = 8, RA_MMA_WARP = 9, RA_EPI_WARPS = 4, RA_THREADS = (10 + RA_EPI_WARPS) * 32;
-constexpr int RA_KB = 4, RA_BSTAGES = 2;
-constexpr size_t RA_EPI_BYTES = size_t(RA_EPI_WARPS) * TC_EPI_WARP_FLOATS * 4;
-constexpr size_t RA_SMEM_BYTES = size_t(RA_KB) * 2 * TC_PART_BYTES + size_t(RA_BSTAGES) * TC_B_BLOB_BYTES + RA_EPI_BYTES +
-                                 768 /*align slack*/ + 256 /*barriers*/;
-static_assert(RA_SMEM_BYTES <= 227 * 1024, "resident-A kernel exceeds the shared memory of an SM");
-
-__global__ void __launch_bounds__(RA_THREADS, 1) gemm_tc_resa_kernel(const TcArgs args) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    uint8_t* a_res = smem;                                             // [RA_KB][A_hi part, A_lo part]
-    uint8_t* b_stage = smem + size_t(RA_KB) * 2 * TC_PART_BYTES;      // [RA_BSTAGES][B_hi part, B_lo part]
-    float* epi_stage = reinterpret_cast<float*>(b_stage + size_t(RA_BSTAGES) * TC_B_BLOB_BYTES);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(reinterpret_cast<uint8_t*>(epi_stage) + RA_EPI_BYTES);
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 10);
-    const uint32_t bar0 = smem_u32(bars);
-    const uint32_t a_full = bar0, a_empty = bar0 + 8;
-    auto b_full = [&](int s) { return bar0 + 8u * (2 + s); };
-    auto b_empty = [&](int s) { return bar0 + 8u * (4 + s); };
-    auto tfull_bar = [&](int a) { return bar0 + 8u * (6 + a); };
-    auto tempty_bar = [&](int a) { return bar0 + 8u * (8 + a); };
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-    if (threadIdx.x == 0) {
-        mbar_init(a_full, RA_PRODUCER_WARPS);
-        mbar_init(a_empty, 1);
-        for (int i = 0; i < RA_BSTAGES; ++i) { mbar_init(b_full(i), 1); mbar_init(b_empty(i), 1); }
-        for (int a = 0; a < 2; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), RA_EPI_WARPS); }
-        fence_barrier_init();
-    }
-    if (warp == RA_MMA_WARP) tmem_alloc(smem_u32(tmem_slot), TC_TMEM_COLS);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-    const int kblocks = args.kblocks, tiles_n = args.tiles_n, tiles_m = args.tiles_m;
-
-    if (warp < RA_PRODUCER_WARPS) {
-        const bool a_vec = (args.lda % 4 == 0) && ((reinterpret_cast<uintptr_t>(args.A) & 15) == 0);
-        const int group = warp >> 2, tid = threadIdx.x & 127;
-        int it = 0;
-        for (int mi = blockIdx.x; mi < tiles_m; mi += gridDim.x, ++it) {
-            float4 va[2][8];
-#pragma unroll
-            for (int hh = 0; hh < 2; ++hh) {
-                const int kb = group + 2 * hh;
-                if (kb < kblocks) fetch_operand<true>(args.A, args.lda, mi * TC_BM, args.M, kb * TC_BK, args.K, a_vec, tid, va[hh]);
-            }
-            mbar_wait(a_empty, (it & 1) ^ 1);            // the MMAs of the previous row tile have retired
-#pragma unroll
-            for (int hh = 0; hh < 2; ++hh) {
-                const int kb = group + 2 * hh;
-                if (kb < kblocks) {
-                    float* st = reinterpret_cast<float*>(a_res + size_t(kb) * 2 * TC_PART_BYTES);
-                    store_operand<true>(st, st + TC_PART_BYTES / 4, tid, va[hh]);
-                }
-            }
-            fence_proxy_async();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(a_full);
-        }
-    } else if (warp == RA_LOADER_WARP) {
-        if (lane == 0) {
-            int q = 0;
-            for (int mi = blockIdx.x; mi < tiles_m; mi += gridDim.x)
-                for (int n = 0; n < tiles_n; ++n)
-                    for (int kb = 0; kb < kblocks; ++kb, ++q) {
-                        const int stage = q % RA_BSTAGES;
-                        mbar_wait(b_empty(stage), ((q / RA_BSTAGES) & 1) ^ 1);
-                        const uint8_t* blob = args.Bpre + (static_cast<size_t>(n) * kblocks + kb) * TC_B_BLOB_BYTES;
-                        mbar_arrive_expect_tx(b_full(stage), TC_B_BLOB_BYTES);
-                        bulk_copy_g2s(smem_u32(b_stage + size_t(stage) * TC_B_BLOB_BYTES), blob, TC_B_BLOB_BYTES, b_full(stage));
-                    }
-        }
-        __syncwarp();
-    } else if (warp == RA_MMA_WARP) {
-        if (lane == 0) {
-            int q = 0, acc = 0, it = 0;
-            uint32_t acc_phase = 0;
-            constexpr uint32_t IDESC = (1u << 4) | (2u << 7) | (2u << 10) | ((TC_BN >> 3) << 17) | ((TC_BM >> 4) << 24);
-            for (int mi = blockIdx.x; mi < tiles_m; mi += gridDim.x, ++it) {
-                mbar_wait(a_full, it & 1);
-                tc_fence_after();
-                for (int n = 0; n < tiles_n; ++n) {
-                    mbar_wait(tempty_bar(acc), acc_phase ^ 1);
-                    tc_fence_after();
-                    const uint32_t d_tmem = tmem_base + static_cast<uint32_t>(acc * TC_BN);
-                    uint32_t accumulate = 0;
-                    for (int kb = 0; kb < kblocks; ++kb, ++q) {
-                        const int stage = q % RA_BSTAGES;
-                        mbar_wait(b_full(stage), (q / RA_BSTAGES) & 1);
-                        tc_fence_after();
-                        const uint32_t a_hi = smem_u32(a_res + size_t(kb) * 2 * TC_PART_BYTES), a_lo = a_hi + TC_PART_BYTES;
-                        const uint32_t b_hi = smem_u32(b_stage + size_t(stage) * TC_B_BLOB_BYTES), b_lo = b_hi + TC_PART_BYTES;
-#pragma unroll
-                        for (int kk = 0; kk < TC_BK / 8; ++kk) {
-                            const uint32_t koff = kk * 2 * TC_PLANE_BYTES;
-                            umma_tf32(d_tmem, make_desc(a_lo + koff), make_desc(b_hi + koff), IDESC, accumulate);
-                            umma_tf32(d_tmem, make_desc(a_hi + koff), make_desc(b_lo + koff), IDESC, 1u);
-                            umma_tf32(d_tmem, make_desc(a_hi + koff), make_desc(b_hi + koff), IDESC, 1u);
-                            accumulate = 1u;
-                        }
-                        umma_commit(b_empty(stage));
-                    }
-                    umma_commit(tfull_bar(acc));
-                    if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-                }
-                umma_commit(a_empty);                    // the resident operand may be replaced once these retire
-            }
-        }
-        __syncwarp();
-    } else {
-        // RA_EPI_WARPS / 4 warps per TMEM lane quarter, each a share of the columns.  (8 warps were measured: no faster --
-        // with two 33 KB weight stages the MMA issuer waits on bulk-copy latency, not on the epilogue.)
-        const int quarter = warp & 3, ew = warp - (RA_MMA_WARP + 1);
-        constexpr int CH = (TC_BN / 32) / (RA_EPI_WARPS / 4);
-        float* stg = epi_stage + ew * TC_EPI_WARP_FLOATS;
-        int acc = 0;
-        uint32_t acc_phase = 0;
-        for (int mi = blockIdx.x; mi < tiles_m; mi += gridDim.x)
-            for (int n = 0; n < tiles_n; ++n) {
-                mbar_wait(tfull_bar(acc), acc_phase);
-                tc_fence_after();
-                tc_epilogue_tile(args, tmem_base, acc, tempty_bar(acc), quarter, stg, mi * TC_BM, n * TC_BN, 0, 0, true, lane,
-                                 (ew / 4) * CH, CH);
-                if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-            }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == RA_MMA_WARP) tmem_dealloc(tmem_base, TC_TMEM_COLS);
-}
-
-// ---- K <= 128 projections, row operand resident in TENSOR MEMORY ------------------------------------------
-// Same idea as gemm_tc_resa_kernel, but the split row operand (128 rows x K <= 128, hi and lo) lives in TMEM
-// columns 256..511 (tcgen05.st from the producers' registers, row = lane) and is read by tcgen05.mma as the A
-// operand; shared memory then holds nothing but weight blobs: six 33 KB stages instead of two, which is what the
-// bulk-copy latency needs.  TMEM: accumulators [0,128) and [128,256), A_hi [256,384), A_lo [384,512).
+// ---- K <= 128 projections with a weight operand, row operand resident in TENSOR MEMORY ----------------------
+// x W with W = [128, H*128]: the H column tiles of a 128-row tile share the row operand, so it is split ONCE per row
+// tile (128 rows x K <= 128, hi and lo) into TMEM columns 256..511 (tcgen05.st from the producers' registers,
+// row = lane) and read by tcgen05.mma as the A operand, while the weight blobs stream through five 33 KB shared-memory
+// stages by bulk copy.  The producers work once per H tiles instead of once per tile; what remains is MMA issue and the
+// 64 KB-per-tile store.  Roles: warps 0-7 producers (TMEM lane quarter warp & 3, K half warp >> 2), warp 8 blob loader,
+// warp 9 MMA issuer, warps 10-17 epilogue (two per TMEM lane quarter, a column half each).
+// TMEM: accumulators [0,128) and [128,256), A_hi [256,384), A_lo [384,512).
+constexpr int TA_PRODUCER_WARPS = 8, TA_LOADER_WARP = 8, TA_MMA_WARP = 9, TA_KB = 4;
 constexpr int TA_BSTAGES = 5, TA_EPI_WARPS = 8, TA_THREADS = (10 + TA_EPI_WARPS) * 32;
 constexpr size_t TA_EPI_BYTES = size_t(TA_EPI_WARPS) * TC_EPI_WARP_FLOATS * 4;
 constexpr size_t TA_SMEM_BYTES = size_t(TA_BSTAGES) * TC_B_BLOB_BYTES + TA_EPI_BYTES + 768 + 256;
@@ -744,20 +610,20 @@ __global__ void __launch_bounds__(TA_THREADS, 1) gemm_tc_tmema_kernel(const TcAr
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
     if (threadIdx.x == 0) {
-        mbar_init(a_full, RA_PRODUCER_WARPS);
+        mbar_init(a_full, TA_PRODUCER_WARPS);
         mbar_init(a_empty, 1);
         for (int a = 0; a < 2; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), TA_EPI_WARPS); }
         for (int i = 0; i < TA_BSTAGES; ++i) { mbar_init(b_full(i), 1); mbar_init(b_empty(i), 1); }
         fence_barrier_init();
     }
-    if (warp == RA_MMA_WARP) tmem_alloc(smem_u32(tmem_slot), 512);
+    if (warp == TA_MMA_WARP) tmem_alloc(smem_u32(tmem_slot), 512);
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     const int kblocks = args.kblocks, tiles_n = args.tiles_n, tiles_m = args.tiles_m;
 
-    if (warp < RA_PRODUCER_WARPS) {
+    if (warp < TA_PRODUCER_WARPS) {
         // warp -> TMEM lane quarter (warp & 3) and K half (warp >> 2); lane = row of the quarter
         const int quarter = warp & 3, khalf = warp >> 2;
         const bool a_vec = (args.lda % 4 == 0) && ((reinterpret_cast<uintptr_t>(args.A) & 15) == 0);
@@ -811,7 +677,7 @@ __global__ void __launch_bounds__(TA_THREADS, 1) gemm_tc_tmema_kernel(const TcAr
             __syncwarp();
             if (lane == 0) mbar_arrive(a_full);
         }
-    } else if (warp == RA_LOADER_WARP) {
+    } else if (warp == TA_LOADER_WARP) {
         if (lane == 0) {
             int q = 0;
             for (int mi = blockIdx.x; mi < tiles_m; mi += gridDim.x)
@@ -825,7 +691,7 @@ __global__ void __launch_bounds__(TA_THREADS, 1) gemm_tc_tmema_kernel(const TcAr
                     }
         }
         __syncwarp();
-    } else if (warp == RA_MMA_WARP) {
+    } else if (warp == TA_MMA_WARP) {
         if (lane == 0) {
             int q = 0, acc = 0, it = 0;
             uint32_t acc_phase = 0;
@@ -862,7 +728,7 @@ __global__ void __launch_bounds__(TA_THREADS, 1) gemm_tc_tmema_kernel(const TcAr
         }
         __syncwarp();
     } else {
-        const int quarter = warp & 3, ew = warp - (RA_MMA_WARP + 1);
+        const int quarter = warp & 3, ew = warp - (TA_MMA_WARP + 1);
         constexpr int CH = (TC_BN / 32) / (TA_EPI_WARPS / 4);
         float* stg = epi_stage + ew * TC_EPI_WARP_FLOATS;
         int acc = 0;
@@ -959,7 +825,7 @@ __global__ void __launch_bounds__(TA_THREADS, 1) gemm_tc_tmema_kernel(const TcAr
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == RA_MMA_WARP) tmem_dealloc(tmem_base, 512);
+    if (warp == TA_MMA_WARP) tmem_dealloc(tmem_base, 512);
 }
 
 // One blob per (128-column tile nt, 32-wide K block kb) of the N x K operand op(B)^T: exactly the B_hi / B_lo half of
@@ -993,26 +859,8 @@ size_t gemm_presplit_bytes(int rows) {
     return static_cast<size_t>(ceil_div(rows < 0 ? 0 : rows, TC_BK)) * TC_B_BLOB_BYTES;
 }
 
-bool gemm_tc_bpre_enabled() {
-    static int cached = -1;
-    if (cached < 0) {
-        const char* e = getenv("GCGCN_GEMM_BPRE");
-        cached = (e != nullptr && e[0] == '0') ? 0 : 1;   // GCGCN_GEMM_BPRE=0 disables
-    }
-    return cached == 1;
-}
-
 int launch_splitk_reduce(const float* partial, int splits, int M, int N, float alpha, float beta, float* C,
                          int ldc, const float* bias, cudaStream_t st, int batch, long long sC);
-
-bool gemm_tc_enabled() {
-    static int cached = -1;
-    if (cached < 0) {
-        const char* e = getenv("GCGCN_GEMM");
-        cached = (e != nullptr && (e[0] == 's' || e[0] == 'S')) ? 0 : 1;   // GCGCN_GEMM=simt disables
-    }
-    return cached == 1;
-}
 
 // returns 1 if the launch was taken by the tensor-core path, 0 if the caller should use the SIMT kernel
 int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float* A, int lda, const float* B,
@@ -1020,7 +868,7 @@ int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float
                    cudaStream_t st, int* taken, int batch, long long sA, long long sB, long long sC, void* pre_ws,
                    size_t pre_bytes, const float* bscale, int lds) {
     *taken = 0;
-    if (!gemm_tc_enabled() || K < 1 || batch < 1) return GCGCN_OK;
+    if (K < 1 || batch < 1) return GCGCN_OK;
     if (static_cast<double>(M) * N * K * batch < 2.0e6) return GCGCN_OK;   // tiny: not worth a 128x128 tile
     TcArgs a;
     a.M = M; a.N = N; a.K = K; a.lda = lda; a.ldb = ldb; a.ldc = ldc;
@@ -1072,7 +920,7 @@ int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float
     a.kblocks = ceil_div(K, TC_BK);
     // weight-like B operand (small, reused by every 128-row tile of a tall A): pre-split it once per call
     const size_t blob_total = static_cast<size_t>(a.tiles_n) * a.kblocks * TC_B_BLOB_BYTES;
-    const bool bpre = gemm_tc_bpre_enabled() && batch == 1 && splits == 1 && !seq && !ta && M >= 4096 &&
+    const bool bpre = batch == 1 && splits == 1 && !seq && !ta && M >= 4096 &&
                       static_cast<size_t>(N) * K * sizeof(float) <= (size_t(8) << 20) && ws != nullptr &&
                       blob_total <= ws_bytes && (reinterpret_cast<uintptr_t>(ws) & 15) == 0;
     if (bpre) {
@@ -1080,21 +928,15 @@ int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float
         GCGCN_CHECK_LAUNCH("gemm_presplit_b");
         a.Bpre = static_cast<const uint8_t*>(ws);
     }
-    // weight gradients: short M (the [rows, 128] operand, transposed), K = every row, one tile per CTA after split-K
+    // generated-operand weight gradient: the short [rows, <= 256] operand (A, transposed) is pre-split into blobs that
+    // every column tile re-uses.  The other weight gradients run MN-major: blobs only pay for themselves where the
+    // wide operand has to be generated (measured on [119808 x 128]^T [119808 x N]: N = 256: 95 us with blobs, 66 us
+    // MN-major; N = 1024: 230 us against 216 us).
     a.Apre = nullptr;
     const size_t ablob_total = static_cast<size_t>(a.tiles_m) * a.kblocks * TC_B_BLOB_BYTES;
-    // (worth it only when several column tiles re-use the blobs: a 128-wide output reads the operand once anyway;
-    //  GCGCN_APRE_MIN_TILES=1 switches it on for the one-tile weight gradients too -- measured, see DESIGN.md)
-    static const int apre_min_tiles = getenv("GCGCN_APRE_MIN_TILES") != nullptr ? atoi(getenv("GCGCN_APRE_MIN_TILES")) : 2;
-    static const bool mn_on = getenv("GCGCN_GEMM_MN") == nullptr || getenv("GCGCN_GEMM_MN")[0] != '0';   // =0: K-major route with register transposes
-    // (since the MN-major route exists the pre-split A blobs only pay for themselves where they are required: the
-    //  generated Khatri-Rao operand of the bilinear weight gradient.  Measured on [119808 x 128]^T [119808 x N]:
-    //  N = 256: 95 us with blobs, 66 us MN-major; N = 1024: 230 us against 216 us.)
-    const bool apre = gemm_tc_bpre_enabled() && !bpre && batch == 1 && ta && !tb && K >= 8192 && M <= 2 * TC_BM &&
-                      a.tiles_n >= apre_min_tiles && (bscale != nullptr || !mn_on) &&
-                      (seq ? (a.partial != nullptr || tiles <= sms) : tiles * splits <= sms) && pre_ws != nullptr &&
-                      ablob_total <= pre_bytes &&
-                      (reinterpret_cast<uintptr_t>(pre_ws) & 15) == 0;
+    const bool apre = bscale != nullptr && !bpre && batch == 1 && ta && !tb && K >= 8192 && M <= 2 * TC_BM &&
+                      a.tiles_n >= 2 && (seq ? (a.partial != nullptr || tiles <= sms) : tiles * splits <= sms) &&
+                      pre_ws != nullptr && ablob_total <= pre_bytes && (reinterpret_cast<uintptr_t>(pre_ws) & 15) == 0;
     if (bscale != nullptr && !apre)
         return fail(GCGCN_ERR_UNSUPPORTED, "gemm: the generated-operand product needs the pre-split weight-gradient path "
                     "(A transposed, K >= 8192, M <= 256, N >= 256, a pre-split workspace)");
@@ -1107,37 +949,19 @@ int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float
     // op(A)[m,k]: stored [M][K] (K contiguous) when !ta, [K][M] when ta.
     // op(B)[k,n] as the N x K operand: stored [N][K] (K contiguous) when tb, [K][N] when !tb.
     const bool a_kc = !ta, b_kc = (tb != 0);
-#define GCGCN_TC_LAUNCH(AK, BK, G, ...)                                                                  \
-    do {                                                                                                 \
-        static std::atomic<unsigned long long> attr_done{0};                                             \
-        if (!device_prepared(attr_done)) {                                                               \
-            GCGCN_TRY(cuda_ok(cudaFuncSetAttribute(gemm_tc_kernel<AK, BK, G, __VA_ARGS__>,               \
-                                                   cudaFuncAttributeMaxDynamicSharedMemorySize,          \
-                                                   static_cast<int>(TC_SMEM_BYTES)), "gemm_tc smem"));   \
-            device_mark_prepared(attr_done);                                                             \
-        }                                                                                                \
-        gemm_tc_kernel<AK, BK, G, __VA_ARGS__><<<grid, tc_threads(G), TC_SMEM_BYTES, st>>>(a);           \
+#define GCGCN_TC_LAUNCH(AK, BK, G, ...)                                                                                 \
+    do {                                                                                                                \
+        static std::atomic<unsigned long long> prepared{0};                                                             \
+        GCGCN_TRY(set_smem_once(prepared, gemm_tc_kernel<AK, BK, G, __VA_ARGS__>, TC_SMEM_BYTES, "gemm_tc smem"));      \
+        gemm_tc_kernel<AK, BK, G, __VA_ARGS__><<<grid, tc_threads(G), TC_SMEM_BYTES, st>>>(a);                          \
     } while (0)
-    static const bool resa_on = getenv("GCGCN_GEMM_RESA") == nullptr || getenv("GCGCN_GEMM_RESA")[0] != '0';
-    static const int resa_min_tiles = getenv("GCGCN_RESA_MIN_TILES") != nullptr ? atoi(getenv("GCGCN_RESA_MIN_TILES")) : 1;   // (one column tile: 40 us against 44 us for [119808,128]x[128,128])
-    const bool resa = bpre && resa_on && a.kblocks <= RA_KB && a.tiles_n >= resa_min_tiles && a.partial == nullptr;
-    static const bool tmema_on = getenv("GCGCN_GEMM_TMEMA") == nullptr || getenv("GCGCN_GEMM_TMEMA")[0] != '0';   // =0: shared-memory resident-A kernel
-    if (resa && tmema_on && !ta) {
-        static std::atomic<unsigned long long> attr_done2{0};
-        if (!device_prepared(attr_done2)) {
-            GCGCN_TRY(cuda_ok(cudaFuncSetAttribute(gemm_tc_tmema_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                   static_cast<int>(TA_SMEM_BYTES)), "gemm_tc_tmema smem"));
-            device_mark_prepared(attr_done2);
-        }
+    // K <= 128 with a pre-split weight operand: the row operand stays resident in tensor memory across the column tiles
+    // (also for a single column tile: 40 us against 44 us for [119808,128]x[128,128])
+    const bool tmema = bpre && a.kblocks <= TA_KB;
+    if (tmema) {
+        static std::atomic<unsigned long long> prepared{0};
+        GCGCN_TRY(set_smem_once(prepared, gemm_tc_tmema_kernel<0>, TA_SMEM_BYTES, "gemm_tc_tmema smem"));
         gemm_tc_tmema_kernel<0><<<std::min(sms, a.tiles_m), TA_THREADS, TA_SMEM_BYTES, st>>>(a);
-    } else if (resa) {
-        static std::atomic<unsigned long long> attr_done{0};
-        if (!device_prepared(attr_done)) {
-            GCGCN_TRY(cuda_ok(cudaFuncSetAttribute(gemm_tc_resa_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                   static_cast<int>(RA_SMEM_BYTES)), "gemm_tc_resa smem"));
-            device_mark_prepared(attr_done);
-        }
-        gemm_tc_resa_kernel<<<std::min(sms, a.tiles_m), RA_THREADS, RA_SMEM_BYTES, st>>>(a);
     } else if (apre) GCGCN_TC_LAUNCH(false, false, 2, false, true);
     else if (bpre) GCGCN_TC_LAUNCH(true, true, 3, true);
     else if (a_kc && b_kc) GCGCN_TC_LAUNCH(true, true, 3, false);
@@ -1145,14 +969,13 @@ int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float
     else if (!a_kc && b_kc) GCGCN_TC_LAUNCH(false, true, 3, false);
     // (never more producer groups than stages: a group two stage-rounds ahead would pass its parity wait on the
     //  empty barrier one phase early and overwrite a stage the MMA warp has not consumed -- 4 groups hang)
-    else if (mn_on) GCGCN_TC_LAUNCH(false, false, 3, false, false, true);
-    else GCGCN_TC_LAUNCH(false, false, 2, false);
+    else GCGCN_TC_LAUNCH(false, false, 3, false, false, true);
 #undef GCGCN_TC_LAUNCH
     timing_set_work(2.0 * M * N * K * batch);
-    GCGCN_CHECK_LAUNCH(resa ? ((tmema_on && !ta) ? "gemm_tc_nn<A in TMEM>" : "gemm_tc_nn<resident A>")
-                            : apre ? "gemm_tc_tn<presplit A>"
-                            : bpre ? (tb ? "gemm_tc_nt<presplit B>" : "gemm_tc_nn<presplit B>")
-                            : ta ? (tb ? "gemm_tc_tt" : (mn_on ? "gemm_tc_tn<MN-major>" : "gemm_tc_tn")) : (tb ? "gemm_tc_nt" : "gemm_tc_nn"));
+    GCGCN_CHECK_LAUNCH(tmema ? "gemm_tc_nn<A in TMEM>"
+                             : apre ? "gemm_tc_tn<presplit A>"
+                             : bpre ? (tb ? "gemm_tc_nt<presplit B>" : "gemm_tc_nn<presplit B>")
+                             : ta ? (tb ? "gemm_tc_tt" : "gemm_tc_tn<MN-major>") : (tb ? "gemm_tc_nt" : "gemm_tc_nn"));
     if (splits > 1 && a.partial != nullptr)
         GCGCN_TRY(launch_splitk_reduce(a.partial, splits, M, N, alpha, beta, C, ldc, bias, st, batch, sC));
     *taken = 1;
@@ -1169,8 +992,8 @@ int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float
 int launch_gemm_rowop(int mode, int M, int N, int K, const float* A, int lda, const float* B, int ldb, const float* T,
                       float* out, long long ld, void* ws, size_t ws_bytes, cudaStream_t st) {
     if (M <= 0 || N <= 0) return GCGCN_OK;
-    if (K < 1 || K > RA_KB * TC_BK || N % TC_BN != 0)
-        return fail(GCGCN_ERR_UNSUPPORTED, "gemm_rowop: needs 1 <= K <= %d and N a multiple of %d (K %d, N %d)", RA_KB * TC_BK,
+    if (K < 1 || K > TA_KB * TC_BK || N % TC_BN != 0)
+        return fail(GCGCN_ERR_UNSUPPORTED, "gemm_rowop: needs 1 <= K <= %d and N a multiple of %d (K %d, N %d)", TA_KB * TC_BK,
                     TC_BN, K, N);
     TcArgs a;
     a.M = M; a.N = N; a.K = K; a.lda = lda; a.ldb = ldb; a.ldc = 0;
@@ -1186,20 +1009,12 @@ int launch_gemm_rowop(int mode, int M, int N, int K, const float* A, int lda, co
     a.Bpre = static_cast<const uint8_t*>(ws);
     const int grid = std::min(sm_count(), a.tiles_m);
     if (mode == 1) {
-        static std::atomic<unsigned long long> attr_done{0};
-        if (!device_prepared(attr_done)) {
-            GCGCN_TRY(cuda_ok(cudaFuncSetAttribute(gemm_tc_tmema_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                   static_cast<int>(TA_SMEM_BYTES)), "gemm_tc_rowdot smem"));
-            device_mark_prepared(attr_done);
-        }
+        static std::atomic<unsigned long long> prepared{0};
+        GCGCN_TRY(set_smem_once(prepared, gemm_tc_tmema_kernel<1>, TA_SMEM_BYTES, "gemm_tc_rowdot smem"));
         gemm_tc_tmema_kernel<1><<<grid, TA_THREADS, TA_SMEM_BYTES, st>>>(a);
     } else {
-        static std::atomic<unsigned long long> attr_done{0};
-        if (!device_prepared(attr_done)) {
-            GCGCN_TRY(cuda_ok(cudaFuncSetAttribute(gemm_tc_tmema_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                   static_cast<int>(TA_SMEM_BYTES)), "gemm_tc_rowacc smem"));
-            device_mark_prepared(attr_done);
-        }
+        static std::atomic<unsigned long long> prepared{0};
+        GCGCN_TRY(set_smem_once(prepared, gemm_tc_tmema_kernel<2>, TA_SMEM_BYTES, "gemm_tc_rowacc smem"));
         gemm_tc_tmema_kernel<2><<<grid, TA_THREADS, TA_SMEM_BYTES, st>>>(a);
     }
     timing_set_work(2.0 * M * N * K);

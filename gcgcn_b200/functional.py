@@ -542,9 +542,7 @@ def gemm(a: torch.Tensor, b: torch.Tensor, trans_a=False, trans_b=False, bias=No
     N = b.shape[0] if trans_b else b.shape[1]
     if out is None:      # beta == 0 overwrites every element: no fill needed
         out = torch.empty(M, N, device=a.device) if (beta == 0.0 and K > 0) else torch.zeros(M, N, device=a.device)
-    # 24 MB of split-K partials / pre-split weight blobs, plus (weight-gradient shapes only) the pre-split short operand
-    pre = ((K + 31) // 32) * 33024 * ((M + 127) // 128) if (trans_a and not trans_b and M <= 256) else 0
-    ws = workspace(a.device, (24 << 20) + pre + 4096)
+    ws = workspace(a.device, (24 << 20) + 4096)     # split-K partials / pre-split weight blobs
     _lib.call("gcgcn_gemm", int(trans_a), int(trans_b), M, N, K, float(alpha), _p(a), a.shape[1], _p(b),
               b.shape[1], float(beta), _p(out), out.shape[1], _p(bias), ws.data_ptr(), ws.numel(),
               _stream(a.device))

@@ -1,5 +1,5 @@
-"""Device time of the weight-gradient GEMMs C = A^T B (A [K, M], B [K, N], K = every node row of a step).
-Environment: GCGCN_GEMM_MN=0 -> K-major route with register transposes; GCGCN_APRE_MIN_TILES=1000 -> no pre-split A."""
+"""Device time of the weight-gradient GEMMs C = A^T B (A [K, M], B [K, N], K = every node row of a step), which run on
+the MN-major tensor-core route."""
 import os
 import sys
 

@@ -18,7 +18,7 @@ DEV = "cuda:0"
                                    (64, 64, 40000), (37, 51, 77), (300, 8, 3),
                                    # tall A, weight-like B: the pre-split-B (bulk copy) variant, ragged edges included
                                    (4224, 1024, 128), (5000, 130, 129), (4100, 128, 1000),
-                                   # short M, K = "every node row": the pre-split-A weight-gradient variant (with ta=1, tb=0)
+                                   # short M, K = "every node row": the MN-major weight-gradient variant (with ta=1, tb=0)
                                    (128, 1024, 20000), (100, 260, 9001), (256, 128, 8200),
                                    # K <= 128 with several column tiles: row operand resident in tensor memory
                                    (4100, 300, 100), (8192, 1024, 64), (4097, 256, 128)])

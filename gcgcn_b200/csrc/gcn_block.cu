@@ -9,7 +9,7 @@
 //             then, without leaving the CTA, the softmax backward dS = P (dA - rowsum(dA P)) and either
 //             dq_h = scale (dS + dS^T) q_h  (MHA)  or dS itself (GAT; the edge pass consumes it).
 //
-// Why a second generation of the stack kernel (gcn_stack_mma.cu), and what ncu said at each step:
+// Why these kernels replaced a plain per-document mma.sync stack kernel, and what ncu said at each step:
 //   1. the first kernel was latency bound (long-scoreboard stalls on five dependent global round trips per
 //      CTA): here the per-sub-layer projection tiles arrive by cp.async into a two-deep ring and the epilogue
 //      operands are loaded ahead of the MMA loop that precedes their use; the attention map and its gradient
@@ -25,7 +25,7 @@
 //
 // All small matrix products run on the tensor cores (mma.sync m16n8k8 TF32, 3xTF32 split, see
 // mma_tf32.cuh).  Block configuration only: slab = in_dim = 128, ReLU + residual, no dropout masks
-// (train-mode masks take the general path in gcn_stack_mma.cu).
+// (keep masks passed in as tensors take the row-tiled kernels of gcn_stack_tiled.cu).
 #include "common.cuh"
 #include "mma_tf32.cuh"
 

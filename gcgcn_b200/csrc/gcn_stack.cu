@@ -13,8 +13,12 @@
 //
 // The three O(n^2 g) products -- A Z_l forward, dN Z^T and A^T dN backward -- run on the tensor cores
 // (mma.sync m16n8k8 TF32 with the 3xTF32 split of mma_tf32.cuh, fp32 parity); the row-local O(n g^2)
-// dense-connect products and the element-wise epilogues stay on the CUDA cores.  This is the path of
-// config 4's 128/256-entity graphs; DocRED-sized graphs (n <= 64) take gcn_block.cu / gcn_stack_mma.cu.
+// dense-connect products and the element-wise epilogues stay on the CUDA cores.
+//
+// launch_stack_fwd / launch_stack_bwd choose one of three kernel families from the shape alone:
+//   gcn_block.cu        the block configuration (slab 128, ReLU + residual, no keep mask) on graphs of n <= 64;
+//   gcn_stack_tiled.cu  otherwise, sub-layer width 32 or 64 with n <= 256 and at most 65,535 documents;
+//   this file           everything else: sub-layer width 16 or 128, n > 256, or more than 65,535 documents.
 #include "common.cuh"
 #include "mma_tf32.cuh"
 
@@ -403,16 +407,7 @@ static size_t stack_bwd_smem(int n, int layers, int gd) {
     return fl * sizeof(float);
 }
 
-// tensor-core (mma.sync 3xTF32) versions for n <= 64, gcn_stack_mma.cu
-bool stack_mma_usable(const gcgcn_batch* bt, int layers, int slab);
-int launch_stack_fwd_mma(const gcgcn_batch* bt, int heads, int layers, int slab, int flags, const float* A,
-                         float* Z, const float* E, const float* Winner, const float* keep, const float* x,
-                         float* G, float* F, cudaStream_t st);
-int launch_stack_bwd_mma(const gcgcn_batch* bt, int heads, int layers, int slab, int flags, const float* A,
-                         const float* Z, const float* G, const float* Winner, const float* keep, const float* dF,
-                         float* dZ, float* dE, float* dA, cudaStream_t st);
-
-// row-tiled tensor-core versions for 65 <= max n <= 256, gcn_stack_tiled.cu
+// row-tiled tensor-core versions for max n <= 256 and sub-layer width 32 or 64, gcn_stack_tiled.cu
 bool stack_tiled_usable(const gcgcn_batch* bt, int layers, int slab);
 int launch_stack_fwd_tiled(const gcgcn_batch* bt, int heads, int layers, int slab, int flags, const float* A,
                            float* Z, const float* E, const float* Winner, const float* keep, const float* x,
@@ -441,8 +436,6 @@ int launch_stack_fwd(const gcgcn_batch* bt, int heads, int layers, int slab, int
     if (bt->num_docs == 0) return GCGCN_OK;
     if (block_config(bt, heads, layers, slab, flags, keep) && (frag_ws != nullptr || layers < 2))
         return launch_block_fwd(bt, heads, layers, A, nullptr, nullptr, Z, E, Winner, x, G, F, frag_ws, BlockDrop{}, st);
-    if (stack_mma_usable(bt, layers, slab))
-        return launch_stack_fwd_mma(bt, heads, layers, slab, flags, A, Z, E, Winner, keep, x, G, F, st);
     if (stack_tiled_usable(bt, layers, slab))
         return launch_stack_fwd_tiled(bt, heads, layers, slab, flags, A, Z, E, Winner, keep, x, G, F, st);
     if (layers < 1 || slab % layers != 0)
@@ -479,8 +472,6 @@ int launch_stack_bwd(const gcgcn_batch* bt, int heads, int layers, int slab, int
     if (block_config(bt, heads, layers, slab, flags, keep) && (frag_ws != nullptr || layers < 2))
         return launch_block_bwd(bt, heads, layers, /*BK_OUT_DA*/ 0, A, nullptr, Z, G, Winner, dF, dZ, dE, dA, frag_ws,
                                 BlockDrop{}, st);
-    if (stack_mma_usable(bt, layers, slab))
-        return launch_stack_bwd_mma(bt, heads, layers, slab, flags, A, Z, G, Winner, keep, dF, dZ, dE, dA, st);
     if (stack_tiled_usable(bt, layers, slab))
         return launch_stack_bwd_tiled(bt, heads, layers, slab, flags, A, Z, G, Winner, keep, dF, dZ, dE, dA, st);
     if (layers < 1 || slab % layers != 0)

@@ -1,5 +1,7 @@
-// Dense-connected GraphConv stack for LARGE graphs (65..256 entities: BASELINE.json configs[3], the
-// 128 / 256-entity sweep): one CTA per (document, head, 32-row tile) and one launch per sub-layer.
+// Dense-connected GraphConv stack for graphs of up to 256 entities with sub-layer width 32 or 64 that the block
+// kernels of gcn_block.cu do not take: the 128 / 256-entity sweep (BASELINE.json configs[3]), keep masks passed
+// in as tensors, and a GraphConv used on its own.  One CTA per (document, head, 32-row tile) and one launch per
+// sub-layer.
 //
 // Same contract and math as gcn_stack.cu (G:36-50 inside G:67-76 / G:103-113).  That kernel gives one CTA a
 // whole (document, head): at n = 256 it owns 220 KB of shared memory, so one CTA of eight warps per SM walks
@@ -497,11 +499,11 @@ static size_t tile_cols_smem(int n, int layers, int gd) {
     return std::max(static_cast<size_t>(k8) * (gd + 8) + static_cast<size_t>(k8) * (TL_ROWS + 8), recycled) * sizeof(float);
 }
 
-// graphs of 65 .. 256 entities with sub-layer width 32 or 64
+// graphs of up to 256 entities with sub-layer width 32 or 64 (the document index is blockIdx.z)
 bool stack_tiled_usable(const gcgcn_batch* bt, int layers, int slab) {
     if (layers < 1 || slab % layers != 0) return false;
     const int gd = slab / layers;
-    return bt->max_nodes > 64 && bt->max_nodes <= 256 && bt->num_docs <= 65535 && (gd == 32 || gd == 64);
+    return bt->max_nodes <= 256 && bt->num_docs <= 65535 && (gd == 32 || gd == 64);
 }
 
 int launch_stack_fwd_tiled(const gcgcn_batch* bt, int heads, int layers, int slab, int flags, const float* A,

@@ -1,4 +1,4 @@
-// Warp-level TF32 tensor-core helpers shared by the per-document kernels (gcn_stack_mma.cu, gcn_block.cu).
+// Warp-level TF32 tensor-core helpers shared by the graph-stack kernels (gcn_block.cu, gcn_stack*.cu, gcn_tile.cu).
 //
 // fp32 parity (<= 1e-4 abs vs the reference) is kept by the 3xTF32 operand split: x = hi + lo with hi
 // exactly representable in TF32, and  a*b ~= lo_a*hi_b + hi_a*lo_b + hi_a*hi_b  (fp32 accumulate).

@@ -239,8 +239,8 @@ def test_full_size_shard_properties():
 
 @pytest.mark.parametrize("layers,heads", [(2, 8), (4, 4)])
 def test_large_and_small_documents_in_one_batch(layers, heads):
-    """max n > 64 routes the whole batch to the row-tiled stack kernels (gcn_stack_tiled.cu): documents smaller
-    than a tile, tile-boundary sizes and non-multiples of 8 in the same launch."""
+    """max n > 64 takes the whole batch off the block kernels onto the row-tiled stack kernels (gcn_stack_tiled.cu):
+    documents smaller than a tile, tile-boundary sizes and non-multiples of 8 in the same launch."""
     gb, state = device_blocks(layers, heads)
     # document ids picked so that no relu pre-activation lies within 4e-6 of zero for either configuration
     # (helpers.relu_margin; DESIGN.md section 2: a pre-activation inside float rounding of 0 may flip one unit)

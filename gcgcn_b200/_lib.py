@@ -189,7 +189,11 @@ SIGNATURES = {
     "gcgcn_pair_bce_bwd": (c_int32, [_BT, _P, _P, c_int32, _P, _P, _P]),
     "gcgcn_rank_ws_bytes": (c_size_t, [c_int64]),
     "gcgcn_rank_candidates": (c_int32, [_BT, _P, c_int32, _P, _P, c_int64, _P, _P, _P, _P]),
+    "gcgcn_rank_candidates_at": (c_int32, [_BT, _P, c_int32, _P, _P, _P, _P, _P, _P, _P]),
     "gcgcn_rank_sort": (c_int32, [_P, _P, c_int64, _P, _P, _P, c_size_t, _P]),
+    "gcgcn_rank_merge_ws_bytes": (c_size_t, [c_int64]),
+    "gcgcn_rank_merge": (c_int32, [_P, _P, c_int64, _P, _P, c_int64, _P, _P, _P, c_size_t, _P]),
+    "gcgcn_rank_curve_points": (c_int32, [_P, c_int64, c_int64, c_int32, _P, _P, _P, _P, c_size_t, _P]),
     "gcgcn_rank_curve": (c_int32, [_P, _P, c_int64, c_int64, c_int32, ctypes.c_double, _P, _P, c_size_t, _P]),
     "gcgcn_rank_decode": (c_int32, [_P, _P, c_int64, c_int64, _P, _P, c_int32, c_int32, _P, _P, _P, _P, _P, _P]),
     "gcgcn_adam_step": (c_int32, [_P, _P, _P, _P, c_int64] + [c_float] * 6 + [c_int32, _P]),

@@ -128,6 +128,15 @@ int launch_rank_sort(const float* score, const uint32_t* payload, long long coun
                      uint32_t* sorted_payload, void* ws, size_t ws_bytes, cudaStream_t st);
 int launch_rank_curve(const uint32_t* key, const uint32_t* pay, long long count, long long T, int has_intrain,
                       double input_theta, gcgcn_rank_result* res, void* ws, size_t ws_bytes, cudaStream_t st);
+int launch_rank_candidates_at(const gcgcn_batch* bt, const float* z, const float* labels, const uint8_t* intrain,
+                              int R, const long long* doc_first, float* score, uint32_t* payload,
+                              unsigned long long* counters, cudaStream_t st);
+size_t rank_merge_ws_bytes(long long count);
+int launch_rank_merge(const uint32_t* key_a, const uint32_t* pay_a, long long na, const uint32_t* key_b,
+                      const uint32_t* pay_b, long long nb, uint32_t* key_out, uint32_t* pay_out, void* ws,
+                      size_t ws_bytes, cudaStream_t st);
+int launch_rank_curve_points(const uint32_t* pay, long long count, long long T, int has_intrain, float* x, float* y,
+                             float* yi, void* ws, size_t ws_bytes, cudaStream_t st);
 int launch_rank_decode(const uint32_t* key, const uint32_t* pay, long long rows, const long long* doc_off,
                        const int* doc_n, int docs, int R, int* doc, int* row, int* col, int* rel, float* score,
                        cudaStream_t st);
@@ -1243,6 +1252,29 @@ int gcgcn_rank_candidates(const gcgcn_batch* bt, const float* logits, int32_t re
     return launch_rank_candidates(bt, logits, labels, intrain, relations, base_id, score, payload,
                                   reinterpret_cast<unsigned long long*>(counters), static_cast<cudaStream_t>(stream));
 }
+int gcgcn_rank_candidates_at(const gcgcn_batch* bt, const float* logits, int32_t relations, const float* labels,
+                             const uint8_t* intrain, const int64_t* doc_base, float* score, uint32_t* payload,
+                             int64_t* counters, void* stream) {
+    GCGCN_API_ENTER(stream);
+    GCGCN_TRY(check_batch(bt));
+    GCGCN_REQUIRE(relations >= 2, "rank_candidates_at: relations < 2 (relation 0 is not a candidate)");
+    const long long count = (bt->total_pairs - bt->total_nodes) * static_cast<long long>(relations - 1);
+    GCGCN_REQUIRE(count >= 0, "rank_candidates_at: total_pairs < total_nodes");
+    if (count >= GCGCN_RANK_MAX_CANDIDATES)
+        return fail(GCGCN_ERR_UNSUPPORTED, "rank_candidates_at: %lld candidates, one evaluation holds fewer than 2^30",
+                    count);
+    GCGCN_TRY(check_device_ptr(counters, "counters"));
+    if (count == 0) return GCGCN_OK;
+    GCGCN_TRY(check_device_ptr(logits, "logits"));
+    if (labels != nullptr) GCGCN_TRY(check_device_ptr(labels, "labels"));
+    if (intrain != nullptr) GCGCN_TRY(check_device_ptr(intrain, "intrain"));
+    GCGCN_TRY(check_device_ptr(doc_base, "doc_base"));
+    GCGCN_TRY(check_device_ptr(score, "score"));
+    GCGCN_TRY(check_device_ptr(payload, "payload"));
+    return launch_rank_candidates_at(bt, logits, labels, intrain, relations, reinterpret_cast<const long long*>(doc_base),
+                                     score, payload, reinterpret_cast<unsigned long long*>(counters),
+                                     static_cast<cudaStream_t>(stream));
+}
 int gcgcn_rank_sort(const float* score, const uint32_t* payload, int64_t count, uint32_t* sorted_key,
                     uint32_t* sorted_payload, void* ws, size_t ws_bytes, void* stream) {
     GCGCN_API_ENTER(stream);
@@ -1274,6 +1306,50 @@ int gcgcn_rank_curve(const uint32_t* sorted_key, const uint32_t* sorted_payload,
                   rank_ws_bytes(count));
     return launch_rank_curve(sorted_key, sorted_payload, count, total_recall < 1 ? 1 : total_recall, has_intrain ? 1 : 0,
                              input_theta, result, ws, ws_bytes, static_cast<cudaStream_t>(stream));
+}
+size_t gcgcn_rank_merge_ws_bytes(int64_t count) { return rank_merge_ws_bytes(count); }
+int gcgcn_rank_merge(const uint32_t* key_a, const uint32_t* payload_a, int64_t na, const uint32_t* key_b,
+                     const uint32_t* payload_b, int64_t nb, uint32_t* key_out, uint32_t* payload_out, void* ws,
+                     size_t ws_bytes, void* stream) {
+    GCGCN_API_ENTER(stream);
+    GCGCN_REQUIRE(na >= 0 && nb >= 0, "rank_merge: negative run length");
+    GCGCN_REQUIRE(na + nb < GCGCN_RANK_MAX_CANDIDATES, "rank_merge: %lld + %lld candidates, one evaluation holds fewer than 2^30",
+                  static_cast<long long>(na), static_cast<long long>(nb));
+    if (na + nb == 0) return GCGCN_OK;
+    if (na > 0) {
+        GCGCN_TRY(check_device_ptr(key_a, "key_a"));
+        GCGCN_TRY(check_device_ptr(payload_a, "payload_a"));
+    }
+    if (nb > 0) {
+        GCGCN_TRY(check_device_ptr(key_b, "key_b"));
+        GCGCN_TRY(check_device_ptr(payload_b, "payload_b"));
+    }
+    GCGCN_TRY(check_device_ptr(key_out, "key_out"));
+    GCGCN_TRY(check_device_ptr(payload_out, "payload_out"));
+    GCGCN_REQUIRE(((reinterpret_cast<uintptr_t>(key_out) | reinterpret_cast<uintptr_t>(payload_out)) & 15) == 0,
+                  "rank_merge: key_out / payload_out not 16-byte aligned");
+    GCGCN_TRY(check_device_ptr(ws, "ws"));
+    GCGCN_REQUIRE(ws_bytes >= rank_merge_ws_bytes(na + nb), "rank_merge: ws_bytes %zu < gcgcn_rank_merge_ws_bytes = %zu",
+                  ws_bytes, rank_merge_ws_bytes(na + nb));
+    return launch_rank_merge(key_a, payload_a, na, key_b, payload_b, nb, key_out, payload_out, ws, ws_bytes,
+                             static_cast<cudaStream_t>(stream));
+}
+int gcgcn_rank_curve_points(const uint32_t* sorted_payload, int64_t count, int64_t total_recall, int32_t has_intrain,
+                            float* x, float* y, float* y_ign, void* ws, size_t ws_bytes, void* stream) {
+    GCGCN_API_ENTER(stream);
+    GCGCN_REQUIRE(count >= 1 && count < GCGCN_RANK_MAX_CANDIDATES, "rank_curve_points: count %lld outside [1, 2^30)",
+                  static_cast<long long>(count));
+    GCGCN_TRY(check_device_ptr(sorted_payload, "sorted_payload"));
+    GCGCN_REQUIRE((reinterpret_cast<uintptr_t>(sorted_payload) & 15) == 0,
+                  "rank_curve_points: sorted_payload not 16-byte aligned");
+    GCGCN_TRY(check_device_ptr(x, "x"));
+    GCGCN_TRY(check_device_ptr(y, "y"));
+    if (has_intrain) GCGCN_TRY(check_device_ptr(y_ign, "y_ign"));
+    GCGCN_TRY(check_device_ptr(ws, "ws"));
+    GCGCN_REQUIRE(ws_bytes >= rank_ws_bytes(count), "rank_curve_points: ws_bytes %zu < gcgcn_rank_ws_bytes = %zu",
+                  ws_bytes, rank_ws_bytes(count));
+    return launch_rank_curve_points(sorted_payload, count, total_recall < 1 ? 1 : total_recall, has_intrain ? 1 : 0, x,
+                                    y, y_ign, ws, ws_bytes, static_cast<cudaStream_t>(stream));
 }
 int gcgcn_rank_decode(const uint32_t* sorted_key, const uint32_t* sorted_payload, int64_t rows, int64_t count,
                       const int64_t* doc_offsets, const int32_t* doc_n, int32_t num_docs, int32_t relations, int32_t* doc,

@@ -9,8 +9,10 @@
 //   curve       per-tile flag counts -> exclusive scan -> x, y, f1 (+ Ign) per position, per-tile first argmax and
 //               float64 AUC partials -> one-block finish (fixed-order reduction, w, result struct)
 //   decode      ranked ids of the first w + 1 candidates -> (doc, row, col, relation, score)
+//   merge       two rankings of disjoint candidate sets with global ids -> the ranking of their union (merge path)
 //
-// Everything is deterministic: integer counts, a stable sort and float64 sums in a fixed order.
+// Everything is deterministic: integer counts, a stable sort, a merge without atomics and float64 sums in a fixed
+// order.
 #include "common.cuh"
 
 namespace gcgcn {
@@ -30,13 +32,19 @@ __device__ __forceinline__ uint32_t score_key(float s) { return ~__float_as_uint
 __device__ __forceinline__ float key_score(uint32_t k) { return __uint_as_float(~k); }
 
 // ---- candidates --------------------------------------------------------------------------------------------------
-// One CTA per pair row (document b, row i): its n pairs x R cells are contiguous in logits.  Candidates of document b
-// start at base_id + (pair_ptr[b] - node_ptr[b]) (R - 1) (every earlier document has n(n-1) off-diagonal pairs).
-__global__ void __launch_bounds__(256)
-rank_candidates_kernel(const int* __restrict__ node_ptr, const long long* __restrict__ pair_ptr,
-                       const int* __restrict__ row_doc, const float* __restrict__ z, const float* __restrict__ labels,
-                       const uint8_t* __restrict__ intrain, int R, long long base_id, float* __restrict__ score,
-                       uint32_t* __restrict__ payload, unsigned long long* __restrict__ counters) {
+// One CTA per pair row (document b, row i): its n pairs x R cells are contiguous in logits.  A candidate's output
+// position in this batch is (pair_ptr[b] - node_ptr[b]) (R - 1) + its rank inside document b (every earlier document
+// of the batch has n(n-1) off-diagonal pairs).  Its id is that position + base_id, or, with AT, the position inside
+// document b + doc_first[b] (the document's first id in a global candidate numbering).
+template <bool AT>
+__device__ __forceinline__ void rank_candidates_body(const int* __restrict__ node_ptr,
+                                                     const long long* __restrict__ pair_ptr,
+                                                     const int* __restrict__ row_doc, const float* __restrict__ z,
+                                                     const float* __restrict__ labels,
+                                                     const uint8_t* __restrict__ intrain, int R, long long base_id,
+                                                     const long long* __restrict__ doc_first, float* __restrict__ score,
+                                                     uint32_t* __restrict__ payload,
+                                                     unsigned long long* __restrict__ counters) {
     __shared__ unsigned int red[2][8];
     const int row = blockIdx.x;
     const int b = row_doc[row];
@@ -44,6 +52,9 @@ rank_candidates_kernel(const int* __restrict__ node_ptr, const long long* __rest
     const long long cell0 = (pair_ptr[b] + static_cast<long long>(i) * n) * R;
     const long long doc_base = base_id + (pair_ptr[b] - node_ptr[b]) * (R - 1);
     const long long row_base = doc_base + static_cast<long long>(i) * (n - 1) * (R - 1);
+    // AT: positions and ids are below 2^30, so 32 bits hold both (no more registers live across the loop than without)
+    const uint32_t row_pos = static_cast<uint32_t>(row_base);
+    const uint32_t row_id = AT ? static_cast<uint32_t>(doc_first[b] + static_cast<long long>(i) * (n - 1) * (R - 1)) : 0u;
     const int cells = n * R;
     unsigned int pos = 0, nan = 0;
     for (int c = threadIdx.x; c < cells; c += blockDim.x) {
@@ -52,9 +63,15 @@ rank_candidates_kernel(const int* __restrict__ node_ptr, const long long* __rest
         const float s = logit_sigmoid(z[cell0 + c]);
         const uint32_t corr = (labels != nullptr && labels[cell0 + c] > 0.5f) ? 1u : 0u;
         const uint32_t intr = (intrain != nullptr && intrain[cell0 + c] != 0) ? 2u : 0u;
-        const long long id = row_base + static_cast<long long>(j - (j > i)) * (R - 1) + (r - 1);
-        score[id - base_id] = s;
-        payload[id - base_id] = (static_cast<uint32_t>(id) << 2) | intr | corr;
+        if constexpr (AT) {
+            const uint32_t off = static_cast<uint32_t>((j - (j > i)) * (R - 1) + (r - 1));
+            score[row_pos + off] = s;
+            payload[row_pos + off] = ((row_id + off) << 2) | intr | corr;
+        } else {
+            const long long id = row_base + static_cast<long long>(j - (j > i)) * (R - 1) + (r - 1);
+            score[id - base_id] = s;
+            payload[id - base_id] = (static_cast<uint32_t>(id) << 2) | intr | corr;
+        }
         pos += corr;
         nan += (s != s) ? 1u : 0u;
     }
@@ -72,6 +89,25 @@ rank_candidates_kernel(const int* __restrict__ node_ptr, const long long* __rest
         if (p) atomicAdd(counters, static_cast<unsigned long long>(p));
         if (q) atomicAdd(counters + 1, static_cast<unsigned long long>(q));
     }
+}
+
+__global__ void __launch_bounds__(256)
+rank_candidates_kernel(const int* __restrict__ node_ptr, const long long* __restrict__ pair_ptr,
+                       const int* __restrict__ row_doc, const float* __restrict__ z, const float* __restrict__ labels,
+                       const uint8_t* __restrict__ intrain, int R, long long base_id, float* __restrict__ score,
+                       uint32_t* __restrict__ payload, unsigned long long* __restrict__ counters) {
+    rank_candidates_body<false>(node_ptr, pair_ptr, row_doc, z, labels, intrain, R, base_id, nullptr, score, payload,
+                                counters);
+}
+
+__global__ void __launch_bounds__(256)
+rank_candidates_at_kernel(const int* __restrict__ node_ptr, const long long* __restrict__ pair_ptr,
+                          const int* __restrict__ row_doc, const float* __restrict__ z,
+                          const float* __restrict__ labels, const uint8_t* __restrict__ intrain, int R,
+                          const long long* __restrict__ doc_first, float* __restrict__ score,
+                          uint32_t* __restrict__ payload, unsigned long long* __restrict__ counters) {
+    rank_candidates_body<true>(node_ptr, pair_ptr, row_doc, z, labels, intrain, R, 0LL, doc_first, score, payload,
+                               counters);
 }
 
 // ---- block-wide exclusive scan of one value per thread (blockDim.x = NT) -----------------------------------------
@@ -352,6 +388,18 @@ int launch_rank_candidates(const gcgcn_batch* bt, const float* z, const float* l
     return GCGCN_OK;
 }
 
+int launch_rank_candidates_at(const gcgcn_batch* bt, const float* z, const float* labels, const uint8_t* intrain,
+                              int R, const long long* doc_first, float* score, uint32_t* payload,
+                              unsigned long long* counters, cudaStream_t st) {
+    if (bt->total_nodes <= 0) return GCGCN_OK;
+    rank_candidates_at_kernel<<<bt->total_nodes, 256, 0, st>>>(bt->node_ptr,
+                                                               reinterpret_cast<const long long*>(bt->pair_ptr),
+                                                               bt->row_doc, z, labels, intrain, R, doc_first, score,
+                                                               payload, counters);
+    GCGCN_CHECK_LAUNCH("rank_candidates_at");
+    return GCGCN_OK;
+}
+
 int launch_rank_sort(const float* score, const uint32_t* payload, long long count, uint32_t* sorted_key,
                      uint32_t* sorted_payload, void* ws, size_t ws_bytes, cudaStream_t st) {
     if (count <= 0) return GCGCN_OK;
@@ -379,6 +427,130 @@ int launch_rank_sort(const float* score, const uint32_t* payload, long long coun
         kin = kout;
         vin = vout;
     }
+    return GCGCN_OK;
+}
+
+// ---- merge of two sorted runs ------------------------------------------------------------------------------------
+// Runs A and B ascend by (key, payload) read as one 64-bit value (key in the high word).  Merge path: output tile t
+// holds outputs [t TILE, (t + 1) TILE); the partition kernel finds, for every tile boundary d, how many of the first d
+// outputs come from A (a binary search along the diagonal a + b = d).  One CTA per tile stages its A and B slices in
+// shared memory, each thread finds its own 16-output diagonal in them and merges 16 outputs, and the tile is written
+// back through shared memory as 16-byte stores.  On equal values A comes first.
+__device__ __forceinline__ unsigned long long merge_value(uint32_t key, uint32_t pay) {
+    return (static_cast<unsigned long long>(key) << 32) | pay;
+}
+
+// split[t] = number of A items among the first min(t TILE, na + nb) outputs, t = 0 .. tiles
+__global__ void __launch_bounds__(256)
+merge_partition_kernel(const uint32_t* __restrict__ key_a, const uint32_t* __restrict__ pay_a, long long na,
+                       const uint32_t* __restrict__ key_b, const uint32_t* __restrict__ pay_b, long long nb, int tiles,
+                       long long* __restrict__ split) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t > tiles) return;
+    const long long d = min(static_cast<long long>(t) * RK_TILE, na + nb);
+    long long lo = max(0LL, d - nb), hi = min(d, na);
+    while (lo < hi) {                      // first i whose A[i] comes after B[d - 1 - i]
+        const long long mid = (lo + hi) >> 1;
+        const long long j = d - 1 - mid;
+        if (merge_value(key_a[mid], pay_a[mid]) <= merge_value(key_b[j], pay_b[j])) lo = mid + 1;
+        else hi = mid;
+    }
+    split[t] = lo;
+}
+
+constexpr int MG_PAD = RK_TILE + RK_TILE / WARP;   // output staging: one padding word per 32 (conflict-free)
+__device__ __forceinline__ int merge_slot(int p) { return p + (p >> 5); }
+
+__global__ void __launch_bounds__(RK_THREADS)
+merge_tile_kernel(const uint32_t* __restrict__ key_a, const uint32_t* __restrict__ pay_a, long long na,
+                  const uint32_t* __restrict__ key_b, const uint32_t* __restrict__ pay_b, long long nb,
+                  const long long* __restrict__ split, uint32_t* __restrict__ key_out, uint32_t* __restrict__ pay_out) {
+    // input staging: A slice then B slice in [0, n) of s_key / s_pay; output staging reuses the same words
+    __shared__ __align__(16) uint32_t smem[2 * MG_PAD];
+    uint32_t* s_key = smem;
+    uint32_t* s_pay = smem + RK_TILE;
+    const long long o0 = static_cast<long long>(blockIdx.x) * RK_TILE;
+    const long long a0 = split[blockIdx.x], a1 = split[blockIdx.x + 1];
+    const long long b0 = o0 - a0;
+    const int n = static_cast<int>(min(static_cast<long long>(RK_TILE), na + nb - o0));
+    const int nA = static_cast<int>(a1 - a0), nB = n - nA;
+    for (int q = threadIdx.x; q < n; q += RK_THREADS) {
+        const bool fa = q < nA;
+        s_key[q] = fa ? key_a[a0 + q] : key_b[b0 + q - nA];
+        s_pay[q] = fa ? pay_a[a0 + q] : pay_b[b0 + q - nA];
+    }
+    __syncthreads();
+    // this thread's outputs [d, d + 16) of the tile start at A index i, B index d - i
+    const int d = min(static_cast<int>(threadIdx.x) * RK_IPT, n);
+    int lo = max(0, d - nB), hi = min(d, nA);
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        const int j = nA + d - 1 - mid;
+        if (merge_value(s_key[mid], s_pay[mid]) <= merge_value(s_key[j], s_pay[j])) lo = mid + 1;
+        else hi = mid;
+    }
+    int i = lo, j = nA + d - lo;                   // j indexes the B slice at its staged position
+    uint32_t ka = i < nA ? s_key[i] : 0u, pa = i < nA ? s_pay[i] : 0u;
+    uint32_t kb = j < n ? s_key[j] : 0u, pb = j < n ? s_pay[j] : 0u;
+    uint32_t ok[RK_IPT], op[RK_IPT];
+#pragma unroll
+    for (int k = 0; k < RK_IPT; ++k) {
+        const bool take_a = i < nA && (j >= n || merge_value(ka, pa) <= merge_value(kb, pb));
+        ok[k] = take_a ? ka : kb;
+        op[k] = take_a ? pa : pb;
+        if (take_a) {
+            ++i;
+            if (i < nA) { ka = s_key[i]; pa = s_pay[i]; }
+        } else {
+            ++j;
+            if (j < n) { kb = s_key[j]; pb = s_pay[j]; }
+        }
+    }
+    __syncthreads();
+    uint32_t* o_key = smem;
+    uint32_t* o_pay = smem + MG_PAD;
+#pragma unroll
+    for (int k = 0; k < RK_IPT; ++k) {
+        if (d + k < n) {
+            o_key[merge_slot(d + k)] = ok[k];
+            o_pay[merge_slot(d + k)] = op[k];
+        }
+    }
+    __syncthreads();
+    // lane-contiguous 16-byte stores: 4 consecutive outputs per thread and step (they never straddle a padding word)
+#pragma unroll
+    for (int q = 0; q < RK_TILE / (4 * RK_THREADS); ++q) {
+        const int p = 4 * (q * RK_THREADS + static_cast<int>(threadIdx.x));
+        const int s0 = merge_slot(p);
+        if (p + 4 <= n) {
+            *reinterpret_cast<uint4*>(key_out + o0 + p) = make_uint4(o_key[s0], o_key[s0 + 1], o_key[s0 + 2], o_key[s0 + 3]);
+            *reinterpret_cast<uint4*>(pay_out + o0 + p) = make_uint4(o_pay[s0], o_pay[s0 + 1], o_pay[s0 + 2], o_pay[s0 + 3]);
+        } else {
+            for (int e = 0; p + e < n; ++e) {
+                key_out[o0 + p + e] = o_key[s0 + e];
+                pay_out[o0 + p + e] = o_pay[s0 + e];
+            }
+        }
+    }
+}
+
+size_t rank_merge_ws_bytes(long long count) {
+    const size_t split_bytes = static_cast<size_t>(rank_tiles(count) + 1) * sizeof(long long);
+    return ((split_bytes + 255) & ~size_t(255)) + 256;              // Arena rounding + the alignment slack
+}
+
+int launch_rank_merge(const uint32_t* key_a, const uint32_t* pay_a, long long na, const uint32_t* key_b,
+                      const uint32_t* pay_b, long long nb, uint32_t* key_out, uint32_t* pay_out, void* ws,
+                      size_t ws_bytes, cudaStream_t st) {
+    if (na + nb <= 0) return GCGCN_OK;
+    Arena a = rank_arena(ws, ws_bytes);
+    const int tiles = rank_tiles(na + nb);
+    long long* split = a.take<long long>(tiles + 1);
+    if (split == nullptr) return fail(GCGCN_ERR_WORKSPACE, "rank_merge: workspace too small (%zu bytes)", ws_bytes);
+    merge_partition_kernel<<<ceil_div(tiles + 1, 256), 256, 0, st>>>(key_a, pay_a, na, key_b, pay_b, nb, tiles, split);
+    GCGCN_CHECK_LAUNCH("rank_merge_partition");
+    merge_tile_kernel<<<tiles, RK_THREADS, 0, st>>>(key_a, pay_a, na, key_b, pay_b, nb, split, key_out, pay_out);
+    GCGCN_CHECK_LAUNCH("rank_merge_tile");
     return GCGCN_OK;
 }
 
@@ -416,11 +588,14 @@ curve_count_kernel(const uint32_t* __restrict__ pay, long long count, unsigned l
 }
 
 // Thread t of tile b owns positions [b TILE + 16 t, +16).  prefix = the scanned tile counts + an in-tile scan.
-__global__ void __launch_bounds__(RK_THREADS)
-curve_main_kernel(const uint32_t* __restrict__ pay, long long count, long long T, int has_intrain,
-                  const unsigned long long* __restrict__ tile_prefix, float* __restrict__ best_f1,
-                  long long* __restrict__ best_pos, float* __restrict__ best_ign, double* __restrict__ auc,
-                  double* __restrict__ ign_auc) {
+// POINTS: write x, y (and yi with intrain) of every position instead of the tile's partials.
+template <bool POINTS>
+__device__ __forceinline__ void curve_main(const uint32_t* __restrict__ pay, long long count, long long T,
+                                           int has_intrain, const unsigned long long* __restrict__ tile_prefix,
+                                           float* __restrict__ best_f1, long long* __restrict__ best_pos,
+                                           float* __restrict__ best_ign, double* __restrict__ auc,
+                                           double* __restrict__ ign_auc, float* __restrict__ px,
+                                           float* __restrict__ py, float* __restrict__ pyi) {
     __shared__ unsigned long long s_warp[33];
     __shared__ float s_f1[RK_THREADS], s_ign[RK_THREADS];
     __shared__ long long s_pos[RK_THREADS];
@@ -452,7 +627,12 @@ curve_main_kernel(const uint32_t* __restrict__ pay, long long count, long long T
                 a += curve_trap(xk, x, yk, y);
                 if (has_intrain) ai += curve_trap(xk, x, yik, yi);
             }
-            if (k < RK_IPT) {            // k == RK_IPT is the next thread's first position: only the term is ours
+            if (POINTS && k < RK_IPT) {
+                px[pos] = x;
+                py[pos] = y;
+                if (has_intrain) pyi[pos] = yi;
+            }
+            if (!POINTS && k < RK_IPT) { // k == RK_IPT is the next thread's first position: only the term is ours
                 const float f = curve_f1(x, y);
                 if (f > f1_best) { f1_best = f; pos_best = pos; }
                 if (has_intrain) ign_best = fmaxf(ign_best, curve_f1(x, yi));
@@ -460,6 +640,7 @@ curve_main_kernel(const uint32_t* __restrict__ pay, long long count, long long T
             }
         }
     }
+    if (POINTS) return;
     s_f1[threadIdx.x] = f1_best;
     s_pos[threadIdx.x] = pos_best;
     s_ign[threadIdx.x] = ign_best;
@@ -487,6 +668,22 @@ curve_main_kernel(const uint32_t* __restrict__ pay, long long count, long long T
         auc[blockIdx.x] = s_auc[0];
         ign_auc[blockIdx.x] = s_iauc[0];
     }
+}
+
+__global__ void __launch_bounds__(RK_THREADS)
+curve_main_kernel(const uint32_t* __restrict__ pay, long long count, long long T, int has_intrain,
+                  const unsigned long long* __restrict__ tile_prefix, float* __restrict__ best_f1,
+                  long long* __restrict__ best_pos, float* __restrict__ best_ign, double* __restrict__ auc,
+                  double* __restrict__ ign_auc) {
+    curve_main<false>(pay, count, T, has_intrain, tile_prefix, best_f1, best_pos, best_ign, auc, ign_auc, nullptr,
+                      nullptr, nullptr);
+}
+
+__global__ void __launch_bounds__(RK_THREADS)
+curve_points_kernel(const uint32_t* __restrict__ pay, long long count, long long T, int has_intrain,
+                    const unsigned long long* __restrict__ tile_prefix, float* __restrict__ x, float* __restrict__ y,
+                    float* __restrict__ yi) {
+    curve_main<true>(pay, count, T, has_intrain, tile_prefix, nullptr, nullptr, nullptr, nullptr, nullptr, x, y, yi);
 }
 
 // One block: fixed-order reduction of the tile partials, w, and the curve values at w.
@@ -592,6 +789,21 @@ int launch_rank_curve(const uint32_t* key, const uint32_t* pay, long long count,
     curve_finish_kernel<<<1, 1024, 0, st>>>(key, pay, count, T, has_intrain, input_theta, tiles, w.flags, w.best_f1,
                                             w.best_pos, w.best_ign, w.auc, w.ign_auc, res);
     GCGCN_CHECK_LAUNCH("rank_curve_finish");
+    return GCGCN_OK;
+}
+
+int launch_rank_curve_points(const uint32_t* pay, long long count, long long T, int has_intrain, float* x, float* y,
+                             float* yi, void* ws, size_t ws_bytes, cudaStream_t st) {
+    Arena a = rank_arena(ws, ws_bytes);
+    CurveWs w;
+    if (!curve_ws_take(a, count, &w))
+        return fail(GCGCN_ERR_WORKSPACE, "rank_curve_points: workspace too small (%zu bytes)", ws_bytes);
+    const int tiles = rank_tiles(count);
+    curve_count_kernel<<<tiles, RK_THREADS, 0, st>>>(pay, count, w.flags);
+    GCGCN_CHECK_LAUNCH("rank_curve_count");
+    GCGCN_TRY(launch_scan<unsigned long long>(w.flags, tiles, w.sums, st));
+    curve_points_kernel<<<tiles, RK_THREADS, 0, st>>>(pay, count, T, has_intrain, w.flags, x, y, yi);
+    GCGCN_CHECK_LAUNCH("rank_curve_points");
     return GCGCN_OK;
 }
 

@@ -14,11 +14,17 @@ one small result struct.  No CPU path.
         ev.add(out["logits"], labels, hb.batch)                  # labels / intrain: [total_pairs, R]
     res = ev.result(input_theta=-1.0)
     pred = ev.predictions(res["theta"])
+
+A set evaluated in shards numbers its candidates globally: ``doc_sizes`` (the entity counts of every document of the
+set, in its order) fixes each document's first candidate id, and ``add(..., doc_index=...)`` names the documents of a
+batch.  Each shard is ranked alone; ``merged`` (one device) or ``all_gather`` (one shard per rank) merges the sorted
+runs into the ranking of the whole set, so every rank computes the result one evaluator over all documents would.
 """
 from __future__ import annotations
 
 import ctypes
-from typing import Optional
+import hashlib
+from typing import Optional, Sequence
 
 import numpy as np
 import torch
@@ -28,16 +34,22 @@ from .batch import RaggedBatch
 from .functional import _cuda, _p, _stream
 
 SORT_TILE = 4096                # GCGCN_RANK_TILE of include/gcgcn_b200.h
-MAX_CANDIDATES = 1 << 30        # one evaluator holds fewer (the payload packs id << 2 | flags)
+MAX_CANDIDATES = 1 << 30        # one evaluator, or one globally numbered set, holds fewer (payload: id << 2 | flags)
 RESULT_BYTES = ctypes.sizeof(_lib.RankResult)
 
 
 class RelationEvaluator:
     """Accumulates the candidates of any number of batches (``add``), ranks them once, lazily, and evaluates the ranking
-    (``result``) or lists its head (``predictions``).  Candidate ids, and so the order of equal scores, follow the
-    order of ``add`` calls and of the documents inside each batch."""
+    (``result``, ``curve``) or lists its head (``predictions``).  Candidate ids, and so the order of equal scores,
+    follow the order of ``add`` calls and of the documents inside each batch.
 
-    def __init__(self, relations: int = 97, device="cuda"):
+    With ``doc_sizes`` (entity counts of every document of the evaluated set, in global order) ids are global instead:
+    document g's candidates start at sum over g' < g of (n_g'^2 - n_g')(relations - 1), ``add`` takes the global
+    indices of its batch's documents, and they must increase strictly across all ``add`` calls.  Evaluators of
+    disjoint document sets of one ``doc_sizes`` combine with ``merged`` or ``all_gather`` into the evaluator of their
+    union, bit for bit."""
+
+    def __init__(self, relations: int = 97, device="cuda", doc_sizes: Optional[Sequence[int]] = None):
         self.relations = int(relations)
         if self.relations < 2:
             raise _lib.GcgcnError("RelationEvaluator: relations must be >= 2 (relation 0 is not a candidate)")
@@ -47,20 +59,38 @@ class RelationEvaluator:
         if self.device.index is None:
             self.device = torch.device("cuda", torch.cuda.current_device())
         _lib.load()
+        self._doc_sizes = None          # global mode: entity count of every document of the set
+        self._doc_first = None          # global mode: first candidate id of every document, [G + 1]
+        if doc_sizes is not None:
+            n = np.asarray(doc_sizes, dtype=np.int64).reshape(-1)
+            if (n < 0).any():
+                raise _lib.GcgcnError("RelationEvaluator: doc_sizes must be >= 0")
+            first = np.zeros(n.size + 1, dtype=np.int64)
+            np.cumsum((n * n - n) * (self.relations - 1), out=first[1:])
+            if first[-1] >= MAX_CANDIDATES:
+                raise _lib.GcgcnError(f"RelationEvaluator: doc_sizes hold {int(first[-1])} candidates, one evaluated "
+                                      "set holds fewer than 2^30")
+            self._doc_sizes, self._doc_first = n, first
         self.count = 0
         self._chunks = []               # (score f32, payload) of every add() in order
         self._doc_n = []                # entity count of every document, add() order
+        self._docs = []                 # global mode: global index of every document added, ascending
         self._labeled = True
         self._has_intrain = False
+        self._merged = False            # the result of merged() / all_gather(): ranked, holds no scores
         self._counters = torch.zeros(2, dtype=torch.int64, device=self.device)   # correct candidates, NaN scores
         self._host_counters = None
         self._ranked = None             # (sorted_key, sorted_payload, ws) while no add() follows
 
     # ---------------------------------------------------------------------------------------------------------------
     def add(self, logits: torch.Tensor, labels: Optional[torch.Tensor], batch: RaggedBatch,
-            intrain: Optional[torch.Tensor] = None) -> None:
+            intrain: Optional[torch.Tensor] = None, doc_index: Optional[Sequence[int]] = None) -> None:
         """Score the candidates of one batch.  logits, labels (multi-hot; > 0.5 is a fact) and intrain (non-zero = the
-        fact was seen in training) are ``[batch.total_pairs, relations]``; labels None for an unlabeled set."""
+        fact was seen in training) are ``[batch.total_pairs, relations]``; labels None for an unlabeled set.
+        ``doc_index`` (with ``doc_sizes`` only, and then required): the global index of each document of the batch."""
+        if self._merged:
+            raise _lib.GcgcnError("RelationEvaluator.add: a merged evaluator is final")
+        doc_first = self._global_doc_first(batch, doc_index)
         shape = (batch.total_pairs, self.relations)
         logits = _cuda(logits.detach(), "logits")
         if tuple(logits.shape) != shape:
@@ -86,8 +116,13 @@ class RelationEvaluator:
         count = int(((n * n - n).sum())) * (self.relations - 1)
         score = torch.empty(count, dtype=torch.float32, device=self.device)
         payload = torch.empty(count, dtype=torch.int32, device=self.device)
-        _lib.call("gcgcn_rank_candidates", batch.ref, _p(logits), self.relations, _p(labels), _p(intrain), self.count,
-                  _p(score), _p(payload), _p(self._counters), _stream(self.device))
+        if doc_first is None:
+            _lib.call("gcgcn_rank_candidates", batch.ref, _p(logits), self.relations, _p(labels), _p(intrain),
+                      self.count, _p(score), _p(payload), _p(self._counters), _stream(self.device))
+        else:
+            _lib.call("gcgcn_rank_candidates_at", batch.ref, _p(logits), self.relations, _p(labels), _p(intrain),
+                      _p(doc_first), _p(score), _p(payload), _p(self._counters), _stream(self.device))
+            self._docs.extend(int(g) for g in doc_index)
         self._chunks.append((score, payload))
         self._doc_n.extend(int(v) for v in n)
         self.count += count
@@ -95,6 +130,28 @@ class RelationEvaluator:
         self._has_intrain |= intrain is not None
         self._host_counters = None
         self._ranked = None
+
+    def _global_doc_first(self, batch: RaggedBatch, doc_index) -> Optional[torch.Tensor]:
+        """Check doc_index against doc_sizes; the batch documents' first global ids on the device (None: local ids)."""
+        if self._doc_sizes is None:
+            if doc_index is not None:
+                raise _lib.GcgcnError("add: doc_index needs an evaluator built with doc_sizes")
+            return None
+        if doc_index is None:
+            raise _lib.GcgcnError("add: an evaluator built with doc_sizes needs doc_index")
+        idx = np.asarray(doc_index, dtype=np.int64).reshape(-1)
+        if idx.size != batch.num_docs:
+            raise _lib.GcgcnError(f"add: doc_index has {idx.size} entries, the batch {batch.num_docs} documents")
+        if idx.size == 0:
+            return torch.zeros(0, dtype=torch.int64, device=self.device)
+        if idx.min() < 0 or idx.max() >= self._doc_sizes.size:
+            raise _lib.GcgcnError(f"add: doc_index outside [0, {self._doc_sizes.size})")
+        prev = self._docs[-1] if self._docs else -1
+        if idx[0] <= prev or (np.diff(idx) <= 0).any():
+            raise _lib.GcgcnError("add: doc_index must increase strictly across all add() calls")
+        if not np.array_equal(self._doc_sizes[idx], np.asarray(batch.sizes, dtype=np.int64)):
+            raise _lib.GcgcnError("add: the batch's entity counts differ from doc_sizes[doc_index]")
+        return torch.from_numpy(self._doc_first[idx]).to(self.device)
 
     def rank(self) -> None:
         """Sort every candidate added so far (``result`` and ``predictions`` do this when they need it)."""
@@ -114,7 +171,9 @@ class RelationEvaluator:
 
     @property
     def scores(self) -> torch.Tensor:
-        """float32 score of every candidate added so far, in id (insertion) order."""
+        """float32 score of every candidate added so far, in insertion order."""
+        if self._merged:
+            raise _lib.GcgcnError("RelationEvaluator.scores: a merged evaluator holds its ranking only")
         if len(self._chunks) > 1:
             self._chunks = [(torch.cat([c[0] for c in self._chunks]), torch.cat([c[1] for c in self._chunks]))]
         return self._chunks[0][0] if self._chunks else torch.zeros(0, device=self.device)
@@ -131,12 +190,15 @@ class RelationEvaluator:
             self._host_counters = [int(v) for v in self._counters.cpu()]
         return self._host_counters
 
-    def _curve(self, input_theta: float, total_recall: Optional[int]) -> _lib.RankResult:
+    def _total_recall(self, total_recall: Optional[int]) -> int:
         self.rank()
         positives, nans = self._counts()
         if nans:
             raise _lib.GcgcnError(f"RelationEvaluator: {nans} NaN scores (NaN logits)")
-        T = positives if total_recall is None else int(total_recall)
+        return positives if total_recall is None else int(total_recall)
+
+    def _curve(self, input_theta: float, total_recall: Optional[int]) -> _lib.RankResult:
+        T = self._total_recall(total_recall)
         key, pay, ws = self._ranked
         out = torch.empty(RESULT_BYTES, dtype=torch.uint8, device=self.device)
         _lib.call("gcgcn_rank_curve", _p(key), _p(pay), self.count, T, int(self._has_intrain), float(input_theta),
@@ -158,16 +220,35 @@ class RelationEvaluator:
                 "ign_f1": float(r.ign_f1) if ign else None, "ign_auc": float(r.ign_auc) if ign else None,
                 "ign_f1_at_w": float(r.ign_f1_at_w) if ign else None}
 
+    def curve(self, total_recall: Optional[int] = None) -> dict:
+        """The precision/recall curve at every ranked position (the reference's ``pr_x``, ``pr_y`` and, with intrain,
+        the Ign ``pr_y``): float32 device tensors ``x``, ``y`` and ``y_ign`` (None unless some ``add`` passed
+        intrain) of length ``count``.  ``total_recall`` as in ``result``."""
+        if not self._labeled:
+            raise _lib.GcgcnError("RelationEvaluator.curve: a batch was added without labels")
+        T = self._total_recall(total_recall)
+        _, pay, ws = self._ranked
+        x = torch.empty(self.count, dtype=torch.float32, device=self.device)
+        y = torch.empty_like(x)
+        y_ign = torch.empty_like(x) if self._has_intrain else None
+        _lib.call("gcgcn_rank_curve_points", _p(pay), self.count, T, int(self._has_intrain), _p(x), _p(y), _p(y_ign),
+                  _p(ws), ws.numel(), _stream(self.device))
+        return {"x": x, "y": y, "y_ign": y_ign}
+
     def predictions(self, input_theta: float = -1.0, total_recall: Optional[int] = None) -> dict:
         """The first w + 1 ranked candidates (the list the reference dumps, C:551-554) as int32 tensors ``doc`` (index of
-        the document in add() order), ``row``, ``col``, ``relation`` and float32 ``score``, on the device."""
+        the document in add() order; its global index with ``doc_sizes``), ``row``, ``col``, ``relation`` and float32
+        ``score``, on the device."""
         if input_theta == -1.0 and not self._labeled:
             raise _lib.GcgcnError("RelationEvaluator.predictions: the best-F1 threshold needs labels; pass input_theta")
         r = self._curve(input_theta, total_recall)
         rows = int(r.w) + 1
-        n = np.asarray(self._doc_n, dtype=np.int64)
-        off = np.zeros(n.size + 1, dtype=np.int64)
-        np.cumsum((n * n - n) * (self.relations - 1), out=off[1:])
+        if self._doc_sizes is None:
+            n = np.asarray(self._doc_n, dtype=np.int64)
+            off = np.zeros(n.size + 1, dtype=np.int64)
+            np.cumsum((n * n - n) * (self.relations - 1), out=off[1:])
+        else:
+            n, off = self._doc_sizes, self._doc_first
         doc_off = torch.from_numpy(off).to(self.device)
         doc_n = torch.from_numpy(n.astype(np.int32)).to(self.device)
         out = {k: torch.empty(rows, dtype=torch.int32, device=self.device) for k in ("doc", "row", "col", "relation")}
@@ -176,4 +257,124 @@ class RelationEvaluator:
         _lib.call("gcgcn_rank_decode", _p(key), _p(pay), rows, self.count, _p(doc_off), _p(doc_n), int(n.size), self.relations,
                   _p(out["doc"]), _p(out["row"]), _p(out["col"]), _p(out["relation"]), _p(out["score"]),
                   _stream(self.device))
+        return out
+
+    # --------------------------------------------------------------------------------------------------- sharded sets
+    @classmethod
+    def merged(cls, parts: Sequence["RelationEvaluator"]) -> "RelationEvaluator":
+        """The evaluator of the union of ``parts``: evaluators on one device with the same ``relations`` and
+        ``doc_sizes`` and disjoint documents.  Each part is ranked, then the sorted runs merge pairwise in a fixed
+        tree order (csrc/rank.cu, ``gcgcn_rank_merge``).  ``result``, ``curve``, ``predictions`` and ``ranked`` of
+        the result are bit-identical to those of one evaluator fed the union in ascending global order.  The result
+        is final: ``add`` and ``scores`` raise."""
+        parts = list(parts)
+        if not parts:
+            raise _lib.GcgcnError("RelationEvaluator.merged: no parts")
+        head = parts[0]
+        for p in parts:
+            if p._doc_sizes is None:
+                raise _lib.GcgcnError("RelationEvaluator.merged: every part needs doc_sizes (global candidate ids)")
+            if p.relations != head.relations:
+                raise _lib.GcgcnError(f"RelationEvaluator.merged: relations {p.relations} != {head.relations}")
+            if p.device != head.device:
+                raise _lib.GcgcnError(f"RelationEvaluator.merged: parts on {p.device} and {head.device}")
+            if not np.array_equal(p._doc_sizes, head._doc_sizes):
+                raise _lib.GcgcnError("RelationEvaluator.merged: the parts' doc_sizes differ")
+        total = sum(p.count for p in parts)
+        if total >= MAX_CANDIDATES:
+            raise _lib.GcgcnError(f"RelationEvaluator.merged: {total} candidates, one evaluated set holds fewer than 2^30")
+        runs = [p.ranked for p in parts if p.count > 0]
+        counters = torch.stack([p._counters for p in parts]).sum(0)
+        return cls._from_runs(head, runs, counters, [p._docs for p in parts], all(p._labeled for p in parts),
+                              any(p._has_intrain for p in parts))
+
+    def all_gather(self, group=None) -> "RelationEvaluator":
+        """The evaluator of the documents of every rank of ``group`` (default: the world), on every rank.  Each rank
+        ranks its own candidates; the ranks exchange their sorted runs and a few counts with all_gather_into_tensor
+        (on the device under NCCL, through the host under other backends), and every rank merges the runs in rank
+        order.  So every rank holds the same bits and reaches the same threshold and checkpoint decisions.  Without a
+        process group, or with one rank, this is ``merged([self])``.  Errors are raised on every rank alike."""
+        import torch.distributed as dist
+        if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+            return type(self).merged([self])
+        world = dist.get_world_size(group)
+        comm = self.device if dist.get_backend(group) == "nccl" else torch.device("cpu")
+        if self.count > 0:
+            self.rank()
+
+        def gather(t):                           # 1-D t -> [world, t.numel()], rank r's t in row r
+            out = torch.empty(world * t.numel(), dtype=t.dtype, device=comm)
+            dist.all_gather_into_tensor(out, t.to(comm).contiguous(), group=group)
+            return out.view(world, -1)
+
+        # metadata first, so that every rank sees the same inconsistency and raises the same error
+        sizes = self._doc_sizes
+        digest = 0 if sizes is None else int.from_bytes(hashlib.blake2b(sizes.tobytes(), digest_size=7).digest(), "little")
+        meta = torch.tensor([self.count, int(sizes is not None), 0 if sizes is None else sizes.size, digest,
+                             self.relations, int(self._labeled), int(self._has_intrain), len(self._docs)],
+                            dtype=torch.int64)
+        m = gather(torch.cat([meta.to(self.device), self._counters])).cpu()
+        if not bool((m[:, 1] == 1).all()):
+            raise _lib.GcgcnError("RelationEvaluator.all_gather: every rank's evaluator needs doc_sizes")
+        if not bool((m[:, 4] == m[0, 4]).all()):
+            raise _lib.GcgcnError("RelationEvaluator.all_gather: the ranks' relations differ")
+        if not bool((m[:, 2:4] == m[0, 2:4]).all()):
+            raise _lib.GcgcnError("RelationEvaluator.all_gather: the ranks' doc_sizes differ")
+        counts = [int(c) for c in m[:, 0]]
+        if sum(counts) >= MAX_CANDIDATES:
+            raise _lib.GcgcnError(f"RelationEvaluator.all_gather: {sum(counts)} candidates, one evaluated set holds "
+                                  "fewer than 2^30")
+        ndocs = [int(d) for d in m[:, 7]]
+        docs = torch.full((max(max(ndocs), 1),), -1, dtype=torch.int64)
+        docs[:len(self._docs)] = torch.tensor(self._docs, dtype=torch.int64)
+        d = gather(docs).cpu().numpy()
+        doc_lists = [d[r, :ndocs[r]].tolist() for r in range(world)]
+        # the runs, padded to the longest (a multiple of 4: every rank's payload run starts 16-byte aligned)
+        maxc = (max(counts) + 3) // 4 * 4
+        runs = []
+        if maxc > 0:
+            send = torch.zeros(2 * maxc, dtype=torch.int32, device=self.device)
+            if self.count > 0:
+                key, pay = self.ranked
+                send[:self.count] = key
+                send[maxc:maxc + self.count] = pay
+            recv = gather(send).to(self.device)
+            runs = [(recv[r, :c], recv[r, maxc:maxc + c]) for r, c in enumerate(counts) if c > 0]
+        counters = m[:, 8:10].sum(0).to(self.device)
+        return type(self)._from_runs(self, runs, counters, doc_lists, bool((m[:, 5] == 1).all()),
+                                     bool((m[:, 6] == 1).any()))
+
+    @classmethod
+    def _from_runs(cls, like, runs, counters, doc_lists, labeled, has_intrain) -> "RelationEvaluator":
+        """The merged evaluator over sorted (key, payload) runs of disjoint documents of ``like``'s doc_sizes."""
+        docs = np.concatenate([np.asarray(d, dtype=np.int64) for d in doc_lists])
+        if np.unique(docs).size != docs.size:
+            raise _lib.GcgcnError("RelationEvaluator: the parts share documents")
+        if not runs:
+            raise _lib.GcgcnError("RelationEvaluator: no candidates (every document has fewer than 2 entities)")
+        out = cls(like.relations, like.device, doc_sizes=like._doc_sizes)
+        dev, st = out.device, _stream(out.device)
+        lib = _lib.load()
+        total = sum(int(k.numel()) for k, _ in runs)
+        ws = torch.empty(int(lib.gcgcn_rank_merge_ws_bytes(total)), dtype=torch.uint8, device=dev)
+        while len(runs) > 1:                     # pairwise rounds: (0, 1), (2, 3), ...; an odd last run moves up
+            nxt = []
+            for (ka, pa), (kb, pb) in zip(runs[0::2], runs[1::2]):
+                n = ka.numel() + kb.numel()
+                key = torch.empty(n, dtype=torch.int32, device=dev)
+                pay = torch.empty(n, dtype=torch.int32, device=dev)
+                _lib.call("gcgcn_rank_merge", _p(ka), _p(pa), ka.numel(), _p(kb), _p(pb), kb.numel(), _p(key), _p(pay),
+                          _p(ws), ws.numel(), st)
+                nxt.append((key, pay))
+            if len(runs) % 2:
+                nxt.append(runs[-1])
+            runs = nxt
+        key, pay = runs[0]
+        out.count = total
+        out._ranked = (key, pay, torch.empty(int(lib.gcgcn_rank_ws_bytes(total)), dtype=torch.uint8, device=dev))
+        out._counters = counters
+        out._docs = np.sort(docs).tolist()
+        out._labeled = labeled
+        out._has_intrain = has_intrain
+        out._merged = True
         return out

@@ -450,6 +450,10 @@ int gcgcn_pair_bce_bwd(const gcgcn_batch* bt, const float* logits, const float* 
 /* ---- relation evaluation (config/Config.py:432-561; Ign F1 of config/Config_bert.py:626-650) ---------------------
  * The DocRED baseline evaluation on the device.  A candidate is (document, row i, column j, relation r) with i != j and
  * 1 <= r < R; its id is its position in insertion order (batches in call order, then documents, i, j, r ascending).
+ * Global ids (gcgcn_rank_candidates_at) number the candidates of a whole evaluated set of G documents instead: document
+ * g's first id is sum_{g' < g} (n_g'^2 - n_g')(R - 1), and inside a document the order is i, j, r as above.  A set
+ * evaluated in shards (one per GPU) then ranks each shard with gcgcn_rank_sort and merges the sorted runs with
+ * gcgcn_rank_merge; the merged ranking equals the ranking of the whole set.
  *   score   = 1 / (1 + exp(-logit))                float32, the loss kernel's sigmoid
  *   correct = labels[p][r] > 0.5;  intrain = intrain[p][r] != 0 (counts only where correct)
  * Ranking: score descending, stable (equal scores keep id order).  At ranked position k (0-based), with c_k / t_k the
@@ -461,7 +465,8 @@ int gcgcn_pair_bce_bwd(const gcgcn_batch* bt, const float* logits, const float* 
  *   np.trapezoid forms them in float32, summed in float64 in a fixed order; 0 for one candidate)
  *   w = best_pos if input_theta == -1, else the last position whose score > input_theta (0 if none).
  * One evaluator holds fewer than 2^30 candidates (the payload packs id << 2 | intrain << 1 | correct):
- * GCGCN_ERR_UNSUPPORTED beyond that.  Every result is bit-reproducible.                                             */
+ * GCGCN_ERR_UNSUPPORTED beyond that; with global ids the whole set's candidates count.  Every result is
+ * bit-reproducible.                                                                                                */
 #define GCGCN_RANK_TILE 4096          /* candidates per CTA of the sort and curve kernels */
 #define GCGCN_RANK_MAX_CANDIDATES (1LL << 30)
 
@@ -493,6 +498,12 @@ size_t gcgcn_rank_ws_bytes(int64_t count);
 int gcgcn_rank_candidates(const gcgcn_batch* bt, const float* logits, int32_t relations, const float* labels,
                           const uint8_t* intrain, int64_t base_id, float* score, uint32_t* payload, int64_t* counters,
                           void* stream);
+/* The same with global ids: doc_base [num_docs] int64 (device) is the first global id of each document of the batch.
+ * score / payload receive the batch's candidates compactly from position 0, exactly as gcgcn_rank_candidates with
+ * base_id 0 would; only the id packed in the payload differs.  The caller keeps every id below 2^30.              */
+int gcgcn_rank_candidates_at(const gcgcn_batch* bt, const float* logits, int32_t relations, const float* labels,
+                             const uint8_t* intrain, const int64_t* doc_base, float* score, uint32_t* payload,
+                             int64_t* counters, void* stream);
 /* Stable ranking of `count` candidates: sorted_key[k] = ~bits(score) of the k-th ranked candidate (ascending keys =
  * descending scores), sorted_payload[k] its payload.  ws >= gcgcn_rank_ws_bytes(count).                           */
 int gcgcn_rank_sort(const float* score, const uint32_t* payload, int64_t count, uint32_t* sorted_key,
@@ -503,6 +514,20 @@ int gcgcn_rank_sort(const float* score, const uint32_t* payload, int64_t count, 
 int gcgcn_rank_curve(const uint32_t* sorted_key, const uint32_t* sorted_payload, int64_t count, int64_t total_recall,
                      int32_t has_intrain, double input_theta, gcgcn_rank_result* result, void* ws, size_t ws_bytes,
                      void* stream);
+/* Workspace of gcgcn_rank_merge for na + nb = count outputs (8 bytes per 4096 outputs; any alignment).          */
+size_t gcgcn_rank_merge_ws_bytes(int64_t count);
+/* Merge two rankings, each ascending by (key, payload) read as one 64-bit value (key high): the output, na + nb long,
+ * ascends the same way; on an exact duplicate the item of A comes first.  Rankings of disjoint candidate sets with
+ * distinct (global) ids merge into the ranking of their union.  Deterministic, no atomics; na or nb may be 0.
+ * Outputs 16-byte aligned and disjoint from the inputs; na + nb < 2^30.  Moves 16 bytes per output.             */
+int gcgcn_rank_merge(const uint32_t* key_a, const uint32_t* payload_a, int64_t na, const uint32_t* key_b,
+                     const uint32_t* payload_b, int64_t nb, uint32_t* key_out, uint32_t* payload_out, void* ws,
+                     size_t ws_bytes, void* stream);
+/* The curve's points at every ranked position k (the reference's pr_x, pr_y and the Ign pr_y): x[k] = x_k,
+ * y[k] = y_k, y_ign[k] = yi_k (written only if has_intrain), float32 [count].  total_recall < 1 means 1;
+ * ws >= gcgcn_rank_ws_bytes(count); sorted_payload 16-byte aligned.                                              */
+int gcgcn_rank_curve_points(const uint32_t* sorted_payload, int64_t count, int64_t total_recall, int32_t has_intrain,
+                            float* x, float* y, float* y_ign, void* ws, size_t ws_bytes, void* stream);
 /* The first `rows` ranked candidates (rows <= count, the ranking's length) as (doc, row, col, relation, score) int32 /
  * float32 [rows].  doc_offsets
  * [num_docs + 1] int64: first candidate id of each document, (n_b^2 - n_b)(relations - 1) apart; doc_n [num_docs]

@@ -196,6 +196,10 @@ SIGNATURES = {
     "gcgcn_rank_curve_points": (c_int32, [_P, c_int64, c_int64, c_int32, _P, _P, _P, _P, c_size_t, _P]),
     "gcgcn_rank_curve": (c_int32, [_P, _P, c_int64, c_int64, c_int32, ctypes.c_double, _P, _P, c_size_t, _P]),
     "gcgcn_rank_decode": (c_int32, [_P, _P, c_int64, c_int64, _P, _P, c_int32, c_int32, _P, _P, _P, _P, _P, _P]),
+    "gcgcn_rank_relations_ws_bytes": (c_size_t, [c_int64, c_int32]),
+    "gcgcn_rank_by_relation": (c_int32, [_P, _P, c_int64, c_int32, _P, _P, _P, c_size_t, _P]),
+    "gcgcn_rank_curve_relations": (c_int32, [_P, _P, c_int64, c_int32, _P, c_int32, _P, _P, _P, c_size_t, _P]),
+    "gcgcn_rank_select": (c_int32, [_P, _P, c_int64, c_int32, _P, _P, _P, _P, _P, c_size_t, _P]),
     "gcgcn_adam_step": (c_int32, [_P, _P, _P, _P, c_int64] + [c_float] * 6 + [c_int32, _P]),
     "gcgcn_gemm": (c_int32, [c_int32, c_int32, c_int32, c_int32, c_int32, c_float, _P, c_int32, _P,
                              c_int32, c_float, _P, c_int32, _P, _P, c_size_t, _P]),

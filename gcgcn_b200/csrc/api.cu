@@ -137,6 +137,15 @@ int launch_rank_merge(const uint32_t* key_a, const uint32_t* pay_a, long long na
                       size_t ws_bytes, cudaStream_t st);
 int launch_rank_curve_points(const uint32_t* pay, long long count, long long T, int has_intrain, float* x, float* y,
                              float* yi, void* ws, size_t ws_bytes, cudaStream_t st);
+size_t rank_relations_ws_bytes(long long count, int R);
+int launch_rank_by_relation(const uint32_t* key, const uint32_t* pay, long long count, int R, uint32_t* rel_key,
+                            uint32_t* rel_pay, void* ws, size_t ws_bytes, cudaStream_t st);
+int launch_rank_curve_relations(const uint32_t* key, const uint32_t* pay, long long count, int R,
+                                const long long* total_recall, int has_intrain, const double* input_theta,
+                                gcgcn_rank_result* res, void* ws, size_t ws_bytes, cudaStream_t st);
+int launch_rank_select(const uint32_t* key, const uint32_t* pay, long long count, int R, const float* theta,
+                       uint32_t* out_key, uint32_t* out_pay, long long* counts, void* ws, size_t ws_bytes,
+                       cudaStream_t st);
 int launch_rank_decode(const uint32_t* key, const uint32_t* pay, long long rows, const long long* doc_off,
                        const int* doc_n, int docs, int R, int* doc, int* row, int* col, int* rel, float* score,
                        cudaStream_t st);
@@ -1370,6 +1379,79 @@ int gcgcn_rank_decode(const uint32_t* sorted_key, const uint32_t* sorted_payload
     GCGCN_TRY(check_device_ptr(score, "score"));
     return launch_rank_decode(sorted_key, sorted_payload, rows, reinterpret_cast<const long long*>(doc_offsets), doc_n,
                               num_docs, relations, doc, row, col, relation, score, static_cast<cudaStream_t>(stream));
+}
+
+// ---- relation evaluation per relation --------------------------------------------------------------------------
+// count in [1, 2^30), a multiple of R - 1, and R - 1 <= 256 (one 8-bit digit)
+static int check_relations(const char* what, int64_t count, int32_t relations) {
+    if (relations < 2) return fail(GCGCN_ERR_INVALID_ARG, "%s: relations < 2 (relation 0 is not a candidate)", what);
+    if (relations - 1 > 256)
+        return fail(GCGCN_ERR_UNSUPPORTED, "%s: %d relations r >= 1, at most 256 (one 8-bit digit)", what,
+                    relations - 1);
+    if (count < 1 || count >= GCGCN_RANK_MAX_CANDIDATES)
+        return fail(GCGCN_ERR_INVALID_ARG, "%s: count %lld outside [1, 2^30)", what, static_cast<long long>(count));
+    if (count % (relations - 1) != 0)
+        return fail(GCGCN_ERR_INVALID_ARG, "%s: count %lld is not a multiple of relations - 1 = %d", what,
+                    static_cast<long long>(count), relations - 1);
+    return GCGCN_OK;
+}
+static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+size_t gcgcn_rank_relations_ws_bytes(int64_t count, int32_t relations) {
+    return rank_relations_ws_bytes(count, relations);
+}
+int gcgcn_rank_by_relation(const uint32_t* sorted_key, const uint32_t* sorted_payload, int64_t count, int32_t relations,
+                           uint32_t* rel_key, uint32_t* rel_payload, void* ws, size_t ws_bytes, void* stream) {
+    GCGCN_API_ENTER(stream);
+    GCGCN_TRY(check_relations("rank_by_relation", count, relations));
+    GCGCN_TRY(check_device_ptr(sorted_key, "sorted_key"));
+    GCGCN_TRY(check_device_ptr(sorted_payload, "sorted_payload"));
+    GCGCN_TRY(check_device_ptr(rel_key, "rel_key"));
+    GCGCN_TRY(check_device_ptr(rel_payload, "rel_payload"));
+    GCGCN_TRY(check_device_ptr(ws, "ws"));
+    GCGCN_REQUIRE(ws_bytes >= rank_relations_ws_bytes(count, relations),
+                  "rank_by_relation: ws_bytes %zu < gcgcn_rank_relations_ws_bytes = %zu", ws_bytes,
+                  rank_relations_ws_bytes(count, relations));
+    return launch_rank_by_relation(sorted_key, sorted_payload, count, relations, rel_key, rel_payload, ws, ws_bytes,
+                                   static_cast<cudaStream_t>(stream));
+}
+int gcgcn_rank_curve_relations(const uint32_t* rel_key, const uint32_t* rel_payload, int64_t count, int32_t relations,
+                               const int64_t* total_recall, int32_t has_intrain, const double* input_theta,
+                               gcgcn_rank_result* results, void* ws, size_t ws_bytes, void* stream) {
+    GCGCN_API_ENTER(stream);
+    GCGCN_TRY(check_relations("rank_curve_relations", count, relations));
+    GCGCN_TRY(check_device_ptr(rel_key, "rel_key"));
+    GCGCN_TRY(check_device_ptr(rel_payload, "rel_payload"));
+    GCGCN_REQUIRE(aligned16(rel_payload), "rank_curve_relations: rel_payload not 16-byte aligned");
+    if (total_recall != nullptr) GCGCN_TRY(check_device_ptr(total_recall, "total_recall"));
+    GCGCN_TRY(check_device_ptr(input_theta, "input_theta"));
+    GCGCN_TRY(check_device_ptr(results, "results"));
+    GCGCN_TRY(check_device_ptr(ws, "ws"));
+    GCGCN_REQUIRE(ws_bytes >= rank_relations_ws_bytes(count, relations),
+                  "rank_curve_relations: ws_bytes %zu < gcgcn_rank_relations_ws_bytes = %zu", ws_bytes,
+                  rank_relations_ws_bytes(count, relations));
+    return launch_rank_curve_relations(rel_key, rel_payload, count, relations,
+                                       reinterpret_cast<const long long*>(total_recall), has_intrain ? 1 : 0,
+                                       input_theta, results, ws, ws_bytes, static_cast<cudaStream_t>(stream));
+}
+int gcgcn_rank_select(const uint32_t* sorted_key, const uint32_t* sorted_payload, int64_t count, int32_t relations,
+                      const float* theta, uint32_t* out_key, uint32_t* out_payload, int64_t* counts, void* ws,
+                      size_t ws_bytes, void* stream) {
+    GCGCN_API_ENTER(stream);
+    GCGCN_TRY(check_relations("rank_select", count, relations));
+    GCGCN_TRY(check_device_ptr(sorted_key, "sorted_key"));
+    GCGCN_TRY(check_device_ptr(sorted_payload, "sorted_payload"));
+    GCGCN_REQUIRE(aligned16(sorted_key) && aligned16(sorted_payload), "rank_select: inputs not 16-byte aligned");
+    GCGCN_TRY(check_device_ptr(theta, "theta"));
+    GCGCN_TRY(check_device_ptr(out_key, "out_key"));
+    GCGCN_TRY(check_device_ptr(out_payload, "out_payload"));
+    GCGCN_TRY(check_device_ptr(counts, "counts"));
+    GCGCN_TRY(check_device_ptr(ws, "ws"));
+    GCGCN_REQUIRE(ws_bytes >= rank_relations_ws_bytes(count, relations),
+                  "rank_select: ws_bytes %zu < gcgcn_rank_relations_ws_bytes = %zu", ws_bytes,
+                  rank_relations_ws_bytes(count, relations));
+    return launch_rank_select(sorted_key, sorted_payload, count, relations, theta, out_key, out_payload,
+                              reinterpret_cast<long long*>(counts), ws, ws_bytes, static_cast<cudaStream_t>(stream));
 }
 
 // ---- dense projection ------------------------------------------------------------------------

@@ -224,8 +224,20 @@ __device__ __forceinline__ uint32_t load_key(const void* in, long long idx) {
     return reinterpret_cast<const uint32_t*>(in)[idx];
 }
 
-// counts[d * tiles + tile] = number of keys of the tile whose digit at `shift` is d
-template <bool FIRST>
+// Where a pass takes its 8-bit digit: the key formed from the score (the sort's pass 0), the key of the previous pass
+// (digit at bit `arg`), or the candidate's relation from the payload, (id mod (R - 1)) with arg = R - 1 (the stable
+// partition of a ranking by relation, gcgcn_rank_by_relation).
+enum DigitSrc { DIGIT_SCORE, DIGIT_KEY, DIGIT_RELATION };
+
+template <int SRC>
+__device__ __forceinline__ uint32_t radix_digit(uint32_t key, uint32_t pay, int arg) {
+    if (SRC == DIGIT_RELATION) return (pay >> 2) % static_cast<uint32_t>(arg);
+    return (key >> arg) & 255u;
+}
+
+// counts[d * tiles + tile] = number of items of the tile whose digit is d; keys_in holds the payloads for
+// DIGIT_RELATION
+template <int SRC>
 __global__ void __launch_bounds__(RK_THREADS)
 radix_upsweep_kernel(const void* __restrict__ keys_in, long long count, int shift, int tiles,
                      uint32_t* __restrict__ counts) {
@@ -237,7 +249,10 @@ radix_upsweep_kernel(const void* __restrict__ keys_in, long long count, int shif
 #pragma unroll 4
     for (int k = 0; k < RK_IPT; ++k) {
         const long long idx = base + k * RK_THREADS + threadIdx.x;
-        if (idx < count) atomicAdd(&hist[warp][(load_key<FIRST>(keys_in, idx) >> shift) & 255u], 1u);
+        if (idx < count) {
+            const uint32_t x = load_key<SRC == DIGIT_SCORE>(keys_in, idx);
+            atomicAdd(&hist[warp][radix_digit<SRC>(x, x, shift)], 1u);
+        }
     }
     __syncthreads();
     uint32_t s = 0;
@@ -251,7 +266,7 @@ radix_upsweep_kernel(const void* __restrict__ keys_in, long long count, int shif
 // after the warp's running count of that digit.  Tile rank = start of the digit in the tile + the counts of that
 // digit in earlier warps + the warp rank.  The tile is staged in shared memory in digit order, then written out so
 // that each digit's run is contiguous at offsets[d * tiles + tile] (the digit-major exclusive scan of the counts).
-template <bool FIRST>
+template <int SRC>
 __global__ void __launch_bounds__(RK_THREADS)
 radix_downsweep_kernel(const void* __restrict__ keys_in, const uint32_t* __restrict__ vals_in, long long count, int shift,
                        int tiles, const uint32_t* __restrict__ offsets, uint32_t* __restrict__ keys_out,
@@ -275,9 +290,9 @@ radix_downsweep_kernel(const void* __restrict__ keys_in, const uint32_t* __restr
     for (int k = 0; k < RK_IPT; ++k) {
         const int t = warp * (RK_IPT * WARP) + k * WARP + lane;
         const bool ok = t < valid;
-        key[k] = ok ? load_key<FIRST>(keys_in, base + t) : 0u;
+        key[k] = ok ? load_key<SRC == DIGIT_SCORE>(keys_in, base + t) : 0u;
         val[k] = ok ? vals_in[base + t] : 0u;
-        const uint32_t d = ok ? ((key[k] >> shift) & 255u) : 256u;
+        const uint32_t d = ok ? radix_digit<SRC>(key[k], val[k], shift) : 256u;
         const uint32_t peers = __match_any_sync(0xffffffffu, d);
         const uint32_t before = ok ? s_whist[warp][d] : 0u;
         __syncwarp();
@@ -305,7 +320,7 @@ radix_downsweep_kernel(const void* __restrict__ keys_in, const uint32_t* __restr
     for (int k = 0; k < RK_IPT; ++k) {
         const int t = warp * (RK_IPT * WARP) + k * WARP + lane;
         if (t < valid) {
-            const uint32_t d = (key[k] >> shift) & 255u;
+            const uint32_t d = radix_digit<SRC>(key[k], val[k], shift);
             const uint32_t p = s_start[d] + s_whist[warp][d] + rank[k];
             s_keys[p] = key[k];
             s_vals[p] = val[k];
@@ -314,7 +329,7 @@ radix_downsweep_kernel(const void* __restrict__ keys_in, const uint32_t* __restr
     __syncthreads();
     for (int t = threadIdx.x; t < valid; t += RK_THREADS) {
         const uint32_t k = s_keys[t];
-        const uint32_t d = (k >> shift) & 255u;
+        const uint32_t d = radix_digit<SRC>(k, SRC == DIGIT_RELATION ? s_vals[t] : 0u, shift);
         const long long o = static_cast<long long>(s_gout[d]) + (t - static_cast<int>(s_start[d]));
         keys_out[o] = k;
         vals_out[o] = s_vals[t];
@@ -415,14 +430,16 @@ int launch_rank_sort(const float* score, const uint32_t* payload, long long coun
         uint32_t* kout = (pass & 1) ? sorted_key : w.keys;
         uint32_t* vout = (pass & 1) ? sorted_payload : w.vals;
         const int shift = 8 * pass;
-        if (pass == 0) radix_upsweep_kernel<true><<<tiles, RK_THREADS, 0, st>>>(kin, count, shift, tiles, w.counts);
-        else radix_upsweep_kernel<false><<<tiles, RK_THREADS, 0, st>>>(kin, count, shift, tiles, w.counts);
+        if (pass == 0) radix_upsweep_kernel<DIGIT_SCORE><<<tiles, RK_THREADS, 0, st>>>(kin, count, shift, tiles, w.counts);
+        else radix_upsweep_kernel<DIGIT_KEY><<<tiles, RK_THREADS, 0, st>>>(kin, count, shift, tiles, w.counts);
         GCGCN_CHECK_LAUNCH("rank_radix_upsweep");
         GCGCN_TRY(launch_scan<uint32_t>(w.counts, ncounts, w.sums, st));
         if (pass == 0)
-            radix_downsweep_kernel<true><<<tiles, RK_THREADS, 0, st>>>(kin, vin, count, shift, tiles, w.counts, kout, vout);
+            radix_downsweep_kernel<DIGIT_SCORE><<<tiles, RK_THREADS, 0, st>>>(kin, vin, count, shift, tiles, w.counts,
+                                                                             kout, vout);
         else
-            radix_downsweep_kernel<false><<<tiles, RK_THREADS, 0, st>>>(kin, vin, count, shift, tiles, w.counts, kout, vout);
+            radix_downsweep_kernel<DIGIT_KEY><<<tiles, RK_THREADS, 0, st>>>(kin, vin, count, shift, tiles, w.counts, kout,
+                                                                           vout);
         GCGCN_CHECK_LAUNCH("rank_radix_downsweep");
         kin = kout;
         vin = vout;
@@ -587,11 +604,16 @@ curve_count_kernel(const uint32_t* __restrict__ pay, long long count, unsigned l
     if (threadIdx.x == 0) flags[blockIdx.x] = total;
 }
 
-// Thread t of tile b owns positions [b TILE + 16 t, +16).  prefix = the scanned tile counts + an in-tile scan.
+// Tile `tile` of the run pay[0, count): thread t owns positions [tile TILE + 16 t, +16).  prefix = the scanned tile
+// counts at `slot` + an in-tile scan; the tile's partials go to index `slot` of the output arrays.
 // POINTS: write x, y (and yi with intrain) of every position instead of the tile's partials.
-template <bool POINTS>
+// SEGMENT: the run is one relation's segment of a partitioned ranking, with its first tile at slot `first`: its counts
+// are the scanned counts minus those at `first`, and as it starts at any alignment the CTA stages its positions (and
+// the next tile's first) in s_stage [RK_TILE + 4] with coalesced loads instead of 16-byte loads per thread.
+template <bool POINTS, bool SEGMENT>
 __device__ __forceinline__ void curve_main(const uint32_t* __restrict__ pay, long long count, long long T,
-                                           int has_intrain, const unsigned long long* __restrict__ tile_prefix,
+                                           int has_intrain, int tile, const unsigned long long* __restrict__ tile_prefix,
+                                           long long first, uint32_t* __restrict__ s_stage, long long slot,
                                            float* __restrict__ best_f1, long long* __restrict__ best_pos,
                                            float* __restrict__ best_ign, double* __restrict__ auc,
                                            double* __restrict__ ign_auc, float* __restrict__ px,
@@ -600,15 +622,25 @@ __device__ __forceinline__ void curve_main(const uint32_t* __restrict__ pay, lon
     __shared__ float s_f1[RK_THREADS], s_ign[RK_THREADS];
     __shared__ long long s_pos[RK_THREADS];
     __shared__ double s_auc[RK_THREADS], s_iauc[RK_THREADS];
-    const long long base = static_cast<long long>(blockIdx.x) * RK_TILE + threadIdx.x * static_cast<long long>(RK_IPT);
+    const long long base = static_cast<long long>(tile) * RK_TILE + threadIdx.x * static_cast<long long>(RK_IPT);
     uint32_t p[RK_IPT + 1];
-    load16(pay, base, count, *reinterpret_cast<uint32_t(*)[RK_IPT]>(p));
-    p[RK_IPT] = base + RK_IPT < count ? pay[base + RK_IPT] : 0u;
+    if constexpr (SEGMENT) {
+        const long long t0 = static_cast<long long>(tile) * RK_TILE;
+        for (int q = threadIdx.x; q < RK_TILE + 4; q += RK_THREADS) s_stage[q] = t0 + q < count ? pay[t0 + q] : 0u;
+        __syncthreads();
+        const uint4* s4 = reinterpret_cast<const uint4*>(s_stage + threadIdx.x * RK_IPT);
+#pragma unroll
+        for (int q = 0; q < RK_IPT / 4; ++q) reinterpret_cast<uint4*>(p)[q] = s4[q];
+        p[RK_IPT] = s_stage[threadIdx.x * RK_IPT + RK_IPT];
+    } else {
+        load16(pay, base, count, *reinterpret_cast<uint32_t(*)[RK_IPT]>(p));
+        p[RK_IPT] = base + RK_IPT < count ? pay[base + RK_IPT] : 0u;
+    }
     unsigned long long acc = 0;
 #pragma unroll
     for (int k = 0; k < RK_IPT; ++k) acc += (p[k] & 1u) + (static_cast<unsigned long long>((p[k] & 3u) == 3u) << 32);
     const unsigned long long pre = block_excl_scan<unsigned long long, RK_THREADS>(acc, s_warp, nullptr) +
-                                   tile_prefix[blockIdx.x];
+                                   (SEGMENT ? tile_prefix[slot] - tile_prefix[first] : tile_prefix[slot]);
     long long c = static_cast<long long>(pre & 0xffffffffull), t = static_cast<long long>(pre >> 32);
     float f1_best = -1.f, ign_best = -1.f;
     long long pos_best = -1;
@@ -662,11 +694,11 @@ __device__ __forceinline__ void curve_main(const uint32_t* __restrict__ pay, lon
         __syncthreads();
     }
     if (threadIdx.x == 0) {
-        best_f1[blockIdx.x] = s_f1[0];
-        best_pos[blockIdx.x] = s_pos[0];
-        best_ign[blockIdx.x] = s_ign[0];
-        auc[blockIdx.x] = s_auc[0];
-        ign_auc[blockIdx.x] = s_iauc[0];
+        best_f1[slot] = s_f1[0];
+        best_pos[slot] = s_pos[0];
+        best_ign[slot] = s_ign[0];
+        auc[slot] = s_auc[0];
+        ign_auc[slot] = s_iauc[0];
     }
 }
 
@@ -675,24 +707,27 @@ curve_main_kernel(const uint32_t* __restrict__ pay, long long count, long long T
                   const unsigned long long* __restrict__ tile_prefix, float* __restrict__ best_f1,
                   long long* __restrict__ best_pos, float* __restrict__ best_ign, double* __restrict__ auc,
                   double* __restrict__ ign_auc) {
-    curve_main<false>(pay, count, T, has_intrain, tile_prefix, best_f1, best_pos, best_ign, auc, ign_auc, nullptr,
-                      nullptr, nullptr);
+    curve_main<false, false>(pay, count, T, has_intrain, blockIdx.x, tile_prefix, 0, nullptr, blockIdx.x, best_f1,
+                             best_pos, best_ign, auc, ign_auc, nullptr, nullptr, nullptr);
 }
 
 __global__ void __launch_bounds__(RK_THREADS)
 curve_points_kernel(const uint32_t* __restrict__ pay, long long count, long long T, int has_intrain,
                     const unsigned long long* __restrict__ tile_prefix, float* __restrict__ x, float* __restrict__ y,
                     float* __restrict__ yi) {
-    curve_main<true>(pay, count, T, has_intrain, tile_prefix, nullptr, nullptr, nullptr, nullptr, nullptr, x, y, yi);
+    curve_main<true, false>(pay, count, T, has_intrain, blockIdx.x, tile_prefix, 0, nullptr, blockIdx.x, nullptr,
+                            nullptr, nullptr, nullptr, nullptr, x, y, yi);
 }
 
-// One block: fixed-order reduction of the tile partials, w, and the curve values at w.
-__global__ void __launch_bounds__(1024)
-curve_finish_kernel(const uint32_t* __restrict__ key, const uint32_t* __restrict__ pay, long long count, long long T,
-                    int has_intrain, double input_theta, int tiles, const unsigned long long* __restrict__ tile_prefix,
-                    const float* __restrict__ best_f1, const long long* __restrict__ best_pos,
-                    const float* __restrict__ best_ign, const double* __restrict__ auc,
-                    const double* __restrict__ ign_auc, gcgcn_rank_result* __restrict__ res) {
+// One block: fixed-order reduction of the tile partials of the run key / pay [0, count), w, and the curve values at w.
+// tile_prefix[t] - prefix_base = the flag counts before tile t of the run.
+__device__ __forceinline__ void curve_finish(const uint32_t* __restrict__ key, const uint32_t* __restrict__ pay,
+                                             long long count, long long T, int has_intrain, double input_theta,
+                                             int tiles, const unsigned long long* __restrict__ tile_prefix,
+                                             unsigned long long prefix_base, const float* __restrict__ best_f1,
+                                             const long long* __restrict__ best_pos,
+                                             const float* __restrict__ best_ign, const double* __restrict__ auc,
+                                             const double* __restrict__ ign_auc, gcgcn_rank_result* __restrict__ res) {
     __shared__ float s_f1[1024], s_ign[1024];
     __shared__ long long s_pos[1024];
     __shared__ double s_auc[1024], s_iauc[1024];
@@ -752,7 +787,7 @@ curve_finish_kernel(const uint32_t* __restrict__ key, const uint32_t* __restrict
     unsigned long long total;
     block_excl_scan<unsigned long long, 1024>(acc, s_warp, &total);
     if (threadIdx.x == 0) {
-        const unsigned long long pre = total + tile_prefix[w / RK_TILE];
+        const unsigned long long pre = total + (tile_prefix[w / RK_TILE] - prefix_base);
         const long long c = static_cast<long long>(pre & 0xffffffffull), t = static_cast<long long>(pre >> 32);
         const float x = curve_ratio(c, T), y = curve_ratio(c, w + 1);
         gcgcn_rank_result r;
@@ -772,6 +807,16 @@ curve_finish_kernel(const uint32_t* __restrict__ key, const uint32_t* __restrict
         r.reserved = 0;
         *res = r;
     }
+}
+
+__global__ void __launch_bounds__(1024)
+curve_finish_kernel(const uint32_t* __restrict__ key, const uint32_t* __restrict__ pay, long long count, long long T,
+                    int has_intrain, double input_theta, int tiles, const unsigned long long* __restrict__ tile_prefix,
+                    const float* __restrict__ best_f1, const long long* __restrict__ best_pos,
+                    const float* __restrict__ best_ign, const double* __restrict__ auc,
+                    const double* __restrict__ ign_auc, gcgcn_rank_result* __restrict__ res) {
+    curve_finish(key, pay, count, T, has_intrain, input_theta, tiles, tile_prefix, 0ull, best_f1, best_pos, best_ign,
+                 auc, ign_auc, res);
 }
 
 int launch_rank_curve(const uint32_t* key, const uint32_t* pay, long long count, long long T, int has_intrain,
@@ -805,6 +850,262 @@ int launch_rank_curve_points(const uint32_t* pay, long long count, long long T, 
     curve_points_kernel<<<tiles, RK_THREADS, 0, st>>>(pay, count, T, has_intrain, w.flags, x, y, yi);
     GCGCN_CHECK_LAUNCH("rank_curve_points");
     return GCGCN_OK;
+}
+
+// ---- per relation ------------------------------------------------------------------------------------------------
+// Every document gives n^2 - n candidates to each relation and its first id is a multiple of R - 1, so a candidate's
+// relation is (id mod (R - 1)) + 1 and every relation holds L = count / (R - 1) candidates.  The stable partition of a
+// ranking by relation (one more radix pass, digit from the payload) puts relation r's candidates, in ranked order, at
+// [(r - 1) L, r L).  The per-relation curve tiles every segment from its own start (blockIdx.y = r - 1, blockIdx.x =
+// tile of the segment), so no tile spans two relations: (R - 1) ceil(L / TILE) <= tiles + R - 1 pieces, and the flag
+// counts of a segment are the scanned piece counts minus the value at its first piece.
+int launch_rank_by_relation(const uint32_t* key, const uint32_t* pay, long long count, int R, uint32_t* rel_key,
+                            uint32_t* rel_pay, void* ws, size_t ws_bytes, cudaStream_t st) {
+    if (R == 2) {                                            // one relation: the partition is the ranking
+        GCGCN_TRY(cuda_ok(cudaMemcpyAsync(rel_key, key, count * sizeof(uint32_t), cudaMemcpyDeviceToDevice, st),
+                          "rank_by_relation"));
+        return cuda_ok(cudaMemcpyAsync(rel_pay, pay, count * sizeof(uint32_t), cudaMemcpyDeviceToDevice, st),
+                       "rank_by_relation");
+    }
+    Arena a = rank_arena(ws, ws_bytes);
+    const int tiles = rank_tiles(count);
+    const long long ncounts = static_cast<long long>(tiles) * RK_RADIX;
+    uint32_t* counts = a.take<uint32_t>(ncounts);
+    uint32_t* sums = a.take<uint32_t>(ceil_div(ncounts, SCAN_CHUNK));
+    if (counts == nullptr || sums == nullptr)
+        return fail(GCGCN_ERR_WORKSPACE, "rank_by_relation: workspace too small (%zu bytes)", ws_bytes);
+    radix_upsweep_kernel<DIGIT_RELATION><<<tiles, RK_THREADS, 0, st>>>(pay, count, R - 1, tiles, counts);
+    GCGCN_CHECK_LAUNCH("rank_relation_upsweep");
+    GCGCN_TRY(launch_scan<uint32_t>(counts, ncounts, sums, st));
+    radix_downsweep_kernel<DIGIT_RELATION><<<tiles, RK_THREADS, 0, st>>>(key, pay, count, R - 1, tiles, counts, rel_key,
+                                                                        rel_pay);
+    GCGCN_CHECK_LAUNCH("rank_relation_downsweep");
+    return GCGCN_OK;
+}
+
+// T of segment s: the caller's value, or the segment's correct candidates (flags holds the exclusive scan of the
+// piece counts, one entry past the last piece); < 1 means 1
+__device__ __forceinline__ long long segment_recall(const long long* __restrict__ total_recall,
+                                                    const unsigned long long* __restrict__ flags, int s,
+                                                    int seg_tiles) {
+    const long long v = total_recall != nullptr
+                            ? total_recall[s]
+                            : static_cast<long long>((flags[static_cast<long long>(s + 1) * seg_tiles] -
+                                                      flags[static_cast<long long>(s) * seg_tiles]) & 0xffffffffull);
+    return v < 1 ? 1 : v;
+}
+
+// packed flag counts of every piece (as curve_count_kernel, from coalesced loads of the segment); block (0, 0) also
+// zeroes the entry past the last piece, so that the scan leaves the grand total there
+__global__ void __launch_bounds__(RK_THREADS)
+rel_curve_count_kernel(const uint32_t* __restrict__ pay, long long L, int seg_tiles,
+                       unsigned long long* __restrict__ flags) {
+    __shared__ unsigned long long s_warp[33];
+    const uint32_t* run = pay + static_cast<long long>(blockIdx.y) * L;
+    const long long t0 = static_cast<long long>(blockIdx.x) * RK_TILE;
+    const int n = static_cast<int>(min(static_cast<long long>(RK_TILE), L - t0));
+    unsigned long long acc = 0;
+    for (int q = threadIdx.x; q < n; q += RK_THREADS) {
+        const uint32_t p = run[t0 + q];
+        acc += (p & 1u) + (static_cast<unsigned long long>((p & 3u) == 3u) << 32);
+    }
+    unsigned long long total;
+    block_excl_scan<unsigned long long, RK_THREADS>(acc, s_warp, &total);
+    if (threadIdx.x == 0) {
+        flags[static_cast<long long>(blockIdx.y) * seg_tiles + blockIdx.x] = total;
+        if (blockIdx.x == 0 && blockIdx.y == 0) flags[static_cast<long long>(gridDim.y) * seg_tiles] = 0ull;
+    }
+}
+
+__global__ void __launch_bounds__(RK_THREADS)
+rel_curve_main_kernel(const uint32_t* __restrict__ pay, long long L, int seg_tiles,
+                      const long long* __restrict__ total_recall, int has_intrain,
+                      const unsigned long long* __restrict__ flags, float* __restrict__ best_f1,
+                      long long* __restrict__ best_pos, float* __restrict__ best_ign, double* __restrict__ auc,
+                      double* __restrict__ ign_auc) {
+    __shared__ __align__(16) uint32_t s_stage[RK_TILE + 4];
+    const int s = blockIdx.y;
+    const long long first = static_cast<long long>(s) * seg_tiles, slot = first + blockIdx.x;
+    curve_main<false, true>(pay + s * L, L, segment_recall(total_recall, flags, s, seg_tiles), has_intrain, blockIdx.x,
+                            flags, first, s_stage, slot, best_f1, best_pos, best_ign, auc, ign_auc, nullptr, nullptr,
+                            nullptr);
+}
+
+// one block per relation: curve_finish over the segment's pieces, in tile order
+__global__ void __launch_bounds__(1024)
+rel_curve_finish_kernel(const uint32_t* __restrict__ key, const uint32_t* __restrict__ pay, long long L, int seg_tiles,
+                        const long long* __restrict__ total_recall, int has_intrain,
+                        const double* __restrict__ input_theta, const unsigned long long* __restrict__ flags,
+                        const float* __restrict__ best_f1, const long long* __restrict__ best_pos,
+                        const float* __restrict__ best_ign, const double* __restrict__ auc,
+                        const double* __restrict__ ign_auc, gcgcn_rank_result* __restrict__ res) {
+    const int s = blockIdx.x;
+    const long long first = static_cast<long long>(s) * seg_tiles;
+    curve_finish(key + s * L, pay + s * L, L, segment_recall(total_recall, flags, s, seg_tiles), has_intrain,
+                 input_theta[s], seg_tiles, flags + first, flags[first], best_f1 + first, best_pos + first,
+                 best_ign + first, auc + first, ign_auc + first, res + s);
+}
+
+struct RelCurveWs {
+    unsigned long long *flags, *sums;
+    float *best_f1, *best_ign;
+    long long* best_pos;
+    double *auc, *ign_auc;
+};
+static int seg_tiles_of(long long count, int R) { return rank_tiles(count / (R - 1)); }
+static bool rel_curve_ws_take(Arena& a, long long count, int R, RelCurveWs* w) {
+    const long long pieces = static_cast<long long>(R - 1) * seg_tiles_of(count, R);
+    w->flags = a.take<unsigned long long>(pieces + 1);
+    w->sums = a.take<unsigned long long>(ceil_div(pieces + 1, SCAN_CHUNK));
+    w->best_f1 = a.take<float>(pieces);
+    w->best_ign = a.take<float>(pieces);
+    w->best_pos = a.take<long long>(pieces);
+    w->auc = a.take<double>(pieces);
+    w->ign_auc = a.take<double>(pieces);
+    return w->flags && w->sums && w->best_f1 && w->best_ign && w->best_pos && w->auc && w->ign_auc;
+}
+
+int launch_rank_curve_relations(const uint32_t* key, const uint32_t* pay, long long count, int R,
+                                const long long* total_recall, int has_intrain, const double* input_theta,
+                                gcgcn_rank_result* res, void* ws, size_t ws_bytes, cudaStream_t st) {
+    Arena a = rank_arena(ws, ws_bytes);
+    RelCurveWs w;
+    if (!rel_curve_ws_take(a, count, R, &w))
+        return fail(GCGCN_ERR_WORKSPACE, "rank_curve_relations: workspace too small (%zu bytes)", ws_bytes);
+    const long long L = count / (R - 1);
+    const int seg_tiles = seg_tiles_of(count, R);
+    const dim3 grid(seg_tiles, R - 1);
+    rel_curve_count_kernel<<<grid, RK_THREADS, 0, st>>>(pay, L, seg_tiles, w.flags);
+    GCGCN_CHECK_LAUNCH("rank_relation_curve_count");
+    GCGCN_TRY(launch_scan<unsigned long long>(w.flags, static_cast<long long>(R - 1) * seg_tiles + 1, w.sums, st));
+    rel_curve_main_kernel<<<grid, RK_THREADS, 0, st>>>(pay, L, seg_tiles, total_recall, has_intrain, w.flags,
+                                                       w.best_f1, w.best_pos, w.best_ign, w.auc, w.ign_auc);
+    GCGCN_CHECK_LAUNCH("rank_relation_curve_main");
+    rel_curve_finish_kernel<<<R - 1, 1024, 0, st>>>(key, pay, L, seg_tiles, total_recall, has_intrain, input_theta,
+                                                    w.flags, w.best_f1, w.best_pos, w.best_ign, w.auc, w.ign_auc, res);
+    GCGCN_CHECK_LAUNCH("rank_relation_curve_finish");
+    return GCGCN_OK;
+}
+
+// ---- selection at one threshold per relation -----------------------------------------------------------------------
+// A ranked candidate is selected when its score > theta[relation - 1].  Per tile: counts of (selected) and of (selected
+// and correct | selected, correct and intrain << 32) -> two exclusive scans (one entry past the last tile holds the
+// totals) -> a stable in-tile compaction of the selected (key, payload) pairs.
+__device__ __forceinline__ void load_theta(const float* __restrict__ theta, int rm1, float* s_theta) {
+    for (int r = threadIdx.x; r < rm1; r += RK_THREADS) s_theta[r] = theta[r];
+    __syncthreads();
+}
+
+__global__ void __launch_bounds__(RK_THREADS)
+select_count_kernel(const uint32_t* __restrict__ key, const uint32_t* __restrict__ pay, long long count, int rm1,
+                    const float* __restrict__ theta, int tiles, uint32_t* __restrict__ sel,
+                    unsigned long long* __restrict__ flags) {
+    __shared__ float s_theta[RK_RADIX];
+    __shared__ uint32_t s_warp[33];
+    __shared__ unsigned long long s_warp64[33];
+    load_theta(theta, rm1, s_theta);
+    const long long base = static_cast<long long>(blockIdx.x) * RK_TILE + threadIdx.x * static_cast<long long>(RK_IPT);
+    uint32_t k[RK_IPT], p[RK_IPT];
+    load16(key, base, count, k);
+    load16(pay, base, count, p);
+    uint32_t m = 0;
+    unsigned long long ct = 0;
+#pragma unroll
+    for (int q = 0; q < RK_IPT; ++q) {
+        if (base + q < count && key_score(k[q]) > s_theta[(p[q] >> 2) % static_cast<uint32_t>(rm1)]) {
+            ++m;
+            ct += (p[q] & 1u) + (static_cast<unsigned long long>((p[q] & 3u) == 3u) << 32);
+        }
+    }
+    uint32_t m_total;
+    unsigned long long ct_total;
+    block_excl_scan<uint32_t, RK_THREADS>(m, s_warp, &m_total);
+    block_excl_scan<unsigned long long, RK_THREADS>(ct, s_warp64, &ct_total);
+    if (threadIdx.x == 0) {
+        sel[blockIdx.x] = m_total;
+        flags[blockIdx.x] = ct_total;
+        if (blockIdx.x == 0) { sel[tiles] = 0u; flags[tiles] = 0ull; }
+    }
+}
+
+__global__ void __launch_bounds__(RK_THREADS)
+select_scatter_kernel(const uint32_t* __restrict__ key, const uint32_t* __restrict__ pay, long long count, int rm1,
+                      const float* __restrict__ theta, int tiles, const uint32_t* __restrict__ sel,
+                      const unsigned long long* __restrict__ flags, uint32_t* __restrict__ out_key,
+                      uint32_t* __restrict__ out_pay, long long* __restrict__ counts) {
+    __shared__ float s_theta[RK_RADIX];
+    __shared__ uint32_t s_warp[33];
+    load_theta(theta, rm1, s_theta);
+    const long long base = static_cast<long long>(blockIdx.x) * RK_TILE + threadIdx.x * static_cast<long long>(RK_IPT);
+    uint32_t k[RK_IPT], p[RK_IPT];
+    load16(key, base, count, k);
+    load16(pay, base, count, p);
+    uint32_t pick = 0, m = 0;
+#pragma unroll
+    for (int q = 0; q < RK_IPT; ++q) {
+        const bool on = base + q < count && key_score(k[q]) > s_theta[(p[q] >> 2) % static_cast<uint32_t>(rm1)];
+        pick |= (on ? 1u : 0u) << q;
+        m += on;
+    }
+    long long o = block_excl_scan<uint32_t, RK_THREADS>(m, s_warp, nullptr) + static_cast<long long>(sel[blockIdx.x]);
+#pragma unroll
+    for (int q = 0; q < RK_IPT; ++q) {
+        if ((pick >> q) & 1u) {
+            out_key[o] = k[q];
+            out_pay[o] = p[q];
+            ++o;
+        }
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        counts[0] = sel[tiles];
+        counts[1] = static_cast<long long>(flags[tiles] & 0xffffffffull);
+        counts[2] = static_cast<long long>(flags[tiles] >> 32);
+    }
+}
+
+struct SelectWs {
+    uint32_t *sel, *sel_sums;
+    unsigned long long *flags, *sums;
+};
+static bool select_ws_take(Arena& a, long long count, SelectWs* w) {
+    const long long n = rank_tiles(count) + 1;
+    w->sel = a.take<uint32_t>(n);
+    w->sel_sums = a.take<uint32_t>(ceil_div(n, SCAN_CHUNK));
+    w->flags = a.take<unsigned long long>(n);
+    w->sums = a.take<unsigned long long>(ceil_div(n, SCAN_CHUNK));
+    return w->sel && w->sel_sums && w->flags && w->sums;
+}
+
+int launch_rank_select(const uint32_t* key, const uint32_t* pay, long long count, int R, const float* theta,
+                       uint32_t* out_key, uint32_t* out_pay, long long* counts, void* ws, size_t ws_bytes,
+                       cudaStream_t st) {
+    Arena a = rank_arena(ws, ws_bytes);
+    SelectWs w;
+    if (!select_ws_take(a, count, &w))
+        return fail(GCGCN_ERR_WORKSPACE, "rank_select: workspace too small (%zu bytes)", ws_bytes);
+    const int tiles = rank_tiles(count);
+    select_count_kernel<<<tiles, RK_THREADS, 0, st>>>(key, pay, count, R - 1, theta, tiles, w.sel, w.flags);
+    GCGCN_CHECK_LAUNCH("rank_select_count");
+    GCGCN_TRY(launch_scan<uint32_t>(w.sel, tiles + 1, w.sel_sums, st));
+    GCGCN_TRY(launch_scan<unsigned long long>(w.flags, tiles + 1, w.sums, st));
+    select_scatter_kernel<<<tiles, RK_THREADS, 0, st>>>(key, pay, count, R - 1, theta, tiles, w.sel, w.flags, out_key,
+                                                        out_pay, counts);
+    GCGCN_CHECK_LAUNCH("rank_select_scatter");
+    return GCGCN_OK;
+}
+
+size_t rank_relations_ws_bytes(long long count, int R) {
+    if (count <= 0 || R < 2) return 512;
+    const long long tiles = rank_tiles(count), ncounts = tiles * RK_RADIX;
+    const size_t partition = ((ncounts * sizeof(uint32_t) + 255) & ~size_t(255)) +
+                             ((ceil_div(ncounts, SCAN_CHUNK) * sizeof(uint32_t) + 255) & ~size_t(255));
+    Arena probe(reinterpret_cast<void*>(256), ~size_t(0) >> 1);
+    RelCurveWs c;
+    rel_curve_ws_take(probe, count, R, &c);
+    Arena probe2(reinterpret_cast<void*>(256), ~size_t(0) >> 1);
+    SelectWs s;
+    select_ws_take(probe2, count, &s);
+    return std::max(partition, std::max(probe.off, probe2.off)) + 256;
 }
 
 // ---- decode -----------------------------------------------------------------------------------------------------

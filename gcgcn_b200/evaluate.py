@@ -15,6 +15,10 @@ one small result struct.  No CPU path.
     res = ev.result(input_theta=-1.0)
     pred = ev.predictions(res["theta"])
 
+``per_relation`` evaluates every relation's candidates alone (the same fields as ``result``, one entry per relation),
+and ``result_at`` / ``predictions_at`` score and list the candidates above one threshold per relation, e.g. the θ_r a
+dev set's ``per_relation`` found, applied to a test set.
+
 A set evaluated in shards numbers its candidates globally: ``doc_sizes`` (the entity counts of every document of the
 set, in its order) fixes each document's first candidate id, and ``add(..., doc_index=...)`` names the documents of a
 batch.  Each shard is ranked alone; ``merged`` (one device) or ``all_gather`` (one shard per rank) merges the sorted
@@ -36,6 +40,9 @@ from .functional import _cuda, _p, _stream
 SORT_TILE = 4096                # GCGCN_RANK_TILE of include/gcgcn_b200.h
 MAX_CANDIDATES = 1 << 30        # one evaluator, or one globally numbered set, holds fewer (payload: id << 2 | flags)
 RESULT_BYTES = ctypes.sizeof(_lib.RankResult)
+MAX_RELATIONS = 257             # per_relation / result_at / predictions_at: relations 1 .. 256 (one 8-bit digit)
+_RESULT_DTYPE = np.dtype([(name, np.int64 if ctype is ctypes.c_int64 else np.float64 if ctype is ctypes.c_double
+                           else np.float32) for name, ctype in _lib.RankResult._fields_])
 
 
 class RelationEvaluator:
@@ -81,6 +88,7 @@ class RelationEvaluator:
         self._counters = torch.zeros(2, dtype=torch.int64, device=self.device)   # correct candidates, NaN scores
         self._host_counters = None
         self._ranked = None             # (sorted_key, sorted_payload, ws) while no add() follows
+        self._by_relation = None        # the ranking partitioned by relation (per_relation), while no add() follows
 
     # ---------------------------------------------------------------------------------------------------------------
     def add(self, logits: torch.Tensor, labels: Optional[torch.Tensor], batch: RaggedBatch,
@@ -130,6 +138,7 @@ class RelationEvaluator:
         self._has_intrain |= intrain is not None
         self._host_counters = None
         self._ranked = None
+        self._by_relation = None
 
     def _global_doc_first(self, batch: RaggedBatch, doc_index) -> Optional[torch.Tensor]:
         """Check doc_index against doc_sizes; the batch documents' first global ids on the device (None: local ids)."""
@@ -242,7 +251,11 @@ class RelationEvaluator:
         if input_theta == -1.0 and not self._labeled:
             raise _lib.GcgcnError("RelationEvaluator.predictions: the best-F1 threshold needs labels; pass input_theta")
         r = self._curve(input_theta, total_recall)
-        rows = int(r.w) + 1
+        key, pay, _ = self._ranked
+        return self._decode(key, pay, int(r.w) + 1, self.count)
+
+    def _decode(self, key, pay, rows, count) -> dict:
+        """The first ``rows`` candidates of the run (key, pay) of length ``count`` as ``predictions`` lists them."""
         if self._doc_sizes is None:
             n = np.asarray(self._doc_n, dtype=np.int64)
             off = np.zeros(n.size + 1, dtype=np.int64)
@@ -253,11 +266,105 @@ class RelationEvaluator:
         doc_n = torch.from_numpy(n.astype(np.int32)).to(self.device)
         out = {k: torch.empty(rows, dtype=torch.int32, device=self.device) for k in ("doc", "row", "col", "relation")}
         out["score"] = torch.empty(rows, dtype=torch.float32, device=self.device)
-        key, pay, _ = self._ranked
-        _lib.call("gcgcn_rank_decode", _p(key), _p(pay), rows, self.count, _p(doc_off), _p(doc_n), int(n.size), self.relations,
+        _lib.call("gcgcn_rank_decode", _p(key), _p(pay), rows, count, _p(doc_off), _p(doc_n), int(n.size), self.relations,
                   _p(out["doc"]), _p(out["row"]), _p(out["col"]), _p(out["relation"]), _p(out["score"]),
                   _stream(self.device))
         return out
+
+    # ------------------------------------------------------------------------------------------------- per relation
+    def _per_relation_values(self, values, dtype, what, scalar_ok=False) -> np.ndarray:
+        """``values`` as one host value per relation r >= 1 (a scalar stands for all of them if ``scalar_ok``)."""
+        v = np.asarray(values, dtype=dtype)
+        if v.ndim == 0 and scalar_ok:
+            v = np.full(self.relations - 1, v, dtype=dtype)
+        if v.shape != (self.relations - 1,):
+            raise _lib.GcgcnError(f"RelationEvaluator: {what} must hold relations - 1 = {self.relations - 1} values, "
+                                  f"got shape {list(v.shape)}")
+        return v
+
+    def _relation_ws(self) -> torch.Tensor:
+        """The ranking's workspace when it is large enough for the per-relation entry points, else a new one."""
+        need = int(_lib.load().gcgcn_rank_relations_ws_bytes(self.count, self.relations))
+        ws = self._ranked[2]
+        return ws if ws.numel() >= need else torch.empty(need, dtype=torch.uint8, device=self.device)
+
+    def per_relation(self, input_theta=-1.0, total_recall: Optional[Sequence[int]] = None) -> dict:
+        """``result`` for every relation r >= 1 on its own: relation r's candidates, in their order in the ranking (the
+        stable ranking of those candidates alone).  Host NumPy arrays of length relations - 1, entry r - 1 for
+        relation r: the fields of ``result`` (Ign fields None unless some ``add`` passed intrain) and ``relation``.
+        ``input_theta``: a scalar or one value per relation (-1: the relation's best-F1 position; otherwise its last
+        score above the value).  ``total_recall``: None (each relation's correct candidates) or one value per
+        relation.  At most 256 relations r >= 1."""
+        if not self._labeled:
+            raise _lib.GcgcnError("RelationEvaluator.per_relation: a batch was added without labels")
+        self._total_recall(None)                            # ranks; raises on NaN scores
+        theta = self._per_relation_values(input_theta, np.float64, "input_theta", scalar_ok=True)
+        tr = None if total_recall is None else self._per_relation_values(total_recall, np.int64, "total_recall")
+        key, pay, _ = self._ranked
+        ws = self._relation_ws()
+        st = _stream(self.device)
+        if self._by_relation is None:
+            rel_key, rel_pay = torch.empty_like(key), torch.empty_like(pay)
+            _lib.call("gcgcn_rank_by_relation", _p(key), _p(pay), self.count, self.relations, _p(rel_key), _p(rel_pay),
+                      _p(ws), ws.numel(), st)
+            self._by_relation = (rel_key, rel_pay)
+        rel_key, rel_pay = self._by_relation
+        theta_d = torch.from_numpy(theta).to(self.device)
+        tr_d = None if tr is None else torch.from_numpy(tr).to(self.device)
+        out = torch.empty((self.relations - 1) * RESULT_BYTES, dtype=torch.uint8, device=self.device)
+        _lib.call("gcgcn_rank_curve_relations", _p(rel_key), _p(rel_pay), self.count, self.relations, _p(tr_d),
+                  int(self._has_intrain), _p(theta_d), _p(out), _p(ws), ws.numel(), st)
+        r = out.cpu().numpy().view(_RESULT_DTYPE)
+        ign = self._has_intrain
+        res = {k: r[k].copy() for k in ("count", "total_recall", "f1", "theta", "best_pos", "auc", "w", "f1_at_w",
+                                         "precision_at_w", "recall_at_w")}
+        for k in ("ign_f1", "ign_auc", "ign_f1_at_w"):
+            res[k] = r[k].copy() if ign else None
+        res["relation"] = np.arange(1, self.relations, dtype=np.int64)
+        return res
+
+    def _select(self, theta):
+        """The candidates above theta[relation - 1], in ranked order: (key, payload) runs of length m, and (m, c, t)."""
+        self._total_recall(None)                            # ranks; raises on NaN scores
+        theta = self._per_relation_values(theta, np.float32, "theta")
+        key, pay, _ = self._ranked
+        ws = self._relation_ws()
+        out_key, out_pay = torch.empty_like(key), torch.empty_like(pay)
+        counts = torch.empty(3, dtype=torch.int64, device=self.device)
+        _lib.call("gcgcn_rank_select", _p(key), _p(pay), self.count, self.relations,
+                  _p(torch.from_numpy(theta).to(self.device)), _p(out_key), _p(out_pay), _p(counts), _p(ws), ws.numel(),
+                  _stream(self.device))
+        m, c, t = (int(v) for v in counts.cpu())
+        return out_key, out_pay, m, c, t
+
+    def result_at(self, theta, total_recall: Optional[int] = None) -> dict:
+        """Precision, recall, F1 and Ign F1 of the candidates whose score is above ``theta[relation - 1]`` (one float32
+        threshold per relation r >= 1, e.g. ``per_relation()["theta"]`` of a dev set): ``count_selected`` (m),
+        ``correct`` (c), precision = c / m (0 when m = 0), recall = c / total_recall (default: the correct candidates;
+        < 1 counts as 1), f1 and ``ign_f1`` (None unless some ``add`` passed intrain), rounded as ``result``."""
+        if not self._labeled:
+            raise _lib.GcgcnError("RelationEvaluator.result_at: a batch was added without labels")
+        T = max(self._total_recall(total_recall), 1)
+        _, _, m, c, t = self._select(theta)
+        f32 = np.float32
+
+        def f1(x, y):                                       # float32, every operation rounded (rank.cu, curve_f1)
+            return f32(f32(f32(2) * x) * y) / f32(f32(x + y) + f32(1e-20))
+
+        precision = f32(c / m) if m else f32(0)
+        recall = f32(c / T)
+        out = {"count_selected": m, "correct": c, "precision": float(precision), "recall": float(recall),
+               "f1": float(f1(recall, precision)), "ign_f1": None}
+        if self._has_intrain:
+            ign = f32(0) if t == c else f32((c - t) / (m - t))
+            out["ign_f1"] = float(f1(recall, ign))
+        return out
+
+    def predictions_at(self, theta) -> dict:
+        """``predictions`` for the candidates whose score is above ``theta[relation - 1]`` (one float32 threshold per
+        relation r >= 1), in ranked order.  Needs no labels: dev-set thresholds applied to a test set."""
+        key, pay, m, _, _ = self._select(theta)
+        return self._decode(key, pay, m, m)
 
     # --------------------------------------------------------------------------------------------------- sharded sets
     @classmethod

@@ -536,6 +536,39 @@ int gcgcn_rank_decode(const uint32_t* sorted_key, const uint32_t* sorted_payload
                       const int64_t* doc_offsets, const int32_t* doc_n, int32_t num_docs, int32_t relations, int32_t* doc,
                       int32_t* row, int32_t* col, int32_t* relation, float* score, void* stream);
 
+/* ---- relation evaluation per relation -----------------------------------------------------------------------------
+ * A candidate's relation is (id mod (R - 1)) + 1 (every document's first id is a multiple of R - 1, for local and
+ * global ids), and each relation holds exactly count / (R - 1) of the candidates of a ranking.
+ * Per-relation result: entry r - 1 is what gcgcn_rank_curve returns when given only relation r's candidates, in their
+ * order in the ranking (which, the ranking being stable, is the stable ranking of those candidates alone); every field
+ * keeps its meaning with positions counted inside the relation's own ranking.  T_r = total_recall[r - 1], or else the
+ * number of correct candidates of r; < 1 means 1.  input_theta[r - 1] = -1 selects the relation's best-F1 position;
+ * any other value the last position whose score > input_theta[r - 1], or 0 if there is none.
+ * Selection at per-relation thresholds: every candidate whose score > theta[relation - 1], in ranked order.  With m
+ * candidates selected, c of them correct and t correct and intrain, and T the total recall: precision =
+ * f32(c / m) (0 when m = 0), recall = f32(c / T), f1 = (2 recall precision) / ((recall + precision) + 1e-20) and Ign
+ * f1 the same with the Ign precision of (c, t, m) (the roundings of the curve above).
+ * At most 256 relations r >= 1 (R <= 257: one 8-bit digit).  Every entry point is deterministic and bit-reproducible,
+ * writes only the caller's memory and enqueues on the stream.                                                       */
+/* workspace of gcgcn_rank_by_relation, gcgcn_rank_curve_relations and gcgcn_rank_select (any alignment)            */
+size_t gcgcn_rank_relations_ws_bytes(int64_t count, int32_t relations);
+/* Stable partition of a ranking (gcgcn_rank_sort / gcgcn_rank_merge) by relation: relation r's candidates, in ranked
+ * order, at [(r - 1) count / (R - 1), r count / (R - 1)).  count % (R - 1) != 0: GCGCN_ERR_INVALID_ARG; R - 1 > 256:
+ * GCGCN_ERR_UNSUPPORTED.  Outputs disjoint from the inputs.  Moves 20 bytes per candidate.                         */
+int gcgcn_rank_by_relation(const uint32_t* sorted_key, const uint32_t* sorted_payload, int64_t count, int32_t relations,
+                           uint32_t* rel_key, uint32_t* rel_payload, void* ws, size_t ws_bytes, void* stream);
+/* The per-relation results over a partition from gcgcn_rank_by_relation: results [R - 1] (device memory).
+ * total_recall [R - 1] int64 (device) or NULL; input_theta [R - 1] double (device).  rel_payload 16-byte aligned.  */
+int gcgcn_rank_curve_relations(const uint32_t* rel_key, const uint32_t* rel_payload, int64_t count, int32_t relations,
+                               const int64_t* total_recall, int32_t has_intrain, const double* input_theta,
+                               gcgcn_rank_result* results, void* ws, size_t ws_bytes, void* stream);
+/* Selection of a ranking at theta [R - 1] float32 (device): out_key / out_payload [count] receive the selected
+ * candidates, in ranked order, from position 0 (gcgcn_rank_decode lists them); counts [3] int64 (device) = m, c, t.
+ * Inputs 16-byte aligned; outputs disjoint from them.                                                               */
+int gcgcn_rank_select(const uint32_t* sorted_key, const uint32_t* sorted_payload, int64_t count, int32_t relations,
+                      const float* theta, uint32_t* out_key, uint32_t* out_payload, int64_t* counts, void* ws,
+                      size_t ws_bytes, void* stream);
+
 /* ---- training step of config 5 (new work: the reference has no multi-GPU path, SURVEY.md 8e) ----
  * Fused Adam over ONE flat float32 buffer holding every hot-path parameter, with the semantics of
  * torch.optim.Adam as the reference's trainer constructs it (config/Config.py:300: lr only, betas

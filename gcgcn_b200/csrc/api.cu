@@ -1127,12 +1127,14 @@ int gcgcn_bilinear_fwd(const float* h, const float* t, const float* Wm, const fl
     GCGCN_TRY(check_device_ptr(t, "t"));
     GCGCN_TRY(check_device_ptr(Wm, "Wm"));
     GCGCN_TRY(check_device_ptr(out, "out"));
+    const size_t need = gcgcn_bilinear_ws_bytes(rows, relations);
+    if (ws == nullptr || ws_bytes < need)
+        return fail(GCGCN_ERR_WORKSPACE, "bilinear_fwd: workspace of %zu bytes needed, got %zu", need, ws_bytes);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     Arena ar(ws, ws_bytes);
     const size_t ld = (static_cast<size_t>(rows) + 31) & ~size_t(31);
     uint8_t* blobs = ar.take<uint8_t>(static_cast<size_t>(relations) * 4 * 33024);
     float* part = ar.take<float>(2 * static_cast<size_t>(relations) * ld);
-    if (blobs == nullptr || part == nullptr) return fail(GCGCN_ERR_WORKSPACE, "bilinear_fwd: workspace too small");
     GCGCN_TRY(launch_gemm_rowop(1, rows, relations * D, D, h, D, Wm, relations * D, t, part, static_cast<long long>(ld), blobs,
                                 static_cast<size_t>(relations) * 4 * 33024, st));
     return launch_bilinear_finish(part, static_cast<long long>(ld), bias, rows, relations, accumulate, out, ldo, st);
@@ -1156,6 +1158,9 @@ int gcgcn_bilinear_bwd(const float* h, const float* t, const float* Wm, const fl
                     "gcgcn_bilinear_outer_bwd / gcgcn_bilinear_dt_bwd with gcgcn_gemm", rows);
     const void* ps[] = {h, t, Wm, Wm2, dout, dh, dt, dWm};
     for (const void* p : ps) GCGCN_TRY(check_device_ptr(p, "bilinear_bwd operand"));
+    const size_t need = gcgcn_bilinear_bwd_ws_bytes(rows, relations);
+    if (ws == nullptr || ws_bytes < need)
+        return fail(GCGCN_ERR_WORKSPACE, "bilinear_bwd: workspace of %zu bytes needed, got %zu", need, ws_bytes);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     Arena ar(ws, ws_bytes);
     const size_t blob_bytes = static_cast<size_t>(relations) * 4 * 33024, pre_bytes = gemm_presplit_bytes(rows);
@@ -1164,8 +1169,6 @@ int gcgcn_bilinear_bwd(const float* h, const float* t, const float* Wm, const fl
     uint8_t* blobs = ar.take<uint8_t>(blob_bytes);
     uint8_t* gws = ar.take<uint8_t>(gws_bytes);
     uint8_t* pre = ar.take<uint8_t>(pre_bytes);
-    if (blobs == nullptr || gws == nullptr || pre == nullptr)
-        return fail(GCGCN_ERR_WORKSPACE, "bilinear_bwd: workspace too small");
     const int N = relations * D;
     GCGCN_TRY(launch_gemm_rowop(2, rows, N, D, h, D, Wm, N, dout, dt, relations, blobs, blob_bytes, st));
     GCGCN_TRY(launch_gemm_rowop(2, rows, N, D, t, D, Wm2, N, dout, dh, relations, blobs, blob_bytes, st));

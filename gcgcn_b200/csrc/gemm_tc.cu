@@ -935,11 +935,11 @@ int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float
     a.Apre = nullptr;
     const size_t ablob_total = static_cast<size_t>(a.tiles_m) * a.kblocks * TC_B_BLOB_BYTES;
     const bool apre = bscale != nullptr && !bpre && batch == 1 && ta && !tb && K >= 8192 && M <= 2 * TC_BM &&
-                      a.tiles_n >= 2 && (seq ? (a.partial != nullptr || tiles <= sms) : tiles * splits <= sms) &&
+                      (seq ? (a.partial != nullptr || tiles <= sms) : tiles * splits <= sms) &&
                       pre_ws != nullptr && ablob_total <= pre_bytes && (reinterpret_cast<uintptr_t>(pre_ws) & 15) == 0;
     if (bscale != nullptr && !apre)
         return fail(GCGCN_ERR_UNSUPPORTED, "gemm: the generated-operand product needs the pre-split weight-gradient path "
-                    "(A transposed, K >= 8192, M <= 256, N >= 256, a pre-split workspace)");
+                    "(A transposed, K >= 8192, M <= 256, a pre-split workspace)");
     if (apre) {
         tc_presplit_b_kernel<<<dim3(a.tiles_m * a.kblocks, 4), 256, 0, st>>>(A, lda, /*kcontig=*/0, M, K, a.kblocks,
                                                                   static_cast<uint8_t*>(pre_ws));

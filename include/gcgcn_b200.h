@@ -411,7 +411,7 @@ int gcgcn_colsum(const float* X, int32_t M, int32_t N, int32_t ldx, float* out, 
 /* Fused forward: out[p][r] (+)= sum_{a,b} h[p][a] W'[a][r*128 + b] t[p][b] + bias[r] in ONE tensor-core pass -- h stays
  * resident in tensor memory per 128-pair tile, W' streams through shared memory as pre-split blobs, and the epilogue
  * contracts every 128 x 128 accumulator tile (one relation) with t straight out of TMEM, so h W' never exists.
- * Wm = W' [128, relations*128] row-major; ws >= gcgcn_bilinear_ws_bytes(rows, relations).                       */
+ * Wm = W' [128, relations*128] row-major; ws >= gcgcn_bilinear_ws_bytes(rows, relations), else GCGCN_ERR_WORKSPACE. */
 size_t gcgcn_bilinear_ws_bytes(int32_t rows, int32_t relations);
 int gcgcn_bilinear_fwd(const float* h, const float* t, const float* Wm, const float* bias, int32_t rows,
                        int32_t relations, int32_t accumulate, float* out, int32_t ldo, void* ws, size_t ws_bytes,
@@ -422,7 +422,7 @@ int gcgcn_bilinear_fwd(const float* h, const float* t, const float* Wm, const fl
  *   dh[p][a] = sum_r dout[p][r] (t W'')[p][r*128 + a]     the same with A = t, B = Wm2 (W viewed as [128 (b), relations*128 (r, a)])
  *   dWm[a][r*128 + b] = beta dWm + sum_p h[p][a] dout[p][r] t[p][b]   weight-gradient GEMM whose [rows, relations*128]
  *                       operand is generated in the producers from t and dout (never stored)
- * dout [rows, relations] row-major.  ws >= gcgcn_bilinear_bwd_ws_bytes(rows, relations).                          */
+ * dout [rows, relations] row-major.  ws >= gcgcn_bilinear_bwd_ws_bytes(rows, relations), else GCGCN_ERR_WORKSPACE.   */
 size_t gcgcn_bilinear_bwd_ws_bytes(int32_t rows, int32_t relations);
 int gcgcn_bilinear_bwd(const float* h, const float* t, const float* Wm, const float* Wm2, const float* dout, int32_t rows,
                        int32_t relations, float beta, float* dh, float* dt, float* dWm, void* ws, size_t ws_bytes,

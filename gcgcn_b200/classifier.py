@@ -6,7 +6,8 @@
 one dense n^2-scale contraction of the model (2 * 128 * 128 * 97 flop per pair): it runs on this package's tcgen05 GEMM
 (3xTF32) as ``Y = h W'`` with ``W'`` the ``[R, 128, 128]`` weight viewed as ``[128, R*128]``, then a row-wise reduction
 against ``t``; the pairs are walked in chunks so that ``Y`` (R*128 floats per pair) stays inside a fixed workspace.
-No CPU path.
+``relation_logits(..., dtype=torch.bfloat16)`` runs the bilinear form on bf16-rounded operands instead (``BilinearBf16Fn``:
+one ``kind::f16`` tensor-core pass, fp32 accumulation; parameters, inputs and gradients stay fp32).  No CPU path.
 """
 from __future__ import annotations
 
@@ -95,6 +96,50 @@ class BilinearFn(Function):
         return dh, dt, dW, dbias
 
 
+class BilinearBf16Fn(Function):
+    """The bilinear form with bf16 operands and fp32 accumulation (include/gcgcn_b200.h, gcgcn_bilinear_bf16_fwd):
+    out[p, r] = sum_b (sum_a bf16(h[p,a]) bf16(W[r,a,b])) t[p,b] + bias[r].  h, t, W, bias and every gradient are fp32;
+    dW[r,a,b] = sum_p bf16(h[p,a]) bf16(dout[p,r] t[p,b]).  The fused kernels take any number of pairs: the backward makes
+    host calls of at most FUSED_CHUNK_PAIRS pairs that accumulate dW' through beta = 1, and has no chunked path."""
+
+    @staticmethod
+    def forward(ctx, h, t, W, bias):
+        h, t, W, bias = _cuda(h, "h"), _cuda(t, "t"), _cuda(W, "weight"), _cuda(bias, "bias")
+        P, R, dev = h.shape[0], W.shape[0], h.device
+        if W.shape[1:] != (D, D) or h.shape[1] != D or t.shape != h.shape:
+            raise _lib.GcgcnError(f"bilinear: expected h, t [P, {D}] and weight [R, {D}, {D}]")
+        Wm = _wmat(W)
+        out = torch.empty(P, R, device=dev)
+        if P > 0:
+            ws = workspace(dev, int(_lib.load().gcgcn_bilinear_bf16_ws_bytes(P, R)))
+            _lib.call("gcgcn_bilinear_bf16_fwd", _p(h), _p(t), _p(Wm), _p(bias), P, R, 0, _p(out), R, ws.data_ptr(),
+                      ws.numel(), _stream(dev))
+        ctx.save_for_backward(h, t, Wm)
+        ctx.R = R
+        return out
+
+    @staticmethod
+    def backward(ctx, dout):
+        h, t, Wm = ctx.saved_tensors
+        R, dev, P = ctx.R, h.device, h.shape[0]
+        dout = _cuda(dout, "dout")
+        dh, dt = torch.empty_like(h), torch.empty_like(t)
+        dWm = torch.zeros_like(Wm)
+        Wm2 = Wm.view(D, R, D).permute(2, 1, 0).reshape(D, R * D).contiguous()       # W viewed as [b][(r, a)]
+        lib = _lib.load()
+        for p0 in range(0, P, FUSED_CHUNK_PAIRS):
+            p1 = min(P, p0 + FUSED_CHUNK_PAIRS)
+            rows = p1 - p0
+            ws = workspace(dev, int(lib.gcgcn_bilinear_bf16_bwd_ws_bytes(rows, R)))
+            _lib.call("gcgcn_bilinear_bf16_bwd", _p(h[p0:p1]), _p(t[p0:p1]), _p(Wm), _p(Wm2), _p(dout[p0:p1]), rows, R,
+                      1.0, _p(dh[p0:p1]), _p(dt[p0:p1]), _p(dWm), ws.data_ptr(), ws.numel(), _stream(dev))
+        dbias = torch.empty(R, device=dev)
+        ws = workspace(dev, 8 << 20)
+        _lib.call("gcgcn_colsum", _p(dout), P, R, R, _p(dbias), ws.data_ptr(), ws.numel(), _stream(dev))
+        dW = dWm.view(D, R, D).permute(1, 0, 2).contiguous()
+        return dh, dt, dW, dbias
+
+
 class PairBceFn(Function):
     """Per-document loss of config/Config.py:355-364 from logits and multi-hot labels [total_pairs, R]."""
 
@@ -141,13 +186,17 @@ class DocBiasFn(Function):
 
 
 def relation_logits(h: torch.Tensor, t: torch.Tensor, bili: nn.Bilinear, cls: nn.Linear, cls_feature=None,
-                    batch: RaggedBatch = None) -> torch.Tensor:
+                    batch: RaggedBatch = None, dtype=torch.float32) -> torch.Tensor:
     """G:356-358: ``bili(h, t) + cls(cat[h, t])`` without forming the concatenation (the linear layer is split by
     input columns into its h and t halves).  ``cls_feature`` [num_docs, R] (with ``batch``) adds the BERT variant's
-    per-document term, B:346-347."""
+    per-document term, B:346-347.  ``dtype`` is the operand type of the bilinear form: torch.float32 (3xTF32, fp32
+    parity) or torch.bfloat16 (BilinearBf16Fn); the linear layer, the logits and every gradient are fp32 either way."""
+    if dtype not in (torch.float32, torch.bfloat16):
+        raise _lib.GcgcnError(f"relation_logits: dtype must be torch.float32 or torch.bfloat16, got {dtype}")
     w = cls.weight
     lin = LinearFn.apply(h, w[:, :D], cls.bias) + LinearFn.apply(t, w[:, D:], None)
-    z = BilinearFn.apply(h, t, bili.weight, bili.bias) + lin
+    bilinear = BilinearBf16Fn if dtype == torch.bfloat16 else BilinearFn
+    z = bilinear.apply(h, t, bili.weight, bili.bias) + lin
     return z if cls_feature is None else DocBiasFn.apply(z, cls_feature, batch)
 
 

@@ -106,6 +106,12 @@ int launch_gemm_rowop(int mode, int M, int N, int K, const float* A, int lda, co
 int launch_gemm_wgrad_scaled(int M, int tiles, int K, const float* A, int lda, const float* T, const float* scale, int lds,
                              float beta, float* C, int ldc, void* ws, size_t ws_bytes, cudaStream_t st, void* pre_ws,
                              size_t pre_bytes);
+size_t gemm_bf16_blob_bytes(int N, int K);
+int launch_gemm_rowop_bf16(int mode, int M, int N, int K, const float* A, int lda, const float* B, int ldb, const float* T,
+                           float* out, long long ld, void* ws, size_t ws_bytes, cudaStream_t st);
+int launch_bilinear_wgrad_bf16(int relations, int rows, const float* h, const float* T, const float* scale, int lds,
+                               float beta, float* C, void* ws, size_t ws_bytes, void* pre, size_t pre_bytes,
+                               cudaStream_t st);
 int launch_bilinear_outer(const float* dout, int ldd, const float* t, int rows, int R, float* dY, cudaStream_t st);
 int launch_bilinear_dt(const float* dout, int ldd, const float* Y, int rows, int R, float* dt, cudaStream_t st);
 int launch_doc_bias_fwd(const gcgcn_batch* bt, const float* v, int R, float* z, cudaStream_t st);
@@ -1174,6 +1180,69 @@ int gcgcn_bilinear_bwd(const float* h, const float* t, const float* Wm, const fl
     GCGCN_TRY(launch_gemm_rowop(2, rows, N, D, t, D, Wm2, N, dout, dh, relations, blobs, blob_bytes, st));
     return launch_gemm_wgrad_scaled(D, relations, rows, h, D, t, dout, relations, beta, dWm, N, gws, gws_bytes, st, pre,
                                     pre_bytes);
+}
+
+// ---- the bilinear form on bf16-rounded operands (single-pass kind::f16, fp32 accumulation) ----
+size_t gcgcn_bilinear_bf16_ws_bytes(int32_t rows, int32_t relations) {
+    const int r = relations < 0 ? 0 : relations;
+    const size_t m = static_cast<size_t>(rows < 0 ? 0 : rows), ld = (m + 31) & ~size_t(31);
+    return align256(gemm_bf16_blob_bytes(r * D, D)) + align256(2 * static_cast<size_t>(r) * ld * sizeof(float)) + 4096;
+}
+
+int gcgcn_bilinear_bf16_fwd(const float* h, const float* t, const float* Wm, const float* bias, int32_t rows,
+                            int32_t relations, int32_t accumulate, float* out, int32_t ldo, void* ws, size_t ws_bytes,
+                            void* stream) {
+    GCGCN_API_ENTER(stream);
+    GCGCN_REQUIRE(rows >= 0 && relations >= 0 && ldo >= relations, "bilinear_bf16_fwd: bad shape");
+    if (rows == 0 || relations == 0) return GCGCN_OK;
+    GCGCN_TRY(check_device_ptr(h, "h"));
+    GCGCN_TRY(check_device_ptr(t, "t"));
+    GCGCN_TRY(check_device_ptr(Wm, "Wm"));
+    GCGCN_TRY(check_device_ptr(out, "out"));
+    const size_t need = gcgcn_bilinear_bf16_ws_bytes(rows, relations);
+    if (ws == nullptr || ws_bytes < need)
+        return fail(GCGCN_ERR_WORKSPACE, "bilinear_bf16_fwd: workspace of %zu bytes needed, got %zu", need, ws_bytes);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    Arena ar(ws, ws_bytes);
+    const size_t ld = (static_cast<size_t>(rows) + 31) & ~size_t(31), blob_bytes = gemm_bf16_blob_bytes(relations * D, D);
+    uint8_t* blobs = ar.take<uint8_t>(blob_bytes);
+    float* part = ar.take<float>(2 * static_cast<size_t>(relations) * ld);
+    GCGCN_TRY(launch_gemm_rowop_bf16(1, rows, relations * D, D, h, D, Wm, relations * D, t, part, static_cast<long long>(ld),
+                                     blobs, blob_bytes, st));
+    return launch_bilinear_finish(part, static_cast<long long>(ld), bias, rows, relations, accumulate, out, ldo, st);
+}
+
+size_t gcgcn_bilinear_bf16_bwd_ws_bytes(int32_t rows, int32_t relations) {
+    const int r = relations < 0 ? 0 : relations, m = rows < 0 ? 0 : rows;
+    // bf16 W' (then W'') blobs, one [128, relations*128] partial per 4096-row range when there are several, bf16 h blobs
+    const size_t ranges = (static_cast<size_t>(m) + 4095) / 4096;
+    return align256(gemm_bf16_blob_bytes(r * D, D)) + align256(ranges > 1 ? ranges * D * r * D * sizeof(float) : 0) +
+           align256(gemm_bf16_blob_bytes(D, m)) + 4096;
+}
+
+int gcgcn_bilinear_bf16_bwd(const float* h, const float* t, const float* Wm, const float* Wm2, const float* dout,
+                            int32_t rows, int32_t relations, float beta, float* dh, float* dt, float* dWm, void* ws,
+                            size_t ws_bytes, void* stream) {
+    GCGCN_API_ENTER(stream);
+    GCGCN_REQUIRE(rows >= 0 && relations >= 1, "bilinear_bf16_bwd: bad shape");
+    if (rows == 0) return GCGCN_OK;
+    const void* ps[] = {h, t, Wm, Wm2, dout, dh, dt, dWm};
+    for (const void* p : ps) GCGCN_TRY(check_device_ptr(p, "bilinear_bf16_bwd operand"));
+    const size_t need = gcgcn_bilinear_bf16_bwd_ws_bytes(rows, relations);
+    if (ws == nullptr || ws_bytes < need)
+        return fail(GCGCN_ERR_WORKSPACE, "bilinear_bf16_bwd: workspace of %zu bytes needed, got %zu", need, ws_bytes);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    Arena ar(ws, ws_bytes);
+    const int N = relations * D;
+    const size_t blob_bytes = gemm_bf16_blob_bytes(N, D), pre_bytes = gemm_bf16_blob_bytes(D, rows);
+    const size_t ranges = (static_cast<size_t>(rows) + 4095) / 4096;
+    const size_t part_bytes = ranges > 1 ? ranges * D * static_cast<size_t>(N) * sizeof(float) : 0;
+    uint8_t* blobs = ar.take<uint8_t>(blob_bytes);
+    uint8_t* part = ar.take<uint8_t>(part_bytes);
+    uint8_t* pre = ar.take<uint8_t>(pre_bytes);
+    GCGCN_TRY(launch_gemm_rowop_bf16(2, rows, N, D, h, D, Wm, N, dout, dt, relations, blobs, blob_bytes, st));
+    GCGCN_TRY(launch_gemm_rowop_bf16(2, rows, N, D, t, D, Wm2, N, dout, dh, relations, blobs, blob_bytes, st));
+    return launch_bilinear_wgrad_bf16(relations, rows, h, t, dout, relations, beta, dWm, part, part_bytes, pre, pre_bytes, st);
 }
 
 int gcgcn_bilinear_outer_bwd(const float* dout, int32_t ldd, const float* t, int32_t rows, int32_t relations, float* dY,

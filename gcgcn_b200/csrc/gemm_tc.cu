@@ -318,13 +318,58 @@ __device__ __forceinline__ void tc_epilogue_tile(const TcArgs& args, uint32_t tm
 // producers' work, and the registers it frees double-buffer the A loads (two K blocks in flight per group).
 constexpr uint32_t TC_B_BLOB_BYTES = 2 * TC_PART_BYTES;     // B_hi part, B_lo part
 
+// ---- bf16 operands: one kind::f16 MMA (BF16 A and B, fp32 accumulator, K = 16) per 16 K values instead of three
+// kind::tf32 MMAs per 8.  Every operand value is rounded once to bf16 (round to nearest even); the products are exact in
+// fp32 and accumulate in fp32.  Same K-major no-swizzle layout as above with 8 bf16 per 16-byte chunk: a K block of
+// TC_BK values is 4 chunk planes (one blob of 8256 B instead of the 33024 B of a hi/lo pair), and one MMA reads two
+// planes, so make_desc() serves unchanged.
+constexpr uint32_t TC_BF16_BLOB_BYTES = (TC_BK / 8) * TC_PLANE_BYTES;
+// kind::f16 instruction descriptor: D F32 (bits 4-5 = 1), A and B BF16 (bits 7-9, 10-12 = 1), both K-major, N = 128, M = 128
+constexpr uint32_t TC_IDESC_BF16 = (1u << 4) | (1u << 7) | (1u << 10) | ((TC_BN >> 3) << 17) | ((TC_BM >> 4) << 24);
+
+// generated operand of the bf16 weight gradient: thread tid owns row tid, v[i] its K values 4i..4i+3 (tile_coord<false>).
+// pack_operand_bf16 rounds them in place: v[j] (j < 4) then holds the 16-byte chunk (8 K values) of plane j.
+__device__ __forceinline__ void pack_operand_bf16(float4 (&v)[8]) {
+#pragma unroll
+    for (int j = 0; j < TC_BK / 8; ++j) {
+        const float4 a = v[2 * j], b = v[2 * j + 1];
+        v[j] = make_float4(__uint_as_float(pack_bf16x2(a.x, a.y)), __uint_as_float(pack_bf16x2(a.z, a.w)),
+                           __uint_as_float(pack_bf16x2(b.x, b.y)), __uint_as_float(pack_bf16x2(b.z, b.w)));
+    }
+}
+// rows kq..kq+31 of T [K][128] at column tid, in the tile_coord<false> order (v[i] = rows 4i..4i+3), 0 past kend.  The row
+// stride is the constant 128: every load of a whole block is one base register plus an immediate offset.
+__device__ __forceinline__ void fetch_rows128(const float* __restrict__ T, int kq, int kend, int tid, float4 (&v)[8]) {
+    const float* p = T + static_cast<size_t>(kq) * TC_BN + tid;
+    if (kq + TC_BK <= kend) {
+#pragma unroll
+        for (int i = 0; i < 8; ++i)
+            v[i] = make_float4(p[(4 * i) * TC_BN], p[(4 * i + 1) * TC_BN], p[(4 * i + 2) * TC_BN], p[(4 * i + 3) * TC_BN]);
+    } else {
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            float t[4];
+#pragma unroll
+            for (int q = 0; q < 4; ++q) t[q] = kq + 4 * i + q < kend ? p[(4 * i + q) * TC_BN] : 0.f;
+            v[i] = make_float4(t[0], t[1], t[2], t[3]);
+        }
+    }
+}
+__device__ __forceinline__ void store_operand_bf16(uint8_t* base, int tid, const float4 (&v)[8]) {
+#pragma unroll
+    for (int j = 0; j < TC_BK / 8; ++j) *reinterpret_cast<float4*>(base + j * TC_PLANE_BYTES + tid * 16) = v[j];
+}
+
 // APRE: the mirror image for the generated-operand weight gradient of the bilinear form (K = every pair): the small
 // [rows, 128] operand is pre-split into blobs, the producers generate the wide operand (double-buffered).
 // MNMAJ: both operands stored [K][MN] (C = A^T B) and fed to the tensor core MN-major (A_KCONTIG = B_KCONTIG = false).
-template <bool A_KCONTIG, bool B_KCONTIG, int GROUPS, bool BPRE, bool APRE = false, bool MNMAJ = false>
+// BF16 (APRE only): the A blobs hold bf16 (tc_bf16_blobs_kernel), the producers round the generated operand to bf16, and
+// every stage is two kind::f16 MMAs.
+template <bool A_KCONTIG, bool B_KCONTIG, int GROUPS, bool BPRE, bool APRE = false, bool MNMAJ = false, bool BF16 = false>
 __global__ void __launch_bounds__(tc_threads(GROUPS), 1) gemm_tc_kernel(const TcArgs args) {
     constexpr int TC_PRODUCER_WARPS = 4 * GROUPS, TC_MMA_WARP = 4 * GROUPS, TC_GROUPS = GROUPS;
     static_assert(GROUPS <= TC_STAGES, "a producer group may run at most one stage-round ahead of the MMA warp");
+    static_assert(!BF16 || (APRE && !B_KCONTIG && !MNMAJ), "bf16 is the generated-operand weight gradient only");
     // (no integer round trip on this pointer: the compiler must keep seeing shared memory, or every
     //  operand store degrades to a generic ST)
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -406,7 +451,65 @@ __global__ void __launch_bounds__(tc_threads(GROUPS), 1) gemm_tc_kernel(const Tc
                 q += GROUPS;
             }
         }
-        if (APRE) {
+        if (APRE && BF16) {
+            // Same work items, K blocks and stage bookkeeping as below.  fetch only ISSUES loads -- the 32 x 128 block of
+            // T and, per lane, one scale bscale[k0 + lane][nt] -- so that two K blocks per group really are in flight;
+            // commit scales, rounds and stores.  (Multiplying inside fetch, as below, waits for the loads there: the
+            // bf16 MMAs are 6x shorter than the 3xTF32 ones and that wait became the bound.)  The scales go through a
+            // 128-byte slot per warp at TC_PART_BYTES in the stage, bytes that neither the tensor core nor the bulk
+            // copy touch in bf16 mode, and come back as float4 (four K values of one chunk).
+            int jbase = 0;
+            for (int t = blockIdx.x; t < total_tiles; t += gridDim.x) {
+                const int ks = t / tiles_mn, rem = t - ks * tiles_mn;
+                const int mtile = rem / args.tiles_n, nt = rem % args.tiles_n;
+                const int kbeg = ks * args.k_per_split, kend = min(args.K, kbeg + args.k_per_split);
+                const int total_q = kend > kbeg ? (kend - kbeg + TC_BK - 1) / TC_BK : 0;
+                auto fetch = [&](int q, float4 (&v)[8], float& sc) {
+                    const int kq = kbeg + q * TC_BK;
+                    fetch_rows128(args.B, kq, kend, tid, v);
+                    sc = kq + lane < kend ? args.bscale[static_cast<size_t>(kq + lane) * args.lds + nt] : 0.f;
+                };
+                auto commit = [&](int q, float4 (&v)[8], float sc) {
+                    const int j = jbase + q, stage = j % TC_STAGES;
+                    const uint32_t phase = (j / TC_STAGES) & 1;
+                    mbar_wait(empty_bar(stage), phase ^ 1);
+                    uint8_t* stb = smem + size_t(stage) * TC_STAGE_BYTES;
+                    if (tid == 0) {
+                        const uint8_t* blob = args.Apre + (static_cast<size_t>(mtile) * args.kblocks + kbeg / TC_BK + q) * TC_BF16_BLOB_BYTES;
+                        mbar_arrive_expect_tx(full_bar(stage), TC_BF16_BLOB_BYTES);
+                        bulk_copy_g2s(smem_u32(stb), blob, TC_BF16_BLOB_BYTES, full_bar(stage));
+                    }
+                    float* slot = reinterpret_cast<float*>(stb + TC_PART_BYTES) + (warp & 3) * 32;
+                    slot[lane] = sc;
+                    __syncwarp();
+#pragma unroll
+                    for (int i = 0; i < 8; ++i) {           // v[i] = K values 4i..4i+3 of row tid (tile_coord<false>)
+                        const float4 s4 = *reinterpret_cast<const float4*>(slot + 4 * i);
+                        v[i].x *= s4.x; v[i].y *= s4.y; v[i].z *= s4.z; v[i].w *= s4.w;
+                    }
+                    pack_operand_bf16(v);
+                    store_operand_bf16(stb + 2 * TC_PART_BYTES, tid, v);
+                    fence_proxy_async();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive(full_bar(stage));
+                };
+                float4 vb0[8], vb1[8];
+                float s0 = 0.f, s1 = 0.f;
+                int q = ((group - jbase) % GROUPS + GROUPS) % GROUPS;
+                if (q < total_q) fetch(q, vb0, s0);
+                while (q < total_q) {
+                    if (q + GROUPS < total_q) fetch(q + GROUPS, vb1, s1);
+                    commit(q, vb0, s0);
+                    q += GROUPS;
+                    if (q >= total_q) break;
+                    if (q + GROUPS < total_q) fetch(q + GROUPS, vb0, s0);
+                    commit(q, vb1, s1);
+                    q += GROUPS;
+                }
+                jbase += total_q;
+            }
+        }
+        if (APRE && !BF16) {
             // (batch == 1)  work items t = blockIdx.x, + gridDim.x, ...; jbase = K blocks of the earlier items, so that the
             // stage / phase bookkeeping runs on across items exactly like the MMA warp's
             int jbase = 0;
@@ -521,7 +624,15 @@ __global__ void __launch_bounds__(tc_threads(GROUPS), 1) gemm_tc_kernel(const Tc
                     mbar_wait(full_bar(stage), phase);
                     tc_fence_after();
                     const uint32_t sa = smem_u32(smem + size_t(stage) * TC_STAGE_BYTES);
-                    if (MNMAJ) {
+                    if constexpr (BF16) {
+                        const uint32_t sb = sa + 2 * TC_PART_BYTES;
+#pragma unroll
+                        for (int kk = 0; kk < TC_BK / 16; ++kk) {
+                            const uint32_t koff = kk * 2 * TC_PLANE_BYTES;   // two 16-byte K chunks (16 bf16) per MMA
+                            umma_bf16(d_tmem, make_desc(sa + koff), make_desc(sb + koff), TC_IDESC_BF16, accumulate);
+                            accumulate = 1u;
+                        }
+                    } else if (MNMAJ) {
                         const uint32_t a_hi = sa, a_lo = sa + TC_MN_PART_BYTES;
                         const uint32_t b_hi = sa + 2 * TC_MN_PART_BYTES, b_lo = sa + 3 * TC_MN_PART_BYTES;
 #pragma unroll
@@ -576,7 +687,9 @@ __global__ void __launch_bounds__(tc_threads(GROUPS), 1) gemm_tc_kernel(const Tc
 
     tc_fence_before();
     __syncthreads();
-    if (warp == TC_MMA_WARP) tmem_dealloc(tmem_base, TC_TMEM_COLS);
+    // (bf16: the base is read again rather than kept live through the producers' loop, where it would be spilled)
+    if (warp == TC_MMA_WARP)
+        tmem_dealloc(BF16 ? *reinterpret_cast<volatile uint32_t*>(tmem_slot) : tmem_base, TC_TMEM_COLS);
 }
 
 // ---- K <= 128 projections with a weight operand, row operand resident in TENSOR MEMORY ----------------------
@@ -592,38 +705,95 @@ constexpr int TA_BSTAGES = 5, TA_EPI_WARPS = 8, TA_THREADS = (10 + TA_EPI_WARPS)
 constexpr size_t TA_EPI_BYTES = size_t(TA_EPI_WARPS) * TC_EPI_WARP_FLOATS * 4;
 constexpr size_t TA_SMEM_BYTES = size_t(TA_BSTAGES) * TC_B_BLOB_BYTES + TA_EPI_BYTES + 768 + 256;
 constexpr uint32_t TA_COL_AHI = 256, TA_COL_ALO = 384;
+// BF16: the row tile is rounded to bf16 once and packed two values per TMEM column into [256, 320) -- 64 columns instead
+// of the 256 of the hi/lo pair -- and the bf16 weight blobs (a quarter of the bytes) stream through 12 stages of 8256 B
+// (20 stages measured no faster).
+// One kind::f16 MMA per 16 K values.  Four producer warps (one per TMEM lane quarter, the whole row each: 64 packed
+// registers) instead of eight, so that the CTA has 14 warps and every thread 128 registers: the epilogues then keep
+// their 64 per-row values and a 32-column accumulator slice in registers without spilling.  Accumulators, epilogues,
+// loader and MMA roles are those of the fp32 kernel.
+constexpr int TA_BSTAGES_BF16 = 12, TA_PRODUCER_WARPS_BF16 = 4;
+constexpr int ta_threads(bool bf16) { return ((bf16 ? TA_PRODUCER_WARPS_BF16 : TA_PRODUCER_WARPS) + 2 + TA_EPI_WARPS) * 32; }
+constexpr uint32_t TA_COL_A16 = 256;
+constexpr size_t TA_SMEM_BYTES_BF16 = size_t(TA_BSTAGES_BF16) * TC_BF16_BLOB_BYTES + TA_EPI_BYTES + 768 + 256;
+static_assert(8 * (6 + 2 * TA_BSTAGES_BF16) + 4 <= 256, "barriers and the TMEM slot fit their 256 bytes");
 
-template <int MODE>      // 0: store the tiles, 1: row-dot epilogue, 2: row-accumulate epilogue
-__global__ void __launch_bounds__(TA_THREADS, 1) gemm_tc_tmema_kernel(const TcArgs args) {
+template <int MODE, bool BF16 = false>      // MODE 0: store the tiles, 1: row-dot epilogue, 2: row-accumulate epilogue
+__global__ void __launch_bounds__(ta_threads(BF16), 1) gemm_tc_tmema_kernel(const TcArgs args) {
     constexpr bool ROWDOT = MODE == 1, ROWACC = MODE == 2;
+    constexpr int PRODUCERS = BF16 ? TA_PRODUCER_WARPS_BF16 : TA_PRODUCER_WARPS;
+    constexpr int LOADER = BF16 ? PRODUCERS : TA_LOADER_WARP, MMA = BF16 ? PRODUCERS + 1 : TA_MMA_WARP;
+    constexpr int BSTAGES = BF16 ? TA_BSTAGES_BF16 : TA_BSTAGES;
+    constexpr uint32_t BLOB = BF16 ? TC_BF16_BLOB_BYTES : TC_B_BLOB_BYTES;
+    static_assert(!BF16 || MODE != 0, "bf16 serves the row-dot and row-accumulate epilogues");
     extern __shared__ __align__(1024) uint8_t smem[];
-    uint8_t* b_stage = smem;                                           // [TA_BSTAGES][B_hi part, B_lo part]
-    float* epi_stage = reinterpret_cast<float*>(b_stage + size_t(TA_BSTAGES) * TC_B_BLOB_BYTES);
+    uint8_t* b_stage = smem;                                           // [BSTAGES][B_hi part, B_lo part] (bf16: [BSTAGES][B])
+    float* epi_stage = reinterpret_cast<float*>(b_stage + size_t(BSTAGES) * BLOB);
     uint64_t* bars = reinterpret_cast<uint64_t*>(reinterpret_cast<uint8_t*>(epi_stage) + TA_EPI_BYTES);
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 6 + 2 * TA_BSTAGES);
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 6 + 2 * BSTAGES);
     const uint32_t bar0 = smem_u32(bars);
     const uint32_t a_full = bar0, a_empty = bar0 + 8;
     auto tfull_bar = [&](int a) { return bar0 + 8u * (2 + a); };
     auto tempty_bar = [&](int a) { return bar0 + 8u * (4 + a); };
     auto b_full = [&](int s) { return bar0 + 8u * (6 + s); };
-    auto b_empty = [&](int s) { return bar0 + 8u * (6 + TA_BSTAGES + s); };
+    auto b_empty = [&](int s) { return bar0 + 8u * (6 + BSTAGES + s); };
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
     if (threadIdx.x == 0) {
-        mbar_init(a_full, TA_PRODUCER_WARPS);
+        mbar_init(a_full, PRODUCERS);
         mbar_init(a_empty, 1);
         for (int a = 0; a < 2; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), TA_EPI_WARPS); }
-        for (int i = 0; i < TA_BSTAGES; ++i) { mbar_init(b_full(i), 1); mbar_init(b_empty(i), 1); }
+        for (int i = 0; i < BSTAGES; ++i) { mbar_init(b_full(i), 1); mbar_init(b_empty(i), 1); }
         fence_barrier_init();
     }
-    if (warp == TA_MMA_WARP) tmem_alloc(smem_u32(tmem_slot), 512);
+    if (warp == MMA) tmem_alloc(smem_u32(tmem_slot), 512);
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     const int kblocks = args.kblocks, tiles_n = args.tiles_n, tiles_m = args.tiles_m;
 
-    if (warp < TA_PRODUCER_WARPS) {
+    if (BF16 && warp < PRODUCERS) {
+        // warp -> TMEM lane quarter, lane = row of the quarter; the row is loaded and packed (two bf16 per column) BEFORE
+        // the wait for the A region of tensor memory, as in the fp32 producers below
+        const int quarter = warp;
+        const bool a_vec = (args.lda % 4 == 0) && ((reinterpret_cast<uintptr_t>(args.A) & 15) == 0);
+        int it = 0;
+        for (int mi = blockIdx.x; mi < tiles_m; mi += gridDim.x, ++it) {
+            const int row = mi * TC_BM + quarter * 32 + lane;
+            const float* src = args.A + static_cast<size_t>(row) * args.lda;
+            uint32_t pk[64];
+#pragma unroll
+            for (int j = 0; j < 32; ++j) {
+                const int k = 4 * j;
+                float4 v;
+                if (row < args.M && a_vec && k + 4 <= args.K) {
+                    v = *reinterpret_cast<const float4*>(src + k);
+                } else {
+                    float t[4];
+#pragma unroll
+                    for (int e = 0; e < 4; ++e) t[e] = (row < args.M && k + e < args.K) ? src[k + e] : 0.f;
+                    v = make_float4(t[0], t[1], t[2], t[3]);
+                }
+                pk[2 * j] = pack_bf16x2(v.x, v.y);
+                pk[2 * j + 1] = pack_bf16x2(v.z, v.w);
+            }
+            mbar_wait(a_empty, (it & 1) ^ 1);            // the MMAs of the previous row tile have retired
+            tc_fence_after();
+#pragma unroll
+            for (int c = 0; c < 4; ++c) {                // 32 K values (16 columns) per tcgen05.st
+                if (c * 32 >= kblocks * TC_BK) break;
+                uint32_t part[16];
+#pragma unroll
+                for (int j = 0; j < 16; ++j) part[j] = pk[16 * c + j];
+                tmem_st16(tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + TA_COL_A16 + 16 * c, part);
+            }
+            asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(a_full);
+        }
+    } else if (warp < PRODUCERS) {
         // warp -> TMEM lane quarter (warp & 3) and K half (warp >> 2); lane = row of the quarter
         const int quarter = warp & 3, khalf = warp >> 2;
         const bool a_vec = (args.lda % 4 == 0) && ((reinterpret_cast<uintptr_t>(args.A) & 15) == 0);
@@ -677,21 +847,21 @@ __global__ void __launch_bounds__(TA_THREADS, 1) gemm_tc_tmema_kernel(const TcAr
             __syncwarp();
             if (lane == 0) mbar_arrive(a_full);
         }
-    } else if (warp == TA_LOADER_WARP) {
+    } else if (warp == LOADER) {
         if (lane == 0) {
             int q = 0;
             for (int mi = blockIdx.x; mi < tiles_m; mi += gridDim.x)
                 for (int n = 0; n < tiles_n; ++n)
                     for (int kb = 0; kb < kblocks; ++kb, ++q) {
-                        const int stage = q % TA_BSTAGES;
-                        mbar_wait(b_empty(stage), ((q / TA_BSTAGES) & 1) ^ 1);
-                        const uint8_t* blob = args.Bpre + (static_cast<size_t>(n) * kblocks + kb) * TC_B_BLOB_BYTES;
-                        mbar_arrive_expect_tx(b_full(stage), TC_B_BLOB_BYTES);
-                        bulk_copy_g2s(smem_u32(b_stage + size_t(stage) * TC_B_BLOB_BYTES), blob, TC_B_BLOB_BYTES, b_full(stage));
+                        const int stage = q % BSTAGES;
+                        mbar_wait(b_empty(stage), ((q / BSTAGES) & 1) ^ 1);
+                        const uint8_t* blob = args.Bpre + (static_cast<size_t>(n) * kblocks + kb) * BLOB;
+                        mbar_arrive_expect_tx(b_full(stage), BLOB);
+                        bulk_copy_g2s(smem_u32(b_stage + size_t(stage) * BLOB), blob, BLOB, b_full(stage));
                     }
         }
         __syncwarp();
-    } else if (warp == TA_MMA_WARP) {
+    } else if (warp == MMA) {
         if (lane == 0) {
             int q = 0, acc = 0, it = 0;
             uint32_t acc_phase = 0;
@@ -705,18 +875,29 @@ __global__ void __launch_bounds__(TA_THREADS, 1) gemm_tc_tmema_kernel(const TcAr
                     const uint32_t d_tmem = tmem_base + static_cast<uint32_t>(acc * TC_BN);
                     uint32_t accumulate = 0;
                     for (int kb = 0; kb < kblocks; ++kb, ++q) {
-                        const int stage = q % TA_BSTAGES;
-                        mbar_wait(b_full(stage), (q / TA_BSTAGES) & 1);
+                        const int stage = q % BSTAGES;
+                        mbar_wait(b_full(stage), (q / BSTAGES) & 1);
                         tc_fence_after();
-                        const uint32_t b_hi = smem_u32(b_stage + size_t(stage) * TC_B_BLOB_BYTES), b_lo = b_hi + TC_PART_BYTES;
+                        if constexpr (BF16) {
+                            const uint32_t b = smem_u32(b_stage + size_t(stage) * BLOB);
 #pragma unroll
-                        for (int kk = 0; kk < TC_BK / 8; ++kk) {
-                            const uint32_t koff = kk * 2 * TC_PLANE_BYTES;
-                            const uint32_t acol = static_cast<uint32_t>(kb * TC_BK + kk * 8);
-                            umma_tf32_ts(d_tmem, tmem_base + TA_COL_ALO + acol, make_desc(b_hi + koff), IDESC, accumulate);
-                            umma_tf32_ts(d_tmem, tmem_base + TA_COL_AHI + acol, make_desc(b_lo + koff), IDESC, 1u);
-                            umma_tf32_ts(d_tmem, tmem_base + TA_COL_AHI + acol, make_desc(b_hi + koff), IDESC, 1u);
-                            accumulate = 1u;
+                            for (int kk = 0; kk < TC_BK / 16; ++kk) {
+                                const uint32_t acol = static_cast<uint32_t>((kb * TC_BK + kk * 16) / 2);   // two bf16 a column
+                                umma_bf16_ts(d_tmem, tmem_base + TA_COL_A16 + acol, make_desc(b + kk * 2 * TC_PLANE_BYTES),
+                                             TC_IDESC_BF16, accumulate);
+                                accumulate = 1u;
+                            }
+                        } else {
+                            const uint32_t b_hi = smem_u32(b_stage + size_t(stage) * BLOB), b_lo = b_hi + TC_PART_BYTES;
+#pragma unroll
+                            for (int kk = 0; kk < TC_BK / 8; ++kk) {
+                                const uint32_t koff = kk * 2 * TC_PLANE_BYTES;
+                                const uint32_t acol = static_cast<uint32_t>(kb * TC_BK + kk * 8);
+                                umma_tf32_ts(d_tmem, tmem_base + TA_COL_ALO + acol, make_desc(b_hi + koff), IDESC, accumulate);
+                                umma_tf32_ts(d_tmem, tmem_base + TA_COL_AHI + acol, make_desc(b_lo + koff), IDESC, 1u);
+                                umma_tf32_ts(d_tmem, tmem_base + TA_COL_AHI + acol, make_desc(b_hi + koff), IDESC, 1u);
+                                accumulate = 1u;
+                            }
                         }
                         umma_commit(b_empty(stage));
                     }
@@ -728,7 +909,7 @@ __global__ void __launch_bounds__(TA_THREADS, 1) gemm_tc_tmema_kernel(const TcAr
         }
         __syncwarp();
     } else {
-        const int quarter = warp & 3, ew = warp - (TA_MMA_WARP + 1);
+        const int quarter = warp & 3, ew = warp - (MMA + 1);
         constexpr int CH = (TC_BN / 32) / (TA_EPI_WARPS / 4);
         float* stg = epi_stage + ew * TC_EPI_WARP_FLOATS;
         int acc = 0;
@@ -825,7 +1006,7 @@ __global__ void __launch_bounds__(TA_THREADS, 1) gemm_tc_tmema_kernel(const TcAr
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == TA_MMA_WARP) tmem_dealloc(tmem_base, 512);
+    if (warp == MMA) tmem_dealloc(tmem_base, 512);
 }
 
 // One blob per (128-column tile nt, 32-wide K block kb) of the N x K operand op(B)^T: exactly the B_hi / B_lo half of
@@ -857,6 +1038,37 @@ tc_presplit_b_kernel(const float* __restrict__ B, int ldb, int b_kcontig, int N,
 // bytes of the pre-split blob array of a [rows, <= 128] operand used as the short side of a weight-gradient GEMM
 size_t gemm_presplit_bytes(int rows) {
     return static_cast<size_t>(ceil_div(rows < 0 ? 0 : rows, TC_BK)) * TC_B_BLOB_BYTES;
+}
+
+// The bf16 counterpart of tc_presplit_b_kernel for an MN-contiguous source (W', W'' and h all are): one blob per
+// (128-row tile nt, 32-wide K block kb) of the N x K operand whose element (n, k) is src[k * ld + n], every value rounded
+// to bf16 (nearest even).  Lanes walk n, so the loads coalesce and each warp stores 512 contiguous bytes of a plane.
+__global__ void __launch_bounds__(256)
+tc_bf16_blobs_kernel(const float* __restrict__ src, int ld, int N, int K, int kblocks, uint8_t* __restrict__ blobs) {
+    const int blob = blockIdx.x, nt = blob / kblocks, kb = blob - nt * kblocks;
+    const int n0 = nt * TC_BN, k0 = kb * TC_BK;
+    uint8_t* dst = blobs + static_cast<size_t>(blob) * TC_BF16_BLOB_BYTES;
+    for (int idx = threadIdx.x; idx < TC_BN * (TC_BK / 8); idx += 256) {
+        const int r = idx & (TC_BN - 1), c = idx >> 7;
+        const int n = n0 + r, k = k0 + 8 * c;
+        float v[8];
+#pragma unroll
+        for (int e = 0; e < 8; ++e) v[e] = (n < N && k + e < K) ? src[static_cast<size_t>(k + e) * ld + n] : 0.f;
+        *reinterpret_cast<uint4*>(dst + c * TC_PLANE_BYTES + r * 16) =
+            make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
+    }
+}
+
+// bytes of the bf16 blobs of an N x K operand
+size_t gemm_bf16_blob_bytes(int N, int K) {
+    return static_cast<size_t>(ceil_div(N < 0 ? 0 : N, TC_BN)) * ceil_div(K < 0 ? 0 : K, TC_BK) * TC_BF16_BLOB_BYTES;
+}
+
+static int launch_bf16_blobs(const float* src, int ld, int N, int K, uint8_t* blobs, cudaStream_t st) {
+    const int kblocks = ceil_div(K, TC_BK);
+    tc_bf16_blobs_kernel<<<ceil_div(N, TC_BN) * kblocks, 256, 0, st>>>(src, ld, N, K, kblocks, blobs);
+    GCGCN_CHECK_LAUNCH("tc_bf16_blobs");
+    return GCGCN_OK;
 }
 
 int launch_splitk_reduce(const float* partial, int splits, int M, int N, float alpha, float beta, float* C,
@@ -1019,6 +1231,76 @@ int launch_gemm_rowop(int mode, int M, int N, int K, const float* A, int lda, co
     }
     timing_set_work(2.0 * M * N * K);
     GCGCN_CHECK_LAUNCH(mode == 1 ? "gemm_tc_rowdot<A in TMEM>" : "gemm_tc_rowacc<A in TMEM>");
+    return GCGCN_OK;
+}
+
+// launch_gemm_rowop on bf16-rounded operands (single-pass kind::f16): A is rounded as it enters tensor memory, B is
+// converted to bf16 blobs first (ws >= gemm_bf16_blob_bytes(N, K)).
+int launch_gemm_rowop_bf16(int mode, int M, int N, int K, const float* A, int lda, const float* B, int ldb, const float* T,
+                           float* out, long long ld, void* ws, size_t ws_bytes, cudaStream_t st) {
+    if (M <= 0 || N <= 0) return GCGCN_OK;
+    if (K < 1 || K > TA_KB * TC_BK || N % TC_BN != 0)
+        return fail(GCGCN_ERR_UNSUPPORTED, "gemm_rowop_bf16: needs 1 <= K <= %d and N a multiple of %d (K %d, N %d)",
+                    TA_KB * TC_BK, TC_BN, K, N);
+    TcArgs a;
+    a.M = M; a.N = N; a.K = K; a.lda = lda; a.ldb = ldb; a.ldc = 0;
+    a.A = A; a.B = B; a.bias = nullptr; a.C = nullptr; a.partial = nullptr; a.alpha = 1.f; a.beta = 0.f;
+    a.tiles_m = ceil_div(M, TC_BM); a.tiles_n = N / TC_BN; a.k_splits = 1; a.k_per_split = K;
+    a.kblocks = ceil_div(K, TC_BK); a.batch = 1; a.sA = a.sB = a.sC = 0; a.Apre = nullptr;
+    a.rd_t = T; a.rd_out = out; a.rd_ld = ld; a.bscale = nullptr; a.lds = 0; a.seq_k = 0;
+    if (ws == nullptr || gemm_bf16_blob_bytes(N, K) > ws_bytes || (reinterpret_cast<uintptr_t>(ws) & 15) != 0)
+        return fail(GCGCN_ERR_WORKSPACE, "gemm_rowop_bf16: workspace of %zu bytes needed for the bf16 weights",
+                    gemm_bf16_blob_bytes(N, K));
+    GCGCN_TRY(launch_bf16_blobs(B, ldb, N, K, static_cast<uint8_t*>(ws), st));
+    a.Bpre = static_cast<const uint8_t*>(ws);
+    const int grid = std::min(sm_count(), a.tiles_m);
+    if (mode == 1) {
+        static std::atomic<unsigned long long> prepared{0};
+        GCGCN_TRY(set_smem_once(prepared, gemm_tc_tmema_kernel<1, true>, TA_SMEM_BYTES_BF16, "gemm_tc_rowdot<bf16> smem"));
+        gemm_tc_tmema_kernel<1, true><<<grid, ta_threads(true), TA_SMEM_BYTES_BF16, st>>>(a);
+    } else {
+        static std::atomic<unsigned long long> prepared{0};
+        GCGCN_TRY(set_smem_once(prepared, gemm_tc_tmema_kernel<2, true>, TA_SMEM_BYTES_BF16, "gemm_tc_rowacc<bf16> smem"));
+        gemm_tc_tmema_kernel<2, true><<<grid, ta_threads(true), TA_SMEM_BYTES_BF16, st>>>(a);
+    }
+    timing_set_work(2.0 * M * N * K);
+    GCGCN_CHECK_LAUNCH(mode == 1 ? "gemm_tc_rowdot<bf16>" : "gemm_tc_rowacc<bf16>");
+    return GCGCN_OK;
+}
+
+// Weight gradient of the bilinear form on bf16-rounded operands, for any rows >= 1:
+//   C[a][r*128 + b] = beta C + sum_p bf16(h[p][a]) bf16(scale[p * lds + r] T[p][b])
+// h is converted to bf16 blobs (pre >= gemm_bf16_blob_bytes(128, rows)); the producers generate the other operand.  The
+// rows are walked in 4096-row ranges (no tensor-core accumulation runs longer); with more than one range every
+// (relation, range) item is a CTA's work item and the deterministic fp32 split-K reduction adds the partials
+// (ws >= ranges * 128 * relations*128 floats), with one range the epilogue applies beta itself.
+int launch_bilinear_wgrad_bf16(int relations, int rows, const float* h, const float* T, const float* scale, int lds,
+                               float beta, float* C, void* ws, size_t ws_bytes, void* pre, size_t pre_bytes,
+                               cudaStream_t st) {
+    if (rows <= 0 || relations <= 0) return GCGCN_OK;
+    const int N = relations * TC_BN, splits = ceil_div(rows, 4096);
+    const size_t part_bytes = splits > 1 ? static_cast<size_t>(splits) * TC_BM * N * sizeof(float) : 0;
+    if (pre == nullptr || gemm_bf16_blob_bytes(TC_BM, rows) > pre_bytes || (reinterpret_cast<uintptr_t>(pre) & 15) != 0 ||
+        part_bytes > ws_bytes || (part_bytes > 0 && (ws == nullptr || (reinterpret_cast<uintptr_t>(ws) & 15) != 0)))
+        return fail(GCGCN_ERR_WORKSPACE, "bilinear_wgrad_bf16: workspace too small");
+    TcArgs a;
+    a.M = TC_BM; a.N = N; a.K = rows; a.lda = TC_BM; a.ldb = TC_BN; a.ldc = N;
+    a.A = h; a.B = T; a.bias = nullptr; a.C = C; a.alpha = 1.f; a.beta = beta;
+    a.tiles_m = 1; a.tiles_n = relations; a.batch = 1; a.sA = a.sB = a.sC = 0;
+    a.rd_t = nullptr; a.rd_out = nullptr; a.rd_ld = 0; a.bscale = scale; a.lds = lds; a.seq_k = 0;
+    a.k_per_split = 4096; a.k_splits = splits;
+    a.partial = splits > 1 ? static_cast<float*>(ws) : nullptr;
+    a.kblocks = ceil_div(rows, TC_BK); a.Bpre = nullptr;
+    GCGCN_TRY(launch_bf16_blobs(h, TC_BM, TC_BM, rows, static_cast<uint8_t*>(pre), st));
+    a.Apre = static_cast<const uint8_t*>(pre);
+    const int grid = std::min(sm_count(), relations * splits);
+    static std::atomic<unsigned long long> prepared{0};
+    GCGCN_TRY(set_smem_once(prepared, gemm_tc_kernel<false, false, 2, false, true, false, true>, TC_SMEM_BYTES,
+                            "gemm_tc_wgrad<bf16> smem"));
+    gemm_tc_kernel<false, false, 2, false, true, false, true><<<grid, tc_threads(2), TC_SMEM_BYTES, st>>>(a);
+    timing_set_work(2.0 * TC_BM * N * rows);
+    GCGCN_CHECK_LAUNCH("gemm_tc_wgrad<bf16>");
+    if (splits > 1) GCGCN_TRY(launch_splitk_reduce(a.partial, splits, TC_BM, N, 1.f, beta, C, N, nullptr, st, 1, 0));
     return GCGCN_OK;
 }
 

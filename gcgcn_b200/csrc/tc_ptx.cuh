@@ -102,5 +102,33 @@ __device__ __forceinline__ void umma_tf32_ts(uint32_t d_tmem, uint32_t a_tmem, u
         "}" ::"r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
+// D[tmem] (+)= A[smem desc] * B[smem desc], 128 x 128 x 16 BF16 (kind::f16, fp32 accumulator)
+__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
+                                          uint32_t accumulate) {
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "setp.ne.b32 p, %4, 0;\n"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
+        "}" ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
+// D[tmem] (+)= A[tmem] * B[smem desc], 128 x 128 x 16 BF16; A holds two bf16 per 32-bit column (element k in the low half)
+__device__ __forceinline__ void umma_bf16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t idesc,
+                                             uint32_t accumulate) {
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "setp.ne.b32 p, %4, 0;\n"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n"
+        "}" ::"r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
+// bf16(lo) | bf16(hi) << 16, both rounded to nearest even (cvt.rn.bf16x2.f32 puts its first source in the high half)
+__device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
+    uint32_t r;
+    asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+    return r;
+}
 
 }  // namespace gcgcn

@@ -77,10 +77,14 @@ class GraphHead(nn.Module):
         return self
 
     def forward(self, context: torch.Tensor, hb: HeadBatch, edge_dtype=torch.float32, labels: Optional[torch.Tensor] = None,
-                cls_feat: Optional[torch.Tensor] = None):
+                cls_feat: Optional[torch.Tensor] = None, classifier_dtype=torch.float32):
         """context [total_tokens, 128] = ``context_output`` of every document back to back; cls_feat [num_docs, cls_dim]
-        = BERT's first-token feature of every document (BERT variant only, B:277).  Returns a dict with x0, e0, y1, e1,
-        y2, entity_feature_h / _t, logits [total_pairs, R] and, given labels, the per-document loss."""
+        = BERT's first-token feature of every document (BERT variant only, B:277).  ``classifier_dtype`` is the operand
+        type of the relation classifier's bilinear form (torch.float32 or torch.bfloat16, ``classifier.relation_logits``);
+        parameters and their gradients stay fp32.  Returns a dict with x0, e0, y1, e1, y2, entity_feature_h / _t,
+        logits [total_pairs, R] and, given labels, the per-document loss."""
+        if classifier_dtype not in (torch.float32, torch.bfloat16):
+            raise _lib.GcgcnError(f"GraphHead: classifier_dtype must be torch.float32 or torch.bfloat16, got {classifier_dtype}")
         if not context.is_cuda:
             raise _lib.GcgcnError("GraphHead: gcgcn_b200 runs on CUDA only (no CPU fallback)")
         bt, blocks, edge = hb.batch, self._blocks, self._edge
@@ -99,7 +103,8 @@ class GraphHead(nn.Module):
             if cls_feat is None:
                 raise _lib.GcgcnError("GraphHead(cls_dim=...) needs cls_feat [num_docs, cls_dim] (B:277)")
             cls_feature = LinearFn.apply(cls_feat, self.linear_cls.weight, self.linear_cls.bias)              # B:346
-        logits = relation_logits(fh, ft, self.bili_layer_01, self.classification_layer_01, cls_feature, bt)   # G:356-358
+        logits = relation_logits(fh, ft, self.bili_layer_01, self.classification_layer_01, cls_feature, bt,
+                                 dtype=classifier_dtype)                                               # G:356-358
         out = {"x0": x0, "e0": e0, "y1": y1, "e1": e1, "y2": y2, "a0": a0, "a1": a1, "entity_feature_h": fh,
                "entity_feature_t": ft, "logits": logits}
         if labels is not None:

@@ -427,6 +427,24 @@ size_t gcgcn_bilinear_bwd_ws_bytes(int32_t rows, int32_t relations);
 int gcgcn_bilinear_bwd(const float* h, const float* t, const float* Wm, const float* Wm2, const float* dout, int32_t rows,
                        int32_t relations, float beta, float* dh, float* dt, float* dWm, void* ws, size_t ws_bytes,
                        void* stream);
+/* The bilinear form on bf16-rounded operands: the same arguments, shapes, workspace rule and outputs as the two fp32
+ * entry points above, with the numerics of SURVEY.md section 8d config 3 (bf16 operands, fp32 accumulation).  bf16(x)
+ * is x rounded to the nearest bf16, ties to even (torch's .to(torch.bfloat16), cvt.rn.bf16x2.f32).  Every product of
+ * two bf16 values is exact in fp32, every sum is fp32, and h, t, W', dout and all outputs stay fp32 in memory:
+ *   out[p][r]   (+)= sum_b (sum_a bf16(h[p][a]) bf16(W'[a][r*128 + b])) t[p][b] + bias[r]     (t not rounded)
+ *   dt[p][b]     = sum_r dout[p][r] sum_a bf16(h[p][a]) bf16(W'[a][r*128 + b])                 (dout not rounded)
+ *   dh[p][a]     = sum_r dout[p][r] sum_b bf16(t[p][b]) bf16(W''[b][r*128 + a])
+ *   dWm[a][r*128 + b] = beta dWm + sum_p bf16(h[p][a]) bf16(dout[p][r] t[p][b])   (the fp32 product, rounded once)
+ * One tcgen05.mma.kind::f16 per 16 K values.  The backward takes any rows >= 0 (no chunked fallback, no minimum):
+ * rows = 0 returns at once and leaves dWm as it is.  The bias gradient is gcgcn_colsum of dout, as for fp32.            */
+size_t gcgcn_bilinear_bf16_ws_bytes(int32_t rows, int32_t relations);
+int gcgcn_bilinear_bf16_fwd(const float* h, const float* t, const float* Wm, const float* bias, int32_t rows,
+                            int32_t relations, int32_t accumulate, float* out, int32_t ldo, void* ws, size_t ws_bytes,
+                            void* stream);
+size_t gcgcn_bilinear_bf16_bwd_ws_bytes(int32_t rows, int32_t relations);
+int gcgcn_bilinear_bf16_bwd(const float* h, const float* t, const float* Wm, const float* Wm2, const float* dout,
+                            int32_t rows, int32_t relations, float beta, float* dh, float* dt, float* dWm, void* ws,
+                            size_t ws_bytes, void* stream);
 int gcgcn_bilinear_reduce_fwd(const float* Y, const float* t, const float* bias, int32_t rows, int32_t relations,
                               int32_t accumulate, float* out, int32_t ldo, void* stream);
 int gcgcn_bilinear_outer_bwd(const float* dout, int32_t ldd, const float* t, int32_t rows, int32_t relations, float* dY,

@@ -285,17 +285,20 @@ int launch_splitk_reduce(const float* partial, int splits, int M, int N, float a
     const bool vec = N % 4 == 0 && ldc % 4 == 0 && sC % 4 == 0 && (reinterpret_cast<uintptr_t>(C) & 15) == 0 &&
                      (reinterpret_cast<uintptr_t>(partial) & 15) == 0 &&
                      (bias == nullptr || (reinterpret_cast<uintptr_t>(bias) & 15) == 0);
+    // (each kernel under its own timer name, all three starting with "splitk_reduce")
     if (vec && splits >= 16 && total / 4 <= 64 * 1024) {
         dim3 grid(ceil_div(total / 4, 32), batch);
         splitk_reduce4_wide_kernel<<<grid, 256, 0, st>>>(partial, splits, M, N, alpha, beta, C, ldc, bias, sC);
+        GCGCN_CHECK_LAUNCH("splitk_reduce4_wide");
     } else if (vec) {
         dim3 grid(ceil_div(total / 4, 256), batch);
         splitk_reduce4_kernel<<<grid, 256, 0, st>>>(partial, splits, M, N, alpha, beta, C, ldc, bias, sC);
+        GCGCN_CHECK_LAUNCH("splitk_reduce4");
     } else {
         dim3 grid(ceil_div(total, 256), batch);
         splitk_reduce_kernel<<<grid, 256, 0, st>>>(partial, splits, M, N, alpha, beta, C, ldc, bias, sC);
+        GCGCN_CHECK_LAUNCH("splitk_reduce");
     }
-    GCGCN_CHECK_LAUNCH("splitk_reduce");
     return GCGCN_OK;
 }
 
@@ -385,7 +388,7 @@ int launch_colsum(const float* X, int M, int N, int ldx, float* out, void* ws, s
         if (ws == nullptr || ws_bytes < static_cast<size_t>(parts) * N * sizeof(float))
             return fail(GCGCN_ERR_WORKSPACE, "colsum: workspace too small");
         colsum128_partial_kernel<<<parts, 256, 0, st>>>(X, M, ldx, rows_per_block, static_cast<float*>(ws));
-        GCGCN_CHECK_LAUNCH("colsum_partial");
+        GCGCN_CHECK_LAUNCH("colsum128_partial");
         return launch_reduce_partials(static_cast<const float*>(ws), parts, N, out, N, nullptr, st);
     }
     int parts = max(1, min(ceil_div(M, 64), sm_count() * 16));

@@ -69,8 +69,9 @@ struct TcArgs {
     // (B a [K, 128] matrix shared by all column tiles) -- the Khatri-Rao factor of the bilinear weight gradient
     const float* bscale;
     int lds;
-    // seq_k != 0 (APRE path, partial == nullptr): the k_splits K ranges of a tile are walked by ONE CTA in order
-    // (grid = tiles), each accumulated in TMEM from zero and added into C by the epilogue (beta = 1 after the first).
+    // seq_k != 0 (partial == nullptr, batch == 1): the k_splits K ranges of a tile are walked by ONE CTA in order
+    // (grid = tiles), each accumulated in TMEM from zero and added into C by the epilogue (beta = 1 and no bias after
+    // the first).
     // Bounds the length of a single tensor-core accumulation: its fp32 adds truncate, and over tens of thousands of
     // K steps the bias reaches 1e-4 of the result.
     int seq_k;
@@ -238,6 +239,8 @@ __device__ __forceinline__ void tc_epilogue_tile(const TcArgs& args, uint32_t tm
     }
     const int rows_valid = min(32, args.M - row_base);      // may be <= 0 for padding tiles
     const bool final_out = args.partial == nullptr;
+    // (seq_k: the bias goes in with the first K range only, the later ones add their accumulator to C)
+    const float* bias_ptr = final_out && !(args.seq_k && ks > 0) ? args.bias : nullptr;
     const bool vec = (ldo % 4 == 0) && ((reinterpret_cast<uintptr_t>(out_base) & 15) == 0) && (n0 + TC_BN <= args.N);
 #pragma unroll 1
     for (int chunk = chunk0; chunk < chunk0 + chunks; ++chunk) {
@@ -262,7 +265,7 @@ __device__ __forceinline__ void tc_epilogue_tile(const TcArgs& args, uint32_t tm
             // lane -> (row = 4*it + lane/8, float4 column = lane%8): 4 rows x 128 contiguous bytes per store
             const int c4 = (lane & 7) * 4, col = n0 + chunk * 32 + c4;
             float4 bias4 = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (final_out && args.bias != nullptr) bias4 = *reinterpret_cast<const float4*>(args.bias + col);
+            if (bias_ptr != nullptr) bias4 = *reinterpret_cast<const float4*>(bias_ptr + col);
             // beta != 0: fetch the 8 old values first -- interleaved with the stores the compiler must keep
             // each load behind the previous store (possible aliasing) and the epilogue becomes a chain of
             // eight global round trips per 32-column chunk
@@ -297,7 +300,7 @@ __device__ __forceinline__ void tc_epilogue_tile(const TcArgs& args, uint32_t tm
         } else {
             const int col = n0 + chunk * 32 + lane;
             if (col < args.N) {
-                const float bias = (final_out && args.bias != nullptr) ? args.bias[col] : 0.f;
+                const float bias = bias_ptr != nullptr ? bias_ptr[col] : 0.f;
                 for (int rr = 0; rr < rows_valid; ++rr) {
                     float val = stg[rr * 32 + ((((lane >> 2) ^ (rr & 7)) << 2) | (lane & 3))];
                     float* p = out_base + static_cast<size_t>(row_base + rr) * ldo + col;
@@ -1135,6 +1138,15 @@ int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float
     const bool bpre = batch == 1 && splits == 1 && !seq && !ta && M >= 4096 &&
                       static_cast<size_t>(N) * K * sizeof(float) <= (size_t(8) << 20) && ws != nullptr &&
                       blob_total <= ws_bytes && (reinterpret_cast<uintptr_t>(ws) & 15) == 0;
+    // K > 4096 left unsplit (no workspace, or too small a one, for the partials) with at most one tile per CTA: the CTA
+    // walks K in 4096-row ranges like the generated operand above.  One tensor-core accumulation over all of a long K
+    // drifts: [119808 x 128]^T [119808 x 128] came out 8.6e-4 of max|C| off in one pass, 2.7e-5 walked (B200, 1000 W).
+    if (!seq && !bpre && batch == 1 && splits == 1 && K > 4096 && tiles <= sms) {
+        a.k_per_split = 4096;
+        a.k_splits = ceil_div(K, a.k_per_split);
+        a.seq_k = 1;
+        grid = tiles;
+    }
     if (bpre) {
         tc_presplit_b_kernel<<<dim3(a.tiles_n * a.kblocks, 4), 256, 0, st>>>(B, ldb, tb != 0, N, K, a.kblocks, static_cast<uint8_t*>(ws));
         GCGCN_CHECK_LAUNCH("gemm_presplit_b");

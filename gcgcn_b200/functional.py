@@ -535,16 +535,19 @@ class PairDenseFn(Function):
 
 def gemm(a: torch.Tensor, b: torch.Tensor, trans_a=False, trans_b=False, bias=None,
          out: Optional[torch.Tensor] = None, alpha=1.0, beta=0.0) -> torch.Tensor:
-    """Thin test hook over gcgcn_gemm (row-major fp32)."""
+    """Thin test hook over gcgcn_gemm (row-major fp32).  ``out`` may be a row-strided view (e.g. a column slice of a
+    wider buffer): it is written in place with its own row stride; its elements must be contiguous within a row."""
     a, b = _cuda(a, "A"), _cuda(b, "B")
     M = a.shape[1] if trans_a else a.shape[0]
     K = a.shape[0] if trans_a else a.shape[1]
     N = b.shape[0] if trans_b else b.shape[1]
     if out is None:      # beta == 0 overwrites every element: no fill needed
         out = torch.empty(M, N, device=a.device) if (beta == 0.0 and K > 0) else torch.zeros(M, N, device=a.device)
+    if out.stride(1) != 1:
+        raise _lib.GcgcnError(f"gemm: out needs unit column stride (strides {tuple(out.stride())})")
     ws = workspace(a.device, (24 << 20) + 4096)     # split-K partials / pre-split weight blobs
     _lib.call("gcgcn_gemm", int(trans_a), int(trans_b), M, N, K, float(alpha), _p(a), a.shape[1], _p(b),
-              b.shape[1], float(beta), _p(out), out.shape[1], _p(bias), ws.data_ptr(), ws.numel(),
+              b.shape[1], float(beta), _p(out), out.stride(0), _p(bias), ws.data_ptr(), ws.numel(),
               _stream(a.device))
     return out
 

@@ -600,7 +600,12 @@ int gcgcn_adam_step(float* params, const float* grads, float* exp_avg, float* ex
 /* ---- dense projection used by the entry points above (exported for tests) ----------------
  * C = alpha * op(A) op(B) + beta * C (+ bias broadcast over rows), row-major float32.
  * trans_a / trans_b: 0 = as stored, 1 = transposed.  K may be huge (weight gradients reduce
- * over every node row of the batch); the split-K partials live in ws.                      */
+ * over every node row of the batch); the split-K partials live in ws.
+ * Any lda, ldb, ldc (>= the row width) and any 4-byte aligned pointers; C outside its M x N
+ * window is never written.  beta = 0: C is not read (it may hold NaN).  K = 0: C = beta C + bias.
+ * M = 0 or N = 0: nothing is launched and C is left as it is.  ws may be NULL or short: the
+ * result stays within the same bound, only the route changes -- without room for split-K
+ * partials a long K is walked in 4096-row ranges inside one CTA per output tile.             */
 int gcgcn_gemm(int32_t trans_a, int32_t trans_b, int32_t M, int32_t N, int32_t K, float alpha,
                const float* A, int32_t lda, const float* B, int32_t ldb, float beta, float* C,
                int32_t ldc, const float* bias, void* ws, size_t ws_bytes, void* stream);

@@ -21,7 +21,9 @@ DEV = "cuda:0"
                                    # short M, K = "every node row": the MN-major weight-gradient variant (with ta=1, tb=0)
                                    (128, 1024, 20000), (100, 260, 9001), (256, 128, 8200),
                                    # K <= 128 with several column tiles: row operand resident in tensor memory
-                                   (4100, 300, 100), (8192, 1024, 64), (4097, 256, 128)])
+                                   (4100, 300, 100), (8192, 1024, 64), (4097, 256, 128),
+                                   # split K on the CUDA-core kernel (M*N*K < 2e6, K >= 2048), on the scalar reduce
+                                   (16, 16, 5000), (12, 13, 10000), (128, 130, 20000)])
 def test_gemm_against_fp64(ta, tb, M, N, K):
     g = torch.Generator().manual_seed(M * 7 + N * 3 + K)
     a = torch.randn((K, M) if ta else (M, K), generator=g)
@@ -33,6 +35,23 @@ def test_gemm_against_fp64(ta, tb, M, N, K):
     out = F.gemm(a.to(DEV), b.to(DEV), ta, tb, bias=bias.to(DEV), out=c0.clone().to(DEV), alpha=0.5, beta=2.0)
     scale = max(1.0, float(ref.abs().max()))
     assert maxdiff(out, ref) <= 2e-6 * scale * max(1, K) ** 0.5
+
+
+@pytest.mark.parametrize("M,N,K", [(37, 51, 77), (300, 130, 200), (128, 128, 40000)])
+def test_gemm_writes_a_row_strided_out_in_place(M, N, K):
+    """out = a column slice of a wider buffer: written with its own row stride, the other columns left bit-identical;
+    an out whose columns are not contiguous is refused."""
+    g = torch.Generator().manual_seed(M + N + K)
+    a, b = torch.randn(K, M, generator=g), torch.randn(K, N, generator=g)
+    wide = torch.randn(M, N + 9, generator=g).to(DEV)
+    before = wide.clone()
+    out = F.gemm(a.to(DEV), b.to(DEV), True, False, out=wide[:, 5:5 + N])
+    ref = a.double().t() @ b.double()
+    assert maxdiff(wide[:, 5:5 + N], ref) <= 2e-6 * float(ref.abs().max()) * K ** 0.5
+    assert out.data_ptr() == wide[:, 5:].data_ptr()
+    assert torch.equal(wide[:, :5], before[:, :5]) and torch.equal(wide[:, 5 + N:], before[:, 5 + N:])
+    with pytest.raises(_lib.GcgcnError, match="unit column stride"):
+        F.gemm(a.to(DEV), b.to(DEV), True, False, out=torch.zeros(N, M, device=DEV).t())
 
 
 def test_gemm_is_deterministic_with_split_k():

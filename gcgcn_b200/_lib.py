@@ -176,17 +176,11 @@ SIGNATURES = {
     "gcgcn_edge_fill_fwd": (c_int32, [_P, _P, _P, c_int32, c_int64, c_int32, _P, _P]),
     "gcgcn_edge_fill_bwd": (c_int32, [_P, _P, c_int32, c_int64, c_int32, _P, _P, _P, c_size_t, _P]),
     "gcgcn_colsum": (c_int32, [_P, c_int32, c_int32, c_int32, _P, _P, c_size_t, _P]),
-    "gcgcn_bilinear_ws_bytes": (c_size_t, [c_int32, c_int32]),
-    "gcgcn_bilinear_fwd": (c_int32, [_P, _P, _P, _P, c_int32, c_int32, c_int32, _P, c_int32, _P, c_size_t, _P]),
-    "gcgcn_bilinear_bwd_ws_bytes": (c_size_t, [c_int32, c_int32]),
-    "gcgcn_bilinear_bwd": (c_int32, [_P, _P, _P, _P, _P, c_int32, c_int32, c_float, _P, _P, _P, _P, c_size_t, _P]),
-    "gcgcn_bilinear_bf16_ws_bytes": (c_size_t, [c_int32, c_int32]),
-    "gcgcn_bilinear_bf16_fwd": (c_int32, [_P, _P, _P, _P, c_int32, c_int32, c_int32, _P, c_int32, _P, c_size_t, _P]),
-    "gcgcn_bilinear_bf16_bwd_ws_bytes": (c_size_t, [c_int32, c_int32]),
-    "gcgcn_bilinear_bf16_bwd": (c_int32, [_P, _P, _P, _P, _P, c_int32, c_int32, c_float, _P, _P, _P, _P, c_size_t, _P]),
-    "gcgcn_bilinear_reduce_fwd": (c_int32, [_P, _P, _P, c_int32, c_int32, c_int32, _P, c_int32, _P]),
-    "gcgcn_bilinear_outer_bwd": (c_int32, [_P, c_int32, _P, c_int32, c_int32, _P, _P]),
-    "gcgcn_bilinear_dt_bwd": (c_int32, [_P, c_int32, _P, c_int32, c_int32, _P, _P]),
+    "gcgcn_bilinear_ws_bytes": (c_size_t, [c_int32, c_int32, c_int32]),
+    "gcgcn_bilinear_fwd": (c_int32, [_P, _P, _P, _P, c_int32, c_int32, c_int32, c_int32, _P, c_int32, _P, c_size_t, _P]),
+    "gcgcn_bilinear_bwd_ws_bytes": (c_size_t, [c_int32, c_int32, c_int32]),
+    "gcgcn_bilinear_bwd": (c_int32, [_P, _P, _P, _P, _P, c_int32, c_int32, c_int32, c_float, _P, _P, _P, _P, c_size_t,
+                                     _P]),
     "gcgcn_doc_bias_fwd": (c_int32, [_BT, _P, c_int32, _P, _P]),
     "gcgcn_doc_bias_bwd": (c_int32, [_BT, _P, c_int32, _P, _P]),
     "gcgcn_pair_bce_fwd": (c_int32, [_BT, _P, _P, c_int32, _P, _P]),

@@ -4,10 +4,10 @@
 356-358) over every pair of a ragged batch, and the trainer's loss (config/Config.py:355-364).  ``h``, ``t`` are
 ``entity_feature_h`` / ``entity_feature_t`` ``[total_pairs, 128]`` (``modules.pair_dense``).  The bilinear form is the
 one dense n^2-scale contraction of the model (2 * 128 * 128 * 97 flop per pair): it runs on this package's tcgen05 GEMM
-(3xTF32) as ``Y = h W'`` with ``W'`` the ``[R, 128, 128]`` weight viewed as ``[128, R*128]``, then a row-wise reduction
-against ``t``; the pairs are walked in chunks so that ``Y`` (R*128 floats per pair) stays inside a fixed workspace.
-``relation_logits(..., dtype=torch.bfloat16)`` runs the bilinear form on bf16-rounded operands instead (``BilinearBf16Fn``:
-one ``kind::f16`` tensor-core pass, fp32 accumulation; parameters, inputs and gradients stay fp32).  No CPU path.
+with ``W'`` the ``[R, 128, 128]`` weight viewed as ``[128, R*128]``, in fp32 (3xTF32) or, with
+``relation_logits(..., dtype=torch.bfloat16)``, on bf16-rounded operands (one ``kind::f16`` tensor-core pass, fp32
+accumulation; parameters, inputs and gradients stay fp32).  ``h W'`` is contracted with ``t`` in the GEMM's epilogue and
+never stored.  No CPU path.
 """
 from __future__ import annotations
 
@@ -17,13 +17,10 @@ from torch.autograd import Function
 
 from . import _lib
 from .batch import RaggedBatch
-from .functional import D, LinearFn, _cuda, _p, _stream, gemm, workspace
+from .functional import D, LinearFn, _cuda, _p, _stream, workspace
 
-CHUNK_PAIRS = 8192          # 8192 pairs x 97 x 128 floats = 407 MB of Y per chunk
-FUSED_BACKWARD = True       # False: the backward materialises Y / dY chunk by chunk (test hook; also the path below 8192 pairs)
-FUSED_MIN_PAIRS = 8192      # the generated-operand weight-gradient GEMM needs K >= 8192
-FUSED_CHUNK_PAIRS = 1 << 18  # pairs per fused backward call (workspace: 1 KB of pre-split h + 1.6 KB of split-K partials per pair)
-FUSED_FORWARD = True        # False: the forward materialises Y = h W' chunk by chunk like the backward does (test hook)
+FUSED_CHUNK_PAIRS = 1 << 18  # pairs per backward call (workspace: 1 KB of pre-split h + 1.6 KB of split-K partials per pair)
+DTYPES = {torch.float32: _lib.F32, torch.bfloat16: _lib.BF16}
 
 
 def _wmat(W: torch.Tensor) -> torch.Tensor:
@@ -33,111 +30,50 @@ def _wmat(W: torch.Tensor) -> torch.Tensor:
 
 
 class BilinearFn(Function):
-    """out[p, r] = sum_{a,b} h[p,a] W[r,a,b] t[p,b] + bias[r]   (torch.nn.Bilinear, G:275, 358)."""
+    """out[p, r] = sum_{a,b} h[p,a] W[r,a,b] t[p,b] + bias[r]   (torch.nn.Bilinear, G:275, 358), with the operand type
+    ``dtype`` (torch.float32 or torch.bfloat16; include/gcgcn_b200.h, gcgcn_bilinear_fwd, gives both numerics).  h, t, W,
+    bias and every gradient are fp32.  The forward is one call; the backward makes host calls of at most
+    FUSED_CHUNK_PAIRS pairs that accumulate dW' through beta = 1."""
 
     @staticmethod
-    def forward(ctx, h, t, W, bias):
+    def forward(ctx, h, t, W, bias, dtype):
         h, t, W, bias = _cuda(h, "h"), _cuda(t, "t"), _cuda(W, "weight"), _cuda(bias, "bias")
-        P, R, dev = h.shape[0], W.shape[0], h.device
-        if W.shape[1:] != (D, D) or h.shape[1] != D or t.shape != h.shape:
-            raise _lib.GcgcnError(f"bilinear: expected h, t [P, {D}] and weight [R, {D}, {D}]")
-        Wm = _wmat(W)
-        out = torch.empty(P, R, device=dev)
-        if FUSED_FORWARD and P > 0:
-            # one tensor-core pass: the accumulator tiles of h W' are contracted with t in the GEMM's epilogue
-            ws = workspace(dev, int(_lib.load().gcgcn_bilinear_ws_bytes(P, R)))
-            _lib.call("gcgcn_bilinear_fwd", _p(h), _p(t), _p(Wm), _p(bias), P, R, 0, _p(out), R, ws.data_ptr(), ws.numel(),
-                      _stream(dev))
-        else:
-            for p0 in range(0, P, CHUNK_PAIRS):
-                p1 = min(P, p0 + CHUNK_PAIRS)
-                Y = gemm(h[p0:p1], Wm)
-                _lib.call("gcgcn_bilinear_reduce_fwd", _p(Y), _p(t[p0:p1]), _p(bias), p1 - p0, R, 0, _p(out[p0:p1]), R,
-                          _stream(dev))
-                del Y
-        ctx.save_for_backward(h, t, Wm)
-        ctx.R = R
-        return out
-
-    @staticmethod
-    def backward(ctx, dout):
-        h, t, Wm = ctx.saved_tensors
-        R, dev, P = ctx.R, h.device, h.shape[0]
-        dout = _cuda(dout, "dout")
-        dh, dt = torch.empty_like(h), torch.empty_like(t)
-        dWm = torch.zeros_like(Wm)
-        p_done = 0
-        if FUSED_BACKWARD and P >= FUSED_MIN_PAIRS:
-            # three tensor-core passes per chunk, nothing of size [pairs, R*128] is ever stored: dt and dh through the
-            # row-accumulate epilogue, dW' with its Khatri-Rao operand generated in the GEMM's producers
-            Wm2 = Wm.view(D, R, D).permute(2, 1, 0).reshape(D, R * D).contiguous()       # W viewed as [b][(r, a)]
-            lib = _lib.load()
-            while P - p_done >= FUSED_MIN_PAIRS:
-                p1 = P if P - p_done <= FUSED_CHUNK_PAIRS + FUSED_MIN_PAIRS else p_done + FUSED_CHUNK_PAIRS
-                rows = p1 - p_done
-                ws = workspace(dev, int(lib.gcgcn_bilinear_bwd_ws_bytes(rows, R)))
-                _lib.call("gcgcn_bilinear_bwd", _p(h[p_done:p1]), _p(t[p_done:p1]), _p(Wm), _p(Wm2), _p(dout[p_done:p1]), rows,
-                          R, 1.0, _p(dh[p_done:p1]), _p(dt[p_done:p1]), _p(dWm), ws.data_ptr(), ws.numel(), _stream(dev))
-                p_done = p1
-        for p0 in range(p_done, P, CHUNK_PAIRS):
-            p1 = min(P, p0 + CHUNK_PAIRS)
-            rows = p1 - p0
-            Y = gemm(h[p0:p1], Wm)                                               # recomputed, not saved
-            _lib.call("gcgcn_bilinear_dt_bwd", _p(dout[p0:p1]), R, _p(Y), rows, R, _p(dt[p0:p1]), _stream(dev))
-            dY = Y                                                               # same storage
-            _lib.call("gcgcn_bilinear_outer_bwd", _p(dout[p0:p1]), R, _p(t[p0:p1]), rows, R, _p(dY), _stream(dev))
-            gemm(dY, Wm, trans_b=True, out=dh[p0:p1])                            # dh = dY W'^T
-            gemm(h[p0:p1], dY, trans_a=True, out=dWm, beta=1.0)                  # dW' += h^T dY
-            del Y, dY
-        dbias = torch.empty(R, device=dev)
-        ws = workspace(dev, 8 << 20)
-        _lib.call("gcgcn_colsum", _p(dout), P, R, R, _p(dbias), ws.data_ptr(), ws.numel(), _stream(dev))
-        dW = dWm.view(D, R, D).permute(1, 0, 2).contiguous()
-        return dh, dt, dW, dbias
-
-
-class BilinearBf16Fn(Function):
-    """The bilinear form with bf16 operands and fp32 accumulation (include/gcgcn_b200.h, gcgcn_bilinear_bf16_fwd):
-    out[p, r] = sum_b (sum_a bf16(h[p,a]) bf16(W[r,a,b])) t[p,b] + bias[r].  h, t, W, bias and every gradient are fp32;
-    dW[r,a,b] = sum_p bf16(h[p,a]) bf16(dout[p,r] t[p,b]).  The fused kernels take any number of pairs: the backward makes
-    host calls of at most FUSED_CHUNK_PAIRS pairs that accumulate dW' through beta = 1, and has no chunked path."""
-
-    @staticmethod
-    def forward(ctx, h, t, W, bias):
-        h, t, W, bias = _cuda(h, "h"), _cuda(t, "t"), _cuda(W, "weight"), _cuda(bias, "bias")
-        P, R, dev = h.shape[0], W.shape[0], h.device
+        P, R, dev, code = h.shape[0], W.shape[0], h.device, DTYPES[dtype]
         if W.shape[1:] != (D, D) or h.shape[1] != D or t.shape != h.shape:
             raise _lib.GcgcnError(f"bilinear: expected h, t [P, {D}] and weight [R, {D}, {D}]")
         Wm = _wmat(W)
         out = torch.empty(P, R, device=dev)
         if P > 0:
-            ws = workspace(dev, int(_lib.load().gcgcn_bilinear_bf16_ws_bytes(P, R)))
-            _lib.call("gcgcn_bilinear_bf16_fwd", _p(h), _p(t), _p(Wm), _p(bias), P, R, 0, _p(out), R, ws.data_ptr(),
+            # one tensor-core pass: the accumulator tiles of h W' are contracted with t in the GEMM's epilogue
+            ws = workspace(dev, int(_lib.load().gcgcn_bilinear_ws_bytes(P, R, code)))
+            _lib.call("gcgcn_bilinear_fwd", _p(h), _p(t), _p(Wm), _p(bias), P, R, code, 0, _p(out), R, ws.data_ptr(),
                       ws.numel(), _stream(dev))
         ctx.save_for_backward(h, t, Wm)
-        ctx.R = R
+        ctx.R, ctx.code = R, code
         return out
 
     @staticmethod
     def backward(ctx, dout):
         h, t, Wm = ctx.saved_tensors
-        R, dev, P = ctx.R, h.device, h.shape[0]
+        R, code, dev, P = ctx.R, ctx.code, h.device, h.shape[0]
         dout = _cuda(dout, "dout")
         dh, dt = torch.empty_like(h), torch.empty_like(t)
         dWm = torch.zeros_like(Wm)
+        # three tensor-core passes per call, nothing of size [pairs, R*128] is ever stored: dt and dh through the
+        # row-accumulate epilogue, dW' with its Khatri-Rao operand generated in the GEMM's producers
         Wm2 = Wm.view(D, R, D).permute(2, 1, 0).reshape(D, R * D).contiguous()       # W viewed as [b][(r, a)]
         lib = _lib.load()
         for p0 in range(0, P, FUSED_CHUNK_PAIRS):
             p1 = min(P, p0 + FUSED_CHUNK_PAIRS)
             rows = p1 - p0
-            ws = workspace(dev, int(lib.gcgcn_bilinear_bf16_bwd_ws_bytes(rows, R)))
-            _lib.call("gcgcn_bilinear_bf16_bwd", _p(h[p0:p1]), _p(t[p0:p1]), _p(Wm), _p(Wm2), _p(dout[p0:p1]), rows, R,
+            ws = workspace(dev, int(lib.gcgcn_bilinear_bwd_ws_bytes(rows, R, code)))
+            _lib.call("gcgcn_bilinear_bwd", _p(h[p0:p1]), _p(t[p0:p1]), _p(Wm), _p(Wm2), _p(dout[p0:p1]), rows, R, code,
                       1.0, _p(dh[p0:p1]), _p(dt[p0:p1]), _p(dWm), ws.data_ptr(), ws.numel(), _stream(dev))
         dbias = torch.empty(R, device=dev)
         ws = workspace(dev, 8 << 20)
         _lib.call("gcgcn_colsum", _p(dout), P, R, R, _p(dbias), ws.data_ptr(), ws.numel(), _stream(dev))
         dW = dWm.view(D, R, D).permute(1, 0, 2).contiguous()
-        return dh, dt, dW, dbias
+        return dh, dt, dW, dbias, None
 
 
 class PairBceFn(Function):
@@ -190,13 +126,12 @@ def relation_logits(h: torch.Tensor, t: torch.Tensor, bili: nn.Bilinear, cls: nn
     """G:356-358: ``bili(h, t) + cls(cat[h, t])`` without forming the concatenation (the linear layer is split by
     input columns into its h and t halves).  ``cls_feature`` [num_docs, R] (with ``batch``) adds the BERT variant's
     per-document term, B:346-347.  ``dtype`` is the operand type of the bilinear form: torch.float32 (3xTF32, fp32
-    parity) or torch.bfloat16 (BilinearBf16Fn); the linear layer, the logits and every gradient are fp32 either way."""
-    if dtype not in (torch.float32, torch.bfloat16):
+    parity) or torch.bfloat16; the linear layer, the logits and every gradient are fp32 either way."""
+    if dtype not in DTYPES:
         raise _lib.GcgcnError(f"relation_logits: dtype must be torch.float32 or torch.bfloat16, got {dtype}")
     w = cls.weight
     lin = LinearFn.apply(h, w[:, :D], cls.bias) + LinearFn.apply(t, w[:, D:], None)
-    bilinear = BilinearBf16Fn if dtype == torch.bfloat16 else BilinearFn
-    z = bilinear.apply(h, t, bili.weight, bili.bias) + lin
+    z = BilinearFn.apply(h, t, bili.weight, bili.bias, dtype) + lin
     return z if cls_feature is None else DocBiasFn.apply(z, cls_feature, batch)
 
 

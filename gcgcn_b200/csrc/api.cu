@@ -97,23 +97,13 @@ int edge_colsum_parts(long long total_pairs);
 int launch_edge_fill_bwd(const void* de, const void* pair_idx, int pairs, long long total_pairs, int dtype, float* drows,
                          float* dbias, float* partial, cudaStream_t st);
 
-int launch_bilinear_reduce(const float* Y, const float* t, const float* bias, int rows, int R, int accumulate, float* out,
-                           int ldo, cudaStream_t st);
 int launch_bilinear_finish(const float* part, long long ld, const float* bias, int rows, int R, int accumulate, float* out,
                            int ldo, cudaStream_t st);
-int launch_gemm_rowop(int mode, int M, int N, int K, const float* A, int lda, const float* B, int ldb, const float* T,
-                      float* out, long long ld, void* ws, size_t ws_bytes, cudaStream_t st);
-int launch_gemm_wgrad_scaled(int M, int tiles, int K, const float* A, int lda, const float* T, const float* scale, int lds,
-                             float beta, float* C, int ldc, void* ws, size_t ws_bytes, cudaStream_t st, void* pre_ws,
-                             size_t pre_bytes);
+int launch_gemm_rowop(int mode, bool bf16, int M, int N, int K, const float* A, int lda, const float* B, int ldb,
+                      const float* T, float* out, long long ld, void* ws, size_t ws_bytes, cudaStream_t st);
 size_t gemm_bf16_blob_bytes(int N, int K);
-int launch_gemm_rowop_bf16(int mode, int M, int N, int K, const float* A, int lda, const float* B, int ldb, const float* T,
-                           float* out, long long ld, void* ws, size_t ws_bytes, cudaStream_t st);
-int launch_bilinear_wgrad_bf16(int relations, int rows, const float* h, const float* T, const float* scale, int lds,
-                               float beta, float* C, void* ws, size_t ws_bytes, void* pre, size_t pre_bytes,
-                               cudaStream_t st);
-int launch_bilinear_outer(const float* dout, int ldd, const float* t, int rows, int R, float* dY, cudaStream_t st);
-int launch_bilinear_dt(const float* dout, int ldd, const float* Y, int rows, int R, float* dt, cudaStream_t st);
+int launch_bilinear_wgrad(bool bf16, int relations, int rows, const float* h, const float* T, const float* scale, int lds,
+                          float beta, float* C, void* ws, size_t ws_bytes, void* pre, size_t pre_bytes, cudaStream_t st);
 int launch_doc_bias_fwd(const gcgcn_batch* bt, const float* v, int R, float* z, cudaStream_t st);
 int launch_doc_bias_bwd(const gcgcn_batch* bt, const float* dz, int R, float* dv, cudaStream_t st);
 int launch_pair_bce_fwd(const gcgcn_batch* bt, const float* z, const float* y, int R, float* loss, cudaStream_t st);
@@ -1107,164 +1097,80 @@ int gcgcn_colsum(const float* X, int32_t M, int32_t N, int32_t ldx, float* out, 
 }
 
 // ---- relation classifier and loss (SURVEY.md 8f row 2) -----------------------------------------------------
-int gcgcn_bilinear_reduce_fwd(const float* Y, const float* t, const float* bias, int32_t rows, int32_t relations,
-                              int32_t accumulate, float* out, int32_t ldo, void* stream) {
-    GCGCN_API_ENTER(stream);
-    GCGCN_REQUIRE(rows >= 0 && relations >= 0 && ldo >= relations, "bilinear_reduce: bad shape");
-    if (rows == 0 || relations == 0) return GCGCN_OK;
-    GCGCN_TRY(check_device_ptr(Y, "Y"));
-    GCGCN_TRY(check_device_ptr(t, "t"));
-    GCGCN_TRY(check_device_ptr(out, "out"));
-    return launch_bilinear_reduce(Y, t, bias, rows, relations, accumulate, out, ldo, static_cast<cudaStream_t>(stream));
+// bytes of the blobs of an N x K operand of the bilinear form's GEMMs (W': N = relations*128, K = 128; h: N = 128, K = rows)
+static size_t bilinear_blob_bytes(int32_t dtype, int N, int K) {
+    if (dtype == GCGCN_BF16) return gemm_bf16_blob_bytes(N, K);
+    return static_cast<size_t>(ceil_div(N, D)) * gemm_presplit_bytes(K);
 }
-size_t gcgcn_bilinear_ws_bytes(int32_t rows, int32_t relations) {
-    const size_t r = static_cast<size_t>(relations < 0 ? 0 : relations), m = static_cast<size_t>(rows < 0 ? 0 : rows);
-    const size_t ld = (m + 31) & ~size_t(31);
-    return align256(r * 4 * 33024) + align256(2 * r * ld * sizeof(float)) + 4096;      // pre-split W' blobs + partials
+
+size_t gcgcn_bilinear_ws_bytes(int32_t rows, int32_t relations, int32_t dtype) {
+    const int r = relations < 0 ? 0 : relations;
+    const size_t m = static_cast<size_t>(rows < 0 ? 0 : rows), ld = (m + 31) & ~size_t(31);
+    // W' blobs, the two column halves' partial sums per (relation, pair)
+    return align256(bilinear_blob_bytes(dtype, r * D, D)) + align256(2 * static_cast<size_t>(r) * ld * sizeof(float)) + 4096;
 }
 
 int gcgcn_bilinear_fwd(const float* h, const float* t, const float* Wm, const float* bias, int32_t rows,
-                       int32_t relations, int32_t accumulate, float* out, int32_t ldo, void* ws, size_t ws_bytes,
-                       void* stream) {
+                       int32_t relations, int32_t dtype, int32_t accumulate, float* out, int32_t ldo, void* ws,
+                       size_t ws_bytes, void* stream) {
     GCGCN_API_ENTER(stream);
+    GCGCN_REQUIRE(dtype == GCGCN_F32 || dtype == GCGCN_BF16, "bilinear_fwd: dtype %d is neither GCGCN_F32 nor GCGCN_BF16",
+                  dtype);
     GCGCN_REQUIRE(rows >= 0 && relations >= 0 && ldo >= relations, "bilinear_fwd: bad shape");
     if (rows == 0 || relations == 0) return GCGCN_OK;
     GCGCN_TRY(check_device_ptr(h, "h"));
     GCGCN_TRY(check_device_ptr(t, "t"));
     GCGCN_TRY(check_device_ptr(Wm, "Wm"));
     GCGCN_TRY(check_device_ptr(out, "out"));
-    const size_t need = gcgcn_bilinear_ws_bytes(rows, relations);
+    const size_t need = gcgcn_bilinear_ws_bytes(rows, relations, dtype);
     if (ws == nullptr || ws_bytes < need)
         return fail(GCGCN_ERR_WORKSPACE, "bilinear_fwd: workspace of %zu bytes needed, got %zu", need, ws_bytes);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     Arena ar(ws, ws_bytes);
-    const size_t ld = (static_cast<size_t>(rows) + 31) & ~size_t(31);
-    uint8_t* blobs = ar.take<uint8_t>(static_cast<size_t>(relations) * 4 * 33024);
+    const size_t ld = (static_cast<size_t>(rows) + 31) & ~size_t(31), blob_bytes = bilinear_blob_bytes(dtype, relations * D, D);
+    uint8_t* blobs = ar.take<uint8_t>(blob_bytes);
     float* part = ar.take<float>(2 * static_cast<size_t>(relations) * ld);
-    GCGCN_TRY(launch_gemm_rowop(1, rows, relations * D, D, h, D, Wm, relations * D, t, part, static_cast<long long>(ld), blobs,
-                                static_cast<size_t>(relations) * 4 * 33024, st));
+    GCGCN_TRY(launch_gemm_rowop(1, dtype == GCGCN_BF16, rows, relations * D, D, h, D, Wm, relations * D, t, part,
+                                static_cast<long long>(ld), blobs, blob_bytes, st));
     return launch_bilinear_finish(part, static_cast<long long>(ld), bias, rows, relations, accumulate, out, ldo, st);
 }
 
-size_t gcgcn_bilinear_bwd_ws_bytes(int32_t rows, int32_t relations) {
-    const size_t r = static_cast<size_t>(relations < 0 ? 0 : relations);
-    // pre-split W' blobs, one [128, relations*128] partial per 4096-row range of the weight-gradient GEMM, pre-split h
-    const size_t ranges = (static_cast<size_t>(rows < 0 ? 0 : rows) + 4095) / 4096;
-    return align256(r * 4 * 33024) + align256(std::max<size_t>(GEMM_WS_BYTES, ranges * D * r * D * sizeof(float))) +
-           align256(gemm_presplit_bytes(rows < 0 ? 0 : rows)) + 4096;
+size_t gcgcn_bilinear_bwd_ws_bytes(int32_t rows, int32_t relations, int32_t dtype) {
+    const int r = relations < 0 ? 0 : relations, m = rows < 0 ? 0 : rows;
+    // W' (then W'') blobs, one [128, relations*128] partial per 4096-row range when there are several, h's blobs
+    const size_t ranges = (static_cast<size_t>(m) + 4095) / 4096;
+    return align256(bilinear_blob_bytes(dtype, r * D, D)) + align256(ranges > 1 ? ranges * D * r * D * sizeof(float) : 0) +
+           align256(bilinear_blob_bytes(dtype, D, m)) + 4096;
 }
 
 int gcgcn_bilinear_bwd(const float* h, const float* t, const float* Wm, const float* Wm2, const float* dout, int32_t rows,
-                       int32_t relations, float beta, float* dh, float* dt, float* dWm, void* ws, size_t ws_bytes,
-                       void* stream) {
+                       int32_t relations, int32_t dtype, float beta, float* dh, float* dt, float* dWm, void* ws,
+                       size_t ws_bytes, void* stream) {
     GCGCN_API_ENTER(stream);
+    GCGCN_REQUIRE(dtype == GCGCN_F32 || dtype == GCGCN_BF16, "bilinear_bwd: dtype %d is neither GCGCN_F32 nor GCGCN_BF16",
+                  dtype);
     GCGCN_REQUIRE(rows >= 0 && relations >= 1, "bilinear_bwd: bad shape");
-    if (rows < 8192)
-        return fail(GCGCN_ERR_UNSUPPORTED, "bilinear_bwd: the fused backward needs >= 8192 rows (got %d); use "
-                    "gcgcn_bilinear_outer_bwd / gcgcn_bilinear_dt_bwd with gcgcn_gemm", rows);
+    if (rows == 0) return GCGCN_OK;
     const void* ps[] = {h, t, Wm, Wm2, dout, dh, dt, dWm};
     for (const void* p : ps) GCGCN_TRY(check_device_ptr(p, "bilinear_bwd operand"));
-    const size_t need = gcgcn_bilinear_bwd_ws_bytes(rows, relations);
+    const size_t need = gcgcn_bilinear_bwd_ws_bytes(rows, relations, dtype);
     if (ws == nullptr || ws_bytes < need)
         return fail(GCGCN_ERR_WORKSPACE, "bilinear_bwd: workspace of %zu bytes needed, got %zu", need, ws_bytes);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     Arena ar(ws, ws_bytes);
-    const size_t blob_bytes = static_cast<size_t>(relations) * 4 * 33024, pre_bytes = gemm_presplit_bytes(rows);
-    const size_t ranges = (static_cast<size_t>(rows) + 4095) / 4096;
-    const size_t gws_bytes = std::max<size_t>(GEMM_WS_BYTES, ranges * D * static_cast<size_t>(relations) * D * sizeof(float));
-    uint8_t* blobs = ar.take<uint8_t>(blob_bytes);
-    uint8_t* gws = ar.take<uint8_t>(gws_bytes);
-    uint8_t* pre = ar.take<uint8_t>(pre_bytes);
+    const bool bf16 = dtype == GCGCN_BF16;
     const int N = relations * D;
-    GCGCN_TRY(launch_gemm_rowop(2, rows, N, D, h, D, Wm, N, dout, dt, relations, blobs, blob_bytes, st));
-    GCGCN_TRY(launch_gemm_rowop(2, rows, N, D, t, D, Wm2, N, dout, dh, relations, blobs, blob_bytes, st));
-    return launch_gemm_wgrad_scaled(D, relations, rows, h, D, t, dout, relations, beta, dWm, N, gws, gws_bytes, st, pre,
-                                    pre_bytes);
-}
-
-// ---- the bilinear form on bf16-rounded operands (single-pass kind::f16, fp32 accumulation) ----
-size_t gcgcn_bilinear_bf16_ws_bytes(int32_t rows, int32_t relations) {
-    const int r = relations < 0 ? 0 : relations;
-    const size_t m = static_cast<size_t>(rows < 0 ? 0 : rows), ld = (m + 31) & ~size_t(31);
-    return align256(gemm_bf16_blob_bytes(r * D, D)) + align256(2 * static_cast<size_t>(r) * ld * sizeof(float)) + 4096;
-}
-
-int gcgcn_bilinear_bf16_fwd(const float* h, const float* t, const float* Wm, const float* bias, int32_t rows,
-                            int32_t relations, int32_t accumulate, float* out, int32_t ldo, void* ws, size_t ws_bytes,
-                            void* stream) {
-    GCGCN_API_ENTER(stream);
-    GCGCN_REQUIRE(rows >= 0 && relations >= 0 && ldo >= relations, "bilinear_bf16_fwd: bad shape");
-    if (rows == 0 || relations == 0) return GCGCN_OK;
-    GCGCN_TRY(check_device_ptr(h, "h"));
-    GCGCN_TRY(check_device_ptr(t, "t"));
-    GCGCN_TRY(check_device_ptr(Wm, "Wm"));
-    GCGCN_TRY(check_device_ptr(out, "out"));
-    const size_t need = gcgcn_bilinear_bf16_ws_bytes(rows, relations);
-    if (ws == nullptr || ws_bytes < need)
-        return fail(GCGCN_ERR_WORKSPACE, "bilinear_bf16_fwd: workspace of %zu bytes needed, got %zu", need, ws_bytes);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    Arena ar(ws, ws_bytes);
-    const size_t ld = (static_cast<size_t>(rows) + 31) & ~size_t(31), blob_bytes = gemm_bf16_blob_bytes(relations * D, D);
-    uint8_t* blobs = ar.take<uint8_t>(blob_bytes);
-    float* part = ar.take<float>(2 * static_cast<size_t>(relations) * ld);
-    GCGCN_TRY(launch_gemm_rowop_bf16(1, rows, relations * D, D, h, D, Wm, relations * D, t, part, static_cast<long long>(ld),
-                                     blobs, blob_bytes, st));
-    return launch_bilinear_finish(part, static_cast<long long>(ld), bias, rows, relations, accumulate, out, ldo, st);
-}
-
-size_t gcgcn_bilinear_bf16_bwd_ws_bytes(int32_t rows, int32_t relations) {
-    const int r = relations < 0 ? 0 : relations, m = rows < 0 ? 0 : rows;
-    // bf16 W' (then W'') blobs, one [128, relations*128] partial per 4096-row range when there are several, bf16 h blobs
-    const size_t ranges = (static_cast<size_t>(m) + 4095) / 4096;
-    return align256(gemm_bf16_blob_bytes(r * D, D)) + align256(ranges > 1 ? ranges * D * r * D * sizeof(float) : 0) +
-           align256(gemm_bf16_blob_bytes(D, m)) + 4096;
-}
-
-int gcgcn_bilinear_bf16_bwd(const float* h, const float* t, const float* Wm, const float* Wm2, const float* dout,
-                            int32_t rows, int32_t relations, float beta, float* dh, float* dt, float* dWm, void* ws,
-                            size_t ws_bytes, void* stream) {
-    GCGCN_API_ENTER(stream);
-    GCGCN_REQUIRE(rows >= 0 && relations >= 1, "bilinear_bf16_bwd: bad shape");
-    if (rows == 0) return GCGCN_OK;
-    const void* ps[] = {h, t, Wm, Wm2, dout, dh, dt, dWm};
-    for (const void* p : ps) GCGCN_TRY(check_device_ptr(p, "bilinear_bf16_bwd operand"));
-    const size_t need = gcgcn_bilinear_bf16_bwd_ws_bytes(rows, relations);
-    if (ws == nullptr || ws_bytes < need)
-        return fail(GCGCN_ERR_WORKSPACE, "bilinear_bf16_bwd: workspace of %zu bytes needed, got %zu", need, ws_bytes);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    Arena ar(ws, ws_bytes);
-    const int N = relations * D;
-    const size_t blob_bytes = gemm_bf16_blob_bytes(N, D), pre_bytes = gemm_bf16_blob_bytes(D, rows);
+    const size_t blob_bytes = bilinear_blob_bytes(dtype, N, D), pre_bytes = bilinear_blob_bytes(dtype, D, rows);
     const size_t ranges = (static_cast<size_t>(rows) + 4095) / 4096;
     const size_t part_bytes = ranges > 1 ? ranges * D * static_cast<size_t>(N) * sizeof(float) : 0;
     uint8_t* blobs = ar.take<uint8_t>(blob_bytes);
     uint8_t* part = ar.take<uint8_t>(part_bytes);
     uint8_t* pre = ar.take<uint8_t>(pre_bytes);
-    GCGCN_TRY(launch_gemm_rowop_bf16(2, rows, N, D, h, D, Wm, N, dout, dt, relations, blobs, blob_bytes, st));
-    GCGCN_TRY(launch_gemm_rowop_bf16(2, rows, N, D, t, D, Wm2, N, dout, dh, relations, blobs, blob_bytes, st));
-    return launch_bilinear_wgrad_bf16(relations, rows, h, t, dout, relations, beta, dWm, part, part_bytes, pre, pre_bytes, st);
+    GCGCN_TRY(launch_gemm_rowop(2, bf16, rows, N, D, h, D, Wm, N, dout, dt, relations, blobs, blob_bytes, st));
+    GCGCN_TRY(launch_gemm_rowop(2, bf16, rows, N, D, t, D, Wm2, N, dout, dh, relations, blobs, blob_bytes, st));
+    return launch_bilinear_wgrad(bf16, relations, rows, h, t, dout, relations, beta, dWm, part, part_bytes, pre, pre_bytes, st);
 }
 
-int gcgcn_bilinear_outer_bwd(const float* dout, int32_t ldd, const float* t, int32_t rows, int32_t relations, float* dY,
-                             void* stream) {
-    GCGCN_API_ENTER(stream);
-    GCGCN_REQUIRE(rows >= 0 && relations >= 0 && ldd >= relations, "bilinear_outer: bad shape");
-    if (rows == 0 || relations == 0) return GCGCN_OK;
-    GCGCN_TRY(check_device_ptr(dout, "dout"));
-    GCGCN_TRY(check_device_ptr(t, "t"));
-    GCGCN_TRY(check_device_ptr(dY, "dY"));
-    return launch_bilinear_outer(dout, ldd, t, rows, relations, dY, static_cast<cudaStream_t>(stream));
-}
-int gcgcn_bilinear_dt_bwd(const float* dout, int32_t ldd, const float* Y, int32_t rows, int32_t relations, float* dt,
-                          void* stream) {
-    GCGCN_API_ENTER(stream);
-    GCGCN_REQUIRE(rows >= 0 && relations >= 0 && ldd >= relations, "bilinear_dt: bad shape");
-    if (rows == 0 || relations == 0) return GCGCN_OK;
-    GCGCN_TRY(check_device_ptr(dout, "dout"));
-    GCGCN_TRY(check_device_ptr(Y, "Y"));
-    GCGCN_TRY(check_device_ptr(dt, "dt"));
-    return launch_bilinear_dt(dout, ldd, Y, rows, relations, dt, static_cast<cudaStream_t>(stream));
-}
 int gcgcn_doc_bias_fwd(const gcgcn_batch* bt, const float* v, int32_t relations, float* z, void* stream) {
     GCGCN_API_ENTER(stream);
     GCGCN_TRY(check_batch(bt));

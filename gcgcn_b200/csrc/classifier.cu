@@ -2,78 +2,16 @@
 // products of  logits = Bilinear(128, 128, R)(h, t) + Linear(256, R)(cat[h, t])  (G:275-276, 356-358)  and the
 // trainer's loss (config/Config.py:355-364).
 //
-// The bilinear form  out[p, r] = sum_{a,b} h[p,a] W[r,a,b] t[p,b]  is run as the one genuinely dense n^2-scale
-// contraction of the model on the tcgen05 GEMM:  Y = h W'  with W' = W viewed as [128, R*128]  (gcgcn_gemm, 3xTF32),
-// followed by the row-wise reduction against t below; the backward is two more GEMMs (dh = dY W'^T, dW' = h^T dY with
-// dY[p, r*128 + b] = dout[p, r] t[p, b]) and the reduction dt[p, b] = sum_r dout[p, r] Y[p, r*128 + b].  The caller
-// (gcgcn_b200/classifier.py) walks the pairs in chunks so that Y never exceeds a fixed workspace.
+// The bilinear form  out[p, r] = sum_{a,b} h[p,a] W[r,a,b] t[p,b]  is the one genuinely dense n^2-scale contraction of
+// the model.  It runs on the tensor-memory GEMM of gemm_tc.cu (launch_gemm_rowop, launch_bilinear_wgrad) in fp32
+// (3xTF32) or on bf16 operands, with W' = W viewed as [128, R*128]: the forward contracts each accumulator tile of h W'
+// with t in the GEMM's epilogue, and the backward forms dh and dt the same way and generates the weight gradient's
+// [pairs, R*128] operand from t and dout in the GEMM's producers, so that no [pairs, R*128] intermediate is ever stored.
+// This file holds the kernels around them: the final transpose of the forward's partial sums, the per-document bias
+// and the loss.
 #include "common.cuh"
 
 namespace gcgcn {
-
-__device__ __forceinline__ float4 cl_ld4(const float* p) { return *reinterpret_cast<const float4*>(p); }
-
-// out[p][r] (+)= sum_b Y[p][r*128 + b] t[p][b] (+ bias[r]);  one warp per pair, lane = 4 columns
-__global__ void __launch_bounds__(256)
-bilinear_reduce_kernel(const float* __restrict__ Y, const float* __restrict__ t, const float* __restrict__ bias, int rows,
-                       int R, int accumulate, float* __restrict__ out, int ldo) {
-    const int lane = threadIdx.x & 31;
-    const int p = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (p >= rows) return;
-    const float4 tv = cl_ld4(t + static_cast<size_t>(p) * D + 4 * lane);
-    const float* y = Y + static_cast<size_t>(p) * R * D + 4 * lane;
-    float* o = out + static_cast<size_t>(p) * ldo;
-    for (int r0 = 0; r0 < R; r0 += 32) {
-        float mine = 0.f;
-        const int rn = min(32, R - r0);
-        for (int k = 0; k < rn; ++k) {
-            const float4 v = Vec4<float>::load(y + static_cast<size_t>(r0 + k) * D);
-            const float s = warp_sum(v.x * tv.x + v.y * tv.y + v.z * tv.z + v.w * tv.w);
-            if (lane == k) mine = s;
-        }
-        if (lane < rn) {
-            const int r = r0 + lane;
-            float v = mine + (bias != nullptr ? bias[r] : 0.f);
-            if (accumulate) v += o[r];
-            o[r] = v;
-        }
-    }
-}
-
-// dY[p][r*128 + b] = dout[p][r] t[p][b]
-__global__ void __launch_bounds__(256)
-bilinear_outer_kernel(const float* __restrict__ dout, int ldd, const float* __restrict__ t, int rows, int R,
-                      float* __restrict__ dY) {
-    const int lane = threadIdx.x & 31;
-    const int p = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (p >= rows) return;
-    const float4 tv = cl_ld4(t + static_cast<size_t>(p) * D + 4 * lane);
-    const float* d = dout + static_cast<size_t>(p) * ldd;
-    float* y = dY + static_cast<size_t>(p) * R * D + 4 * lane;
-    for (int r = 0; r < R; ++r) {
-        const float s = d[r];
-        Vec4<float>::store(y + static_cast<size_t>(r) * D, make_float4(s * tv.x, s * tv.y, s * tv.z, s * tv.w));
-    }
-}
-
-// dt[p][b] = sum_r dout[p][r] Y[p][r*128 + b]
-__global__ void __launch_bounds__(256)
-bilinear_dt_kernel(const float* __restrict__ dout, int ldd, const float* __restrict__ Y, int rows, int R,
-                   float* __restrict__ dt) {
-    const int lane = threadIdx.x & 31;
-    const int p = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (p >= rows) return;
-    const float* d = dout + static_cast<size_t>(p) * ldd;
-    const float* y = Y + static_cast<size_t>(p) * R * D + 4 * lane;
-    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll 4
-    for (int r = 0; r < R; ++r) {
-        const float s = d[r];
-        const float4 v = Vec4<float>::load(y + static_cast<size_t>(r) * D);
-        acc.x += s * v.x; acc.y += s * v.y; acc.z += s * v.z; acc.w += s * v.w;
-    }
-    *reinterpret_cast<float4*>(dt + static_cast<size_t>(p) * D + 4 * lane) = acc;
-}
 
 // ---- the trainer's loss (C:355-364): per document, mean over the ordered pairs i != j of BCELoss(sigmoid(z), y) ----
 // torch's arithmetic: p = sigmoid(z); bce = (y - 1) max(log1p(-p), -100) - y max(log(p), -100)   (ATen Loss.cpp)
@@ -212,25 +150,6 @@ int launch_bilinear_finish(const float* part, long long ld, const float* bias, i
     return GCGCN_OK;
 }
 
-int launch_bilinear_reduce(const float* Y, const float* t, const float* bias, int rows, int R, int accumulate, float* out,
-                           int ldo, cudaStream_t st) {
-    if (rows <= 0 || R <= 0) return GCGCN_OK;
-    bilinear_reduce_kernel<<<cl_grid(rows), 256, 0, st>>>(Y, t, bias, rows, R, accumulate, out, ldo);
-    GCGCN_CHECK_LAUNCH("bilinear_reduce");
-    return GCGCN_OK;
-}
-int launch_bilinear_outer(const float* dout, int ldd, const float* t, int rows, int R, float* dY, cudaStream_t st) {
-    if (rows <= 0 || R <= 0) return GCGCN_OK;
-    bilinear_outer_kernel<<<cl_grid(rows), 256, 0, st>>>(dout, ldd, t, rows, R, dY);
-    GCGCN_CHECK_LAUNCH("bilinear_outer");
-    return GCGCN_OK;
-}
-int launch_bilinear_dt(const float* dout, int ldd, const float* Y, int rows, int R, float* dt, cudaStream_t st) {
-    if (rows <= 0 || R <= 0) return GCGCN_OK;
-    bilinear_dt_kernel<<<cl_grid(rows), 256, 0, st>>>(dout, ldd, Y, rows, R, dt);
-    GCGCN_CHECK_LAUNCH("bilinear_dt");
-    return GCGCN_OK;
-}
 int launch_pair_bce_fwd(const gcgcn_batch* bt, const float* z, const float* y, int R, float* loss, cudaStream_t st) {
     if (bt->num_docs <= 0) return GCGCN_OK;
     pair_bce_fwd_kernel<<<bt->num_docs, 256, 0, st>>>(bt->node_ptr, reinterpret_cast<const long long*>(bt->pair_ptr), z, y,

@@ -304,8 +304,7 @@ int launch_splitk_reduce(const float* partial, int splits, int M, int N, float a
 
 int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float* A, int lda, const float* B,
                    int ldb, float beta, float* C, int ldc, const float* bias, void* ws, size_t ws_bytes,
-                   cudaStream_t st, int* taken, int batch, long long sA, long long sB, long long sC, void* pre_ws,
-                   size_t pre_bytes, const float* bscale = nullptr, int lds = 0);
+                   cudaStream_t st, int* taken, int batch, long long sA, long long sB, long long sC);
 
 int launch_gemm(int ta, int tb, int M, int N, int K, float alpha, const float* A, int lda,
                 const float* B, int ldb, float beta, float* C, int ldc, const float* bias, void* ws,
@@ -314,7 +313,7 @@ int launch_gemm(int ta, int tb, int M, int N, int K, float alpha, const float* A
     if (K < 0) return fail(GCGCN_ERR_INVALID_ARG, "gemm: K < 0");
     int taken = 0;
     GCGCN_TRY(launch_gemm_tc(ta, tb, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, bias, ws, ws_bytes, st, &taken,
-                             1, 0, 0, 0, nullptr, 0));
+                             1, 0, 0, 0));
     if (taken) return GCGCN_OK;
     const int tiles = ceil_div(M, GM) * ceil_div(N, GN);
     int splits = 1;
@@ -349,19 +348,6 @@ int launch_gemm(int ta, int tb, int M, int N, int K, float alpha, const float* A
     return GCGCN_OK;
 }
 
-// C[M, tiles * 128] (+)= A^T [M, K] x KR, column tile nt of KR being  scale[k][nt] * T[k][0..127]  (T a [K, 128] matrix):
-// the weight gradient of a bilinear form, dW'[a][(r, b)] = sum_p h[p][a] dout[p][r] t[p][b], without materialising the
-// [K, tiles * 128] operand.  Tensor-core path only (K >= 8192, M <= 256): GCGCN_ERR_UNSUPPORTED otherwise.
-int launch_gemm_wgrad_scaled(int M, int tiles, int K, const float* A, int lda, const float* T, const float* scale, int lds,
-                             float beta, float* C, int ldc, void* ws, size_t ws_bytes, cudaStream_t st, void* pre_ws,
-                             size_t pre_bytes) {
-    int taken = 0;
-    GCGCN_TRY(launch_gemm_tc(1, 0, M, tiles * 128, K, 1.f, A, lda, T, 128, beta, C, ldc, nullptr, ws, ws_bytes, st, &taken, 1, 0,
-                             0, 0, pre_ws, pre_bytes, scale, lds));
-    if (!taken) return fail(GCGCN_ERR_UNSUPPORTED, "gemm_wgrad_scaled: shape not covered by the tensor-core path");
-    return GCGCN_OK;
-}
-
 // `batch` independent products with the same shapes and strided operands (the per-head dense-connect
 // weight gradients): one tensor-core launch when possible, else a loop over the single-product path
 int launch_gemm_batched(int ta, int tb, int M, int N, int K, float alpha, const float* A, int lda, const float* B,
@@ -370,7 +356,7 @@ int launch_gemm_batched(int ta, int tb, int M, int N, int K, float alpha, const 
     if (M <= 0 || N <= 0 || batch <= 0) return GCGCN_OK;
     int taken = 0;
     GCGCN_TRY(launch_gemm_tc(ta, tb, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, nullptr, ws, ws_bytes, st, &taken,
-                             batch, sA, sB, sC, nullptr, 0));
+                             batch, sA, sB, sC));
     if (taken) return GCGCN_OK;
     for (int b = 0; b < batch; ++b)
         GCGCN_TRY(launch_gemm(ta, tb, M, N, K, alpha, A + b * sA, lda, B + b * sB, ldb, beta, C + b * sC, ldc, nullptr,

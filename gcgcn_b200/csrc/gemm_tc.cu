@@ -1080,8 +1080,7 @@ int launch_splitk_reduce(const float* partial, int splits, int M, int N, float a
 // returns 1 if the launch was taken by the tensor-core path, 0 if the caller should use the SIMT kernel
 int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float* A, int lda, const float* B,
                    int ldb, float beta, float* C, int ldc, const float* bias, void* ws, size_t ws_bytes,
-                   cudaStream_t st, int* taken, int batch, long long sA, long long sB, long long sC, void* pre_ws,
-                   size_t pre_bytes, const float* bscale, int lds) {
+                   cudaStream_t st, int* taken, int batch, long long sA, long long sB, long long sC) {
     *taken = 0;
     if (K < 1 || batch < 1) return GCGCN_OK;
     if (static_cast<double>(M) * N * K * batch < 2.0e6) return GCGCN_OK;   // tiny: not worth a 128x128 tile
@@ -1091,7 +1090,8 @@ int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float
     a.tiles_m = ceil_div(M, TC_BM);
     a.tiles_n = ceil_div(N, TC_BN);
     a.batch = batch; a.sA = sA; a.sB = sB; a.sC = sC;
-    a.rd_t = nullptr; a.rd_out = nullptr; a.rd_ld = 0; a.bscale = bscale; a.lds = lds; a.seq_k = 0;
+    a.rd_t = nullptr; a.rd_out = nullptr; a.rd_ld = 0; a.bscale = nullptr; a.lds = 0; a.seq_k = 0;
+    a.Apre = nullptr;
     const int tiles = a.tiles_m * a.tiles_n * batch;
     const int sms = sm_count();
     int splits = 1;
@@ -1112,36 +1112,17 @@ int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float
     }
     a.k_splits = splits;
     int grid = std::min(sms, tiles * splits);
-    // generated-operand weight gradient (K = every pair of the batch): one CTA per tile walks the K ranges in order and
-    // adds each range's accumulator into C, so that no single tensor-core accumulation is longer than 4096 rows
-    const bool seq = bscale != nullptr;
-    if (seq) {
-        a.k_per_split = 4096;
-        a.k_splits = splits = ceil_div(K, a.k_per_split);
-        const size_t per = static_cast<size_t>(M) * N * sizeof(float);
-        if (splits > 1 && ws != nullptr && per * splits <= ws_bytes && (reinterpret_cast<uintptr_t>(ws) & 15) == 0) {
-            // room for one partial per range: plain split-K over the ranges, every CTA takes (tile, range) items
-            // round-robin (all SMs busy), the fp32 reduction adds them up
-            a.partial = static_cast<float*>(ws);
-            a.seq_k = 0;
-            grid = std::min(sms, tiles * splits);
-        } else {
-            a.partial = nullptr;
-            a.seq_k = splits > 1 ? 1 : 0;
-            grid = std::min(sms, tiles);
-        }
-    }
     a.Bpre = nullptr;
     a.kblocks = ceil_div(K, TC_BK);
     // weight-like B operand (small, reused by every 128-row tile of a tall A): pre-split it once per call
     const size_t blob_total = static_cast<size_t>(a.tiles_n) * a.kblocks * TC_B_BLOB_BYTES;
-    const bool bpre = batch == 1 && splits == 1 && !seq && !ta && M >= 4096 &&
+    const bool bpre = batch == 1 && splits == 1 && !ta && M >= 4096 &&
                       static_cast<size_t>(N) * K * sizeof(float) <= (size_t(8) << 20) && ws != nullptr &&
                       blob_total <= ws_bytes && (reinterpret_cast<uintptr_t>(ws) & 15) == 0;
     // K > 4096 left unsplit (no workspace, or too small a one, for the partials) with at most one tile per CTA: the CTA
-    // walks K in 4096-row ranges like the generated operand above.  One tensor-core accumulation over all of a long K
-    // drifts: [119808 x 128]^T [119808 x 128] came out 8.6e-4 of max|C| off in one pass, 2.7e-5 walked (B200, 1000 W).
-    if (!seq && !bpre && batch == 1 && splits == 1 && K > 4096 && tiles <= sms) {
+    // walks K in 4096-row ranges, adding each range's accumulator into C.  One tensor-core accumulation over all of a long
+    // K drifts: [119808 x 128]^T [119808 x 128] came out 8.6e-4 of max|C| off in one pass, 2.7e-5 walked (B200, 1000 W).
+    if (!bpre && batch == 1 && splits == 1 && K > 4096 && tiles <= sms) {
         a.k_per_split = 4096;
         a.k_splits = ceil_div(K, a.k_per_split);
         a.seq_k = 1;
@@ -1151,24 +1132,6 @@ int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float
         tc_presplit_b_kernel<<<dim3(a.tiles_n * a.kblocks, 4), 256, 0, st>>>(B, ldb, tb != 0, N, K, a.kblocks, static_cast<uint8_t*>(ws));
         GCGCN_CHECK_LAUNCH("gemm_presplit_b");
         a.Bpre = static_cast<const uint8_t*>(ws);
-    }
-    // generated-operand weight gradient: the short [rows, <= 256] operand (A, transposed) is pre-split into blobs that
-    // every column tile re-uses.  The other weight gradients run MN-major: blobs only pay for themselves where the
-    // wide operand has to be generated (measured on [119808 x 128]^T [119808 x N]: N = 256: 95 us with blobs, 66 us
-    // MN-major; N = 1024: 230 us against 216 us).
-    a.Apre = nullptr;
-    const size_t ablob_total = static_cast<size_t>(a.tiles_m) * a.kblocks * TC_B_BLOB_BYTES;
-    const bool apre = bscale != nullptr && !bpre && batch == 1 && ta && !tb && K >= 8192 && M <= 2 * TC_BM &&
-                      (seq ? (a.partial != nullptr || tiles <= sms) : tiles * splits <= sms) &&
-                      pre_ws != nullptr && ablob_total <= pre_bytes && (reinterpret_cast<uintptr_t>(pre_ws) & 15) == 0;
-    if (bscale != nullptr && !apre)
-        return fail(GCGCN_ERR_UNSUPPORTED, "gemm: the generated-operand product needs the pre-split weight-gradient path "
-                    "(A transposed, K >= 8192, M <= 256, a pre-split workspace)");
-    if (apre) {
-        tc_presplit_b_kernel<<<dim3(a.tiles_m * a.kblocks, 4), 256, 0, st>>>(A, lda, /*kcontig=*/0, M, K, a.kblocks,
-                                                                  static_cast<uint8_t*>(pre_ws));
-        GCGCN_CHECK_LAUNCH("gemm_presplit_a");
-        a.Apre = static_cast<const uint8_t*>(pre_ws);
     }
     // op(A)[m,k]: stored [M][K] (K contiguous) when !ta, [K][M] when ta.
     // op(B)[k,n] as the N x K operand: stored [N][K] (K contiguous) when tb, [K][N] when !tb.
@@ -1186,8 +1149,7 @@ int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float
         static std::atomic<unsigned long long> prepared{0};
         GCGCN_TRY(set_smem_once(prepared, gemm_tc_tmema_kernel<0>, TA_SMEM_BYTES, "gemm_tc_tmema smem"));
         gemm_tc_tmema_kernel<0><<<std::min(sms, a.tiles_m), TA_THREADS, TA_SMEM_BYTES, st>>>(a);
-    } else if (apre) GCGCN_TC_LAUNCH(false, false, 2, false, true);
-    else if (bpre) GCGCN_TC_LAUNCH(true, true, 3, true);
+    } else if (bpre) GCGCN_TC_LAUNCH(true, true, 3, true);
     else if (a_kc && b_kc) GCGCN_TC_LAUNCH(true, true, 3, false);
     else if (a_kc && !b_kc) GCGCN_TC_LAUNCH(true, false, 3, false);
     else if (!a_kc && b_kc) GCGCN_TC_LAUNCH(false, true, 3, false);
@@ -1197,24 +1159,24 @@ int launch_gemm_tc(int ta, int tb, int M, int N, int K, float alpha, const float
 #undef GCGCN_TC_LAUNCH
     timing_set_work(2.0 * M * N * K * batch);
     GCGCN_CHECK_LAUNCH(tmema ? "gemm_tc_nn<A in TMEM>"
-                             : apre ? "gemm_tc_tn<presplit A>"
                              : bpre ? (tb ? "gemm_tc_nt<presplit B>" : "gemm_tc_nn<presplit B>")
                              : ta ? (tb ? "gemm_tc_tt" : "gemm_tc_tn<MN-major>") : (tb ? "gemm_tc_nt" : "gemm_tc_nn"));
-    if (splits > 1 && a.partial != nullptr)
-        GCGCN_TRY(launch_splitk_reduce(a.partial, splits, M, N, alpha, beta, C, ldc, bias, st, batch, sC));
+    if (splits > 1) GCGCN_TRY(launch_splitk_reduce(a.partial, splits, M, N, alpha, beta, C, ldc, bias, st, batch, sC));
     *taken = 1;
     return GCGCN_OK;
 }
 
 // Row-dot / row-accumulate GEMMs over a [M, K <= 128] row operand that stays resident in tensor memory per row tile
-// (split hi/lo) while B [K, N] (N a multiple of 128) streams through shared memory as pre-split blobs; the accumulator
-// tiles are consumed from TMEM and never stored:
+// while B [K, N] (N a multiple of 128) streams through shared memory as blobs; the accumulator tiles are consumed from
+// TMEM and never stored:
 //   mode 1  part[(nt * 2 + half) * ld + m] = sum_{c in half of tile nt} (A B)[m][128 nt + c] T[m][c]
 //           -- the bilinear form out[p, r] = sum_b (h W')[p, r*128 + b] t[p, b]
 //   mode 2  out[m][c] = sum_nt T[m * ld + nt] (A B)[m][128 nt + c]
 //           -- its input gradients, dt[p, b] = sum_r dout[p, r] (h W')[p, r*128 + b]
-int launch_gemm_rowop(int mode, int M, int N, int K, const float* A, int lda, const float* B, int ldb, const float* T,
-                      float* out, long long ld, void* ws, size_t ws_bytes, cudaStream_t st) {
+// fp32 (3xTF32): A is split hi/lo, B is pre-split (ws >= gemm_presplit_bytes(K) per column tile).  bf16 (single-pass
+// kind::f16): A is rounded as it enters tensor memory, B is converted to bf16 blobs (ws >= gemm_bf16_blob_bytes(N, K)).
+int launch_gemm_rowop(int mode, bool bf16, int M, int N, int K, const float* A, int lda, const float* B, int ldb,
+                      const float* T, float* out, long long ld, void* ws, size_t ws_bytes, cudaStream_t st) {
     if (M <= 0 || N <= 0) return GCGCN_OK;
     if (K < 1 || K > TA_KB * TC_BK || N % TC_BN != 0)
         return fail(GCGCN_ERR_UNSUPPORTED, "gemm_rowop: needs 1 <= K <= %d and N a multiple of %d (K %d, N %d)", TA_KB * TC_BK,
@@ -1225,76 +1187,52 @@ int launch_gemm_rowop(int mode, int M, int N, int K, const float* A, int lda, co
     a.tiles_m = ceil_div(M, TC_BM); a.tiles_n = N / TC_BN; a.k_splits = 1; a.k_per_split = K;
     a.kblocks = ceil_div(K, TC_BK); a.batch = 1; a.sA = a.sB = a.sC = 0; a.Apre = nullptr;
     a.rd_t = T; a.rd_out = out; a.rd_ld = ld; a.bscale = nullptr; a.lds = 0; a.seq_k = 0;
-    const size_t blob_total = static_cast<size_t>(a.tiles_n) * a.kblocks * TC_B_BLOB_BYTES;
+    const size_t blob_total = bf16 ? gemm_bf16_blob_bytes(N, K) : static_cast<size_t>(a.tiles_n) * gemm_presplit_bytes(K);
     if (ws == nullptr || blob_total > ws_bytes || (reinterpret_cast<uintptr_t>(ws) & 15) != 0)
-        return fail(GCGCN_ERR_WORKSPACE, "gemm_rowop: workspace of %zu bytes needed for the pre-split weights", blob_total);
-    tc_presplit_b_kernel<<<dim3(a.tiles_n * a.kblocks, 4), 256, 0, st>>>(B, ldb, 0, N, K, a.kblocks, static_cast<uint8_t*>(ws));
-    GCGCN_CHECK_LAUNCH("gemm_presplit_b");
+        return fail(GCGCN_ERR_WORKSPACE, "gemm_rowop: workspace of %zu bytes needed for the weight blobs", blob_total);
+    if (bf16) {
+        GCGCN_TRY(launch_bf16_blobs(B, ldb, N, K, static_cast<uint8_t*>(ws), st));
+    } else {
+        tc_presplit_b_kernel<<<dim3(a.tiles_n * a.kblocks, 4), 256, 0, st>>>(B, ldb, 0, N, K, a.kblocks, static_cast<uint8_t*>(ws));
+        GCGCN_CHECK_LAUNCH("gemm_presplit_b");
+    }
     a.Bpre = static_cast<const uint8_t*>(ws);
     const int grid = std::min(sm_count(), a.tiles_m);
-    if (mode == 1) {
-        static std::atomic<unsigned long long> prepared{0};
-        GCGCN_TRY(set_smem_once(prepared, gemm_tc_tmema_kernel<1>, TA_SMEM_BYTES, "gemm_tc_rowdot smem"));
-        gemm_tc_tmema_kernel<1><<<grid, TA_THREADS, TA_SMEM_BYTES, st>>>(a);
-    } else {
-        static std::atomic<unsigned long long> prepared{0};
-        GCGCN_TRY(set_smem_once(prepared, gemm_tc_tmema_kernel<2>, TA_SMEM_BYTES, "gemm_tc_rowacc smem"));
-        gemm_tc_tmema_kernel<2><<<grid, TA_THREADS, TA_SMEM_BYTES, st>>>(a);
-    }
-    timing_set_work(2.0 * M * N * K);
-    GCGCN_CHECK_LAUNCH(mode == 1 ? "gemm_tc_rowdot<A in TMEM>" : "gemm_tc_rowacc<A in TMEM>");
+#define GCGCN_ROWOP_LAUNCH(MODE, BF16, NAME)                                                                            \
+    do {                                                                                                                \
+        constexpr size_t smem = BF16 ? TA_SMEM_BYTES_BF16 : TA_SMEM_BYTES;                                              \
+        static std::atomic<unsigned long long> prepared{0};                                                             \
+        GCGCN_TRY(set_smem_once(prepared, gemm_tc_tmema_kernel<MODE, BF16>, smem, NAME " smem"));                      \
+        gemm_tc_tmema_kernel<MODE, BF16><<<grid, ta_threads(BF16), smem, st>>>(a);                                      \
+        timing_set_work(2.0 * M * N * K);                                                                               \
+        GCGCN_CHECK_LAUNCH(NAME);                                                                                       \
+    } while (0)
+    if (mode == 1 && !bf16) GCGCN_ROWOP_LAUNCH(1, false, "gemm_tc_rowdot<A in TMEM>");
+    else if (mode == 1) GCGCN_ROWOP_LAUNCH(1, true, "gemm_tc_rowdot<bf16>");
+    else if (!bf16) GCGCN_ROWOP_LAUNCH(2, false, "gemm_tc_rowacc<A in TMEM>");
+    else GCGCN_ROWOP_LAUNCH(2, true, "gemm_tc_rowacc<bf16>");
+#undef GCGCN_ROWOP_LAUNCH
     return GCGCN_OK;
 }
 
-// launch_gemm_rowop on bf16-rounded operands (single-pass kind::f16): A is rounded as it enters tensor memory, B is
-// converted to bf16 blobs first (ws >= gemm_bf16_blob_bytes(N, K)).
-int launch_gemm_rowop_bf16(int mode, int M, int N, int K, const float* A, int lda, const float* B, int ldb, const float* T,
-                           float* out, long long ld, void* ws, size_t ws_bytes, cudaStream_t st) {
-    if (M <= 0 || N <= 0) return GCGCN_OK;
-    if (K < 1 || K > TA_KB * TC_BK || N % TC_BN != 0)
-        return fail(GCGCN_ERR_UNSUPPORTED, "gemm_rowop_bf16: needs 1 <= K <= %d and N a multiple of %d (K %d, N %d)",
-                    TA_KB * TC_BK, TC_BN, K, N);
-    TcArgs a;
-    a.M = M; a.N = N; a.K = K; a.lda = lda; a.ldb = ldb; a.ldc = 0;
-    a.A = A; a.B = B; a.bias = nullptr; a.C = nullptr; a.partial = nullptr; a.alpha = 1.f; a.beta = 0.f;
-    a.tiles_m = ceil_div(M, TC_BM); a.tiles_n = N / TC_BN; a.k_splits = 1; a.k_per_split = K;
-    a.kblocks = ceil_div(K, TC_BK); a.batch = 1; a.sA = a.sB = a.sC = 0; a.Apre = nullptr;
-    a.rd_t = T; a.rd_out = out; a.rd_ld = ld; a.bscale = nullptr; a.lds = 0; a.seq_k = 0;
-    if (ws == nullptr || gemm_bf16_blob_bytes(N, K) > ws_bytes || (reinterpret_cast<uintptr_t>(ws) & 15) != 0)
-        return fail(GCGCN_ERR_WORKSPACE, "gemm_rowop_bf16: workspace of %zu bytes needed for the bf16 weights",
-                    gemm_bf16_blob_bytes(N, K));
-    GCGCN_TRY(launch_bf16_blobs(B, ldb, N, K, static_cast<uint8_t*>(ws), st));
-    a.Bpre = static_cast<const uint8_t*>(ws);
-    const int grid = std::min(sm_count(), a.tiles_m);
-    if (mode == 1) {
-        static std::atomic<unsigned long long> prepared{0};
-        GCGCN_TRY(set_smem_once(prepared, gemm_tc_tmema_kernel<1, true>, TA_SMEM_BYTES_BF16, "gemm_tc_rowdot<bf16> smem"));
-        gemm_tc_tmema_kernel<1, true><<<grid, ta_threads(true), TA_SMEM_BYTES_BF16, st>>>(a);
-    } else {
-        static std::atomic<unsigned long long> prepared{0};
-        GCGCN_TRY(set_smem_once(prepared, gemm_tc_tmema_kernel<2, true>, TA_SMEM_BYTES_BF16, "gemm_tc_rowacc<bf16> smem"));
-        gemm_tc_tmema_kernel<2, true><<<grid, ta_threads(true), TA_SMEM_BYTES_BF16, st>>>(a);
-    }
-    timing_set_work(2.0 * M * N * K);
-    GCGCN_CHECK_LAUNCH(mode == 1 ? "gemm_tc_rowdot<bf16>" : "gemm_tc_rowacc<bf16>");
-    return GCGCN_OK;
-}
-
-// Weight gradient of the bilinear form on bf16-rounded operands, for any rows >= 1:
-//   C[a][r*128 + b] = beta C + sum_p bf16(h[p][a]) bf16(scale[p * lds + r] T[p][b])
-// h is converted to bf16 blobs (pre >= gemm_bf16_blob_bytes(128, rows)); the producers generate the other operand.  The
-// rows are walked in 4096-row ranges (no tensor-core accumulation runs longer); with more than one range every
-// (relation, range) item is a CTA's work item and the deterministic fp32 split-K reduction adds the partials
+// Weight gradient of the bilinear form, for any rows >= 1:
+//   C[a][r*128 + b] = beta C + sum_p h[p][a] (scale[p * lds + r] T[p][b])
+// fp32 (3xTF32): h is pre-split into hi/lo blobs (pre >= gemm_presplit_bytes(rows)).  bf16: h is converted to bf16 blobs
+// (pre >= gemm_bf16_blob_bytes(128, rows)) and both factors are rounded to bf16.  The producers generate the other
+// operand (the general weight gradients run MN-major: blobs only pay for themselves where the wide operand has to be
+// generated; measured on [119808 x 128]^T [119808 x N]: N = 256: 95 us with blobs, 66 us MN-major; N = 1024: 230 us
+// against 216 us).  The rows are walked in 4096-row ranges (no tensor-core accumulation runs longer); with more than one range
+// every (relation, range) item is a CTA's work item and the deterministic fp32 split-K reduction adds the partials
 // (ws >= ranges * 128 * relations*128 floats), with one range the epilogue applies beta itself.
-int launch_bilinear_wgrad_bf16(int relations, int rows, const float* h, const float* T, const float* scale, int lds,
-                               float beta, float* C, void* ws, size_t ws_bytes, void* pre, size_t pre_bytes,
-                               cudaStream_t st) {
+int launch_bilinear_wgrad(bool bf16, int relations, int rows, const float* h, const float* T, const float* scale, int lds,
+                          float beta, float* C, void* ws, size_t ws_bytes, void* pre, size_t pre_bytes, cudaStream_t st) {
     if (rows <= 0 || relations <= 0) return GCGCN_OK;
     const int N = relations * TC_BN, splits = ceil_div(rows, 4096);
     const size_t part_bytes = splits > 1 ? static_cast<size_t>(splits) * TC_BM * N * sizeof(float) : 0;
-    if (pre == nullptr || gemm_bf16_blob_bytes(TC_BM, rows) > pre_bytes || (reinterpret_cast<uintptr_t>(pre) & 15) != 0 ||
+    const size_t pre_need = bf16 ? gemm_bf16_blob_bytes(TC_BM, rows) : gemm_presplit_bytes(rows);
+    if (pre == nullptr || pre_need > pre_bytes || (reinterpret_cast<uintptr_t>(pre) & 15) != 0 ||
         part_bytes > ws_bytes || (part_bytes > 0 && (ws == nullptr || (reinterpret_cast<uintptr_t>(ws) & 15) != 0)))
-        return fail(GCGCN_ERR_WORKSPACE, "bilinear_wgrad_bf16: workspace too small");
+        return fail(GCGCN_ERR_WORKSPACE, "bilinear_wgrad: workspace too small");
     TcArgs a;
     a.M = TC_BM; a.N = N; a.K = rows; a.lda = TC_BM; a.ldb = TC_BN; a.ldc = N;
     a.A = h; a.B = T; a.bias = nullptr; a.C = C; a.alpha = 1.f; a.beta = beta;
@@ -1303,15 +1241,27 @@ int launch_bilinear_wgrad_bf16(int relations, int rows, const float* h, const fl
     a.k_per_split = 4096; a.k_splits = splits;
     a.partial = splits > 1 ? static_cast<float*>(ws) : nullptr;
     a.kblocks = ceil_div(rows, TC_BK); a.Bpre = nullptr;
-    GCGCN_TRY(launch_bf16_blobs(h, TC_BM, TC_BM, rows, static_cast<uint8_t*>(pre), st));
+    if (bf16) {
+        GCGCN_TRY(launch_bf16_blobs(h, TC_BM, TC_BM, rows, static_cast<uint8_t*>(pre), st));
+    } else {
+        tc_presplit_b_kernel<<<dim3(a.kblocks, 4), 256, 0, st>>>(h, TC_BM, /*kcontig=*/0, TC_BM, rows, a.kblocks,
+                                                                 static_cast<uint8_t*>(pre));
+        GCGCN_CHECK_LAUNCH("gemm_presplit_a");
+    }
     a.Apre = static_cast<const uint8_t*>(pre);
     const int grid = std::min(sm_count(), relations * splits);
-    static std::atomic<unsigned long long> prepared{0};
-    GCGCN_TRY(set_smem_once(prepared, gemm_tc_kernel<false, false, 2, false, true, false, true>, TC_SMEM_BYTES,
-                            "gemm_tc_wgrad<bf16> smem"));
-    gemm_tc_kernel<false, false, 2, false, true, false, true><<<grid, tc_threads(2), TC_SMEM_BYTES, st>>>(a);
-    timing_set_work(2.0 * TC_BM * N * rows);
-    GCGCN_CHECK_LAUNCH("gemm_tc_wgrad<bf16>");
+#define GCGCN_WGRAD_LAUNCH(BF16, NAME)                                                                                  \
+    do {                                                                                                                \
+        static std::atomic<unsigned long long> prepared{0};                                                             \
+        GCGCN_TRY(set_smem_once(prepared, gemm_tc_kernel<false, false, 2, false, true, false, BF16>, TC_SMEM_BYTES,     \
+                                NAME " smem"));                                                                         \
+        gemm_tc_kernel<false, false, 2, false, true, false, BF16><<<grid, tc_threads(2), TC_SMEM_BYTES, st>>>(a);       \
+        timing_set_work(2.0 * TC_BM * N * rows);                                                                        \
+        GCGCN_CHECK_LAUNCH(NAME);                                                                                       \
+    } while (0)
+    if (bf16) GCGCN_WGRAD_LAUNCH(true, "gemm_tc_wgrad<bf16>");
+    else GCGCN_WGRAD_LAUNCH(false, "gemm_tc_tn<presplit A>");
+#undef GCGCN_WGRAD_LAUNCH
     if (splits > 1) GCGCN_TRY(launch_splitk_reduce(a.partial, splits, TC_BM, N, 1.f, beta, C, N, nullptr, st, 1, 0));
     return GCGCN_OK;
 }

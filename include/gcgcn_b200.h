@@ -402,55 +402,40 @@ int gcgcn_colsum(const float* X, int32_t M, int32_t N, int32_t ldx, float* out, 
 
 /* ---- relation classifier and loss (SURVEY.md 8f row 2, second half) -------------------------------------------
  * logits = bili_layer_01(h, t) + classification_layer_01(cat[h, t])  (G:356-358) with h, t = entity_feature_h / _t
- * [total_pairs, 128] from gcgcn_pair_dense_fwd.  The bilinear form runs on gcgcn_gemm as Y = h W' (W' = the
- * [R, 128, 128] weight viewed as [128, R*128], 3xTF32 tcgen05 tiles) followed by the reductions below; the caller
- * (gcgcn_b200/classifier.py) walks the pairs in chunks so that Y stays within a fixed workspace.
- *   reduce: out[p][r] (+)= sum_b Y[p][r*128 + b] t[p][b] (+ bias[r])        Y [rows, R*128], out row stride ldo
- *   outer:  dY[p][r*128 + b] = dout[p][r] t[p][b]                            (then dh = dY W'^T, dW' = h^T dY)
- *   dt:     dt[p][b] = sum_r dout[p][r] Y[p][r*128 + b]                                                        */
-/* Fused forward: out[p][r] (+)= sum_{a,b} h[p][a] W'[a][r*128 + b] t[p][b] + bias[r] in ONE tensor-core pass -- h stays
- * resident in tensor memory per 128-pair tile, W' streams through shared memory as pre-split blobs, and the epilogue
- * contracts every 128 x 128 accumulator tile (one relation) with t straight out of TMEM, so h W' never exists.
- * Wm = W' [128, relations*128] row-major; ws >= gcgcn_bilinear_ws_bytes(rows, relations), else GCGCN_ERR_WORKSPACE. */
-size_t gcgcn_bilinear_ws_bytes(int32_t rows, int32_t relations);
-int gcgcn_bilinear_fwd(const float* h, const float* t, const float* Wm, const float* bias, int32_t rows,
-                       int32_t relations, int32_t accumulate, float* out, int32_t ldo, void* ws, size_t ws_bytes,
-                       void* stream);
-/* Fused backward of the bilinear form for rows >= 8192 (GCGCN_ERR_UNSUPPORTED below that: use the three kernels
- * further down), no [rows, relations*128] intermediate:
- *   dt[p][b] = sum_r dout[p][r] (h W')[p][r*128 + b]      row-accumulate epilogue on the TMEM-resident GEMM, A = h, B = Wm
- *   dh[p][a] = sum_r dout[p][r] (t W'')[p][r*128 + a]     the same with A = t, B = Wm2 (W viewed as [128 (b), relations*128 (r, a)])
+ * [total_pairs, 128] from gcgcn_pair_dense_fwd.  The bilinear form, with W' = the [R, 128, 128] weight viewed as
+ * [128, R*128] (Wm, row-major) and W'' = the same weight viewed as [128 (b), R*128 (r, a)] (Wm2), runs in tensor-core
+ * passes that never store a [rows, relations*128] intermediate:
+ *   out[p][r] (+)= sum_{a,b} h[p][a] W'[a][r*128 + b] t[p][b] + bias[r]  in ONE pass -- h stays resident in tensor memory
+ *                  per 128-pair tile, W' streams through shared memory as blobs, and the epilogue contracts every
+ *                  128 x 128 accumulator tile (one relation) with t straight out of TMEM; out has row stride ldo, bias
+ *                  may be null, accumulate != 0 adds to out
+ *   dt[p][b] = sum_r dout[p][r] (h W')[p][r*128 + b]      row-accumulate epilogue on the same GEMM, A = h, B = Wm
+ *   dh[p][a] = sum_r dout[p][r] (t W'')[p][r*128 + a]     the same with A = t, B = Wm2
  *   dWm[a][r*128 + b] = beta dWm + sum_p h[p][a] dout[p][r] t[p][b]   weight-gradient GEMM whose [rows, relations*128]
- *                       operand is generated in the producers from t and dout (never stored)
- * dout [rows, relations] row-major.  ws >= gcgcn_bilinear_bwd_ws_bytes(rows, relations), else GCGCN_ERR_WORKSPACE.   */
-size_t gcgcn_bilinear_bwd_ws_bytes(int32_t rows, int32_t relations);
-int gcgcn_bilinear_bwd(const float* h, const float* t, const float* Wm, const float* Wm2, const float* dout, int32_t rows,
-                       int32_t relations, float beta, float* dh, float* dt, float* dWm, void* ws, size_t ws_bytes,
-                       void* stream);
-/* The bilinear form on bf16-rounded operands: the same arguments, shapes, workspace rule and outputs as the two fp32
- * entry points above, with the numerics of SURVEY.md section 8d config 3 (bf16 operands, fp32 accumulation).  bf16(x)
- * is x rounded to the nearest bf16, ties to even (torch's .to(torch.bfloat16), cvt.rn.bf16x2.f32).  Every product of
- * two bf16 values is exact in fp32, every sum is fp32, and h, t, W', dout and all outputs stay fp32 in memory:
+ *                       operand is generated in the producers from t and dout, walked in 4096-row ranges
+ * dout [rows, relations] row-major.  The bias gradient is gcgcn_colsum of dout.  The backward takes any rows >= 0:
+ * rows = 0 returns at once and leaves dWm as it is.  ws >= gcgcn_bilinear_ws_bytes / gcgcn_bilinear_bwd_ws_bytes of the
+ * same rows, relations and dtype, else GCGCN_ERR_WORKSPACE; a dtype other than GCGCN_F32 or GCGCN_BF16 is
+ * GCGCN_ERR_INVALID_ARG.  Both types keep h, t, W', dout and every output fp32 in memory.
+ *
+ * dtype GCGCN_F32: 3xTF32 tcgen05 tiles (hi/lo split operands), fp32 accumulation.
+ *
+ * dtype GCGCN_BF16: the numerics of SURVEY.md section 8d config 3 (bf16 operands, fp32 accumulation).  bf16(x) is x
+ * rounded to the nearest bf16, ties to even (torch's .to(torch.bfloat16), cvt.rn.bf16x2.f32).  Every product of two
+ * bf16 values is exact in fp32 and every sum is fp32:
  *   out[p][r]   (+)= sum_b (sum_a bf16(h[p][a]) bf16(W'[a][r*128 + b])) t[p][b] + bias[r]     (t not rounded)
  *   dt[p][b]     = sum_r dout[p][r] sum_a bf16(h[p][a]) bf16(W'[a][r*128 + b])                 (dout not rounded)
  *   dh[p][a]     = sum_r dout[p][r] sum_b bf16(t[p][b]) bf16(W''[b][r*128 + a])
  *   dWm[a][r*128 + b] = beta dWm + sum_p bf16(h[p][a]) bf16(dout[p][r] t[p][b])   (the fp32 product, rounded once)
- * One tcgen05.mma.kind::f16 per 16 K values.  The backward takes any rows >= 0 (no chunked fallback, no minimum):
- * rows = 0 returns at once and leaves dWm as it is.  The bias gradient is gcgcn_colsum of dout, as for fp32.            */
-size_t gcgcn_bilinear_bf16_ws_bytes(int32_t rows, int32_t relations);
-int gcgcn_bilinear_bf16_fwd(const float* h, const float* t, const float* Wm, const float* bias, int32_t rows,
-                            int32_t relations, int32_t accumulate, float* out, int32_t ldo, void* ws, size_t ws_bytes,
-                            void* stream);
-size_t gcgcn_bilinear_bf16_bwd_ws_bytes(int32_t rows, int32_t relations);
-int gcgcn_bilinear_bf16_bwd(const float* h, const float* t, const float* Wm, const float* Wm2, const float* dout,
-                            int32_t rows, int32_t relations, float beta, float* dh, float* dt, float* dWm, void* ws,
-                            size_t ws_bytes, void* stream);
-int gcgcn_bilinear_reduce_fwd(const float* Y, const float* t, const float* bias, int32_t rows, int32_t relations,
-                              int32_t accumulate, float* out, int32_t ldo, void* stream);
-int gcgcn_bilinear_outer_bwd(const float* dout, int32_t ldd, const float* t, int32_t rows, int32_t relations, float* dY,
-                             void* stream);
-int gcgcn_bilinear_dt_bwd(const float* dout, int32_t ldd, const float* Y, int32_t rows, int32_t relations, float* dt,
-                          void* stream);
+ * One tcgen05.mma.kind::f16 per 16 K values.                                                                      */
+size_t gcgcn_bilinear_ws_bytes(int32_t rows, int32_t relations, int32_t dtype);
+int gcgcn_bilinear_fwd(const float* h, const float* t, const float* Wm, const float* bias, int32_t rows,
+                       int32_t relations, int32_t dtype, int32_t accumulate, float* out, int32_t ldo, void* ws,
+                       size_t ws_bytes, void* stream);
+size_t gcgcn_bilinear_bwd_ws_bytes(int32_t rows, int32_t relations, int32_t dtype);
+int gcgcn_bilinear_bwd(const float* h, const float* t, const float* Wm, const float* Wm2, const float* dout, int32_t rows,
+                       int32_t relations, int32_t dtype, float beta, float* dh, float* dt, float* dWm, void* ws,
+                       size_t ws_bytes, void* stream);
 /* cls_feature of the BERT variant (models/GraphCNN_multihead_bert_gate_cls.py:346-347): a per-document vector
  * v[b] = linear_cls(cls_feat_b) added to the logits of every pair of document b.  z [total_pairs, relations] in place;
  * bwd: dv[b] = sum of dz over the document's pairs.                                                              */

@@ -2,7 +2,7 @@
     python scripts/run_classifier.py [pairs] [iters] [--bwd] [--dtype fp32|bf16]
 
 --dtype both [--out PATH] times the bilinear form's two operand types against each other in one process, alternating
-them: BilinearFn (3xTF32) and BilinearBf16Fn (bf16 operands) alone and inside relation_logits, forward and forward +
+them: BilinearFn in fp32 (3xTF32) and on bf16 operands, alone and inside relation_logits, forward and forward +
 backward, at 99 312 and 794 496 pairs (the bench's 12-document batch x 16 and x 128), then a GraphHead forward +
 backward (loss included) on a 192-document synthetic batch in both classifier dtypes.  CUDA events around ITERS steps
 after a warm-up, the median of REPS such windows; per-kernel device times from the library's timing hooks.  Writes one
@@ -18,7 +18,7 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from gcgcn_b200 import _lib                                   # noqa: E402
-from gcgcn_b200.classifier import BilinearBf16Fn, BilinearFn, relation_logits            # noqa: E402
+from gcgcn_b200.classifier import BilinearFn, relation_logits            # noqa: E402
 
 DTYPES = {"fp32": torch.float32, "bf16": torch.bfloat16}
 
@@ -98,9 +98,8 @@ def both(out_path, iters, reps):
         allp = [h, t] + list(bili.parameters()) + list(cls.parameters())
         steps = {}
         for key, dt in DTYPES.items():
-            fn = BilinearBf16Fn if dt == torch.bfloat16 else BilinearFn
-            steps[("bilinear", "fwd", key)] = lambda fn=fn: fn.apply(*leaves)
-            steps[("bilinear", "fwd+bwd", key)] = lambda fn=fn: torch.autograd.grad(fn.apply(*leaves), leaves, up)
+            steps[("bilinear", "fwd", key)] = lambda dt=dt: BilinearFn.apply(*leaves, dt)
+            steps[("bilinear", "fwd+bwd", key)] = lambda dt=dt: torch.autograd.grad(BilinearFn.apply(*leaves, dt), leaves, up)
             steps[("classifier", "fwd", key)] = lambda dt=dt: relation_logits(h, t, bili, cls, dtype=dt)
             steps[("classifier", "fwd+bwd", key)] = lambda dt=dt: torch.autograd.grad(
                 relation_logits(h, t, bili, cls, dtype=dt), allp, up)

@@ -1,5 +1,5 @@
-"""Float64 reference of the relation classifier's bilinear form on bf16-rounded operands (gcgcn_bilinear_bf16_fwd / _bwd,
-classifier.BilinearBf16Fn), restated from the definitions in include/gcgcn_b200.h:
+"""Float64 reference of the relation classifier's bilinear form on bf16-rounded operands (gcgcn_bilinear_fwd / _bwd
+with dtype GCGCN_BF16, classifier.BilinearFn with torch.bfloat16), restated from the definitions in include/gcgcn_b200.h:
 
   out[p, r]     = sum_b (sum_a bf16(h[p, a]) bf16(W[r, a, b])) t[p, b] + bias[r]
   dt[p, b]      = sum_r dout[p, r] sum_a bf16(h[p, a]) bf16(W[r, a, b])

@@ -1,21 +1,12 @@
-"""-m gpu: the bilinear form on bf16 operands (gcgcn_bilinear_bf16_fwd / _bwd, classifier.BilinearBf16Fn,
-relation_logits(dtype=torch.bfloat16), GraphHead(classifier_dtype=torch.bfloat16)).
+"""-m gpu: the bilinear form on bf16 operands against the fp32 route (relation_logits(dtype=torch.bfloat16),
+GraphHead(classifier_dtype=torch.bfloat16)).  Both routes against float64 are in test_gpu_classifier_fp64.py.
 
-Against float64 of the rounded operands (tests/classifier_bf16_oracle.py) the only error left is the kernels' fp32
-accumulation, so the bounds sit at the scale of the fp32 route's own float64 tests (test_gpu_classifier_fp64.py), each
-at least 4x above the error measured on a B200 (noted beside it): a wrong instruction descriptor, operand layout or
-rounding shows up as errors of 1e-3 and more.  Against the fp32 route the difference is the bf16 rounding itself, and
-the bound is relative (max |difference| / max |fp32 value|).
-
-P runs on both sides of every boundary of the kernels: 128-pair row tiles, 4096-row ranges of the weight gradient (one
-range: the epilogue applies beta; several: split-K partials and the fp32 reduction), and the host calls of
-FUSED_CHUNK_PAIRS pairs; R from one relation to more relation tiles than the B200's 148 SMs.
+The difference between the two routes is the bf16 rounding of the operands itself, and the bound is relative
+(max |difference| / max |fp32 value|).
 """
 import pytest
 import torch
 
-from classifier_bf16_oracle import bilinear_bf16
-from oracle import classifier_oracle as CO
 from gcgcn_b200 import _lib
 from gcgcn_b200 import classifier as C
 from gcgcn_b200 import synthetic as S
@@ -25,17 +16,9 @@ from gcgcn_b200.sharding import FlatTrainer
 pytestmark = pytest.mark.gpu
 DEV = torch.device("cuda:0")
 D = 128
-ERR_WORKSPACE = -4
-ROWDOT, ROWACC, WGRAD = "gemm_tc_rowdot<bf16>", "gemm_tc_rowacc<bf16>", "gemm_tc_wgrad<bf16>"
+ROWDOT, WGRAD = "gemm_tc_rowdot<bf16>", "gemm_tc_wgrad<bf16>"
 FP32_ROUTE = ("gemm_tc_rowdot<A in TMEM>", "gemm_tc_rowacc<A in TMEM>", "gemm_tc_tn<presplit A>", "gemm_presplit_b",
-              "gemm_presplit_a", "bilinear_reduce", "bilinear_outer", "bilinear_dt")
-
-# max |got - ref| / max |ref| against float64 of the rounded operands; the worst value measured on a B200 beside each
-TOL = {"out": 1.2e-6,       # 2.5e-7
-       "dh": 2.5e-6,        # 5.9e-7 (P 532481)
-       "dt": 3e-6,          # 6.9e-7 (P 8193, R 150)
-       "dW": 2.5e-5,        # 5.4e-6 (P 4096: one 4096-row accumulation); 2.8e-7 below 128 rows
-       "dbias": 1.2e-6}     # 3.0e-7
+              "gemm_presplit_a")
 # relative bound against the fp32 route (the bf16 rounding of the operands)
 VS_FP32 = 2e-2
 
@@ -48,158 +31,6 @@ def rel_err(got, ref):
     got, ref = got.double(), ref.double()
     assert got.shape == ref.shape, (got.shape, ref.shape)
     return float((got - ref).abs().max()) / max(float(ref.abs().max()), 1e-30)
-
-
-def bilinear_inputs(P, R, seed):
-    """h, t as pair_dense leaves them (tanh), W and bias with nn.Bilinear's init, a random upstream gradient."""
-    gen = torch.Generator(device=DEV).manual_seed(seed)
-    h = torch.tanh(torch.randn(P, D, generator=gen, device=DEV))
-    t = torch.tanh(torch.randn(P, D, generator=gen, device=DEV))
-    W = (torch.rand(R, D, D, generator=gen, device=DEV) * 2 - 1) / D ** 0.5
-    bias = (torch.rand(R, generator=gen, device=DEV) * 2 - 1) / D ** 0.5
-    dout = torch.randn(P, R, generator=gen, device=DEV)
-    return h, t, W, bias, dout
-
-
-def run_bilinear(h, t, W, bias, dout):
-    """BilinearBf16Fn forward and backward; returns (out, dh, dt, dW, dbias) and {kernel: launches}."""
-    leaves = [x.clone().requires_grad_(True) for x in (h, t, W, bias)]
-    torch.cuda.synchronize()
-    _lib.timing_begin(stream())
-    out = C.BilinearBf16Fn.apply(*leaves)
-    out.backward(dout)
-    ran = {k: v[0] for k, v in _lib.timing_end(stream()).items()}
-    torch.cuda.synchronize()
-    return (out.detach(),) + tuple(x.grad for x in leaves), ran
-
-
-ROUTES = ([(P, 97) for P in (1, 127, 128, 129, 4095, 4096, 4097, 8191, 8192, 270336, 532481)]
-          + [(P, R) for R in (1, 2, 33, 150) for P in (127, 8193)])
-
-
-@pytest.mark.parametrize("P,R", ROUTES)
-def test_bilinear_bf16_against_float64(P, R):
-    """4096 / 4097: one range / two, the second of one row; 270336: two host calls (262144 + 8192); 532481: three, the
-    last of one pair.  Only the bf16 kernels run."""
-    h, t, W, bias, dout = bilinear_inputs(P, R, seed=P * 1000 + R)
-    got, ran = run_bilinear(h, t, W, bias, dout)
-    calls = -(-P // C.FUSED_CHUNK_PAIRS)
-    assert ran.get(ROWDOT) == 1 and ran.get(ROWACC) == 2 * calls and ran.get(WGRAD) == calls, ran
-    assert not [k for k in ran if k in FP32_ROUTE or (k.startswith("gemm") and "<bf16>" not in k)], ran
-    ref = bilinear_bf16(h, t, W, bias, dout)
-    errs = {k: rel_err(g, r) for k, g, r in zip(TOL, got, ref)}
-    print(f"P {P} R {R}: " + ", ".join(f"{k} {e:.2e}" for k, e in errs.items()))
-    for k, e in errs.items():
-        assert e <= TOL[k], f"P {P} R {R} {k}: {e:.3e} > {TOL[k]:.1e}"
-
-
-def test_bilinear_bf16_is_deterministic():
-    """Fixed-order reductions, no atomics: two runs are bitwise equal."""
-    args = bilinear_inputs(12289, 97, seed=7)
-    a, _ = run_bilinear(*args)
-    b, _ = run_bilinear(*args)
-    for k, x, y in zip(TOL, a, b):
-        assert torch.equal(x, y), k
-
-
-# ---- the C entry points ---------------------------------------------------------------------------------------------
-def lib():
-    return _lib.load()
-
-
-def p(x):
-    return None if x is None else x.data_ptr()
-
-
-def weights(W):
-    return CO.wprime(W.double()).float().contiguous(), CO.wsecond(W.double()).float().contiguous()
-
-
-def test_fwd_accumulates_into_a_strided_output_without_bias():
-    """accumulate = 1 into a prefilled out of row stride ldo > R, bias null: out[:, :R] += the bilinear form, columns
-    R.. untouched; a workspace of exactly gcgcn_bilinear_bf16_ws_bytes suffices."""
-    P, R, ldo = 1000, 33, 40
-    h, t, W, _, _ = bilinear_inputs(P, R, seed=11)
-    Wm, _ = weights(W)
-    gen = torch.Generator(device=DEV).manual_seed(12)
-    out = torch.full((P, ldo), -7.25, device=DEV)
-    out[:, :R] = torch.randn(P, R, generator=gen, device=DEV)
-    before = out.clone()
-    ws = torch.empty(int(lib().gcgcn_bilinear_bf16_ws_bytes(P, R)), dtype=torch.uint8, device=DEV)
-    _lib.call("gcgcn_bilinear_bf16_fwd", p(h), p(t), p(Wm), None, P, R, 1, p(out), ldo, p(ws), ws.numel(), stream())
-    torch.cuda.synchronize()
-    assert torch.equal(out[:, R:], before[:, R:])
-    e = rel_err(out[:, :R], before[:, :R].double() + bilinear_bf16(h, t, W))
-    print(f"fwd accumulate: {e:.2e}")
-    assert e <= TOL["out"]                                                  # 1.8e-7
-
-
-@pytest.mark.parametrize("P", [100, 8193])
-@pytest.mark.parametrize("beta", [0.0, 1.0])
-def test_bwd_beta(P, beta):
-    """beta = 0 overwrites dWm (NaN before: never read), beta = 1 adds to it; dh and dt are written whole.  P = 100: one
-    4096-row range (the epilogue applies beta); 8193: three (the split-K reduction does)."""
-    R = 33
-    h, t, W, _, dout = bilinear_inputs(P, R, seed=21 + P)
-    Wm, Wm2 = weights(W)
-    gen = torch.Generator(device=DEV).manual_seed(22)
-    prior = torch.randn(D, R * D, generator=gen, device=DEV) if beta else torch.full((D, R * D), float("nan"), device=DEV)
-    dWm = prior.clone()
-    dh = torch.full_like(h, float("nan"))
-    dt = torch.full_like(t, float("nan"))
-    ws = torch.empty(int(lib().gcgcn_bilinear_bf16_bwd_ws_bytes(P, R)), dtype=torch.uint8, device=DEV)
-    _lib.call("gcgcn_bilinear_bf16_bwd", p(h), p(t), p(Wm), p(Wm2), p(dout), P, R, beta, p(dh), p(dt), p(dWm), p(ws),
-              ws.numel(), stream())
-    torch.cuda.synchronize()
-    _, rdh, rdt, rdW, _ = bilinear_bf16(h, t, W, None, dout)
-    want = CO.wprime(rdW) + (prior.double() if beta else 0.0)
-    errs = {"dh": rel_err(dh, rdh), "dt": rel_err(dt, rdt), "dW": rel_err(dWm, want)}
-    print(f"bwd P {P} beta {beta}: " + ", ".join(f"{k} {v:.2e}" for k, v in errs.items()))
-    for k, e in errs.items():
-        assert e <= TOL[k], f"{k}: {e:.3e} > {TOL[k]:.1e}"
-
-
-def test_zero_rows_launch_nothing():
-    R = 97
-    h, t, W, bias, dout = bilinear_inputs(4, R, seed=31)
-    Wm, Wm2 = weights(W)
-    out = torch.full((4, R), 3.0, device=DEV)
-    dh, dt, dWm = torch.full_like(h, 3.0), torch.full_like(t, 3.0), torch.full((D, R * D), 3.0, device=DEV)
-    ws = torch.empty(4096, dtype=torch.uint8, device=DEV)
-    before = _lib.launch_count()
-    assert lib().gcgcn_bilinear_bf16_fwd(p(h), p(t), p(Wm), p(bias), 0, R, 0, p(out), R, p(ws), ws.numel(), stream()) == 0
-    assert lib().gcgcn_bilinear_bf16_bwd(p(h), p(t), p(Wm), p(Wm2), p(dout), 0, R, 0.0, p(dh), p(dt), p(dWm), p(ws),
-                                         ws.numel(), stream()) == 0
-    assert _lib.launch_count() == before
-    torch.cuda.synchronize()
-    assert bool((out == 3).all() and (dh == 3).all() and (dt == 3).all() and (dWm == 3).all())
-    # and through the autograd function: an empty forward and backward
-    leaves = [x[:0].clone().requires_grad_(True) for x in (h, t)] + [W.clone().requires_grad_(True),
-                                                                     bias.clone().requires_grad_(True)]
-    z = C.BilinearBf16Fn.apply(*leaves)
-    z.backward(torch.zeros_like(z))
-    assert z.shape == (0, R) and not leaves[2].grad.any() and not leaves[3].grad.any()
-
-
-@pytest.mark.parametrize("which", ["fwd", "bwd"])
-def test_workspace_one_byte_short_is_refused_before_any_launch(which):
-    P, R = 8192, 97
-    h, t, W, bias, dout = bilinear_inputs(P, R, seed=51)
-    Wm, Wm2 = weights(W)
-    out = torch.zeros(P, R, device=DEV)
-    dh, dt, dWm = torch.zeros_like(h), torch.zeros_like(t), torch.zeros(D, R * D, device=DEV)
-    need = int(lib().gcgcn_bilinear_bf16_ws_bytes(P, R) if which == "fwd" else lib().gcgcn_bilinear_bf16_bwd_ws_bytes(P, R))
-    ws = torch.empty(need, dtype=torch.uint8, device=DEV)
-    before = _lib.launch_count()
-    if which == "fwd":
-        rc = lib().gcgcn_bilinear_bf16_fwd(p(h), p(t), p(Wm), p(bias), P, R, 0, p(out), R, p(ws), need - 1, stream())
-    else:
-        rc = lib().gcgcn_bilinear_bf16_bwd(p(h), p(t), p(Wm), p(Wm2), p(dout), P, R, 0.0, p(dh), p(dt), p(dWm), p(ws),
-                                           need - 1, stream())
-    assert rc == ERR_WORKSPACE, (rc, lib().gcgcn_last_error())
-    assert _lib.launch_count() == before
-    torch.cuda.synchronize()
-    assert not out.any() and not dh.any() and not dt.any() and not dWm.any()
 
 
 # ---- against the fp32 route -----------------------------------------------------------------------------------------

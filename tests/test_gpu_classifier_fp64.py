@@ -1,21 +1,26 @@
-"""-m gpu: the relation classifier and the trainer's loss against the float64 oracle (oracle/classifier_oracle.py) on
-every route.
+"""-m gpu: the relation classifier and the trainer's loss against float64 on every route, the bilinear form in both its
+operand types.
 
-The bilinear form runs on three tensor-core modes of gemm_tc.cu: the row-dot epilogue (forward), the row-accumulate
-epilogue (dh, dt) and the weight-gradient GEMM whose [pairs, R*128] operand its producers generate from t and dout,
-split-K over 4096-row ranges with an fp32 reduction (dW').  BilinearFn takes that fused backward from 8192 pairs on,
-in host calls of up to 262144 pairs that accumulate dW' through beta = 1; below 8192 pairs it materialises h W' chunk
-by chunk.  The cases below put P on both sides of every one of those boundaries and R from 1 to past the 148 SMs of a
-B200, call the C entry points with the strides, accumulation and beta the header documents, and run the loss and the
-per-document bias on a ragged batch with a document of 65 536 pairs.
+The bilinear form runs on three tensor-core modes of gemm_tc.cu, in fp32 (3xTF32) or on bf16 operands: the row-dot
+epilogue (forward), the row-accumulate epilogue (dh, dt) and the weight-gradient GEMM whose [pairs, R*128] operand its
+producers generate from t and dout, walked in 4096-row ranges (one range: the epilogue applies beta; several: split-K
+partials and an fp32 reduction) (dW').  BilinearFn makes the backward in host calls of up to FUSED_CHUNK_PAIRS pairs
+that accumulate dW' through beta = 1.  The cases below put P on both sides of every one of those boundaries and of the
+128-pair row tiles, and R from 1 to past the 148 SMs of a B200, call the C entry points with the strides, accumulation
+and beta the header documents, and run the loss and the per-document bias on a ragged batch with a document of 65 536
+pairs.
 
-Every bound sits at least 4x above the error measured on a B200 (noted beside it) and well below the 1e-4 that a
-3xTF32 route which lost one of its three products would still meet on some quantities; the exception is a sum that one
-tensor-core accumulator carries over thousands of rows (LONG_TOL).
+fp32 is checked against float64 (oracle/classifier_oracle.py), bf16 against float64 of the rounded operands
+(tests/classifier_bf16_oracle.py): either way only the kernels' fp32 accumulation is left.  Every bound sits at least 4x
+above the error measured on a B200 (noted beside it) and well below the 1e-4 that a 3xTF32 route which lost one of its
+three products would still meet on some quantities (bf16: a wrong instruction descriptor, operand layout or rounding
+shows up as errors of 1e-3 and more); the exception is an fp32 sum that one tensor-core accumulator carries over
+thousands of rows (LONG_TOL).
 """
 import pytest
 import torch
 
+from classifier_bf16_oracle import bilinear_bf16
 from oracle import classifier_oracle as CO
 from gcgcn_b200 import _lib
 from gcgcn_b200 import classifier as C
@@ -24,26 +29,36 @@ from gcgcn_b200.batch import RaggedBatch
 pytestmark = pytest.mark.gpu
 DEV = torch.device("cuda:0")
 D = 128
-ERR_UNSUPPORTED, ERR_WORKSPACE = -2, -4
-FUSED_WGRAD = "gemm_tc_tn<presplit A>"           # the generated-operand weight-gradient GEMM, once per fused host call
-ROWDOT = "gemm_tc_rowdot<A in TMEM>"
+ERR_INVALID_ARG, ERR_WORKSPACE = -1, -4
+F32, BF16 = torch.float32, torch.bfloat16
+DTYPES = [pytest.param(F32, id="f32"), pytest.param(BF16, id="bf16")]
+ORACLE = {F32: CO.bilinear, BF16: bilinear_bf16}
+# row-dot forward, row-accumulate dh and dt, the generated-operand weight gradient; then the operand converters
+KERNELS = {F32: ("gemm_tc_rowdot<A in TMEM>", "gemm_tc_rowacc<A in TMEM>", "gemm_tc_tn<presplit A>",
+                 "gemm_presplit_b", "gemm_presplit_a"),
+           BF16: ("gemm_tc_rowdot<bf16>", "gemm_tc_rowacc<bf16>", "gemm_tc_wgrad<bf16>")}
 
-# max |got - ref| / max |ref| against float64; the worst value measured over ROUTES on a B200 (1000 W) beside each
-TOL = {"out": 6e-6,        # 1.5e-6
-       "dh": 2e-5,         # 4.4e-6 (P 127, R 150: chunked, 512-row split-K ranges); fused 1.7e-6
-       "dt": 7e-6,         # 1.7e-6
-       "dW": 8e-6,         # 1.8e-6 (P 127)
-       "dbias": 1.2e-6}    # 2.9e-7
-# One tensor-core accumulator fed by thousands of rows comes out small by about 2.5e-5 per 4096 rows (its fp32 adds
-# truncate, DESIGN.md section 4a).  Measured: dW' of the fused backward (4096-row ranges) 2.7e-5 to 3.9e-5 at every P
-# from 8192 to 532481 (3.0e-5 at 532481), and dh, dW' of the chunked backward at P = 8191 (accumulators of 6208 and
-# 8191 rows) 5.5e-5 and 6.9e-5.  Four times that would pass 1e-4, so these keep DESIGN.md section 2's 1e-4.
+# max |got - ref| / max |ref| against float64 (of the rounded operands for bf16); the worst value measured over ROUTES
+# on a B200 (1000 W) beside each
+TOL = {F32: {"out": 6e-6,        # 1.5e-6
+             "dh": 7e-6,         # 1.7e-6
+             "dt": 7e-6,         # 1.7e-6
+             "dW": 8e-6,         # 2.2e-6 (P 128: 3.6x below)
+             "dbias": 1.2e-6},   # 3.0e-7
+       BF16: {"out": 1.2e-6,     # 2.5e-7
+              "dh": 2.5e-6,      # 5.9e-7 (P 532481)
+              "dt": 3e-6,        # 6.9e-7 (P 8193, R 150)
+              "dW": 2.5e-5,      # 5.4e-6 (P 4096: one 4096-row accumulation); 2.8e-7 below 128 rows
+              "dbias": 1.2e-6}}  # 3.0e-7
+# One fp32 tensor-core accumulator fed by thousands of rows comes out small by about 2.5e-5 per 4096 rows (its fp32 adds
+# truncate, DESIGN.md section 4a).  dW' takes one accumulator per min(P, 4096)-row range, so from a few hundred pairs on
+# that drift outgrows TOL's margin.  Measured: dW' 2.7e-5 to 3.9e-5 at every P from 4095 to 532481 (3.1e-5 at 4095,
+# 3.0e-5 at 532481).  Four times that would pass 1e-4, so these keep DESIGN.md section 2's 1e-4.
 LONG_TOL = 1e-4
 
 
-def tol(k, P):
-    long_sum = (k == "dW" and P >= 4096) or (k == "dh" and 4096 <= P < C.FUSED_MIN_PAIRS)
-    return LONG_TOL if long_sum else TOL[k]
+def tol(dtype, k, P):
+    return LONG_TOL if dtype == F32 and k == "dW" and P >= 256 else TOL[dtype][k]
 
 
 def stream():
@@ -67,54 +82,48 @@ def bilinear_inputs(P, R, seed):
     return h, t, W, bias, dout
 
 
-def run_bilinear(h, t, W, bias, dout):
+def run_bilinear(dtype, h, t, W, bias, dout):
     """BilinearFn forward and backward; returns (out, dh, dt, dW, dbias) and {kernel: launches}."""
     leaves = [x.clone().requires_grad_(True) for x in (h, t, W, bias)]
     torch.cuda.synchronize()
     _lib.timing_begin(stream())
-    out = C.BilinearFn.apply(*leaves)
+    out = C.BilinearFn.apply(*leaves, dtype)
     out.backward(dout)
     ran = {k: v[0] for k, v in _lib.timing_end(stream()).items()}
     torch.cuda.synchronize()
     return (out.detach(),) + tuple(x.grad for x in leaves), ran
 
 
-def fused_calls(P):
-    """Host calls of the fused backward that BilinearFn makes for P pairs."""
-    calls, rest = 0, P
-    while rest >= C.FUSED_MIN_PAIRS:
-        rest -= rest if rest <= C.FUSED_CHUNK_PAIRS + C.FUSED_MIN_PAIRS else C.FUSED_CHUNK_PAIRS
-        calls += 1
-    return calls
-
-
-ROUTES = ([(P, 97) for P in (1, 127, 8191, 8192, 8193, 12289, 270336, 532481)]
+ROUTES = ([(P, 97) for P in (1, 127, 128, 129, 4095, 4096, 4097, 8191, 8192, 8193, 12289, 270336, 532481)]
           + [(P, R) for R in (1, 2, 33, 150) for P in (127, 8193)])
 
 
+@pytest.mark.parametrize("dtype", DTYPES)
 @pytest.mark.parametrize("P,R", ROUTES)
-def test_bilinear_against_float64(P, R):
-    """P = 1, 127, 8191: chunked backward; 8192: the fused minimum, two whole 4096-row ranges; 8193: three ranges, the
-    last of one row; 12289: four ranges and a row; 270336: the largest single fused call; 532481: three calls of
-    262144, 262144 and 8193 pairs.  R = 1: one relation tile; R = 150: more relation tiles than SMs."""
+def test_bilinear_against_float64(P, R, dtype):
+    """128 / 129: one row tile / two; 4096 / 4097: one 4096-row range / two, the second of one row; 8193: three ranges,
+    the last of one row; 12289: four ranges and a row; 270336: two host calls (262144 + 8192); 532481: three, the last
+    of one pair.  R = 1: one relation tile; R = 150: more relation tiles than SMs.  Only the kernels of dtype run."""
     h, t, W, bias, dout = bilinear_inputs(P, R, seed=P * 1000 + R)
-    got, ran = run_bilinear(h, t, W, bias, dout)
-    assert ran.get(ROWDOT) == 1, ran
-    assert ran.get(FUSED_WGRAD, 0) == fused_calls(P), ran
-    assert fused_calls(P) == {8192: 1, 8193: 1, 12289: 1, 270336: 1, 532481: 3}.get(P, 0)
-    ref = CO.bilinear(h, t, W, bias, dout)
-    errs = {k: rel_err(g, r) for k, g, r in zip(TOL, got, ref)}
-    print(f"P {P} R {R}: " + ", ".join(f"{k} {e:.2e}" for k, e in errs.items()))
+    got, ran = run_bilinear(dtype, h, t, W, bias, dout)
+    rowdot, rowacc, wgrad = KERNELS[dtype][:3]
+    calls = -(-P // C.FUSED_CHUNK_PAIRS)
+    assert ran.get(rowdot) == 1 and ran.get(rowacc) == 2 * calls and ran.get(wgrad) == calls, ran
+    assert not [k for k in ran if k.startswith("gemm") and k not in KERNELS[dtype]], ran
+    ref = ORACLE[dtype](h, t, W, bias, dout)
+    errs = {k: rel_err(g, r) for k, g, r in zip(TOL[dtype], got, ref)}
+    print(f"{dtype} P {P} R {R}: " + ", ".join(f"{k} {e:.2e}" for k, e in errs.items()))
     for k, e in errs.items():
-        assert e <= tol(k, P), f"P {P} R {R} {k}: {e:.3e} > {tol(k, P):.1e}"
+        assert e <= tol(dtype, k, P), f"P {P} R {R} {k}: {e:.3e} > {tol(dtype, k, P):.1e}"
 
 
-def test_bilinear_is_deterministic():
+@pytest.mark.parametrize("dtype", DTYPES)
+def test_bilinear_is_deterministic(dtype):
     """Fixed-order reductions, no atomics: two runs are bitwise equal."""
     args = bilinear_inputs(12289, 97, seed=7)
-    a, _ = run_bilinear(*args)
-    b, _ = run_bilinear(*args)
-    for k, x, y in zip(TOL, a, b):
+    a, _ = run_bilinear(dtype, *args)
+    b, _ = run_bilinear(dtype, *args)
+    for k, x, y in zip(TOL[dtype], a, b):
         assert torch.equal(x, y), k
 
 
@@ -131,109 +140,113 @@ def weights(W):
     return CO.wprime(W.double()).float().contiguous(), CO.wsecond(W.double()).float().contiguous()
 
 
-def test_fwd_accumulates_into_a_strided_output_without_bias():
-    """accumulate = 1 into a prefilled out of row stride ldo > R, bias null: out[:, :R] += h W t, columns R.. untouched;
-    a workspace of exactly gcgcn_bilinear_ws_bytes suffices."""
-    P, R, ldo = 1000, 33, 40
+@pytest.mark.parametrize("dtype", DTYPES)
+def test_fwd_accumulates_into_a_strided_output_without_bias(dtype):
+    """accumulate = 1 into a prefilled out of row stride ldo > R, bias null: out[:, :R] += the bilinear form, columns
+    R.. untouched; a workspace of exactly gcgcn_bilinear_ws_bytes suffices."""
+    P, R, ldo, code = 1000, 33, 40, C.DTYPES[dtype]
     h, t, W, _, _ = bilinear_inputs(P, R, seed=11)
     Wm, _ = weights(W)
     gen = torch.Generator(device=DEV).manual_seed(12)
     out = torch.full((P, ldo), -7.25, device=DEV)
     out[:, :R] = torch.randn(P, R, generator=gen, device=DEV)
     before = out.clone()
-    ws = torch.empty(int(lib().gcgcn_bilinear_ws_bytes(P, R)), dtype=torch.uint8, device=DEV)
-    _lib.call("gcgcn_bilinear_fwd", p(h), p(t), p(Wm), None, P, R, 1, p(out), ldo, p(ws), ws.numel(), stream())
+    ws = torch.empty(int(lib().gcgcn_bilinear_ws_bytes(P, R, code)), dtype=torch.uint8, device=DEV)
+    _lib.call("gcgcn_bilinear_fwd", p(h), p(t), p(Wm), None, P, R, code, 1, p(out), ldo, p(ws), ws.numel(), stream())
     torch.cuda.synchronize()
     assert torch.equal(out[:, R:], before[:, R:])
-    e = rel_err(out[:, :R], before[:, :R].double() + CO.bilinear(h, t, W))
-    print(f"fwd accumulate: {e:.2e}")
-    assert e <= TOL["out"]                                                  # 1.2e-6
+    e = rel_err(out[:, :R], before[:, :R].double() + ORACLE[dtype](h, t, W))
+    print(f"{dtype} fwd accumulate: {e:.2e}")
+    assert e <= TOL[dtype]["out"]                                           # fp32 1.2e-6, bf16 1.8e-7
 
 
+@pytest.mark.parametrize("dtype", DTYPES)
+@pytest.mark.parametrize("P", [100, 8193])
 @pytest.mark.parametrize("beta", [0.0, 1.0])
-def test_fused_bwd_beta(beta):
-    """beta = 0 overwrites dWm (NaN before: never read), beta = 1 adds to it; dh and dt are written whole."""
-    P, R = 8193, 33
-    h, t, W, _, dout = bilinear_inputs(P, R, seed=21)
+def test_fused_bwd_beta(beta, P, dtype):
+    """beta = 0 overwrites dWm (NaN before: never read), beta = 1 adds to it; dh and dt are written whole.  P = 100: one
+    4096-row range (the epilogue applies beta); 8193: three (the split-K reduction does)."""
+    R, code = 33, C.DTYPES[dtype]
+    h, t, W, _, dout = bilinear_inputs(P, R, seed=21 + P)
     Wm, Wm2 = weights(W)
     gen = torch.Generator(device=DEV).manual_seed(22)
     prior = torch.randn(D, R * D, generator=gen, device=DEV) if beta else torch.full((D, R * D), float("nan"), device=DEV)
     dWm = prior.clone()
     dh = torch.full_like(h, float("nan"))
     dt = torch.full_like(t, float("nan"))
-    ws = torch.empty(int(lib().gcgcn_bilinear_bwd_ws_bytes(P, R)), dtype=torch.uint8, device=DEV)
-    _lib.call("gcgcn_bilinear_bwd", p(h), p(t), p(Wm), p(Wm2), p(dout), P, R, beta, p(dh), p(dt), p(dWm), p(ws),
+    ws = torch.empty(int(lib().gcgcn_bilinear_bwd_ws_bytes(P, R, code)), dtype=torch.uint8, device=DEV)
+    _lib.call("gcgcn_bilinear_bwd", p(h), p(t), p(Wm), p(Wm2), p(dout), P, R, code, beta, p(dh), p(dt), p(dWm), p(ws),
               ws.numel(), stream())
     torch.cuda.synchronize()
-    _, rdh, rdt, rdW, _ = CO.bilinear(h, t, W, None, dout)
+    _, rdh, rdt, rdW, _ = ORACLE[dtype](h, t, W, None, dout)
     want = CO.wprime(rdW) + (prior.double() if beta else 0.0)
     errs = {"dh": rel_err(dh, rdh), "dt": rel_err(dt, rdt), "dW": rel_err(dWm, want)}
-    print(f"bwd beta {beta}: " + ", ".join(f"{k} {v:.2e}" for k, v in errs.items()))
-    for k, e in errs.items():                                               # dh 1.4e-6, dt 1.3e-6, dW' 3.3e-5
-        assert e <= tol(k, P), f"{k}: {e:.3e} > {tol(k, P):.1e}"
+    print(f"{dtype} bwd P {P} beta {beta}: " + ", ".join(f"{k} {v:.2e}" for k, v in errs.items()))
+    for k, e in errs.items():                                               # fp32 P 8193: dh 1.4e-6, dt 1.3e-6, dW' 3.3e-5
+        assert e <= tol(dtype, k, P), f"{k}: {e:.3e} > {tol(dtype, k, P):.1e}"
 
 
-def test_chunked_kernels_with_strided_dout():
-    """gcgcn_bilinear_reduce_fwd (accumulate, bias, ldo > R), gcgcn_bilinear_outer_bwd and gcgcn_bilinear_dt_bwd with
-    dout of row stride ldd > R (NaN past column R: never read), R = 33 (one relation past a warp's 32)."""
-    P, R, ldd, ldo = 300, 33, 37, 41
-    h, t, W, bias, dout = bilinear_inputs(P, R, seed=31)
-    Y = (h.double() @ CO.wprime(W.double())).float()                     # [P, R*128], the chunked route's h W'
-    dpad = torch.full((P, ldd), float("nan"), device=DEV)
-    dpad[:, :R] = dout
-    gen = torch.Generator(device=DEV).manual_seed(32)
-    out = torch.full((P, ldo), -7.25, device=DEV)
-    out[:, :R] = torch.randn(P, R, generator=gen, device=DEV)
-    before = out.clone()
-    dY = torch.empty(P, R * D, device=DEV)
-    dt = torch.full_like(t, float("nan"))
-    _lib.call("gcgcn_bilinear_reduce_fwd", p(Y), p(t), p(bias), P, R, 1, p(out), ldo, stream())
-    _lib.call("gcgcn_bilinear_outer_bwd", p(dpad), ldd, p(t), P, R, p(dY), stream())
-    _lib.call("gcgcn_bilinear_dt_bwd", p(dpad), ldd, p(Y), P, R, p(dt), stream())
-    torch.cuda.synchronize()
-    Y3 = Y.double().view(P, R, D)
-    assert torch.equal(out[:, R:], before[:, R:])
-    e_out = rel_err(out[:, :R], before[:, :R].double() + torch.einsum("prb,pb->pr", Y3, t.double()) + bias.double())
-    assert torch.equal(dY, (dout[:, :, None] * t[:, None, :]).reshape(P, R * D))        # one fp32 product each
-    e_dt = rel_err(dt, torch.einsum("pr,prb->pb", dout.double(), Y3))
-    print(f"reduce_fwd {e_out:.2e}, dt_bwd {e_dt:.2e}")
-    assert e_out <= 5e-7 and e_dt <= 8e-7                                   # 1.0e-7, 1.9e-7
-
-
-def test_bwd_below_the_fused_minimum_is_refused_before_any_launch():
-    P, R = 8191, 97
-    h, t, W, _, dout = bilinear_inputs(P, R, seed=41)
+@pytest.mark.parametrize("dtype", DTYPES)
+def test_zero_rows_launch_nothing(dtype):
+    R, code = 97, C.DTYPES[dtype]
+    h, t, W, bias, dout = bilinear_inputs(4, R, seed=31)
     Wm, Wm2 = weights(W)
-    dh, dt, dWm = torch.zeros_like(h), torch.zeros_like(t), torch.zeros(D, R * D, device=DEV)
-    ws = torch.empty(int(lib().gcgcn_bilinear_bwd_ws_bytes(P, R)), dtype=torch.uint8, device=DEV)
+    out = torch.full((4, R), 3.0, device=DEV)
+    dh, dt, dWm = torch.full_like(h, 3.0), torch.full_like(t, 3.0), torch.full((D, R * D), 3.0, device=DEV)
+    ws = torch.empty(4096, dtype=torch.uint8, device=DEV)
     before = _lib.launch_count()
-    rc = lib().gcgcn_bilinear_bwd(p(h), p(t), p(Wm), p(Wm2), p(dout), P, R, 0.0, p(dh), p(dt), p(dWm), p(ws),
-                                  ws.numel(), stream())
-    assert rc == ERR_UNSUPPORTED, lib().gcgcn_last_error()
+    assert lib().gcgcn_bilinear_fwd(p(h), p(t), p(Wm), p(bias), 0, R, code, 0, p(out), R, p(ws), ws.numel(), stream()) == 0
+    assert lib().gcgcn_bilinear_bwd(p(h), p(t), p(Wm), p(Wm2), p(dout), 0, R, code, 0.0, p(dh), p(dt), p(dWm), p(ws),
+                                    ws.numel(), stream()) == 0
     assert _lib.launch_count() == before
     torch.cuda.synchronize()
-    assert not dh.any() and not dt.any() and not dWm.any()
+    assert bool((out == 3).all() and (dh == 3).all() and (dt == 3).all() and (dWm == 3).all())
+    # and through the autograd function: an empty forward and backward
+    leaves = [x[:0].clone().requires_grad_(True) for x in (h, t)] + [W.clone().requires_grad_(True),
+                                                                     bias.clone().requires_grad_(True)]
+    z = C.BilinearFn.apply(*leaves, dtype)
+    z.backward(torch.zeros_like(z))
+    assert z.shape == (0, R) and not leaves[2].grad.any() and not leaves[3].grad.any()
 
 
-@pytest.mark.parametrize("which", ["fwd", "bwd"])
-def test_workspace_one_byte_short_is_refused_before_any_launch(which):
-    P, R = 8192, 97
+def call_entry(which, code, ws_bytes, P=8192, R=97):
+    """One call of gcgcn_bilinear_fwd or _bwd on zeroed outputs; returns (rc, launches, whether an output was written)."""
     h, t, W, bias, dout = bilinear_inputs(P, R, seed=51)
     Wm, Wm2 = weights(W)
     out = torch.zeros(P, R, device=DEV)
     dh, dt, dWm = torch.zeros_like(h), torch.zeros_like(t), torch.zeros(D, R * D, device=DEV)
-    need = int(lib().gcgcn_bilinear_ws_bytes(P, R) if which == "fwd" else lib().gcgcn_bilinear_bwd_ws_bytes(P, R))
-    ws = torch.empty(need, dtype=torch.uint8, device=DEV)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=DEV)
     before = _lib.launch_count()
     if which == "fwd":
-        rc = lib().gcgcn_bilinear_fwd(p(h), p(t), p(Wm), p(bias), P, R, 0, p(out), R, p(ws), need - 1, stream())
+        rc = lib().gcgcn_bilinear_fwd(p(h), p(t), p(Wm), p(bias), P, R, code, 0, p(out), R, p(ws), ws_bytes, stream())
     else:
-        rc = lib().gcgcn_bilinear_bwd(p(h), p(t), p(Wm), p(Wm2), p(dout), P, R, 0.0, p(dh), p(dt), p(dWm), p(ws),
-                                      need - 1, stream())
-    assert rc == ERR_WORKSPACE, (rc, lib().gcgcn_last_error())
-    assert _lib.launch_count() == before
+        rc = lib().gcgcn_bilinear_bwd(p(h), p(t), p(Wm), p(Wm2), p(dout), P, R, code, 0.0, p(dh), p(dt), p(dWm), p(ws),
+                                      ws_bytes, stream())
+    launches = _lib.launch_count() - before
     torch.cuda.synchronize()
-    assert not out.any() and not dh.any() and not dt.any() and not dWm.any()
+    return rc, launches, bool(out.any() or dh.any() or dt.any() or dWm.any())
+
+
+@pytest.mark.parametrize("dtype", DTYPES)
+@pytest.mark.parametrize("which", ["fwd", "bwd"])
+def test_workspace_one_byte_short_is_refused_before_any_launch(which, dtype):
+    P, R, code = 8192, 97, C.DTYPES[dtype]
+    need = int(lib().gcgcn_bilinear_ws_bytes(P, R, code) if which == "fwd" else lib().gcgcn_bilinear_bwd_ws_bytes(P, R, code))
+    rc, launches, written = call_entry(which, code, need - 1, P, R)
+    assert rc == ERR_WORKSPACE, (rc, lib().gcgcn_last_error())
+    assert launches == 0 and not written
+
+
+@pytest.mark.parametrize("which", ["fwd", "bwd"])
+def test_unknown_dtype_is_refused_before_any_launch(which):
+    """Only GCGCN_F32 (0) and GCGCN_BF16 (1) name an operand type; a workspace ample for either does not matter."""
+    P, R = 8192, 97
+    need = max(int(f(P, R, code)) for f in (lib().gcgcn_bilinear_ws_bytes, lib().gcgcn_bilinear_bwd_ws_bytes)
+               for code in C.DTYPES.values())
+    for code in (2, -1):
+        rc, launches, written = call_entry(which, code, need, P, R)
+        assert rc == ERR_INVALID_ARG and b"dtype" in lib().gcgcn_last_error(), (rc, lib().gcgcn_last_error())
+        assert launches == 0 and not written
 
 
 # ---- the loss and the per-document bias on a ragged batch ----------------------------------------------------------

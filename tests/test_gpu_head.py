@@ -122,8 +122,7 @@ def test_loss_kernel_alone_matches_torch_bce():
 @pytest.mark.parametrize("P", [1, 127, 1000, 8192 + 77, 20011])
 def test_bilinear_classifier_against_torch(P):
     """G:356-358 on its own: Bilinear(128, 128, 97) + Linear(256, 97) over P pairs (P not a multiple of the 128-row tile,
-    and more than one chunk of the backward) against torch's own modules on the CPU; the fused forward (row-dot
-    epilogue on the tcgen05 GEMM) against the chunked forward that materialises h W'."""
+    and more than one 4096-row range of the weight gradient) against torch's own modules on the CPU."""
     from gcgcn_b200 import classifier as C
     torch.manual_seed(P)
     bili, cls = torch.nn.Bilinear(128, 128, 97), torch.nn.Linear(256, 97)
@@ -150,19 +149,6 @@ def test_bilinear_classifier_against_torch(P):
     for k, g in (("h", hg.grad), ("t", tg.grad), ("W", bg.weight.grad), ("b", bg.bias.grad), ("Wc", cg.weight.grad),
                  ("bc", cg.bias.grad)):
         assert rel(g, ref[k]) <= 1e-4, k
-    C.FUSED_FORWARD = C.FUSED_BACKWARD = False          # the chunked route that materialises h W' and its gradient
-    try:
-        fused = {"h": hg.grad.clone(), "t": tg.grad.clone(), "W": bg.weight.grad.clone()}
-        for m in (bg, cg):
-            m.zero_grad()
-        hg.grad = tg.grad = None
-        chunked = C.relation_logits(hg, tg, bg, cg)
-        (chunked * up.to(DEV)).sum().backward()
-    finally:
-        C.FUSED_FORWARD = C.FUSED_BACKWARD = True
-    assert float((chunked.detach() - got.detach()).abs().max()) <= 2e-5
-    for k, g in (("h", hg.grad), ("t", tg.grad), ("W", bg.weight.grad)):
-        assert rel(fused[k], g) <= 1e-4, k           # two summation orders of 12416-term 3xTF32 sums
 
 
 @pytest.mark.parametrize("idx", [0, 1])
